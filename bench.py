@@ -9,6 +9,18 @@ convex 8x upsampling, backward warp + validity mask of the 3x1088x1920 frame, ma
 
     python bench.py [--gpus N] [--steps K] [--warmup W]            # this repo's CUDA path
     python bench.py --impl reference ...                            # the CPU path on the host cores
+    python bench.py --dump-outputs DIR ...                          # also write the last timed step's outputs
+
+`--dump-outputs DIR` (rank 0): after the timed steps, DIR/<name>.npy holds what the last timed step of the
+           device-resident arm computed -- `corr` (the last lookup), `flow_up`, `warped`, `mask` as float32
+           (pairs, n) arrays, and `epe_state`, the float64 (sum, count) the step returned (the EPE metric
+           accumulated over the timed steps).  Row p of output i (in that order) holds pair p's values at the
+           flat C-order positions np.sort(np.random.default_rng(i).choice(size, n, replace=False)) of its
+           per-pair array, n = 60e6 // (16 * pairs), or at every position when size <= n: under 64 MB in all.
+           The inputs are seeded, so two builds run with the same arguments can be compared output for output.
+           The last micro-batch is sampled after the timed window; with several micro-batches per step the
+           others are sampled inside it (the next one overwrites the shared lookup buffer), which adds a gather
+           of at most 60 MB to the timed time.
 
 `value`  : pairs/s with inputs resident in HBM (CUDA events, barrier + synchronize on both sides,
            max over ranks).
@@ -139,6 +151,40 @@ def make_batch(pairs, device, seed, torch):
     return batch
 
 
+# ------------------------------------------------------------------------------ --dump-outputs
+# per-pair shape of every array hot_path() returns
+DUMP_SHAPES = {"corr": (LEVELS * (2 * RADIUS + 1) ** 2, h8, w8), "flow_up": (2, H, W), "warped": (3, H, W), "mask": (H, W)}
+DUMP_BYTES = 60_000_000
+
+
+class OutputSampler:
+    """Fixed, seeded positions of hot_path()'s outputs, the same in every pair.  `take` gathers them on the device as
+    soon as a micro-batch is done (the next one overwrites the shared lookup buffer); `write` saves the float32
+    (pairs, n) arrays once the timed window has closed."""
+
+    def __init__(self, pairs, device, torch):
+        import numpy as np
+
+        per_output = DUMP_BYTES // (len(DUMP_SHAPES) * 4 * pairs)
+        self.index, self.parts = {}, []
+        for seed, (name, shape) in enumerate(DUMP_SHAPES.items()):
+            n = int(np.prod(shape))
+            pick = np.arange(n) if n <= per_output else np.sort(np.random.default_rng(seed).choice(n, per_output, replace=False))
+            self.index[name] = torch.from_numpy(pick).to(device)
+
+    def take(self, out):
+        self.parts.append({k: out[k].reshape(out[k].shape[0], -1)[:, i] for k, i in self.index.items()})
+
+    def write(self, path, epe_state):
+        import numpy as np
+
+        os.makedirs(path, exist_ok=True)
+        for k in self.index:
+            arr = np.concatenate([p[k].float().cpu().numpy() for p in self.parts])
+            np.save(os.path.join(path, k + ".npy"), arr)
+        np.save(os.path.join(path, "epe_state.npy"), epe_state.double().cpu().numpy())
+
+
 # ------------------------------------------------------------------------------ CPU path (oracle port)
 def cpu_pass(sample):
     """The reference's op sequence for one pass, on the host, through the oracle port."""
@@ -225,7 +271,7 @@ def run_reference(args):
     # oracle library are imported after this point, so the setting takes effect)
     for var in ("OMP_NUM_THREADS", "OPENBLAS_NUM_THREADS", "MKL_NUM_THREADS"):
         os.environ[var] = str(host_cores())
-    steps, warm = max(1, min(args.steps, 3)), max(1, min(args.warmup, 1))
+    steps, warm = args.steps, max(1, min(args.warmup, 1))
     cb = time_cpu(steps, warm, 1)
     line = {
         "impl": "reference", "metric": METRIC, "value": cb["value"], "unit": UNIT, "n_gpus": args.gpus,
@@ -328,16 +374,23 @@ def run_ours(args):
     lookup_out = torch.empty((micro, LEVELS * (2 * RADIUS + 1) ** 2, h8, w8), device=device)
     metric = AverageEndPointError()
 
-    def step(timers=None):
+    def step(timers=None, sampler=None):
+        """One pass over every micro-batch.  With `sampler`, each micro-batch but the last is sampled before the next
+        one overwrites the shared lookup buffer; the last one's outputs are returned, to be sampled by the caller."""
+        out = None
         for v in views:
+            if sampler is not None and out is not None:
+                sampler.take(out)
             lo = lookup_out if v["fmap1"].shape[0] == micro else None
-            hot_path(v, metric, timers=timers, lookup_out=lo, cta_group=args.cta_group)
-        return metric.sync()                           # (sum, count) all-reduce of a copy: the only collective
+            out = hot_path(v, metric, timers=timers, lookup_out=lo, cta_group=args.cta_group)
+        # (sum, count) all-reduce of a copy: the only collective
+        return metric.sync(), (out if sampler is not None else None)
 
     # ---- device-resident arm
     for _ in range(args.warmup):
         step()
     metric.reset()
+    dump = OutputSampler(pairs, device, torch) if args.dump_outputs and rank == 0 else None
     sampler = ClockSampler(dev_index)
     if rank == 0:
         sampler.start()
@@ -348,11 +401,16 @@ def run_ours(args):
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     t_wall0 = time.time()
     e0.record()
-    for _ in range(args.steps):
-        step(timers)
+    for i in range(args.steps):
+        state, last = step(timers, dump if i == args.steps - 1 else None)
     e1.record()
+    if dump is not None:
+        dump.take(last)                                # after e1: the last micro-batch's sample is not timed
     barrier()
     t_wall1 = time.time()
+    if dump is not None:
+        dump.write(args.dump_outputs, state)
+        del dump
     launches = ofb200.launch_count() - l0
     ms = e0.elapsed_time(e1)
     if world > 1:
@@ -506,7 +564,12 @@ def main():
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
     ap.add_argument("--no-named", action="store_true", help="skip the single-kernel named configs")
     ap.add_argument("--no-placement", action="store_true", help="ranks use cuda:LOCAL_RANK without probing the host links")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's outputs to DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3                                   # timing rule: at least 3 warm-up steps
     if args.impl == "reference":

@@ -1,19 +1,23 @@
-"""Import the read-only reference checkout (/root/reference) for golden-vector generation.
+"""Import an unmodified reference checkout (OFB200_REFERENCE, else one staged under oracle/_ref/) for golden-vector
+generation.
 
-Only used by tests/golden/make_golden.py in the authoring container. Nothing in
-tests/, bench.py or the product imports this at run time: /root/reference does
-not exist on the GPU box.
+Only used by tests/golden/make_golden.py. Nothing in tests/, bench.py or the
+product imports this at run time: the stored vectors are all the tests need.
 
 The reference needs pytorch_lightning / torchmetrics (not installed): they are
 stubbed with the minimum surface the hot path touches (SURVEY.md section 8c).
 """
+import os
 import sys
 import types
 
 import torch
 from torch import nn
 
-REF = "/root/reference"
+sys.path.insert(0, os.path.join(os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__)))), "tools"))
+from stage_reference import find_reference  # noqa: E402
+
+REF = find_reference() or ""
 
 
 def _stub_third_party():
@@ -55,6 +59,9 @@ def _stub_third_party():
 
 def load_reference():
     """Returns (optical_flow module, model.corr, model.utils, RAFT class)."""
+    if not os.path.isdir(os.path.join(REF, "methods", "raft", "model")):
+        raise RuntimeError("set OFB200_REFERENCE to a checkout of the upstream torch-optical-flow project, or stage "
+                           "one under oracle/_ref/")
     _stub_third_party()
     for name in list(sys.modules):
         if name == "optical_flow" or name.startswith("optical_flow.") or name == "model" or name.startswith("model."):

@@ -1,7 +1,7 @@
-"""Generate tests/golden/*.npz by running the UNMODIFIED reference (/root/reference) on CPU.
+"""Generate tests/golden/*.npz by running the UNMODIFIED reference on CPU.
 
-Run in the authoring container only (`python tests/golden/make_golden.py`); the GPU box has
-no /root/reference.  Every array stored here is an input or an output of a reference call;
+`OFB200_REFERENCE=<checkout> python tests/golden/make_golden.py`; the tests themselves need
+only the stored vectors.  Every array stored here is an input or an output of a reference call;
 the reference call that produced it is named in the `ref_call` string of each case.
 
 The lookup *index / validity* vectors are produced by replaying, with eager torch fp32 ops,

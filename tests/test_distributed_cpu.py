@@ -25,7 +25,9 @@ def _worker(rank, world, port, total_pairs, q):
     for p in (os.path.join(ROOT, "torch-optical-flow_b200"), ROOT):
         if p not in sys.path:
             sys.path.insert(0, p)
-    os.environ.update(MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port), RANK=str(rank), WORLD_SIZE=str(world))
+    # CPU states on every rank: hide any GPU so an empty shard's state is not created on cuda:0
+    os.environ.update(MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port), RANK=str(rank), WORLD_SIZE=str(world),
+                      CUDA_VISIBLE_DEVICES="")
     dist.init_process_group("gloo", rank=rank, world_size=world)
     try:
         import oracle
