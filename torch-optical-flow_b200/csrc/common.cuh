@@ -2,6 +2,7 @@
 #pragma once
 #include <cuda_runtime.h>
 #include <cuda_bf16.h>
+#include <cuda_fp16.h>
 #include <stdint.h>
 
 #include "../../include/ofb200.h"
@@ -17,9 +18,9 @@ extern int64_t g_ofb_launches;  // api.cu
         if (e__ != cudaSuccess) return (int)e__;   \
     } while (0)
 
-#define OFB_CUDA(call)                             \
+#define OFB_CUDA(...)  /* variadic: the call may contain template-argument commas */ \
     do {                                           \
-        cudaError_t e__ = (call);                  \
+        cudaError_t e__ = (__VA_ARGS__);           \
         if (e__ != cudaSuccess) return (int)e__;   \
     } while (0)
 
@@ -41,6 +42,19 @@ static inline int ofb_num_sms() {
         sms[dev] = n > 0 ? n : 148;
     }
     return sms[dev];
+}
+
+// Raises Kernel's dynamic shared-memory limit to `bytes`, the first time it is called on each device.
+template <auto Kernel>
+static inline cudaError_t ofb_smem_once(int bytes) {
+    static bool configured[OFB_MAX_DEVICES] = {false};
+    const int dev = ofb_device();
+    if (!configured[dev]) {
+        const cudaError_t e = cudaFuncSetAttribute(Kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
+        if (e != cudaSuccess) return e;
+        configured[dev] = true;
+    }
+    return cudaSuccess;
 }
 
 namespace ofb {
@@ -83,6 +97,15 @@ __device__ __forceinline__ float source_index(float g, int size) {
 }
 
 __device__ __forceinline__ float ld_nc(const float* p) { return __ldg(p); }
+
+// input element -> fp32: feature maps and mask logits arrive in fp32, or in half precision from an autocast caller
+__device__ __forceinline__ float ld_f32(const float* p) { return __ldg(p); }
+__device__ __forceinline__ float ld_f32(const __nv_bfloat16* p) {
+    return __uint_as_float((unsigned)__ldg(reinterpret_cast<const unsigned short*>(p)) << 16);
+}
+__device__ __forceinline__ float ld_f32(const __half* p) {
+    return __half2float(__ushort_as_half(__ldg(reinterpret_cast<const unsigned short*>(p))));
+}
 
 __device__ __forceinline__ float warp_sum(float v) {
 #pragma unroll

@@ -228,12 +228,11 @@ OFB_API int ofb_corr_lookup_ondemand(const void* f1_km, const void* const* f2_km
     P.levels = levels; P.radius = radius; P.B = B; P.C = C; P.h = h; P.w = w;
     P.tiles_x = (w + TQ - 1) / TQ; P.tiles_y = (h + TQY - 1) / TQY;
     P.n_items = (long long)B * levels * P.tiles_x * P.tiles_y;
-    static int occ = 0;
-    if (!occ) {
+    static const int occ = [] {
         const char* e = getenv("OFB_ONDEMAND_OCC");                 // resident CTAs per SM (tuning override)
-        occ = e ? atoi(e) : 4;
-        if (occ < 1 || occ > 16) occ = 4;
-    }
+        const int n = e ? atoi(e) : 4;
+        return (n < 1 || n > 16) ? 4 : n;
+    }();
     long long blocks = (long long)ofb_num_sms() * occ;
     if (blocks > P.n_items) blocks = P.n_items;
     cudaStream_t st = (cudaStream_t)stream;

@@ -20,15 +20,6 @@ constexpr int TCMAX = 256;  // channels per tile (the whole K extent of the tens
 
 // One CTA turns a 32-pixel x C-channel tile: reads are 128-byte lines (32 pixels of one channel), 8 in
 // flight per thread; writes are whole 2*C-byte pixel rows of the K-major operand.
-// feature-map element -> fp32: the maps arrive in fp32, or in half precision from an autocast (`precision: 16`) caller
-__device__ __forceinline__ float ld_in(const float* p) { return __ldg(p); }
-__device__ __forceinline__ float ld_in(const __nv_bfloat16* p) {
-    return __uint_as_float((unsigned)__ldg(reinterpret_cast<const unsigned short*>(p)) << 16);
-}
-__device__ __forceinline__ float ld_in(const __half* p) {
-    return __half2float(__ushort_as_half(__ldg(reinterpret_cast<const unsigned short*>(p))));
-}
-
 template <int POOL, typename TIn>
 __global__ void __launch_bounds__(256) prep_kernel(const TIn* __restrict__ in, __nv_bfloat16* __restrict__ out, int C,
                                                    int h, int w, float scale) {
@@ -51,13 +42,13 @@ __global__ void __launch_bounds__(256) prep_kernel(const TIn* __restrict__ in, _
             if (pok && c < Ct) {
                 const TIn* src = src0 + (size_t)c * HW;
                 if (POOL == 1) {
-                    v[u] = ld_in(src);
+                    v[u] = ofb::ld_f32(src);
                 } else {
                     float a = 0.0f;
 #pragma unroll
                     for (int dy = 0; dy < POOL; ++dy)
 #pragma unroll
-                        for (int dx = 0; dx < POOL; ++dx) a += ld_in(src + dy * w + dx);
+                        for (int dx = 0; dx < POOL; ++dx) a += ofb::ld_f32(src + dy * w + dx);
                     v[u] = a * (1.0f / (float)(POOL * POOL));
                 }
             }

@@ -13,12 +13,11 @@
 // Warp roles as in corr_gemm.cu: warp 0 = TMA producer, warp 1 = MMA issuer + TMEM owner, warps 2-5 = epilogue
 // (one TMEM lane quarter each); accumulators are double-buffered so the epilogue of one tile overlaps the K loop of
 // the next.  Every mbarrier wait is bounded (trap instead of hang).
-#include <cuda.h>
-#include <cudaTypedefs.h>
-
-#include "common.cuh"
+#include "sm100.cuh"
 
 namespace {
+
+using namespace ofb;
 
 constexpr int BM = 128, BK = 64, UK = 16;
 constexpr int A_STAGE = BM * BK * 2;                 // 16 KiB
@@ -38,72 +37,6 @@ struct GemmArgs {
     int accumulate;
 };
 
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count));
-}
-__device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(uint32_t bar) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
-}
-__device__ __forceinline__ bool mbar_try_wait(uint32_t bar, uint32_t parity) {
-    uint32_t ok;
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t}"
-        : "=r"(ok) : "r"(bar), "r"(parity) : "memory");
-    return ok != 0;
-}
-__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
-    uint32_t spins = 0;
-    while (!mbar_try_wait(bar, parity)) {
-        if (++spins > (1u << 27)) __trap();          // a protocol bug becomes a trapped launch, never a hung GPU
-    }
-}
-__device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tma_load_3d(uint32_t dst, const CUtensorMap* map, uint32_t bar, int c0, int c1, int c2) {
-    asm volatile(
-        "cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];"
-        ::"r"(dst), "l"(map), "r"(bar), "r"(c0), "r"(c1), "r"(c2) : "memory");
-}
-__device__ __forceinline__ void umma_bf16(uint32_t d_tmem, uint64_t adesc, uint64_t bdesc, uint32_t idesc, uint32_t accumulate) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-        ::"r"(d_tmem), "l"(adesc), "l"(bdesc), "r"(idesc), "r"(accumulate) : "memory");
-}
-__device__ __forceinline__ void umma_commit(uint32_t bar) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
-}
-__device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&v)[32]) {
-    asm volatile(
-        "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
-        "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, "
-        "%16, %17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31}, [%32];"
-        : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]),
-          "=r"(v[8]), "=r"(v[9]), "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15]),
-          "=r"(v[16]), "=r"(v[17]), "=r"(v[18]), "=r"(v[19]), "=r"(v[20]), "=r"(v[21]), "=r"(v[22]), "=r"(v[23]),
-          "=r"(v[24]), "=r"(v[25]), "=r"(v[26]), "=r"(v[27]), "=r"(v[28]), "=r"(v[29]), "=r"(v[30]), "=r"(v[31])
-        : "r"(taddr) : "memory");
-}
-// K-major, 128-byte swizzled operand tile (rows of 128 bytes, 8-row groups 1024 bytes apart): as corr_gemm.cu
-__device__ __forceinline__ uint64_t make_smem_desc(uint32_t saddr) {
-    uint64_t d = 0;
-    d |= (uint64_t)((saddr & 0x3FFFFu) >> 4);
-    d |= (uint64_t)1 << 16;
-    d |= (uint64_t)(1024 >> 4) << 32;
-    d |= (uint64_t)1 << 46;
-    d |= (uint64_t)2 << 61;
-    return d;
-}
-__device__ __forceinline__ uint32_t make_idesc(int M, int N) {
-    return (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
-}
-
 __global__ void __launch_bounds__(NT, 1) gemm_nt_kernel(const __grid_constant__ CUtensorMap map_a,
                                                         const __grid_constant__ CUtensorMap map_b, const GemmArgs G) {
     extern __shared__ uint8_t smem_raw[];
@@ -119,15 +52,14 @@ __global__ void __launch_bounds__(NT, 1) gemm_nt_kernel(const __grid_constant__ 
     const uint32_t off_b = STAGES * A_STAGE;
 
     if (warp == 0 && lane == 0) {
-        asm volatile("prefetch.tensormap [%0];" ::"l"(&map_a) : "memory");
-        asm volatile("prefetch.tensormap [%0];" ::"l"(&map_b) : "memory");
+        prefetch_tmap(&map_a); prefetch_tmap(&map_b);
         for (int s = 0; s < STAGES; ++s) { mbar_init(bar_full + 8 * s, 1); mbar_init(bar_empty + 8 * s, 1); }
         for (int s = 0; s < 2; ++s) { mbar_init(bar_tfull + 8 * s, 1); mbar_init(bar_tempty + 8 * s, 4); }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        fence_barrier_init();
     }
     if (warp == 1) {
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(tmem_slot), "r"(512) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+        tmem_alloc<1>(tmem_slot, 512);
+        tmem_relinquish<1>();
     }
     tc_fence_before();
     __syncthreads();
@@ -164,11 +96,11 @@ __global__ void __launch_bounds__(NT, 1) gemm_nt_kernel(const __grid_constant__ 
                     const uint64_t bdesc = make_smem_desc(sbase + off_b + stage * B_STAGE_MAX);
 #pragma unroll
                     for (int k = 0; k < BK / UK; ++k)
-                        umma_bf16(d_tmem, adesc + (uint64_t)(2 * k), bdesc + (uint64_t)(2 * k), idesc, (uint32_t)((kb | k) != 0));
-                    umma_commit(bar_empty + 8 * stage);
+                        umma_bf16<1>(d_tmem, adesc + (uint64_t)(2 * k), bdesc + (uint64_t)(2 * k), idesc, (uint32_t)((kb | k) != 0));
+                    umma_commit<1>(bar_empty + 8 * stage);
                     if (++stage == STAGES) { stage = 0; phase ^= 1; }
                 }
-                umma_commit(bar_tfull + 8 * acc);
+                umma_commit<1>(bar_tfull + 8 * acc);
                 if (++acc == 2) { acc = 0; tphase ^= 1; }
             }
         }
@@ -186,7 +118,7 @@ __global__ void __launch_bounds__(NT, 1) gemm_nt_kernel(const __grid_constant__ 
             for (int c0 = 0; c0 < G.N; c0 += 32) {
                 uint32_t v[32];
                 tmem_ld32(taddr + c0, v);
-                asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+                tmem_ld_wait();
                 if (row < G.M) {
 #pragma unroll
                     for (int c = 0; c < 32; c += 4) {
@@ -206,7 +138,7 @@ __global__ void __launch_bounds__(NT, 1) gemm_nt_kernel(const __grid_constant__ 
     }
     tc_fence_before();
     __syncthreads();
-    if (warp == 1) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "r"(512) : "memory");
+    if (warp == 1) tmem_dealloc<1>(tmem_base, 512);
 }
 
 // fp32 (rows x cols, tight) -> bf16 copy (pitch pc) and / or bf16 transpose (pitch pr); 32 x 32 tiles through smem
@@ -233,30 +165,12 @@ __global__ void __launch_bounds__(256) cast_bf16_kernel(const float* __restrict_
     }
 }
 
-PFN_cuTensorMapEncodeTiled_v12000 get_encode() {
-    static PFN_cuTensorMapEncodeTiled_v12000 fn = nullptr;
-    static bool tried = false;
-    if (!tried) {
-        tried = true;
-        void* p = nullptr;
-        cudaDriverEntryPointQueryResult qres;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &qres) == cudaSuccess &&
-            qres == cudaDriverEntryPointSuccess)
-            fn = reinterpret_cast<PFN_cuTensorMapEncodeTiled_v12000>(p);
-    }
-    return fn;
-}
-
 bool encode_operand(CUtensorMap* m, const void* base, int K, int rows, int batch, long long ld, long long stride, int box_rows) {
-    PFN_cuTensorMapEncodeTiled_v12000 enc = get_encode();
-    if (!enc) return false;
-    cuuint64_t gdim[3] = {(cuuint64_t)K, (cuuint64_t)rows, (cuuint64_t)batch};
-    cuuint64_t gstr[2] = {(cuuint64_t)ld * 2, (cuuint64_t)stride * 2};
-    cuuint32_t box[3] = {BK, (cuuint32_t)box_rows, 1};
-    cuuint32_t estr[3] = {1, 1, 1};
-    return enc(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, const_cast<void*>(base), gdim, gstr, box, estr,
-               CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-               CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
+    const cuuint64_t gdim[3] = {(cuuint64_t)K, (cuuint64_t)rows, (cuuint64_t)batch};
+    const cuuint64_t gstr[2] = {(cuuint64_t)ld * 2, (cuuint64_t)stride * 2};
+    const cuuint32_t box[3] = {BK, (cuuint32_t)box_rows, 1};
+    return encode_tiled(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, base, gdim, gstr, box, CU_TENSOR_MAP_SWIZZLE_128B,
+                        CU_TENSOR_MAP_L2_PROMOTION_L2_256B);
 }
 
 }  // namespace
@@ -283,12 +197,7 @@ OFB_API int ofb_gemm_nt_bf16(const void* A, const void* B, float* D, int batch, 
     if (items > 0x7fffffffLL) return OFB_EUNSUPPORTED;
     G.items = (int)items;
     G.alpha = alpha; G.accumulate = accumulate;
-    static bool configured[OFB_MAX_DEVICES] = {false};
-    const int dev = ofb_device();
-    if (!configured[dev]) {
-        OFB_CUDA(cudaFuncSetAttribute(gemm_nt_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_ALLOC));
-        configured[dev] = true;
-    }
+    OFB_CUDA(ofb_smem_once<gemm_nt_kernel>(SMEM_ALLOC));
     const int grid = (int)(items < ofb_num_sms() ? items : ofb_num_sms());
     gemm_nt_kernel<<<grid, NT, SMEM_ALLOC, (cudaStream_t)stream>>>(ma, mb, G);
     OFB_LAUNCH_CHECK();

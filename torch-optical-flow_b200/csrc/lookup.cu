@@ -478,19 +478,15 @@ OFB_API int ofb_corr_lookup(const ofb_pyramid* pyr, const float* coords, float* 
     if (tile_ok) {
         const int threads = 32 * pyr->levels;
         const size_t wsm = (size_t)(2 * radius + 3) * threads * 40;               // window slots: rows x (16 + 16 + 8) B
-        static int gr = 0;                                 // window rows per cp.async commit group: 3 (measured ~2 % faster
-        if (!gr) {                                         // than one group for the whole window); OFB_LOOKUP_GR=16 for A/B
+        // window rows per cp.async commit group: 3 (measured ~2 % faster than one group for the whole window);
+        // OFB_LOOKUP_GR=16 for A/B
+        static const int gr = [] {
             const char* e = getenv("OFB_LOOKUP_GR");
-            gr = (e && atoi(e) == 16) ? 16 : 3;
-        }
-        static bool configured[OFB_MAX_DEVICES] = {false};
-        const int dev = ofb_device();
-        if (!configured[dev]) {
-            OFB_CUDA(cudaFuncSetAttribute(lookup_tile_kernel<4, 3>, cudaFuncAttributeMaxDynamicSharedMemorySize, 11 * 128 * 40));
-            OFB_CUDA(cudaFuncSetAttribute(lookup_tile_kernel<4, 16>, cudaFuncAttributeMaxDynamicSharedMemorySize, 11 * 128 * 40));
-            OFB_CUDA(cudaFuncSetAttribute(lookup_tile_kernel<3, 16>, cudaFuncAttributeMaxDynamicSharedMemorySize, 9 * 128 * 40));
-            configured[dev] = true;
-        }
+            return (e && atoi(e) == 16) ? 16 : 3;
+        }();
+        OFB_CUDA(ofb_smem_once<lookup_tile_kernel<4, 3>>(11 * 128 * 40));
+        OFB_CUDA(ofb_smem_once<lookup_tile_kernel<4, 16>>(11 * 128 * 40));
+        OFB_CUDA(ofb_smem_once<lookup_tile_kernel<3, 16>>(9 * 128 * 40));
         if (radius == 4 && gr == 3) lookup_tile_kernel<4, 3><<<(int)blocks, threads, wsm, st>>>(P, coords, out, idx_or_null, valid_or_null);
         else if (radius == 4) lookup_tile_kernel<4, 16><<<(int)blocks, threads, wsm, st>>>(P, coords, out, idx_or_null, valid_or_null);
         else lookup_tile_kernel<3, 16><<<(int)blocks, threads, wsm, st>>>(P, coords, out, idx_or_null, valid_or_null);

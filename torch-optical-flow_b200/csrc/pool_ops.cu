@@ -12,14 +12,6 @@
 
 namespace {
 
-__device__ __forceinline__ float ld_map(const float* p) { return __ldg(p); }
-__device__ __forceinline__ float ld_map(const __nv_bfloat16* p) {
-    return __uint_as_float((unsigned)__ldg(reinterpret_cast<const unsigned short*>(p)) << 16);
-}
-__device__ __forceinline__ float ld_map(const __half* p) {
-    return __half2float(__ushort_as_half(__ldg(reinterpret_cast<const unsigned short*>(p))));
-}
-
 // out[b, c, k] = bf16(mean of the pool x pool block k of fmap[b, c]) for k < (h/pool)*(w/pool), 0 for the padding
 template <typename TIn>
 __global__ void __launch_bounds__(256) pool_cast_kernel(const TIn* __restrict__ in, __nv_bfloat16* __restrict__ out,
@@ -36,7 +28,7 @@ __global__ void __launch_bounds__(256) pool_cast_kernel(const TIn* __restrict__ 
             const TIn* src = in + plane * (long long)h * w + (long long)(yo * pool) * w + xo * pool;
             float a = 0.0f;
             for (int dy = 0; dy < pool; ++dy)
-                for (int dx = 0; dx < pool; ++dx) a += ld_map(src + dy * w + dx);
+                for (int dx = 0; dx < pool; ++dx) a += ofb::ld_f32(src + dy * w + dx);
             v = a * inv;
         }
         out[t] = __float2bfloat16_rn(v);

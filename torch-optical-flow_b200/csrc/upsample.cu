@@ -17,16 +17,6 @@ namespace {
 constexpr int PX = 32;   // coarse pixels per CTA
 constexpr int NT = PX * 8;
 
-// mask logit -> fp32: the mask head's output is fp32, or half precision under the reference's `precision: 16`
-// (autocast convolution; softmax itself autocasts to fp32, raft.py:78)
-__device__ __forceinline__ float ld_logit(const float* p) { return __ldg(p); }
-__device__ __forceinline__ float ld_logit(const __nv_bfloat16* p) {
-    return __uint_as_float((unsigned)__ldg(reinterpret_cast<const unsigned short*>(p)) << 16);
-}
-__device__ __forceinline__ float ld_logit(const __half* p) {
-    return __half2float(__ushort_as_half(__ldg(reinterpret_cast<const unsigned short*>(p))));
-}
-
 template <typename TM>
 __global__ void __launch_bounds__(NT) convex_upsample_kernel(const float* __restrict__ flow,
                                                              const TM* __restrict__ mask,
@@ -53,6 +43,8 @@ __global__ void __launch_bounds__(NT) convex_upsample_kernel(const float* __rest
             nby[ky * 3 + kx] = in ? 8.0f * __ldg(fy + yy * w + xx) : 0.0f;
         }
 
+    // mask logits: fp32, or half precision under the reference's `precision: 16` (autocast convolution; softmax
+    // itself autocasts to fp32, raft.py:78)
     const TM* mp = mask + (size_t)n * 576 * hw + (size_t)(i * 8) * hw + p;
     float ox[8], oy[8];
     // JG sub-columns at a time: 9*JG independent 128-byte-coalesced loads are in flight per warp before
@@ -64,7 +56,7 @@ __global__ void __launch_bounds__(NT) convex_upsample_kernel(const float* __rest
 #pragma unroll
         for (int jj = 0; jj < JG; ++jj)
 #pragma unroll
-            for (int k = 0; k < 9; ++k) m[jj][k] = ld_logit(mp + (size_t)(k * 64 + jg + jj) * hw);
+            for (int k = 0; k < 9; ++k) m[jj][k] = ofb::ld_f32(mp + (size_t)(k * 64 + jg + jj) * hw);
 #pragma unroll
         for (int jj = 0; jj < JG; ++jj) {
             float mx = m[jj][0];

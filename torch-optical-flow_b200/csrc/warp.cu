@@ -394,12 +394,11 @@ int launch_direct(const float* frame, const float* flow, float* out, uint8_t* va
 template <int PAD, bool AC>
 int launch_rows(const float* frame, const float* flow, float* out, uint8_t* valid, int B, int C, int H, int W,
                 FlowMul fm, cudaStream_t st) {
-    static int rpt = 0;
-    if (!rpt) {
+    static const int rpt = [] {
         const char* e = getenv("OFB_WARP_RPT");           // tuning override
-        rpt = e ? atoi(e) : RPT_DEFAULT;
-        if (rpt != 1 && rpt != 2 && rpt != 4 && rpt != 8) rpt = RPT_DEFAULT;
-    }
+        const int r = e ? atoi(e) : RPT_DEFAULT;
+        return (r == 1 || r == 2 || r == 4 || r == 8) ? r : RPT_DEFAULT;
+    }();
     const dim3 block(128);
     const dim3 grid((W + 127) / 128, (H + rpt - 1) / rpt, B);
     if (grid.y > 65535) return OFB_EUNSUPPORTED;
@@ -416,13 +415,7 @@ int launch_staged(const float* frame, const float* flow, float* out, uint8_t* va
                   FlowMul fm, cudaStream_t st) {
     const int cg = C < CG_MAX ? C : CG_MAX;
     const size_t smem = (size_t)cg * WIN_H * WIN_W * sizeof(float);
-    static bool configured[OFB_MAX_DEVICES] = {false};
-    const int dev = ofb_device();
-    if (!configured[dev]) {
-        OFB_CUDA(cudaFuncSetAttribute(warp_staged_kernel<PAD, AC>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                      (int)(CG_MAX * WIN_H * WIN_W * sizeof(float))));
-        configured[dev] = true;
-    }
+    OFB_CUDA(ofb_smem_once<warp_staged_kernel<PAD, AC>>((int)(CG_MAX * WIN_H * WIN_W * sizeof(float))));
     const int vec4 = (W % 4 == 0) && ((reinterpret_cast<uintptr_t>(frame) & 15) == 0);
     dim3 grid((W + TW - 1) / TW, (H + TH - 1) / TH, B);
     warp_staged_kernel<PAD, AC><<<grid, NT, smem, st>>>(frame, flow, out, valid, B, C, H, W, vec4, fm);
@@ -488,11 +481,10 @@ OFB_API int ofb_warp_f32(const float* frame, const float* flow, float* out, uint
         return OFB_EUNSUPPORTED;
     // auto: the row kernel; 1 = direct gather (also nearest / NHWC), 2 = cp.async-staged, 3 = row kernel,
     // 4 = TMA-staged window (warp_tma.cu)
-    static int auto_v = -1;
-    if (auto_v < 0) {
+    static const int auto_v = [] {
         const char* e = getenv("OFB_WARP_VARIANT");       // tuning override for variant 0
-        auto_v = e ? atoi(e) : 0;
-    }
+        return e ? atoi(e) : 0;
+    }();
     int v = variant != 0 ? variant : (auto_v == 4 && can_tma ? 4 : (can_rows ? 3 : 1));
     if (v == 4)
         return ofb_warp_tma_launch(frame, flow, out, valid_or_null, B, C, H, W, padding_mode, align_corners, fm.x, fm.y, st);

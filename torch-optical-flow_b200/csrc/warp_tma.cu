@@ -13,10 +13,7 @@
 //     the row kernel, so the result never depends on the staging.
 // HBM sees every frame line about once (neighbouring windows overlap in L2); L1 sees 4 shared-memory
 // wavefronts per channel per warp instead of up to 4 x 32 sector requests.
-#include <cuda.h>
-#include <cudaTypedefs.h>
-
-#include "common.cuh"
+#include "sm100.cuh"
 
 namespace {
 
@@ -34,39 +31,6 @@ constexpr int STAGES = 2;
 struct FlowMul2 {
     float x, y;
 };
-
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint32_t bar, uint32_t count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(bar), "r"(count));
-}
-__device__ __forceinline__ void mbar_expect_tx(uint32_t bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ bool mbar_try_wait(uint32_t bar, uint32_t parity) {
-    uint32_t ok;
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-        "selp.u32 %0, 1, 0, p;\n\t}"
-        : "=r"(ok) : "r"(bar), "r"(parity) : "memory");
-    return ok != 0;
-}
-// bounded: a protocol bug becomes a trapped launch, never a hung GPU
-__device__ __forceinline__ void mbar_wait(uint32_t bar, uint32_t parity) {
-    uint32_t spins = 0;
-    while (!mbar_try_wait(bar, parity)) {
-        if (++spins > (1u << 26)) __trap();
-    }
-}
-__device__ __forceinline__ void tma_box_3d(uint32_t dst, const CUtensorMap* map, uint32_t bar, int x, int y, int z) {
-    asm volatile(
-        "cp.async.bulk.tensor.3d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4, %5}], [%2];"
-        ::"r"(dst), "l"(map), "r"(bar), "r"(x), "r"(y), "r"(z) : "memory");
-}
-
-__device__ __forceinline__ void mbar_arrive(uint32_t bar) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(bar) : "memory");
-}
 
 struct TileCoord {
     int b, tile_x, tile_y;
@@ -102,7 +66,7 @@ __global__ void __launch_bounds__(NT + 32, 3) warp_tma_kernel(const __grid_const
 
     if (threadIdx.x == 0) {
         for (int s = 0; s < STAGES; ++s) { mbar_init(smem_u32(&s_full[s]), 1); mbar_init(smem_u32(&s_empty[s]), NT / 32); }
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        fence_barrier_init();
     }
     __syncthreads();
 
@@ -135,7 +99,7 @@ __global__ void __launch_bounds__(NT + 32, 3) warp_tma_kernel(const __grid_const
                 const uint32_t full = smem_u32(&s_full[slot]);
                 mbar_expect_tx(full, (uint32_t)(cg * WIN_W * WIN_H * 4));
                 for (int c = 0; c < cg; ++c)
-                    tma_box_3d(win_s + slot * stage_bytes + c * PLANE_BYTES, &map, full, ox, oy, tc.b * C + g * CGRP + c);
+                    tma_load_3d(win_s + slot * stage_bytes + c * PLANE_BYTES, &map, full, ox, oy, tc.b * C + g * CGRP + c);
                 if (++slot == STAGES) { slot = 0; ph ^= 1; }
             }
         }
@@ -237,30 +201,10 @@ __global__ void __launch_bounds__(NT + 32, 3) warp_tma_kernel(const __grid_const
     }
 }
 
-PFN_cuTensorMapEncodeTiled_v12000 get_encode() {
-    static PFN_cuTensorMapEncodeTiled_v12000 fn = nullptr;
-    static bool tried = false;
-    if (!tried) {
-        tried = true;
-        void* p = nullptr;
-        cudaDriverEntryPointQueryResult qres;
-        if (cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &qres) == cudaSuccess &&
-            qres == cudaDriverEntryPointSuccess)
-            fn = reinterpret_cast<PFN_cuTensorMapEncodeTiled_v12000>(p);
-    }
-    return fn;
-}
-
 template <int PAD, bool AC>
 int launch(const CUtensorMap& map, const float* frame, const float* flow, float* out, uint8_t* valid, int B, int C,
            int H, int W, FlowMul2 fm, cudaStream_t st) {
-    static bool configured[OFB_MAX_DEVICES] = {false};
-    const int dev = ofb_device();
-    if (!configured[dev]) {
-        OFB_CUDA(cudaFuncSetAttribute(warp_tma_kernel<PAD, AC>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                      STAGES * CGRP * PLANE_BYTES));
-        configured[dev] = true;
-    }
+    OFB_CUDA(ofb_smem_once<warp_tma_kernel<PAD, AC>>(STAGES * CGRP * PLANE_BYTES));
     const int cg = C < CGRP ? C : CGRP;
     const size_t smem = (size_t)STAGES * cg * PLANE_BYTES;
     const int ntx = (W + TW - 1) / TW, nty = (H + TH - 1) / TH;
@@ -280,16 +224,12 @@ int launch(const CUtensorMap& map, const float* frame, const float* flow, float*
 // (warp.cu) checks that and the 32-bit offset limits.
 int ofb_warp_tma_launch(const float* frame, const float* flow, float* out, uint8_t* valid, int B, int C, int H, int W,
                         int pad, int ac, float fmx, float fmy, cudaStream_t st) {
-    PFN_cuTensorMapEncodeTiled_v12000 enc = get_encode();
-    if (!enc) return OFB_EDRIVER;
     CUtensorMap map;
-    cuuint64_t gdim[3] = {(cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)B * C};
-    cuuint64_t gstr[2] = {(cuuint64_t)W * 4, (cuuint64_t)W * H * 4};
-    cuuint32_t box[3] = {WIN_W, WIN_H, 1};
-    cuuint32_t estr[3] = {1, 1, 1};
-    if (enc(&map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, const_cast<float*>(frame), gdim, gstr, box, estr,
-            CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_128B,
-            CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) != CUDA_SUCCESS)
+    const cuuint64_t gdim[3] = {(cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)B * C};
+    const cuuint64_t gstr[2] = {(cuuint64_t)W * 4, (cuuint64_t)W * H * 4};
+    const cuuint32_t box[3] = {WIN_W, WIN_H, 1};
+    if (!encode_tiled(&map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, frame, gdim, gstr, box, CU_TENSOR_MAP_SWIZZLE_NONE,
+                      CU_TENSOR_MAP_L2_PROMOTION_L2_128B))
         return OFB_EDRIVER;
     const FlowMul2 fm{fmx, fmy};
 #define OFB_CASE(P, A) \
