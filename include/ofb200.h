@@ -15,8 +15,8 @@
  *   - the last argument is the CUDA stream (cudaStream_t passed as void*; NULL = default)
  *   - returns 0 on success, a negative OFB_E* code for a rejected argument, or a positive
  *     cudaError_t for a CUDA failure; never throws, never allocates device memory, never
- *     synchronises (ofb_corr_pyramid_bf16*, ofb_gemm_nt_bf16 and the TMA variant of ofb_warp_f32 are the only
- *     calls that touch the driver outside a stream: they encode TMA descriptors on the host)
+ *     synchronises (ofb_corr_pyramid_bf16*, ofb_corr_pyramid_f16, ofb_gemm_nt_bf16 and the TMA variant of ofb_warp_f32
+ *     are the only calls that touch the driver outside a stream: they encode TMA descriptors on the host)
  *   - there is no CPU compute path: without a CUDA device every call fails
  */
 #ifndef OFB200_H_
@@ -44,7 +44,8 @@ extern "C" {
 
 #define OFB_DTYPE_F32 0
 #define OFB_DTYPE_BF16 1
-#define OFB_DTYPE_F16 2 /* input feature maps of ofb_corr_prep_from, mask of ofb_convex_upsample, ofb_scale_flow */
+#define OFB_DTYPE_F16 2 /* feature maps and operands of ofb_corr_prep_from / _to, correlation pyramids, mask of
+                           ofb_convex_upsample, ofb_scale_flow */
 #define OFB_DTYPE_F64 3 /* ofb_scale_flow only */
 
 #define OFB_MAX_LEVELS 4
@@ -168,8 +169,8 @@ int ofb_sequence_loss_backward_f32(const float* const* preds, float* const* d_pr
  * Level l of query q = (b, y, x) is an h_l x w_l image, h_l = floor(h / 2^l).  Two layouts
  * (strides in ELEMENTS of the pyramid dtype, `np` = row_pitch):
  *   OFB_LAYOUT_ROWS      element (q, yy, xx) at  base[l] + q*q_stride[l] + yy*np + xx
- *   OFB_LAYOUT_BLOCK8X4  8 (x) by 4 (y) element blocks of 32 contiguous elements (64 bytes in bf16 = one
- *                        DRAM atom), blocks raster-ordered:
+ *   OFB_LAYOUT_BLOCK8X4  8 (x) by 4 (y) element blocks of 32 contiguous elements (64 bytes in bf16 or fp16 =
+ *                        one DRAM atom), blocks raster-ordered:
  *                        base[l] + q*q_stride[l] + ((yy>>2)*(np>>3) + (xx>>3))*32 + (yy&3)*8 + (xx&7)
  *                        -- the lookup's 11x11 window touches ~8 atoms instead of ~15.
  *   OFB_LAYOUT_QMINOR8X4 the same 8x4 blocks, but block-major / query-minor: with Q = B*h*w queries,
@@ -182,8 +183,9 @@ int ofb_sequence_loss_backward_f32(const float* const* preds, float* const* d_pr
 * (row_pitch multiple of 16 elements, so every row starts on a 32-byte sector), 2 = padded 8x4
  * blocks (row_pitch multiple of 8, rows padded to a multiple of 4), 3 = the same blocks query-minor.
  * elems[l] receives the element count of level l PER QUERY (= q_stride[l] except for mode 3).
- * The tensor-core builder needs mode 1 or 2 and writes whole 8-element pieces, i.e. zeros into the
- * padding columns; the bf16 lookup kernel relies on padding columns holding finite values.
+ * The tensor-core builder needs mode 1, 2 or 3 and writes whole 8-element pieces, i.e. zeros into the
+ * padding columns; the 16-bit lookup kernel relies on padding columns holding finite values.
+ * The blocked layouts are 16-bit layouts: bf16 or fp16 pyramids, not fp32 ones.
  * ------------------------------------------------------------------------------------- */
 #define OFB_LAYOUT_ROWS 0
 #define OFB_LAYOUT_BLOCK8X4 1
@@ -196,8 +198,8 @@ typedef struct ofb_pyramid {
     int32_t lvl_h[OFB_MAX_LEVELS];
     int32_t lvl_w[OFB_MAX_LEVELS];
     int32_t levels;
-    int32_t dtype;  /* OFB_DTYPE_F32 or OFB_DTYPE_BF16 */
-    int32_t layout; /* OFB_LAYOUT_ROWS, OFB_LAYOUT_BLOCK8X4 or OFB_LAYOUT_QMINOR8X4 (blocked layouts: bf16 only) */
+    int32_t dtype;  /* OFB_DTYPE_F32, OFB_DTYPE_BF16 or OFB_DTYPE_F16 */
+    int32_t layout; /* OFB_LAYOUT_ROWS, OFB_LAYOUT_BLOCK8X4 or OFB_LAYOUT_QMINOR8X4 (blocked layouts: 16-bit only) */
     int32_t reserved;
 } ofb_pyramid;
 
@@ -222,8 +224,9 @@ int ofb_pyramid_layout(int h, int w, int levels, int mode, ofb_pyramid* pyr_host
  *         pyr: layout from ofb_pyramid_layout(padded = 1), dtype BF16.
  *         cta_group: 0 = auto, 1 = one CTA per tile, 2 = CTA pair (cta_group::2), 3 = clusters of two independent
  *         cta_group::1 CTAs with the fmap2 operand ring TMA-multicast into both (query-minor layout only).
- * ofb_corr_pyramid_simt_f32: plain CUDA-core builder (fp32 in, fp32 or bf16 out) used by tests as an
- *         on-device cross-check and for shapes the tensor-core kernel rejects.
+ * ofb_corr_pyramid_simt_f32: plain CUDA-core builder (fp32 in, fp32, bf16 or fp16 out) used by tests as an
+ *         on-device cross-check and for shapes the tensor-core kernel rejects.  Each pooled level is computed from the
+ *         stored level above it, in fp32, and rounded to the pyramid dtype.
  * ------------------------------------------------------------------------------------- */
 int ofb_corr_prep_bf16(const float* fmap_nchw, void* out_km_bf16, int B, int C, int h, int w, int pool,
                        float scale, void* stream);
@@ -233,8 +236,22 @@ int ofb_corr_prep_bf16(const float* fmap_nchw, void* out_km_bf16, int B, int C, 
  * precision anyway; here the half-precision map is the kernel's input (element -> fp32 -> * scale -> bf16). */
 int ofb_corr_prep_from(const void* fmap_nchw, int in_dtype, void* out_km_bf16, int B, int C, int h, int w, int pool,
                        float scale, void* stream);
+/* The same pass with the operand type chosen: out_dtype OFB_DTYPE_BF16 (= ofb_corr_prep_from) or OFB_DTYPE_F16, the
+ * operands of ofb_corr_pyramid_f16 (element -> fp32 -> * scale -> round to nearest even).  An fp16 map prepped to fp16
+ * with pool = 1 and scale = 1 is an exact transpose. */
+int ofb_corr_prep_to(const void* fmap_nchw, int in_dtype, void* out_km, int out_dtype, int B, int C, int h, int w,
+                     int pool, float scale, void* stream);
 int ofb_corr_pyramid_bf16(const void* f1_km, const void* f2_km, const void* f2q_km, const ofb_pyramid* pyr_host,
                           int B, int C, int h, int w, float scale, int cta_group, void* stream);
+/* ofb_corr_pyramid_bf16 in fp16: the precision the reference stores its pyramid in under `precision: 16`
+ * (methods/raft/config/train/default.yaml:20): autocast runs the torch.matmul of corr.py:85 on fp16 operands, and
+ * avg_pool2d keeps fp16 (corr.py:52-54).  f1_km, f2_km, f2q_km: fp16 K-major operands (ofb_corr_prep_to, out_dtype
+ * F16); pyr->dtype must be OFB_DTYPE_F16; everything else as for the bf16 builder.  Prep fmap1 with scale = 1 and pass
+ * scale = 1/sqrt(C) here: it is applied to the fp32 accumulators, the reference's order (an fp16 GEMM of the rounded
+ * maps, then the scale, corr.py:85-87), and keeps fmap1/sqrt(C) out of fp16 subnormals.  Scaled correlations beyond
+ * +-65504 become inf, as in the reference under autocast. */
+int ofb_corr_pyramid_f16(const void* f1_km, const void* f2_km, const void* f2q_km, const ofb_pyramid* pyr_host,
+                         int B, int C, int h, int w, float scale, int cta_group, void* stream);
 /* On-demand correlation lookup (SURVEY.md section 8f row 4): CorrBlock.__call__ (corr.py:56-77) WITHOUT the materialised
  * volume of corr.py:45-54.  avg_pool2d is linear, so level l of the pyramid is f1^T . avgpool_l(f2) / sqrt(C); the kernel
  * evaluates those dot products only at the positions each query's window touches and samples them with the same bit-exact
@@ -267,6 +284,10 @@ int ofb_corr_pyramid_simt_f32(const float* fmap1, const float* fmap2, const ofb_
  *   coords (B,2,h,w) fp32 (ch0 = x, ch1 = y);  out (B, L*(2r+1)^2, h, w) fp32
  *   idx_or_null   (B*h*w, L, 2, 2r+1) int32 floor indices (x taps then y taps)
  *   valid_or_null (B*h*w, L, (2r+1)^2) u8   utils.py:77 predicate per sample
+ * pyr: dtype F32, BF16 or F16.  Floor indices and validity masks do not depend on the dtype.  16-bit pyramids with
+ * radius 3 or 4 take the register-tile kernel, whose 3-tap filter multiplies one in-window column by an exact zero
+ * weight the reference's 2-tap form never reads: an inf stored in that column (an fp16 correlation beyond +-65504)
+ * gives NaN where the reference gives a finite value.
  * ------------------------------------------------------------------------------------- */
 int ofb_corr_lookup(const ofb_pyramid* pyr_host, const float* coords, float* out,
                     int32_t* idx_or_null, uint8_t* valid_or_null, int B, int h, int w, int radius,

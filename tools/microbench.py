@@ -17,6 +17,7 @@ import torch  # noqa: E402
 
 import ofb200  # noqa: E402
 from model.corr import CorrBlock, prepare_operands  # noqa: E402
+from ofb200.ops.corr import _default_pyramid_dtype, build_pyramid  # noqa: E402
 from model.utils import coords_grid  # noqa: E402
 from optical_flow import normalize  # noqa: E402
 
@@ -122,21 +123,20 @@ def _corr_setup(b, c, h, w, seed=1):
 
 
 def bench_corr(name, b, c, h, w, cta_groups=(0,), prep=True):
-    lib = ofb200.load()
     gen, f1, f2 = _corr_setup(b, c, h, w)
     n = h * w
-    st = ofb200.stream_ptr()
     recs = []
-    a_km, b_km, q_km = prepare_operands(f1, f2, 4)
-    ms = timeit(lambda: prepare_operands(f1, f2, 4))
+    # the operands of the pyramid CorrBlock(f1, f2) builds (OFB200_PYRAMID_DTYPE): fp16 for an fp16 pyramid, else bf16
+    op_dt = torch.float16 if _default_pyramid_dtype() == torch.float16 else torch.bfloat16
+    a_km, b_km, q_km = prepare_operands(f1, f2, 4, op_dt)
+    ms = timeit(lambda: prepare_operands(f1, f2, 4, op_dt))
     if prep:
         recs.append(record(f"{name} K2 prep (fmap1, fmap2, fmap2/4x4)", ms, nbytes=b * c * n * (3 * 4 + 2 * 2 + 2 / 16)))
     blk = CorrBlock(f1, f2)
     elems = sum(int(blk._pyr.lvl_h[lv]) * int(blk._pyr.lvl_w[lv]) for lv in range(4)) * b * n
     for cg in cta_groups:
         def run():
-            rc = lib.ofb_corr_pyramid_bf16(ofb200.ptr(a_km), ofb200.ptr(b_km), ofb200.ptr(q_km), ctypes.byref(blk._pyr),
-                                           b, c, h, w, 1.0, cg, st)
+            rc = build_pyramid((a_km, b_km, q_km), blk._pyr, b, c, h, w, op_dt, cg)
             assert rc == 0
         ms = timeit(run, reps=10)
         recs.append(record(f"{name} K2 corr pyramid cta_group={cg}", ms, nbytes=elems * 2 + 2 * b * n * c * 2,
@@ -157,7 +157,8 @@ def bench_lookup(name, blk, gen, b, h, w, iters=12):
     n = h * w
     coords = coords_grid(b, h, w).cuda()[None] + 4 * torch.randn((iters, b, 2, h, w), device="cuda", generator=gen)
     out = torch.empty((b, 324, h, w), device="cuda")
-    esz = 2 if blk._buffers[0].dtype == torch.bfloat16 else 4
+    dt = blk._buffers[0].dtype
+    esz = dt.itemsize
 
     def look():
         for it in range(iters):
@@ -165,7 +166,7 @@ def bench_lookup(name, blk, gen, b, h, w, iters=12):
                                      b, h, w, 4, st)
             assert rc == 0
     ms = timeit(look, reps=5) / iters
-    return record(f"{name} K3 lookup r=4 x{iters} ({'bf16' if esz == 2 else 'fp32'} pyramid), per iteration", ms,
+    return record(f"{name} K3 lookup r=4 x{iters} ({ {torch.bfloat16: 'bf16', torch.float16: 'fp16'}.get(dt, 'fp32')} pyramid), per iteration", ms,
                   nbytes=b * n * (4 * 100 * esz + 8 + 324 * 4), iters_ms=round(iters * ms, 3))
 
 

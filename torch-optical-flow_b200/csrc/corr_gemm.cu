@@ -8,14 +8,16 @@
 // runs twice: on fmap2 (levels 0, 1) and on the 4x4-averaged fmap2 (levels 2, 3) -- pooling is linear,
 // avgpool4(f1^T f2) = f1^T avgpool4(f2), and the second run costs 1/16 of the first.
 //
-//   * operands are K-major bf16 (ofb_corr_prep_bf16: cast + transpose, 1/sqrt(C) folded into fmap1),
-//     fetched by TMA with 128-byte swizzle;
+//   * operands are K-major bf16 (ofb_corr_prep_bf16: cast + transpose, 1/sqrt(C) folded into fmap1) or fp16
+//     (ofb_corr_prep_to; the scale is applied to the accumulators, the reference's order under autocast),
+//     fetched by TMA with 128-byte swizzle.  The storage type T is a template parameter: it reaches only the
+//     instruction descriptor, the tensor maps and the epilogue's pack instruction;
 //   * a CTA owns 128 queries (rows of the volume): their 128 x C slice of fmap1 stays RESIDENT in
 //     shared memory while the CTA walks target tiles; only fmap2 streams through a 96..160 KiB TMA ring;
 //   * a target tile is 256 targets laid out as 4 "chunks" of 2 rows x 32 columns of the target image
 //     (tile shape 32x8, 64x4 or 128x2, whichever wastes least for the image width), fetched as 4-D TMA
 //     boxes (C, x, y, b).  TMA zero-fills outside the image;
-//   * tcgen05.mma (kind::f16, bf16 x bf16 -> fp32) accumulates 128 x 256 in TMEM, two accumulator
+//   * tcgen05.mma (kind::f16, bf16 x bf16 or fp16 x fp16 -> fp32) accumulates 128 x 256 in TMEM, two accumulator
 //     stages (2 x 256 of the 512 columns) so the epilogue of tile n overlaps the MMAs of tile n+1;
 //   * cta_group = 2: a CTA PAIR shares each target tile (each CTA loads half of it, the MMA is M = 256
 //     across the pair) -- halves the L2 -> SM operand traffic, which is what bounds cta_group = 1
@@ -33,6 +35,7 @@
 // Roofline (DESIGN.md section 4): 2*B*N^2*C flops against the bf16 tensor peak and 2 bytes * 1.33 *
 // B*N^2 of pyramid writes against HBM; at C = 256 and 1965 MHz the write is the larger bound.
 #include <cstdlib>
+#include <type_traits>
 
 #include "sm100.cuh"
 
@@ -90,20 +93,21 @@ static_assert(Ring<1, 0>::SMEM_ALLOC <= 232448 && Ring<2, 0>::SMEM_ALLOC <= 2324
               Ring<2, 2>::SMEM_ALLOC <= 232448 && Ring<2, 2>::STAGES <= MAX_STAGES && Ring<1, 2, 1>::SMEM_ALLOC <= 232448 &&
               Ring<2, 2, 1>::SMEM_ALLOC <= 232448, "shared memory budget");
 
-struct LevelOut {
-    __nv_bfloat16* base;
+template <typename T> struct LevelOut {
+    T* base;                     // 16-bit storage: __nv_bfloat16 or __half
     long long q_stride;
     int pitch, h, w;
     int blocked;                 // 8x4 blocks (OFB_LAYOUT_BLOCK8X4 / QMINOR8X4): a 16-byte piece is one block row
     long long blk_stride;        // elements between consecutive blocks: 32, or 32 * Q for the query-minor layout
 };
 // element offset (without the query term q * q_stride) of the 8-element piece starting at (y, x), x % 8 == 0
-__device__ __forceinline__ long long piece_offset(const LevelOut& L, int y, int x) {
+template <typename T>
+__device__ __forceinline__ long long piece_offset(const LevelOut<T>& L, int y, int x) {
     if (L.blocked) return ((long long)(y >> 2) * (L.pitch >> 3) + (x >> 3)) * L.blk_stride + (y & 3) * 8;
     return (long long)y * L.pitch + x;
 }
 
-struct GemmParams {
+template <typename T> struct GemmParams {
     int B, C, kb;
     int Nq;                      // queries per batch element (rows of the volume)
     int th, tw;                  // target image of THIS run (h x w, or h/4 x w/4 for the pooled run)
@@ -114,7 +118,7 @@ struct GemmParams {
     int tiles_per_item, n_chunks, mblk, n_items;
     float scale;
     int apply_scale, has_b;
-    LevelOut la, lb;             // level written from the accumulators, and its 2x2 mean
+    LevelOut<T> la, lb;          // level written from the accumulators, and its 2x2 mean
     int dbg;                     // PROF builds only: bit mask disabling parts of the epilogue (tools/k2_profile.py)
     unsigned long long* prof;    // optional per-CTA wait-cycle counters (ofb_corr_pyramid_bf16_profile)
 };
@@ -134,6 +138,15 @@ __device__ __forceinline__ void mbar_wait_p(uint32_t bar, uint32_t parity, unsig
 __device__ __forceinline__ uint32_t pack_bf16(float lo, float hi) {
     __nv_bfloat162 v = __floats2bfloat162_rn(lo, hi);
     return *reinterpret_cast<uint32_t*>(&v);
+}
+__device__ __forceinline__ uint32_t pack_f16(float lo, float hi) {
+    __half2 v = __floats2half2_rn(lo, hi);
+    return *reinterpret_cast<uint32_t*>(&v);
+}
+// two fp32 values -> one word of the 16-bit storage type T (round to nearest even)
+template <typename T> __device__ __forceinline__ uint32_t pack16(float lo, float hi) {
+    if constexpr (std::is_same<T, __half>::value) return pack_f16(lo, hi);
+    else return pack_bf16(lo, hi);
 }
 __device__ __forceinline__ void st_shared_v4(uint32_t addr, uint32_t a, uint32_t b, uint32_t c, uint32_t d) {
     asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};" ::"r"(addr), "r"(a), "r"(b), "r"(c), "r"(d) : "memory");
@@ -189,7 +202,8 @@ __device__ __forceinline__ void stage_slot(uint32_t slot, uint32_t rot, const ui
 struct ItemCoord {
     int b, chunk, m;
 };
-__device__ __forceinline__ ItemCoord decode_item(const GemmParams& P, int item) {
+template <typename GP>
+__device__ __forceinline__ ItemCoord decode_item(const GP& P, int item) {
     ItemCoord ic;
     ic.m = item % P.mblk;
     const int r = item / P.mblk;
@@ -199,11 +213,11 @@ __device__ __forceinline__ ItemCoord decode_item(const GemmParams& P, int item) 
 }
 
 // The (item, tile) sequence of one worker, as the three roles walk it.
-struct TileIter {
+template <typename T> struct TileIter {
     int item, t, t1;
     ItemCoord ic;
     bool valid;
-    __device__ __forceinline__ void load(const GemmParams& P) {
+    __device__ __forceinline__ void load(const GemmParams<T>& P) {
         valid = item < P.n_items;
         if (valid) {
             ic = decode_item(P, item);
@@ -211,8 +225,8 @@ struct TileIter {
             t1 = min(t + P.tiles_per_item, P.ntiles);
         }
     }
-    __device__ __forceinline__ void init(const GemmParams& P, int worker) { item = worker; load(P); }
-    __device__ __forceinline__ void advance(const GemmParams& P, int n_workers) {
+    __device__ __forceinline__ void init(const GemmParams<T>& P, int worker) { item = worker; load(P); }
+    __device__ __forceinline__ void advance(const GemmParams<T>& P, int n_workers) {
         if (++t >= t1) { item += n_workers; load(P); }
     }
 };
@@ -220,7 +234,8 @@ struct TileIter {
 // EPI_PIPE: one 32-column piece = block rows 2*rh, 2*rh+1 of the chunk's two 8x4 blocks (chunk = 16 x 4 targets, column
 // c = row * 16 + x).  Level 0: one 32-byte sector per block.  Level 1: the piece closes ONE pooled row (8 means); the
 // even piece keeps it in `keep`, the odd piece stores both rows as one sector.
-__device__ __forceinline__ void store_piece(const GemmParams& P, const uint32_t (&v)[32], int rh, int x0, int y0,
+template <typename T>
+__device__ __forceinline__ void store_piece(const GemmParams<T>& P, const uint32_t (&v)[32], int rh, int x0, int y0,
                                             long long qg, bool qok, uint32_t (&keep)[4]) {
     float f[32];
 #pragma unroll
@@ -233,8 +248,8 @@ __device__ __forceinline__ void store_piece(const GemmParams& P, const uint32_t 
                 uint32_t r0[4], r1[4];
 #pragma unroll
                 for (int e = 0; e < 4; ++e) {
-                    r0[e] = pack_bf16(f[b2 * 8 + 2 * e], f[b2 * 8 + 2 * e + 1]);
-                    r1[e] = pack_bf16(f[16 + b2 * 8 + 2 * e], f[16 + b2 * 8 + 2 * e + 1]);
+                    r0[e] = pack16<T>(f[b2 * 8 + 2 * e], f[b2 * 8 + 2 * e + 1]);
+                    r1[e] = pack16<T>(f[16 + b2 * 8 + 2 * e], f[16 + b2 * 8 + 2 * e + 1]);
                 }
                 st_global_v8(P.la.base + qg * P.la.q_stride + piece_offset(P.la, y0, x) + rh * 16, r0, r1);
             }
@@ -247,7 +262,7 @@ __device__ __forceinline__ void store_piece(const GemmParams& P, const uint32_t 
             const int a0 = 4 * e, a1 = 4 * e + 2;
             const float m0 = (((f[a0] + f[a0 + 1]) + f[a0 + 16]) + f[a0 + 17]) * 0.25f;
             const float m1 = (((f[a1] + f[a1 + 1]) + f[a1 + 16]) + f[a1 + 17]) * 0.25f;
-            mk[e] = pack_bf16(m0, m1);
+            mk[e] = pack16<T>(m0, m1);
         }
         if (rh == 0) {
 #pragma unroll
@@ -262,13 +277,14 @@ __device__ __forceinline__ void store_piece(const GemmParams& P, const uint32_t 
 
 // ------------------------------------------------------------------------------------ the kernel
 // LAY: output layout (OFB_LAYOUT_ROWS / BLOCK8X4 / QMINOR8X4)
+// T: 16-bit operand and pyramid storage type (__nv_bfloat16 or __half)
 // MC (CG == 1 only): CTAs run as CLUSTERS OF TWO that walk the same target tiles with their own 128 queries each, their own
 // accumulators and their own cta_group::1 MMAs; every fmap2 stage is fetched half by each CTA and MULTICAST into both, so
 // the L2 -> SM operand stream is halved (as with cta_group::2) while the two epilogues stay independent.
-template <int CG, bool PROF, int LAY, int EPI, bool MC>
+template <typename T, int CG, bool PROF, int LAY, int EPI, bool MC>
 __global__ void __launch_bounds__(NUM_THREADS, 1)
 corr_pyramid_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CUtensorMap map_b,
-                    const GemmParams P) {
+                    const GemmParams<T> P) {
     static_assert(!MC || CG == 1, "multicast clusters issue cta_group::1 MMAs");
     using R = Ring<CG, LAY, EPI>;
     constexpr bool BULK = R::BULK;
@@ -366,7 +382,7 @@ corr_pyramid_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
     } else if (warp == 1) {
         // ============================== MMA issuer (leader CTA, one lane) ====================
         if ((leader || MC) && lane == 0) {
-            constexpr uint32_t idesc = make_idesc(BLOCK_M * CG, TILE_N);
+            constexpr uint32_t idesc = make_idesc(BLOCK_M * CG, TILE_N, F16Format<T>::umma);
             uint32_t stage = 0, bphase = 0, aphase = 0, acc = 0, tphase = 0;
             for (int item = worker; item < P.n_items; item += n_workers) {
                 const ItemCoord ic = decode_item(P, item);
@@ -409,7 +425,7 @@ corr_pyramid_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
         // ============================== epilogue, software-pipelined (8 warps) ===============
         const int q4 = warp & 3, half = (warp - 2) >> 2;
         uint32_t acc = 0, tphase = 0;
-        TileIter it;
+        TileIter<T> it;
         it.init(P, worker);
         if (it.valid) {
             uint32_t buf0[32], buf1[32], keep[4] = {0, 0, 0, 0};
@@ -424,7 +440,7 @@ corr_pyramid_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
                 const int qrow = it.ic.m * m_rows + (int)rank * BLOCK_M + q4 * 32 + lane;     // this lane's query row
                 const bool qok = qrow < P.Nq;
                 const long long qg = (long long)it.ic.b * P.Nq + qrow;
-                TileIter nxt = it;
+                TileIter<T> nxt = it;
                 nxt.advance(P, n_workers);
                 uint32_t taddr_next = 0;
 #pragma unroll
@@ -544,7 +560,7 @@ corr_pyramid_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
                         const int x0 = (tx * P.XB + xb) * P.CW, y0 = (ty * P.YQ + yq) * P.CR;
                         uint32_t pk[32];
 #pragma unroll
-                        for (int c = 0; c < 32; ++c) pk[c] = pack_bf16(f[2 * c], f[2 * c + 1]);
+                        for (int c = 0; c < 32; ++c) pk[c] = pack16<T>(f[2 * c], f[2 * c + 1]);
                         const bool qok = qrow0 + lane < P.Nq;
                         const int nvalid = min(32, P.Nq - qrow0);          // queries of this warp inside the batch element
                         const long long ts0 = PROF ? clock64() : 0;
@@ -571,7 +587,7 @@ corr_pyramid_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
                                     }
                                 } else if (qok && y0 < P.la.h && x < P.la.pitch) {
                                     // direct: one full 32-byte sector (two block rows) per lane and instruction
-                                    __nv_bfloat16* dst = P.la.base + (qglob0 + lane) * P.la.q_stride + piece_offset(P.la, y0, x);
+                                    T* dst = P.la.base + (qglob0 + lane) * P.la.q_stride + piece_offset(P.la, y0, x);
                                     st_global_v8(dst, pk + 4 * b2, pk + 4 * (2 + b2));
                                     st_global_v8(dst + 16, pk + 4 * (4 + b2), pk + 4 * (6 + b2));
                                 }
@@ -584,7 +600,7 @@ corr_pyramid_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
                                 const int a0 = ((2 * c) >> 3) * 32 + ((2 * c) & 7) * 2, a1 = ((2 * c + 1) >> 3) * 32 + ((2 * c + 1) & 7) * 2;
                                 const float m0 = (((f[a0] + f[a0 + 1]) + f[a0 + 16]) + f[a0 + 17]) * 0.25f;
                                 const float m1 = (((f[a1] + f[a1 + 1]) + f[a1 + 16]) + f[a1 + 17]) * 0.25f;
-                                mk[c] = pack_bf16(m0, m1);
+                                mk[c] = pack16<T>(m0, m1);
                             }
                             const int y = y0 >> 1, x = x0 >> 1;
                             if (BULK && bulk_b) {
@@ -616,8 +632,8 @@ corr_pyramid_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
 #pragma unroll
                         for (int p = 0; p < 8; ++p) {
                             const float* s = f + p * 8;
-                            st_shared_v4(wa + ((p ^ wsw_a) << 4), pack_bf16(s[0], s[1]), pack_bf16(s[2], s[3]),
-                                         pack_bf16(s[4], s[5]), pack_bf16(s[6], s[7]));
+                            st_shared_v4(wa + ((p ^ wsw_a) << 4), pack16<T>(s[0], s[1]), pack16<T>(s[2], s[3]),
+                                         pack16<T>(s[4], s[5]), pack16<T>(s[6], s[7]));
                         }
                         if (P.has_b) {
                             // 2x2 means, summed in the reference's raster order then / 4 (corr.py:53)
@@ -631,8 +647,8 @@ corr_pyramid_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
 #pragma unroll
                             for (int p = 0; p < 2; ++p) {
                                 const float* s = m + p * 8;
-                                st_shared_v4(wb + ((p ^ wsw_b) << 4), pack_bf16(s[0], s[1]), pack_bf16(s[2], s[3]),
-                                             pack_bf16(s[4], s[5]), pack_bf16(s[6], s[7]));
+                                st_shared_v4(wb + ((p ^ wsw_b) << 4), pack16<T>(s[0], s[1]), pack16<T>(s[2], s[3]),
+                                             pack16<T>(s[4], s[5]), pack16<T>(s[6], s[7]));
                             }
                         }
                     }
@@ -711,9 +727,9 @@ corr_pyramid_kernel(const __grid_constant__ CUtensorMap map_a, const __grid_cons
 }
 
 // ------------------------------------------------------------------------------------ host side
-template <int CG, bool PROF, int LAY, int EPI, bool MC>
-int launch_gemm(const CUtensorMap& ma, const CUtensorMap& mb, const GemmParams& P, int grid, cudaStream_t st) {
-    OFB_CUDA(ofb_smem_once<corr_pyramid_kernel<CG, PROF, LAY, EPI, MC>>(Ring<CG, LAY, EPI>::SMEM_ALLOC));
+template <typename T, int CG, bool PROF, int LAY, int EPI, bool MC>
+int launch_gemm(const CUtensorMap& ma, const CUtensorMap& mb, const GemmParams<T>& P, int grid, cudaStream_t st) {
+    OFB_CUDA(ofb_smem_once<corr_pyramid_kernel<T, CG, PROF, LAY, EPI, MC>>(Ring<CG, LAY, EPI>::SMEM_ALLOC));
     cudaLaunchConfig_t cfg = {};
     cfg.gridDim = dim3(grid);
     cfg.blockDim = dim3(NUM_THREADS);
@@ -726,13 +742,14 @@ int launch_gemm(const CUtensorMap& ma, const CUtensorMap& mb, const GemmParams& 
     attr[0].val.clusterDim.z = 1;
     cfg.attrs = attr;
     cfg.numAttrs = 1;
-    OFB_CUDA(cudaLaunchKernelEx(&cfg, corr_pyramid_kernel<CG, PROF, LAY, EPI, MC>, ma, mb, P));
+    OFB_CUDA(cudaLaunchKernelEx(&cfg, corr_pyramid_kernel<T, CG, PROF, LAY, EPI, MC>, ma, mb, P));
     OFB_LAUNCH_CHECK();
     return OFB_OK;
 }
 
 // One GEMM run: queries (B, Nq, C) x targets (B, th*tw, C) -> level la_idx (th x tw per query) and, when
-// lb_idx >= 0, its 2x2 mean.
+// lb_idx >= 0, its 2x2 mean.  T: the operands' and the pyramid's 16-bit type.
+template <typename T>
 int run_gemm(const void* f1_km, const void* f2_km, const ofb_pyramid* pyr, int la_idx, int lb_idx, int B, int C, int Nq,
              int th, int tw, float scale, int cg_mode, unsigned long long* prof, int prof_slot, cudaStream_t st) {
     // cg_mode: 1 = one CTA per tile, 2 = CTA pair sharing one 256-row accumulator tile (cta_group::2),
@@ -740,7 +757,7 @@ int run_gemm(const void* f1_km, const void* f2_km, const ofb_pyramid* pyr, int l
     const bool mc = cg_mode == 3;
     const int cg = mc ? 1 : cg_mode;           // tcgen05 cta_group
     const int cl = (cg == 2 || mc) ? 2 : 1;    // CTAs per cluster / work item
-    GemmParams P = {};
+    GemmParams<T> P = {};
     P.B = B; P.C = C; P.kb = C / BLOCK_K; P.Nq = Nq; P.th = th; P.tw = tw;
     P.scale = scale; P.apply_scale = (scale != 1.0f) ? 1 : 0;
     // chunk shape follows the output layout (a chunk must be whole 64/128-byte runs of it); tile shape =
@@ -783,12 +800,12 @@ int run_gemm(const void* f1_km, const void* f2_km, const ofb_pyramid* pyr, int l
     const long long n_items = (long long)B * P.mblk * P.n_chunks;
     if (n_items > 0x7fffffffLL) return OFB_EUNSUPPORTED;
     P.n_items = (int)n_items;
-    P.la.base = reinterpret_cast<__nv_bfloat16*>(pyr->base[la_idx]);
+    P.la.base = reinterpret_cast<T*>(pyr->base[la_idx]);
     P.la.q_stride = pyr->q_stride[la_idx]; P.la.pitch = pyr->row_pitch[la_idx];
     P.la.h = pyr->lvl_h[la_idx]; P.la.w = pyr->lvl_w[la_idx]; P.la.blocked = blk; P.la.blk_stride = blk_stride;
     P.has_b = lb_idx >= 0 ? 1 : 0;
     if (P.has_b) {
-        P.lb.base = reinterpret_cast<__nv_bfloat16*>(pyr->base[lb_idx]);
+        P.lb.base = reinterpret_cast<T*>(pyr->base[lb_idx]);
         P.lb.q_stride = pyr->q_stride[lb_idx]; P.lb.pitch = pyr->row_pitch[lb_idx];
         P.lb.h = pyr->lvl_h[lb_idx]; P.lb.w = pyr->lvl_w[lb_idx]; P.lb.blocked = blk; P.lb.blk_stride = blk_stride;
     }
@@ -804,7 +821,7 @@ int run_gemm(const void* f1_km, const void* f2_km, const ofb_pyramid* pyr, int l
         const cuuint64_t dims[3] = {(cuuint64_t)C, (cuuint64_t)Nq, (cuuint64_t)B};
         const cuuint64_t str[2] = {(cuuint64_t)C * 2, (cuuint64_t)Nq * C * 2};
         const cuuint32_t box[3] = {BLOCK_K, BLOCK_M, 1};
-        if (!encode_tiled(&ma, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 3, f1_km, dims, str, box, CU_TENSOR_MAP_SWIZZLE_128B,
+        if (!encode_tiled(&ma, F16Format<T>::tma, 3, f1_km, dims, str, box, CU_TENSOR_MAP_SWIZZLE_128B,
                           CU_TENSOR_MAP_L2_PROMOTION_L2_256B))
             return OFB_EDRIVER;
     }
@@ -812,45 +829,59 @@ int run_gemm(const void* f1_km, const void* f2_km, const ofb_pyramid* pyr, int l
         const cuuint64_t dims[4] = {(cuuint64_t)C, (cuuint64_t)tw, (cuuint64_t)th, (cuuint64_t)B};
         const cuuint64_t str[3] = {(cuuint64_t)C * 2, (cuuint64_t)tw * C * 2, (cuuint64_t)th * tw * C * 2};
         const cuuint32_t box[4] = {BLOCK_K, (cuuint32_t)P.CW, (cuuint32_t)P.box_rows, 1};
-        if (!encode_tiled(&mb, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, f2_km, dims, str, box, CU_TENSOR_MAP_SWIZZLE_128B,
+        if (!encode_tiled(&mb, F16Format<T>::tma, 4, f2_km, dims, str, box, CU_TENSOR_MAP_SWIZZLE_128B,
                           CU_TENSOR_MAP_L2_PROMOTION_L2_256B))
             return OFB_EDRIVER;
     }
     int grid = workers * cl;
     if ((long long)grid > n_items * cl) grid = (int)(n_items * cl);
-    // epilogue store mode of the query-minor layout (OFB_K2_EPI=direct|bulk overrides; other layouts stage through smem)
-    int epi = EPI_DIRECT;
-    if (const char* e = getenv("OFB_K2_EPI")) epi = (e[0] == 'd' || e[0] == '0') ? EPI_DIRECT : (e[0] == 'p' || e[0] == '2') ? EPI_PIPE : EPI_BULK;
-    if (pyr->layout != OFB_LAYOUT_QMINOR8X4) epi = EPI_DIRECT;
+    if constexpr (std::is_same<T, __half>::value) {
+        // fp16 is built with the direct epilogue only and has no diagnostics variant: OFB_K2_EPI is ignored here
+        if (prof) return OFB_EUNSUPPORTED;
+        if (mc) return pyr->layout == OFB_LAYOUT_QMINOR8X4 ? launch_gemm<T, 1, false, 2, 0, true>(ma, mb, P, grid, st)
+                                                           : OFB_EUNSUPPORTED;
+#define OFB_GEMM_CASE_F16(CGV, LAYV) \
+        if (cg == CGV && pyr->layout == LAYV) return launch_gemm<T, CGV, false, LAYV, EPI_DIRECT, false>(ma, mb, P, grid, st);
+        OFB_GEMM_CASE_F16(1, 0) OFB_GEMM_CASE_F16(1, 1) OFB_GEMM_CASE_F16(1, 2)
+        OFB_GEMM_CASE_F16(2, 0) OFB_GEMM_CASE_F16(2, 1) OFB_GEMM_CASE_F16(2, 2)
+#undef OFB_GEMM_CASE_F16
+        return OFB_EINVAL;
+    } else {
+        // epilogue store mode of the query-minor layout (OFB_K2_EPI=direct|bulk overrides; other layouts stage through smem)
+        int epi = EPI_DIRECT;
+        if (const char* e = getenv("OFB_K2_EPI")) epi = (e[0] == 'd' || e[0] == '0') ? EPI_DIRECT : (e[0] == 'p' || e[0] == '2') ? EPI_PIPE : EPI_BULK;
+        if (pyr->layout != OFB_LAYOUT_QMINOR8X4) epi = EPI_DIRECT;
 #define OFB_GEMM_CASE(CGV, PROFV, LAYV, EPIV) \
-    if (cg == CGV && !mc && (prof != nullptr) == PROFV && pyr->layout == LAYV && epi == EPIV) \
-        return launch_gemm<CGV, PROFV, LAYV, EPIV, false>(ma, mb, P, grid, st);
-    OFB_GEMM_CASE(1, false, 0, 0) OFB_GEMM_CASE(1, false, 1, 0) OFB_GEMM_CASE(1, false, 2, 0) OFB_GEMM_CASE(1, false, 2, 1)
-    OFB_GEMM_CASE(2, false, 0, 0) OFB_GEMM_CASE(2, false, 1, 0) OFB_GEMM_CASE(2, false, 2, 0) OFB_GEMM_CASE(2, false, 2, 1)
-    OFB_GEMM_CASE(1, true, 0, 0) OFB_GEMM_CASE(1, true, 1, 0) OFB_GEMM_CASE(1, true, 2, 0) OFB_GEMM_CASE(1, true, 2, 1)
-    OFB_GEMM_CASE(2, true, 0, 0) OFB_GEMM_CASE(2, true, 1, 0) OFB_GEMM_CASE(2, true, 2, 0) OFB_GEMM_CASE(2, true, 2, 1)
-    OFB_GEMM_CASE(1, false, 2, 2) OFB_GEMM_CASE(2, false, 2, 2) OFB_GEMM_CASE(1, true, 2, 2) OFB_GEMM_CASE(2, true, 2, 2)
-    // multicast clusters: the product layout (query-minor) only
-    if (mc && pyr->layout == OFB_LAYOUT_QMINOR8X4) {
-        if (!prof && epi == EPI_DIRECT) return launch_gemm<1, false, 2, 0, true>(ma, mb, P, grid, st);
-        if (!prof && epi == EPI_BULK) return launch_gemm<1, false, 2, 1, true>(ma, mb, P, grid, st);
-        if (prof && epi == EPI_DIRECT) return launch_gemm<1, true, 2, 0, true>(ma, mb, P, grid, st);
-        if (prof && epi == EPI_BULK) return launch_gemm<1, true, 2, 1, true>(ma, mb, P, grid, st);
-        if (!prof && epi == EPI_PIPE) return launch_gemm<1, false, 2, 2, true>(ma, mb, P, grid, st);
-        if (prof && epi == EPI_PIPE) return launch_gemm<1, true, 2, 2, true>(ma, mb, P, grid, st);
-    }
-    if (mc) return OFB_EUNSUPPORTED;
+        if (cg == CGV && !mc && (prof != nullptr) == PROFV && pyr->layout == LAYV && epi == EPIV) \
+            return launch_gemm<T, CGV, PROFV, LAYV, EPIV, false>(ma, mb, P, grid, st);
+        OFB_GEMM_CASE(1, false, 0, 0) OFB_GEMM_CASE(1, false, 1, 0) OFB_GEMM_CASE(1, false, 2, 0) OFB_GEMM_CASE(1, false, 2, 1)
+        OFB_GEMM_CASE(2, false, 0, 0) OFB_GEMM_CASE(2, false, 1, 0) OFB_GEMM_CASE(2, false, 2, 0) OFB_GEMM_CASE(2, false, 2, 1)
+        OFB_GEMM_CASE(1, true, 0, 0) OFB_GEMM_CASE(1, true, 1, 0) OFB_GEMM_CASE(1, true, 2, 0) OFB_GEMM_CASE(1, true, 2, 1)
+        OFB_GEMM_CASE(2, true, 0, 0) OFB_GEMM_CASE(2, true, 1, 0) OFB_GEMM_CASE(2, true, 2, 0) OFB_GEMM_CASE(2, true, 2, 1)
+        OFB_GEMM_CASE(1, false, 2, 2) OFB_GEMM_CASE(2, false, 2, 2) OFB_GEMM_CASE(1, true, 2, 2) OFB_GEMM_CASE(2, true, 2, 2)
+        // multicast clusters: the product layout (query-minor) only
+        if (mc && pyr->layout == OFB_LAYOUT_QMINOR8X4) {
+            if (!prof && epi == EPI_DIRECT) return launch_gemm<T, 1, false, 2, 0, true>(ma, mb, P, grid, st);
+            if (!prof && epi == EPI_BULK) return launch_gemm<T, 1, false, 2, 1, true>(ma, mb, P, grid, st);
+            if (prof && epi == EPI_DIRECT) return launch_gemm<T, 1, true, 2, 0, true>(ma, mb, P, grid, st);
+            if (prof && epi == EPI_BULK) return launch_gemm<T, 1, true, 2, 1, true>(ma, mb, P, grid, st);
+            if (!prof && epi == EPI_PIPE) return launch_gemm<T, 1, false, 2, 2, true>(ma, mb, P, grid, st);
+            if (prof && epi == EPI_PIPE) return launch_gemm<T, 1, true, 2, 2, true>(ma, mb, P, grid, st);
+        }
+        if (mc) return OFB_EUNSUPPORTED;
 #undef OFB_GEMM_CASE
-    return OFB_EINVAL;
+        return OFB_EINVAL;
+    }
 }
 
-int corr_pyramid_impl(const void* f1_km, const void* f2_km, const void* f2q_km, const ofb_pyramid* pyr, int B, int C, int h,
-                      int w, float scale, int cta_group, unsigned long long* prof, void* stream) {
+// dtype: the 16-bit type of the operands and of the pyramid, OFB_DTYPE_BF16 or OFB_DTYPE_F16
+int corr_pyramid_impl(int dtype, const void* f1_km, const void* f2_km, const void* f2q_km, const ofb_pyramid* pyr, int B,
+                      int C, int h, int w, float scale, int cta_group, unsigned long long* prof, void* stream) {
     if (B == 0) return OFB_OK;   // nothing to do: empty tensors have no storage, their pointers may be null
     if (!f1_km || !f2_km || !pyr || B < 0 || C <= 0 || h <= 0 || w <= 0) return OFB_EINVAL;
     if (cta_group < 0 || cta_group > 3) return OFB_EINVAL;
     if (pyr->levels < 1 || pyr->levels > OFB_MAX_LEVELS) return OFB_EINVAL;
-    if (pyr->dtype != OFB_DTYPE_BF16) return OFB_EUNSUPPORTED;          // fp32 pyramids: ofb_corr_pyramid_simt_f32
+    if (pyr->dtype != dtype) return OFB_EUNSUPPORTED;                   // fp32 pyramids: ofb_corr_pyramid_simt_f32
     if (C % BLOCK_K != 0 || C > MAX_KB * BLOCK_K) return OFB_EUNSUPPORTED;
     if (pyr->levels > 2 && !f2q_km) return OFB_EINVAL;                  // levels 2, 3 come from the 4x4-averaged fmap2
     if (B == 0) return OFB_OK;
@@ -878,22 +909,28 @@ int corr_pyramid_impl(const void* f1_km, const void* f2_km, const void* f2q_km, 
     if (cg == 0) cg = (pyr->layout == OFB_LAYOUT_QMINOR8X4 && h * w > BLOCK_M) ? 3 : 1;
     if (cg == 3 && pyr->layout != OFB_LAYOUT_QMINOR8X4) return OFB_EUNSUPPORTED;
     cudaStream_t st = (cudaStream_t)stream;
-    const int rc = run_gemm(f1_km, f2_km, pyr, 0, pyr->levels > 1 ? 1 : -1, B, C, h * w, h, w, scale, cg, prof, 0, st);
+    const auto run = dtype == OFB_DTYPE_F16 ? run_gemm<__half> : run_gemm<__nv_bfloat16>;
+    const int rc = run(f1_km, f2_km, pyr, 0, pyr->levels > 1 ? 1 : -1, B, C, h * w, h, w, scale, cg, prof, 0, st);
     if (rc != OFB_OK || pyr->levels <= 2) return rc;
-    return run_gemm(f1_km, f2q_km, pyr, 2, pyr->levels > 3 ? 3 : -1, B, C, h * w, h >> 2, w >> 2, scale, cg, prof, 1, st);
+    return run(f1_km, f2q_km, pyr, 2, pyr->levels > 3 ? 3 : -1, B, C, h * w, h >> 2, w >> 2, scale, cg, prof, 1, st);
 }
 
 }  // namespace
 
 OFB_API int ofb_corr_pyramid_bf16(const void* f1_km, const void* f2_km, const void* f2q_km, const ofb_pyramid* pyr, int B,
                                   int C, int h, int w, float scale, int cta_group, void* stream) {
-    return corr_pyramid_impl(f1_km, f2_km, f2q_km, pyr, B, C, h, w, scale, cta_group, nullptr, stream);
+    return corr_pyramid_impl(OFB_DTYPE_BF16, f1_km, f2_km, f2q_km, pyr, B, C, h, w, scale, cta_group, nullptr, stream);
+}
+
+OFB_API int ofb_corr_pyramid_f16(const void* f1_km, const void* f2_km, const void* f2q_km, const ofb_pyramid* pyr, int B,
+                                 int C, int h, int w, float scale, int cta_group, void* stream) {
+    return corr_pyramid_impl(OFB_DTYPE_F16, f1_km, f2_km, f2q_km, pyr, B, C, h, w, scale, cta_group, nullptr, stream);
 }
 
 OFB_API int ofb_corr_pyramid_bf16_profile(const void* f1_km, const void* f2_km, const void* f2q_km, const ofb_pyramid* pyr,
                                           int B, int C, int h, int w, float scale, int cta_group, uint64_t* prof_dev,
                                           void* stream) {
     if (!prof_dev) return OFB_EINVAL;
-    return corr_pyramid_impl(f1_km, f2_km, f2q_km, pyr, B, C, h, w, scale, cta_group,
+    return corr_pyramid_impl(OFB_DTYPE_BF16, f1_km, f2_km, f2q_km, pyr, B, C, h, w, scale, cta_group,
                              reinterpret_cast<unsigned long long*>(prof_dev), stream);
 }

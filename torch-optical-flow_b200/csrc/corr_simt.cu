@@ -1,6 +1,6 @@
 // corr_simt.cu -- operand preparation for K2 and a CUDA-core correlation-pyramid builder.
 //
-//  * ofb_corr_prep_bf16: fmap (B,C,h,w) fp32 NCHW -> (B,(h/pool)*(w/pool),C) bf16, K-major, times
+//  * ofb_corr_prep_bf16 / _from / _to: fmap (B,C,h,w) NCHW -> (B,(h/pool)*(w/pool),C) bf16 or fp16, K-major, times
 //    `scale`, optionally averaged over complete pool x pool blocks.  Replaces the .view /
 //    .transpose(1,2) in CorrBlock.corr (reference methods/raft/model/corr.py:82-85), folds the
 //    1/sqrt(C) of corr.py:87 into fmap1, and -- pool = 4 on fmap2 -- feeds the run that produces
@@ -8,8 +8,10 @@
 //    tensor-core path needs (0.2 GB at the Sintel configuration against 2.1 GB of pyramid).
 //  * ofb_pyramid_layout: strides of the pyramid buffers (see include/ofb200.h).
 //  * ofb_corr_pyramid_simt_f32: fp32 CUDA-core GEMM + successive 2x2 pooling -- the reference's
-//    own op order (corr.py:44-54,79-87).  Not the fast path: tests use it as an on-device
+//    own op order (corr.py:44-54,79-87), fp32, bf16 or fp16 stored.  Not the fast path: tests use it as an on-device
 //    cross-check of the tcgen05 builder at sizes the CPU oracle cannot reach.
+#include <type_traits>
+
 #include "common.cuh"
 
 namespace {
@@ -19,9 +21,9 @@ constexpr int TP = 32;    // pixels per tile
 constexpr int TCMAX = 256;  // channels per tile (the whole K extent of the tensor-core path)
 
 // One CTA turns a 32-pixel x C-channel tile: reads are 128-byte lines (32 pixels of one channel), 8 in
-// flight per thread; writes are whole 2*C-byte pixel rows of the K-major operand.
-template <int POOL, typename TIn>
-__global__ void __launch_bounds__(256) prep_kernel(const TIn* __restrict__ in, __nv_bfloat16* __restrict__ out, int C,
+// flight per thread; writes are whole 2*C-byte pixel rows of the K-major operand (TOut: bf16 or fp16).
+template <int POOL, typename TIn, typename TOut>
+__global__ void __launch_bounds__(256) prep_kernel(const TIn* __restrict__ in, TOut* __restrict__ out, int C,
                                                    int h, int w, float scale) {
     // output pixel p = (yo, xo) of the (h/POOL) x (w/POOL) image = mean of a complete POOL x POOL block
     extern __shared__ float tile[];                       // [Ct][TP + 1]
@@ -60,14 +62,19 @@ __global__ void __launch_bounds__(256) prep_kernel(const TIn* __restrict__ in, _
         }
     }
     __syncthreads();
-    // write: one pixel row (Ct channels) per warp pass, bf16x2 per lane, 128 bytes per instruction
+    // write: one pixel row (Ct channels) per warp pass, two 16-bit elements per lane, 128 bytes per instruction
     for (int q = warp; q < TP; q += 8) {
         const int pp = p0 + q;
         if (pp >= HWo) break;
-        __nv_bfloat16* dst = out + ((size_t)b * HWo + pp) * C + c0;
+        TOut* dst = out + ((size_t)b * HWo + pp) * C + c0;
         for (int cc = 2 * lane; cc < Ct; cc += 64) {
-            __nv_bfloat162 v2 = __floats2bfloat162_rn(tile[cc * (TP + 1) + q], tile[(cc + 1) * (TP + 1) + q]);
-            *reinterpret_cast<__nv_bfloat162*>(dst + cc) = v2;
+            if constexpr (std::is_same<TOut, __half>::value) {
+                __half2 v2 = __floats2half2_rn(tile[cc * (TP + 1) + q], tile[(cc + 1) * (TP + 1) + q]);
+                *reinterpret_cast<__half2*>(dst + cc) = v2;
+            } else {
+                __nv_bfloat162 v2 = __floats2bfloat162_rn(tile[cc * (TP + 1) + q], tile[(cc + 1) * (TP + 1) + q]);
+                *reinterpret_cast<__nv_bfloat162*>(dst + cc) = v2;
+            }
         }
     }
 }
@@ -76,6 +83,7 @@ __global__ void __launch_bounds__(256) prep_kernel(const TIn* __restrict__ in, _
 template <typename T> __device__ __forceinline__ T cvt_out(float v);
 template <> __device__ __forceinline__ float cvt_out<float>(float v) { return v; }
 template <> __device__ __forceinline__ __nv_bfloat16 cvt_out<__nv_bfloat16>(float v) { return __float2bfloat16_rn(v); }
+template <> __device__ __forceinline__ __half cvt_out<__half>(float v) { return __float2half_rn(v); }
 
 constexpr int GT = 32;
 
@@ -119,6 +127,7 @@ __global__ void __launch_bounds__(GT * GT / 4) corr_l0_kernel(const float* __res
 template <typename T> __device__ __forceinline__ float cvt_in(T v);
 template <> __device__ __forceinline__ float cvt_in<float>(float v) { return v; }
 template <> __device__ __forceinline__ float cvt_in<__nv_bfloat16>(__nv_bfloat16 v) { return __bfloat162float(v); }
+template <> __device__ __forceinline__ float cvt_in<__half>(__half v) { return __half2float(v); }
 
 template <typename T>
 __global__ void __launch_bounds__(256) pool2_kernel(const T* __restrict__ src, T* __restrict__ dst, long long Qn,
@@ -161,37 +170,50 @@ int build_simt(const float* f1, const float* f2, const ofb_pyramid* pyr, int B, 
 
 }  // namespace
 
-template <typename TIn>
-static int launch_prep(const void* fmap, __nv_bfloat16* out, int B, int C, int h, int w, int pool, float scale, int HWo,
+template <typename TIn, typename TOut>
+static int launch_prep(const void* fmap, TOut* out, int B, int C, int h, int w, int pool, float scale, int HWo,
                        cudaStream_t st) {
     dim3 grid((HWo + TP - 1) / TP, (C + TCMAX - 1) / TCMAX, B);
     const size_t smem = (size_t)(C < TCMAX ? C : TCMAX) * (TP + 1) * sizeof(float);      // <= 33 KiB
     const TIn* in = reinterpret_cast<const TIn*>(fmap);
-    if (pool == 1) prep_kernel<1, TIn><<<grid, 256, smem, st>>>(in, out, C, h, w, scale);
-    else if (pool == 2) prep_kernel<2, TIn><<<grid, 256, smem, st>>>(in, out, C, h, w, scale);
-    else if (pool == 4) prep_kernel<4, TIn><<<grid, 256, smem, st>>>(in, out, C, h, w, scale);
-    else prep_kernel<8, TIn><<<grid, 256, smem, st>>>(in, out, C, h, w, scale);
+    if (pool == 1) prep_kernel<1, TIn, TOut><<<grid, 256, smem, st>>>(in, out, C, h, w, scale);
+    else if (pool == 2) prep_kernel<2, TIn, TOut><<<grid, 256, smem, st>>>(in, out, C, h, w, scale);
+    else if (pool == 4) prep_kernel<4, TIn, TOut><<<grid, 256, smem, st>>>(in, out, C, h, w, scale);
+    else prep_kernel<8, TIn, TOut><<<grid, 256, smem, st>>>(in, out, C, h, w, scale);
     OFB_LAUNCH_CHECK();
     return OFB_OK;
 }
 
-OFB_API int ofb_corr_prep_from(const void* fmap_nchw, int in_dtype, void* out_km_bf16, int B, int C, int h, int w, int pool,
-                               float scale, void* stream) {
+template <typename TOut>
+static int launch_prep_from(const void* fmap, int in_dtype, TOut* out, int B, int C, int h, int w, int pool, float scale,
+                            int HWo, cudaStream_t st) {
+    if (in_dtype == OFB_DTYPE_F32) return launch_prep<float>(fmap, out, B, C, h, w, pool, scale, HWo, st);
+    if (in_dtype == OFB_DTYPE_BF16) return launch_prep<__nv_bfloat16>(fmap, out, B, C, h, w, pool, scale, HWo, st);
+    return launch_prep<__half>(fmap, out, B, C, h, w, pool, scale, HWo, st);
+}
+
+OFB_API int ofb_corr_prep_to(const void* fmap_nchw, int in_dtype, void* out_km, int out_dtype, int B, int C, int h, int w,
+                             int pool, float scale, void* stream) {
     if (B == 0) return OFB_OK;   // nothing to do: empty tensors have no storage, their pointers may be null
-    if (!fmap_nchw || !out_km_bf16 || B < 0 || C <= 0 || h <= 0 || w <= 0) return OFB_EINVAL;
+    if (!fmap_nchw || !out_km || B < 0 || C <= 0 || h <= 0 || w <= 0) return OFB_EINVAL;
     if (pool != 1 && pool != 2 && pool != 4 && pool != 8) return OFB_EINVAL;
     if (in_dtype != OFB_DTYPE_F32 && in_dtype != OFB_DTYPE_BF16 && in_dtype != OFB_DTYPE_F16) return OFB_EINVAL;
+    if (out_dtype != OFB_DTYPE_BF16 && out_dtype != OFB_DTYPE_F16) return OFB_EINVAL;
     if (C & 1) return OFB_EUNSUPPORTED;
-    if (reinterpret_cast<uintptr_t>(out_km_bf16) & 3) return OFB_EALIGN;
+    if (reinterpret_cast<uintptr_t>(out_km) & 3) return OFB_EALIGN;
     if (reinterpret_cast<uintptr_t>(fmap_nchw) & (in_dtype == OFB_DTYPE_F32 ? 3 : 1)) return OFB_EALIGN;
     const int HWo = (h / pool) * (w / pool);
     if (HWo == 0) return OFB_OK;
     if (B > 65535) return OFB_EUNSUPPORTED;
-    __nv_bfloat16* out = reinterpret_cast<__nv_bfloat16*>(out_km_bf16);
     cudaStream_t st = (cudaStream_t)stream;
-    if (in_dtype == OFB_DTYPE_F32) return launch_prep<float>(fmap_nchw, out, B, C, h, w, pool, scale, HWo, st);
-    if (in_dtype == OFB_DTYPE_BF16) return launch_prep<__nv_bfloat16>(fmap_nchw, out, B, C, h, w, pool, scale, HWo, st);
-    return launch_prep<__half>(fmap_nchw, out, B, C, h, w, pool, scale, HWo, st);
+    if (out_dtype == OFB_DTYPE_F16)
+        return launch_prep_from(fmap_nchw, in_dtype, reinterpret_cast<__half*>(out_km), B, C, h, w, pool, scale, HWo, st);
+    return launch_prep_from(fmap_nchw, in_dtype, reinterpret_cast<__nv_bfloat16*>(out_km), B, C, h, w, pool, scale, HWo, st);
+}
+
+OFB_API int ofb_corr_prep_from(const void* fmap_nchw, int in_dtype, void* out_km_bf16, int B, int C, int h, int w, int pool,
+                               float scale, void* stream) {
+    return ofb_corr_prep_to(fmap_nchw, in_dtype, out_km_bf16, OFB_DTYPE_BF16, B, C, h, w, pool, scale, stream);
 }
 
 OFB_API int ofb_corr_prep_bf16(const float* fmap_nchw, void* out_km_bf16, int B, int C, int h, int w, int pool,
@@ -236,5 +258,6 @@ OFB_API int ofb_corr_pyramid_simt_f32(const float* fmap1, const float* fmap2, co
     cudaStream_t st = (cudaStream_t)stream;
     if (pyr->dtype == OFB_DTYPE_F32) return build_simt<float>(fmap1, fmap2, pyr, B, C, h, w, scale, st);
     if (pyr->dtype == OFB_DTYPE_BF16) return build_simt<__nv_bfloat16>(fmap1, fmap2, pyr, B, C, h, w, scale, st);
+    if (pyr->dtype == OFB_DTYPE_F16) return build_simt<__half>(fmap1, fmap2, pyr, B, C, h, w, scale, st);
     return OFB_EINVAL;
 }

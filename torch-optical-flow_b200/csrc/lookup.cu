@@ -25,6 +25,7 @@
 // HBM roofline per query and iteration (SURVEY.md 8d): L*(2r+2)^2*esize + 8 read, 4*L*(2r+1)^2 written.
 #include <climits>
 #include <cstdlib>
+#include <type_traits>
 
 #include "common.cuh"
 
@@ -43,7 +44,7 @@ struct LookupParams {
     int lh[OFB_MAX_LEVELS];
     int lw[OFB_MAX_LEVELS];
     int levels, radius, B, h, w;
-    int blocked;   // 8x4-blocked layouts (register-tile kernel only)
+    int blocked;   // 8x4-blocked layouts (register-tile kernel only, 16-bit pyramids)
     long long blk_stride;   // elements between consecutive blocks: 32, or 32 * Q (query-minor)
 };
 
@@ -56,8 +57,11 @@ template <> struct Elem<__nv_bfloat16> {
         return __bfloat162float(__ldg(row + x));
     }
 };
+template <> struct Elem<__half> {
+    static __device__ __forceinline__ float get(const __half* row, int x) { return __half2float(__ldg(row + x)); }
+};
 
-// patch load: fp32 -> one element per word; bf16 -> two elements per 4-byte word
+// patch load: fp32 -> one element per word; bf16 / fp16 -> two elements per 4-byte word
 template <typename T>
 __device__ __forceinline__ void load_patch(float* patch, const T* slice, int pitch, int Hl, int Wl, int px0, int py0,
                                            int rows, int lane);
@@ -88,6 +92,25 @@ __device__ __forceinline__ void load_patch<__nv_bfloat16>(float* patch, const __
             const unsigned wd = __ldg(reinterpret_cast<const unsigned*>(slice + (size_t)y * pitch + x));
             v0 = __uint_as_float(wd << 16);
             if (x + 1 < Wl) v1 = __uint_as_float(wd & 0xffff0000u);
+        }
+        patch[r * PD + 2 * cw] = v0;
+        patch[r * PD + 2 * cw + 1] = v1;
+    }
+}
+
+template <>
+__device__ __forceinline__ void load_patch<__half>(float* patch, const __half* slice, int pitch, int Hl, int Wl, int px0,
+                                                   int py0, int rows, int lane) {
+    // px0 is even, pitch is even, the slice base is 4-byte aligned
+#pragma unroll
+    for (int e = lane; e < PD * (PD / 2); e += 32) {
+        const int r = e / (PD / 2), cw = e - r * (PD / 2);
+        const int y = py0 + r, x = px0 + 2 * cw;
+        float v0 = 0.0f, v1 = 0.0f;
+        if (r < rows && y >= 0 && y < Hl && x >= 0 && x < Wl) {
+            const float2 v = __half22float2(__ldg(reinterpret_cast<const __half2*>(slice + (size_t)y * pitch + x)));
+            v0 = v.x;
+            if (x + 1 < Wl) v1 = v.y;
         }
         patch[r * PD + 2 * cw] = v0;
         patch[r * PD + 2 * cw + 1] = v1;
@@ -187,7 +210,7 @@ __global__ void __launch_bounds__(NW * 32) lookup_kernel(const LookupParams P, c
 }
 
 // ------------------------------------------------------------------------------------------------
-// Register-tile lookup for bf16 pyramids (the product path).
+// Register-tile lookup for 16-bit (bf16 / fp16) pyramids (the product path).
 //
 // thread = (query, level): lane <-> query (coordinates in, channel rows out are 128-byte coalesced),
 // warp <-> pyramid level.  Each thread
@@ -199,6 +222,7 @@ __global__ void __launch_bounds__(NW * 32) lookup_kernel(const LookupParams P, c
 //      the reference's 2-tap form plus exact zeros;
 //   3. streams the window row by row: 16-byte aligned chunk loads (2.25 per row on average),
 //      realigned in registers with two select stages (word shift) and a funnel shift (half-word),
+//      widened to fp32 (bf16: a shift or mask of the word; fp16: a conversion of each half),
 //      horizontal filter -> 9 values, vertical filter accumulated into three live output rows;
 //   4. writes each finished output row straight to its 9 channels.
 // No shared memory, no shuffles, ~56 warp instructions per (query, level) against ~230 before.
@@ -251,7 +275,9 @@ __device__ __forceinline__ TapSet<R> make_taps(float center, int size, int32_t* 
     return ts;
 }
 
-template <int R, int GR>
+// T: the pyramid's 16-bit type.  Only the widening of the realigned words depends on it: the coordinates, floor
+// indices, validity masks and filter weights are the same code for both types.
+template <int R, int GR, typename T>
 __global__ void __launch_bounds__(128) lookup_tile_kernel(const LookupParams P, const float* __restrict__ coords,
                                                            float* __restrict__ out, int32_t* __restrict__ idx_out,
                                                            uint8_t* __restrict__ valid_out) {
@@ -301,7 +327,7 @@ __global__ void __launch_bounds__(128) lookup_tile_kernel(const LookupParams P, 
     // the last window column / row only carries weight when some tap slid by one (dmask != 0)
     const int wcols = tx.dmask ? WIN : WIN - 1, wrows = ty.dmask ? WIN : WIN - 1;
     const bool ck2 = (s + wcols > 16) && xa + 16 >= 0 && xa + 24 <= pitch;
-    const __nv_bfloat16* slice = reinterpret_cast<const __nv_bfloat16*>(P.base[l]) + q * P.q_stride[l];
+    const T* slice = reinterpret_cast<const T*>(P.base[l]) + q * P.q_stride[l];
     float* outp = out + (b * (long long)(P.levels * DD) + (long long)l * DD) * HW + p;
 
     float acc[3][D];                                            // output rows j = r, r-1, r-2 in flight
@@ -328,7 +354,7 @@ __global__ void __launch_bounds__(128) lookup_tile_kernel(const LookupParams P, 
             const int y = ys + r;
             const bool rok = !dead && r < wrows && y >= 0 && y < Hl;
             // an aligned 8-element chunk is one row of an 8x4 block (blocked) or 8 consecutive row elements
-            const __nv_bfloat16* row = P.blocked
+            const T* row = P.blocked
                 ? slice + ((long long)(y >> 2) * (pitch >> 3) + (xa >> 3)) * P.blk_stride + (y & 3) * 8
                 : slice + (long long)y * pitch + xa;
 #pragma unroll
@@ -374,9 +400,15 @@ __global__ void __launch_bounds__(128) lookup_tile_kernel(const LookupParams P, 
 #pragma unroll
         for (int k = 0; k < NW; ++k) v[k] = __funnelshift_r(t2[k], t2[k + 1], hs);
         float px[WIN];
+        if constexpr (std::is_same<T, __half>::value) {
 #pragma unroll
-        for (int e = 0; e < WIN; ++e)
-            px[e] = __uint_as_float((e & 1) ? (v[e >> 1] & 0xffff0000u) : (v[e >> 1] << 16));
+            for (int e = 0; e < WIN; ++e)
+                px[e] = __half2float(__ushort_as_half((unsigned short)((e & 1) ? (v[e >> 1] >> 16) : (v[e >> 1] & 0xffffu))));
+        } else {
+#pragma unroll
+            for (int e = 0; e < WIN; ++e)
+                px[e] = __uint_as_float((e & 1) ? (v[e >> 1] & 0xffff0000u) : (v[e >> 1] << 16));
+        }
         // ---- horizontal filter
         float hrow[D];
 #pragma unroll
@@ -435,6 +467,19 @@ __global__ void __launch_bounds__(256) bilinear_sampler_kernel(const float* __re
     }
 }
 
+template <typename T>
+int launch_tile(const LookupParams& P, const float* coords, float* out, int32_t* idx, uint8_t* valid, int radius, int gr,
+                int blocks, int threads, size_t wsm, cudaStream_t st) {
+    OFB_CUDA(ofb_smem_once<lookup_tile_kernel<4, 3, T>>(11 * 128 * 40));
+    OFB_CUDA(ofb_smem_once<lookup_tile_kernel<4, 16, T>>(11 * 128 * 40));
+    OFB_CUDA(ofb_smem_once<lookup_tile_kernel<3, 16, T>>(9 * 128 * 40));
+    if (radius == 4 && gr == 3) lookup_tile_kernel<4, 3, T><<<blocks, threads, wsm, st>>>(P, coords, out, idx, valid);
+    else if (radius == 4) lookup_tile_kernel<4, 16, T><<<blocks, threads, wsm, st>>>(P, coords, out, idx, valid);
+    else lookup_tile_kernel<3, 16, T><<<blocks, threads, wsm, st>>>(P, coords, out, idx, valid);
+    OFB_LAUNCH_CHECK();
+    return OFB_OK;
+}
+
 }  // namespace
 
 OFB_API int ofb_corr_lookup(const ofb_pyramid* pyr, const float* coords, float* out, int32_t* idx_or_null,
@@ -443,7 +488,8 @@ OFB_API int ofb_corr_lookup(const ofb_pyramid* pyr, const float* coords, float* 
     if (!pyr || !coords || !out || B < 0 || h <= 0 || w <= 0) return OFB_EINVAL;
     if (pyr->levels < 1 || pyr->levels > OFB_MAX_LEVELS) return OFB_EINVAL;
     if (radius < 0 || 2 * radius + 1 > MAX_D) return OFB_EUNSUPPORTED;
-    if (pyr->dtype != OFB_DTYPE_F32 && pyr->dtype != OFB_DTYPE_BF16) return OFB_EINVAL;
+    if (pyr->dtype != OFB_DTYPE_F32 && pyr->dtype != OFB_DTYPE_BF16 && pyr->dtype != OFB_DTYPE_F16) return OFB_EINVAL;
+    const bool half16 = pyr->dtype != OFB_DTYPE_F32;      // 16-bit storage: bf16 or fp16
     if (B == 0) return OFB_OK;
     LookupParams P;
     P.levels = pyr->levels; P.radius = radius; P.B = B; P.h = h; P.w = w;
@@ -460,7 +506,7 @@ OFB_API int ofb_corr_lookup(const ofb_pyramid* pyr, const float* coords, float* 
         if (on) {
             if (!P.base[l] || P.lh[l] <= 0 || P.lw[l] <= 0 || P.pitch[l] < P.lw[l]) return OFB_EINVAL;
             if (P.lh[l] > 65536 || P.lw[l] > 65536) return OFB_EUNSUPPORTED;
-            if (pyr->dtype == OFB_DTYPE_BF16 &&
+            if (half16 &&
                 ((P.pitch[l] & 1) || (P.q_stride[l] & 1) || (reinterpret_cast<uintptr_t>(P.base[l]) & 3)))
                 return OFB_EALIGN;
         }
@@ -471,8 +517,8 @@ OFB_API int ofb_corr_lookup(const ofb_pyramid* pyr, const float* coords, float* 
     const long long blocks = (Q + QT - 1) / QT;
     if (blocks > 0x7fffffffLL) return OFB_EUNSUPPORTED;
     cudaStream_t st = (cudaStream_t)stream;
-    // product path: bf16 pyramid with padded rows (pitch multiple of 8, 16-byte aligned slices)
-    bool tile_ok = pyr->dtype == OFB_DTYPE_BF16 && (radius == 4 || radius == 3) && !getenv("OFB_LOOKUP_V1");
+    // product path: 16-bit pyramid with padded rows (pitch multiple of 8, 16-byte aligned slices)
+    bool tile_ok = half16 && (radius == 4 || radius == 3) && !getenv("OFB_LOOKUP_V1");
     for (int l = 0; l < pyr->levels && tile_ok; ++l)
         tile_ok = (P.pitch[l] % 8 == 0) && (P.q_stride[l] % 8 == 0) && ((reinterpret_cast<uintptr_t>(P.base[l]) & 15) == 0);
     if (tile_ok) {
@@ -484,19 +530,18 @@ OFB_API int ofb_corr_lookup(const ofb_pyramid* pyr, const float* coords, float* 
             const char* e = getenv("OFB_LOOKUP_GR");
             return (e && atoi(e) == 16) ? 16 : 3;
         }();
-        OFB_CUDA(ofb_smem_once<lookup_tile_kernel<4, 3>>(11 * 128 * 40));
-        OFB_CUDA(ofb_smem_once<lookup_tile_kernel<4, 16>>(11 * 128 * 40));
-        OFB_CUDA(ofb_smem_once<lookup_tile_kernel<3, 16>>(9 * 128 * 40));
-        if (radius == 4 && gr == 3) lookup_tile_kernel<4, 3><<<(int)blocks, threads, wsm, st>>>(P, coords, out, idx_or_null, valid_or_null);
-        else if (radius == 4) lookup_tile_kernel<4, 16><<<(int)blocks, threads, wsm, st>>>(P, coords, out, idx_or_null, valid_or_null);
-        else lookup_tile_kernel<3, 16><<<(int)blocks, threads, wsm, st>>>(P, coords, out, idx_or_null, valid_or_null);
-        OFB_LAUNCH_CHECK();
-        return OFB_OK;
+        if (pyr->dtype == OFB_DTYPE_F16) return launch_tile<__half>(P, coords, out, idx_or_null, valid_or_null, radius, gr,
+                                                                    (int)blocks, threads, wsm, st);
+        return launch_tile<__nv_bfloat16>(P, coords, out, idx_or_null, valid_or_null, radius, gr, (int)blocks, threads, wsm,
+                                          st);
     }
     if (P.blocked) return OFB_EUNSUPPORTED;   // the generic kernels read rows
     if (pyr->dtype == OFB_DTYPE_BF16) {
         OFB_CUDA(cudaFuncSetAttribute(lookup_kernel<__nv_bfloat16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         lookup_kernel<__nv_bfloat16><<<(int)blocks, NW * 32, smem, st>>>(P, coords, out, idx_or_null, valid_or_null);
+    } else if (pyr->dtype == OFB_DTYPE_F16) {
+        OFB_CUDA(cudaFuncSetAttribute(lookup_kernel<__half>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        lookup_kernel<__half><<<(int)blocks, NW * 32, smem, st>>>(P, coords, out, idx_or_null, valid_or_null);
     } else {
         OFB_CUDA(cudaFuncSetAttribute(lookup_kernel<float>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         lookup_kernel<float><<<(int)blocks, NW * 32, smem, st>>>(P, coords, out, idx_or_null, valid_or_null);

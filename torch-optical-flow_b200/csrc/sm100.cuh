@@ -202,10 +202,22 @@ __device__ __forceinline__ uint64_t make_smem_desc(uint32_t saddr) {
     d |= (uint64_t)2 << 61;                 // SWIZZLE_128B
     return d;
 }
-// kind::f16 instruction descriptor: D fp32, A = B = bf16, both K-major
-__host__ __device__ constexpr uint32_t make_idesc(int M, int N) {
-    return (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
+// kind::f16 operand formats (the a_format [7,10) and b_format [10,13) fields of the instruction descriptor)
+constexpr uint32_t UMMA_F16 = 0, UMMA_BF16 = 1;
+// kind::f16 instruction descriptor: D fp32, A = B = `ab_format` (bf16 by default), both K-major
+__host__ __device__ constexpr uint32_t make_idesc(int M, int N, uint32_t ab_format = UMMA_BF16) {
+    return (1u << 4) | (ab_format << 7) | (ab_format << 10) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
 }
+// The 16-bit operand / storage type T as the tcgen05 and TMA descriptors name it
+template <typename T> struct F16Format;
+template <> struct F16Format<__nv_bfloat16> {
+    static constexpr uint32_t umma = UMMA_BF16;
+    static constexpr CUtensorMapDataType tma = CU_TENSOR_MAP_DATA_TYPE_BFLOAT16;
+};
+template <> struct F16Format<__half> {
+    static constexpr uint32_t umma = UMMA_F16;
+    static constexpr CUtensorMapDataType tma = CU_TENSOR_MAP_DATA_TYPE_FLOAT16;
+};
 
 // ------------------------------------------------------------------------------------ host side
 // cuTensorMapEncodeTiled with no interleave and no out-of-bounds NaN fill (TMA zero-fills outside the tensor).

@@ -68,7 +68,9 @@ SIGNATURES = {
     "ofb_pyramid_layout": (_i, [_i, _i, _i, _i, ctypes.POINTER(Pyramid), ctypes.POINTER(_i64 * MAX_LEVELS)]),
     "ofb_corr_prep_bf16": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _f, _vp]),
     "ofb_corr_prep_from": (_i, [_vp, _i, _vp, _i, _i, _i, _i, _i, _f, _vp]),
+    "ofb_corr_prep_to": (_i, [_vp, _i, _vp, _i, _i, _i, _i, _i, _i, _f, _vp]),
     "ofb_corr_pyramid_bf16": (_i, [_vp, _vp, _vp, ctypes.POINTER(Pyramid), _i, _i, _i, _i, _f, _i, _vp]),
+    "ofb_corr_pyramid_f16": (_i, [_vp, _vp, _vp, ctypes.POINTER(Pyramid), _i, _i, _i, _i, _f, _i, _vp]),
     "ofb_corr_pyramid_bf16_profile": (_i, [_vp, _vp, _vp, ctypes.POINTER(Pyramid), _i, _i, _i, _i, _f, _i, _vp, _vp]),
     "ofb_corr_pyramid_simt_f32": (_i, [_vp, _vp, ctypes.POINTER(Pyramid), _i, _i, _i, _i, _f, _vp]),
     "ofb_gemm_nt_bf16": (_i, [_vp, _vp, _vp, _i, _i, _i, _i] + [ctypes.c_longlong] * 6 + [_f, _i, _vp]),

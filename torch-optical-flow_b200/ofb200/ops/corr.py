@@ -3,9 +3,10 @@ built by the K2 tcgen05 kernel and sampled by the K3 lookup kernel of libofb200.
 
 Differences a caller can observe, all deliberate (DESIGN.md):
   * `corr_pyramid[l]` keeps the reference's shape (B*h*w, 1, h_l, w_l) but is a strided view of a
-    padded buffer (row pitch rounded up to 8 elements for TMA) and is stored in bf16 by default
-    (the reference's shipped configs run `precision: 16`, so its stored volume is half precision
-    too); pass `pyramid_dtype=torch.float32` for an fp32 pyramid (CUDA-core builder).
+    padded buffer (row pitch rounded up to 8 elements for TMA) and is stored in bf16 by default;
+    pass `pyramid_dtype=torch.float16` for the precision the reference's shipped configs store it in
+    (`precision: 16`: an fp16 pyramid, the same bytes and tensor-core path as bf16, 3 more significand
+    bits, but correlations beyond +-65504 become inf), or `torch.float32` for an fp32 pyramid (CUDA-core builder).
   * differentiable with respect to the feature maps (K3 backward kernel + two library GEMMs per level); the
     lookup coordinates get no gradient (the reference's RAFT detaches them, raft.py:127).
 """
@@ -21,7 +22,12 @@ import ofb200
 
 
 def _default_pyramid_dtype() -> torch.dtype:
-    return torch.float32 if os.environ.get("OFB200_PYRAMID_DTYPE", "bf16").lower() in ("fp32", "f32", "float32") else torch.bfloat16
+    name = os.environ.get("OFB200_PYRAMID_DTYPE", "bf16").lower()
+    if name in ("fp32", "f32", "float32"):
+        return torch.float32
+    if name in ("fp16", "f16", "float16", "half"):
+        return torch.float16
+    return torch.bfloat16
 
 
 # optional ofb200.runner.KernelTimers: when set (bench.py), the prep launches and the pyramid kernel get their own
@@ -44,24 +50,48 @@ def _span(name: str, launches: int):
 _IN_DTYPES = {torch.float32: ofb200.DTYPE_F32, torch.bfloat16: ofb200.DTYPE_BF16, torch.float16: ofb200.DTYPE_F16}
 
 
-def prepare_operands(fmap1: Tensor, fmap2: Tensor, num_levels: int):
-    """K-major bf16 operands of the tcgen05 builder: fmap1 * 1/sqrt(C), fmap2, and (for pyramids with
-    more than two levels) fmap2 averaged over complete 4x4 blocks.  (B, C, h, w) CUDA inputs in fp32, bf16 or fp16:
-    half-precision maps (autocast callers) are read as they are, without an fp32 round trip."""
+def prepare_operands(fmap1: Tensor, fmap2: Tensor, num_levels: int, dtype: torch.dtype = torch.bfloat16):
+    """K-major operands of the tcgen05 builder in `dtype` (bf16 or fp16): fmap1, fmap2, and (for pyramids with more
+    than two levels) fmap2 averaged over complete 4x4 blocks.  (B, C, h, w) CUDA inputs in fp32, bf16 or fp16:
+    half-precision maps (autocast callers) are read as they are, without an fp32 round trip.
+
+    bf16 operands carry the 1/sqrt(C) of corr.py:87 folded into fmap1 (build with scale 1.0).  fp16 operands do not:
+    the fp16 builder applies it to its fp32 accumulators, the reference's order under autocast (an fp16 matmul of the
+    rounded maps, then the scale), and fmap1/sqrt(C) stays out of fp16 subnormals.  `operand_scale` says which."""
+    if dtype not in (torch.bfloat16, torch.float16):
+        raise NotImplementedError("prepare_operands: the tcgen05 builder's operands are bf16 or fp16")
     b, c, h, w = fmap1.shape
     dt1, dt2 = _IN_DTYPES[fmap1.dtype], _IN_DTYPES[fmap2.dtype]
+    out_dt = _IN_DTYPES[dtype]
     lib = ofb200.load()
     st = ofb200.stream_ptr()
     dev = fmap1.device
-    a_km = torch.empty((b, h * w, c), dtype=torch.bfloat16, device=dev)
-    b_km = torch.empty((b, h * w, c), dtype=torch.bfloat16, device=dev)
-    q_km = torch.empty((b, (h // 4) * (w // 4), c), dtype=torch.bfloat16, device=dev) if num_levels > 2 else None
-    scale = 1.0 / math.sqrt(float(c))
-    ofb200.check(lib.ofb_corr_prep_from(ofb200.ptr(fmap1), dt1, ofb200.ptr(a_km), b, c, h, w, 1, scale, st), "ofb_corr_prep_from")
-    ofb200.check(lib.ofb_corr_prep_from(ofb200.ptr(fmap2), dt2, ofb200.ptr(b_km), b, c, h, w, 1, 1.0, st), "ofb_corr_prep_from")
+    a_km = torch.empty((b, h * w, c), dtype=dtype, device=dev)
+    b_km = torch.empty((b, h * w, c), dtype=dtype, device=dev)
+    q_km = torch.empty((b, (h // 4) * (w // 4), c), dtype=dtype, device=dev) if num_levels > 2 else None
+    scale = operand_scale(c, dtype)
+    ofb200.check(lib.ofb_corr_prep_to(ofb200.ptr(fmap1), dt1, ofb200.ptr(a_km), out_dt, b, c, h, w, 1, scale, st),
+                 "ofb_corr_prep_to")
+    ofb200.check(lib.ofb_corr_prep_to(ofb200.ptr(fmap2), dt2, ofb200.ptr(b_km), out_dt, b, c, h, w, 1, 1.0, st),
+                 "ofb_corr_prep_to")
     if q_km is not None:
-        ofb200.check(lib.ofb_corr_prep_from(ofb200.ptr(fmap2), dt2, ofb200.ptr(q_km), b, c, h, w, 4, 1.0, st), "ofb_corr_prep_from")
+        ofb200.check(lib.ofb_corr_prep_to(ofb200.ptr(fmap2), dt2, ofb200.ptr(q_km), out_dt, b, c, h, w, 4, 1.0, st),
+                     "ofb_corr_prep_to")
     return a_km, b_km, q_km
+
+
+def operand_scale(c: int, dtype: torch.dtype = torch.bfloat16) -> float:
+    """The factor prepare_operands folds into fmap1: 1/sqrt(C) for bf16 operands, 1 for fp16 ones."""
+    return 1.0 / math.sqrt(float(c)) if dtype == torch.bfloat16 else 1.0
+
+
+def build_pyramid(ops, pyr, b: int, c: int, h: int, w: int, dtype: torch.dtype = torch.bfloat16, cta_group: int = 0) -> int:
+    """Run the tcgen05 builder of `dtype` on prepare_operands' output; returns the library's status code."""
+    lib = ofb200.load()
+    fn = lib.ofb_corr_pyramid_f16 if dtype == torch.float16 else lib.ofb_corr_pyramid_bf16
+    scale = (1.0 / math.sqrt(float(c))) / operand_scale(c, dtype)     # what the operands do not carry yet
+    return fn(ofb200.ptr(ops[0]), ofb200.ptr(ops[1]), ofb200.ptr(ops[2]), ctypes.byref(pyr), b, c, h, w, scale,
+              int(cta_group), ofb200.stream_ptr())
 
 
 class _GradState:
@@ -129,12 +159,15 @@ class _PyramidHandle(torch.autograd.Function):
         task = torch._C._current_graph_task_id() if hasattr(torch._C, "_current_graph_task_id") else None
         if blk.dpyr is not None and blk.task == task:
             scale = 1.0 / math.sqrt(float(c))
-            # The two GEMMs per level.  "tcgen05" (default with a bf16 pyramid): bf16 operands, fp32 accumulation, this
-            # library's long-K tensor-core kernel fed by one cast / transpose pass over the fp32 gradient level --
-            # the precision of a `precision: 16` run of the reference.  "fp32" (default with an fp32 pyramid; matches
-            # the reference's fp32 autograd to 1e-5) and "bf16" go through the library bmm.  OFB200_BWD_GEMM overrides.
+            # The two GEMMs per level.  "tcgen05" (default with a bf16 or fp16 pyramid): bf16 operands, fp32
+            # accumulation, this library's long-K tensor-core kernel fed by one cast / transpose pass over the fp32
+            # gradient level -- the precision of a `precision: 16` run of the reference.  It reads only the fp32 gradient
+            # pyramid and the feature maps, never the stored pyramid, and bf16 keeps the gradients' fp32 range (fp16
+            # operands would underflow without loss scaling).  "fp32" (default with an fp32 pyramid; matches the
+            # reference's fp32 autograd to 1e-5) and "bf16" go through the library bmm.  OFB200_BWD_GEMM overrides.
             tc_ok = c % 32 == 0 and c <= 256
-            mode = os.environ.get("OFB200_BWD_GEMM", "").lower() or ("tcgen05" if blk.pyr_dtype == ofb200.DTYPE_BF16 and tc_ok else "fp32")
+            half_pyr = blk.pyr_dtype in (ofb200.DTYPE_BF16, ofb200.DTYPE_F16)
+            mode = os.environ.get("OFB200_BWD_GEMM", "").lower() or ("tcgen05" if half_pyr and tc_ok else "fp32")
             if mode == "tcgen05" and not tc_ok:
                 raise NotImplementedError("CorrBlock backward: the tcgen05 GEMM needs C to be a multiple of 32, at most 256")
             d_levels = []
@@ -242,11 +275,12 @@ class CorrBlock:
     ) -> None:
         """fmap1, fmap2 (B, C, h, w) in fp32 / bf16 / fp16 (reference corr.py:38-54).
 
-        Extensions (keyword-only, defaults keep the reference's behaviour): `pyramid_dtype` (bf16 default, fp32 selects
-        the CUDA-core builder), `builder`, `cta_group` (K2 launch mode), and `on_demand=True` (or
-        OFB200_CORR_ON_DEMAND=1): nothing is materialised -- every lookup evaluates the correlation values of its own
-        windows from the operand maps (ofb_corr_lookup_ondemand; 22 MB instead of 2.83 GB per 1080p pair, slower per
-        lookup; forward-only)."""
+        Extensions (keyword-only, defaults keep the reference's behaviour): `pyramid_dtype` (bf16 default; fp16 is the
+        precision the reference stores its pyramid in under `precision: 16`; fp32 selects the CUDA-core builder;
+        OFB200_PYRAMID_DTYPE=bf16|fp16|fp32 sets the default; ignored with `on_demand`), `builder`, `cta_group` (K2
+        launch mode), and `on_demand=True` (or OFB200_CORR_ON_DEMAND=1): nothing is materialised -- every lookup
+        evaluates the correlation values of its own windows from the operand maps (ofb_corr_lookup_ondemand; 22 MB
+        instead of 2.83 GB per 1080p pair, slower per lookup; forward-only)."""
         self.num_levels = num_levels
         self.radius = radius
         if fmap1.shape != fmap2.shape or fmap1.dim() != 4:
@@ -255,8 +289,8 @@ class CorrBlock:
             raise NotImplementedError(f"CorrBlock: num_levels must be in [1, {ofb200.MAX_LEVELS}]")
         if pyramid_dtype is None:
             pyramid_dtype = _default_pyramid_dtype()
-        if pyramid_dtype not in (torch.float32, torch.bfloat16):
-            raise NotImplementedError("CorrBlock: pyramid_dtype must be torch.float32 or torch.bfloat16")
+        if pyramid_dtype not in (torch.float32, torch.bfloat16, torch.float16):
+            raise NotImplementedError("CorrBlock: pyramid_dtype must be torch.float32, torch.bfloat16 or torch.float16")
         self._on_host = not fmap1.is_cuda
         # training: keep the differentiable feature maps behind a handle node the lookups depend on
         self._handle = None
@@ -300,24 +334,29 @@ class CorrBlock:
                     levels.append(f2l)
             self._on_demand = (a_km, levels)
             return
-        tc_ok = pyramid_dtype == torch.bfloat16 and c % 64 == 0 and c <= 256
+        tc_ok = pyramid_dtype in (torch.bfloat16, torch.float16) and c % 64 == 0 and c <= 256
         if builder == "auto":
             builder = "tcgen05" if tc_ok else "simt"
         if builder == "tcgen05" and not tc_ok:
-            raise NotImplementedError("CorrBlock: the tcgen05 builder needs a bf16 pyramid and C in {64,128,192,256}")
+            raise NotImplementedError("CorrBlock: the tcgen05 builder needs a bf16 or fp16 pyramid and C in {64,128,192,256}")
         self.builder = builder
-        if builder != "tcgen05" and fmap1.dtype != torch.float32:
-            fmap1, fmap2 = fmap1.float(), fmap2.float()     # the CUDA-core builder reads fp32; the tcgen05 prep reads
-                                                            # bf16 / fp16 maps (autocast callers) as they are
+        if builder != "tcgen05":
+            # the CUDA-core builder reads fp32; the tcgen05 prep reads bf16 / fp16 maps (autocast callers) as they are.
+            # An fp16 pyramid is the correlation of the fp16-rounded maps, whichever builder makes it (autocast's matmul
+            # operands, corr.py:85)
+            if pyramid_dtype == torch.float16 and fmap1.dtype != torch.float16:
+                fmap1, fmap2 = fmap1.half(), fmap2.half()
+            if fmap1.dtype != torch.float32:
+                fmap1, fmap2 = fmap1.float(), fmap2.float()
 
         pyr = ofb200.Pyramid()
         elems = (ctypes.c_int64 * ofb200.MAX_LEVELS)()
-        # tcgen05 builder: 8x4-blocked bf16 levels (what the lookup kernel reads with the fewest DRAM atoms),
+        # tcgen05 builder: 8x4-blocked 16-bit levels (what the lookup kernel reads with the fewest DRAM atoms),
         # query-minor by default (OFB200_PYRAMID_LAYOUT=blocked|qminor); CUDA-core builder: padded rows
         blocked_mode = 2 if os.environ.get("OFB200_PYRAMID_LAYOUT", "qminor").lower() == "blocked" else 3
         mode = blocked_mode if (builder == "tcgen05" and radius in (3, 4)) else 1
         ofb200.check(lib.ofb_pyramid_layout(h, w, num_levels, mode, ctypes.byref(pyr), ctypes.byref(elems)), "ofb_pyramid_layout")
-        pyr.dtype = ofb200.DTYPE_BF16 if pyramid_dtype == torch.bfloat16 else ofb200.DTYPE_F32
+        pyr.dtype = _IN_DTYPES[pyramid_dtype]
         n = h * w
         self._buffers = []
         self._views: Optional[List[Tensor]] = None
@@ -336,11 +375,10 @@ class CorrBlock:
             scale = 1.0 / math.sqrt(float(c))
             if builder == "tcgen05":
                 with _span("corr_prep", 3 if num_levels > 2 else 2):
-                    ops = prepare_operands(fmap1, fmap2, num_levels)
+                    ops = prepare_operands(fmap1, fmap2, num_levels, pyramid_dtype)
                 with _span("corr_pyramid_kernel", 2 if num_levels > 2 else 1):
-                    rc = lib.ofb_corr_pyramid_bf16(ofb200.ptr(ops[0]), ofb200.ptr(ops[1]), ofb200.ptr(ops[2]),
-                                                   ctypes.byref(pyr), b, c, h, w, 1.0, int(cta_group), ofb200.stream_ptr())
-                ofb200.check(rc, "ofb_corr_pyramid_bf16")
+                    rc = build_pyramid(ops, pyr, b, c, h, w, pyramid_dtype, cta_group)
+                ofb200.check(rc, "ofb_corr_pyramid_f16" if pyramid_dtype == torch.float16 else "ofb_corr_pyramid_bf16")
                 # keep the operands alive until the stream has consumed them
                 for t in ops:
                     if t is not None:
@@ -446,7 +484,8 @@ class CorrBlock:
         """All-pairs correlation volume (B, h, w, 1, h, w) / sqrt(C) (reference corr.py:79-87).
 
         The reference's static method is an exact matmul in the inputs' precision, so the default here is the fp32
-        CUDA-core builder (`pyramid_dtype=torch.bfloat16` selects the tcgen05 builder and a bf16-rounded volume).
+        CUDA-core builder (`pyramid_dtype=torch.bfloat16` or `torch.float16` selects the tcgen05 builder and a volume
+        rounded to that type; fp16 is what the reference's matmul returns under autocast).
         Forward-only: the training path goes through the constructor (reference raft.py:112), which is
         differentiable; inputs that require grad raise instead of silently returning a detached volume."""
         if torch.is_grad_enabled() and (fmap1.requires_grad or fmap2.requires_grad):
