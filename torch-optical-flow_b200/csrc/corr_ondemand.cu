@@ -6,8 +6,8 @@
 //     corr_l[q, (y, x)] = < f1[:, q] / sqrt(C) , avgpool_l(f2)[:, y, x] >
 // at the ~(2r+2)^2 positions its window touches.  This kernel evaluates exactly those dot products from the K-major
 // bf16 operands the tcgen05 builder uses (ofb_corr_prep_from: fmap1 * 1/sqrt(C), and fmap2 pooled by 1, 2, 4, 8) and
-// feeds them to the same bit-exact sampling sequence as lookup.cu.  Memory per pair: 4 small operand maps (22 MB at
-// 1080p) instead of the 2.83 GB pyramid; cost: ~100x the arithmetic of a lookup per iteration, on the CUDA cores.
+// samples them as the generic lookup does (ofb::warp_window, common.cuh).  Memory per pair: 4 small operand maps (22 MB
+// at 1080p) instead of the 2.83 GB pyramid; cost: ~100x the arithmetic of a lookup per iteration, on the CUDA cores.
 // It is a capacity feature (batch sizes / resolutions whose pyramid does not fit), not a faster path: see DESIGN.md.
 //
 // Work decomposition: a work item is an 8 x 4 tile of queries at ONE pyramid level; its 4 warps own the 4 tile rows and walk
@@ -18,7 +18,7 @@
 // (default 4 = the register limit) per SM.  Measured (profiles/r02_ondemand.jsonl): with white-noise coordinates
 // (sigma = 4 px, the bench's) consecutive windows overlap by only ~1/3 and the kernel stays at the L2 -> SM limit
 // (9.4 ms per iteration for 8 pairs at 136x240); smooth coordinates reuse their rows from L1.  Per query a warp
-//   1. computes the 2*(2r+1) tap coordinates with the reference's fp32 round trip (lookup.cu, SURVEY.md 8c),
+//   1. computes the 2*(2r+1) tap coordinates with the reference's fp32 round trip (ofb::lookup_tap, SURVEY.md 8c),
 //   2. evaluates the <= 12 x 12 patch of dot products: lane <-> 8 consecutive channels, 32 positions per pass,
 //      one 16-byte load + 8 FMAs per position and lane, then ONE transposing butterfly (31 shuffles) turns the 32 lanes'
 //      partial sums of 32 positions into one finished value per lane,
@@ -32,8 +32,8 @@ namespace {
 
 constexpr int TQ = 8;         // queries per tile row (one warp walks them)
 constexpr int TQY = 4;        // tile rows = warps per CTA
-constexpr int PD = 12;        // patch rows / cols
-constexpr int MAX_D = 9;      // 2*radius+1, radius <= 4
+using ofb::PD;
+using ofb::MAX_D;
 constexpr int MAX_DD = MAX_D * MAX_D;
 
 struct OdParams {
@@ -112,31 +112,15 @@ __global__ void __launch_bounds__(128) ondemand_lookup_kernel(const OdParams P, 
             Slice<CPL>::load(P.f1 + ((long long)b * HW + p) * P.C + lane * CPL, a);
             const float cx0 = __ldg(coords + ((long long)b * 2 + 0) * HW + p);
             const float cy0 = __ldg(coords + ((long long)b * 2 + 1) * HW + p);
-            // ---- 1. tap coordinates: lane t (x taps) and lane 16+t (y taps); same sequence as lookup.cu
-            const int t = lane & 15, isy = lane >> 4;
-            const float cen = __fmul_rn(isy ? cy0 : cx0, inv);
-            const int size = isy ? Hl : Wl;
-            const float pos = __fadd_rn(cen, (float)(t - P.radius));
-            const float sm1 = (float)(size - 1);
-            const float g = __fsub_rn(__fdiv_rn(__fmul_rn(2.0f, pos), sm1), 1.0f);
-            const float ic = __fmul_rn(__fdiv_rn(__fadd_rn(g, 1.0f), 2.0f), sm1);
-            const float fl = floorf(ic);
-            float w1 = __fsub_rn(ic, fl), w0 = __fsub_rn(__fadd_rn(fl, 1.0f), ic);
-            // guard for the int conversion (non-finite / far-away coordinates).  Level sizes are <= 65536 and a window
-            // spans 2r+1 <= 9 taps, so ONE tap outside [-32768, 70000] means every tap of the window is outside the
-            // image: the patch is skipped and the result is 0.  Inside the guard the taps are consecutive integers
-            // (+- the fp32 round-trip slide) and the patch has at most 2r+3 <= 11 columns / rows.
-            int i0 = (fl >= -32768.0f && fl <= 70000.0f) ? (int)fl : -1000000;
-            if (i0 == -1000000) { w0 = 0.0f; w1 = 0.0f; }
-            const int x_first = __shfl_sync(0xffffffffu, i0, 0), x_last = __shfl_sync(0xffffffffu, i0, D - 1);
-            const int y_first = __shfl_sync(0xffffffffu, i0, 16), y_last = __shfl_sync(0xffffffffu, i0, 16 + D - 1);
-            const bool guarded = __any_sync(0xffffffffu, i0 == -1000000 && t < D);
-            const int px0 = x_first, py0 = y_first;
-            const int cols = x_last + 2 - px0, rows = y_last + 2 - py0;
-            const bool patch_ok = !guarded && cols <= PD && rows <= PD && cols > 0 && rows > 0;   // warp-uniform
+            // ---- 1. tap coordinates.  A window with a tap outside the guard lies outside the image (ofb::LookupTap): its
+            // dot products are skipped and its samples are 0
+            ofb::WarpWindow win = ofb::warp_window<false>(cx0, cy0, inv, P.radius, Wl, Hl, lane);
+            const bool guarded = __any_sync(0xffffffffu, win.i0 == ofb::TAP_FAR && (lane & 15) < D);
+            win.patch_ok = win.patch_ok && !guarded;
+            const int px0 = win.px0, py0 = win.py0, cols = win.cols;
             // ---- 2. the patch of dot products, 32 positions per pass
-            if (patch_ok) {
-                const int npos = rows * cols;
+            if (win.patch_ok) {
+                const int npos = win.rows * cols;
                 int r = 0, c = 0;                                     // uniform raster walk over the patch
                 for (int g0 = 0; g0 < npos; g0 += 32) {
                     float part[32];
@@ -173,26 +157,11 @@ __global__ void __launch_bounds__(128) ondemand_lookup_kernel(const OdParams P, 
                 }
             }
             __syncwarp();
-            // ---- 3. (2r+1)^2 samples, 3 per lane; channel k = i*D + j with i moving x (corr.py:64-70)
-#pragma unroll
-            for (int kk = 0; kk < (MAX_DD + 31) / 32; ++kk) {
-                const int k = kk * 32 + lane;
-                const bool active = k < DD;
-                const int i = active ? k / D : 0, j = active ? k - (k / D) * D : 0;
-                const int x0 = __shfl_sync(0xffffffffu, i0, i), y0 = __shfl_sync(0xffffffffu, i0, 16 + j);
-                const float wx0 = __shfl_sync(0xffffffffu, w0, i), wx1 = __shfl_sync(0xffffffffu, w1, i);
-                const float wy0 = __shfl_sync(0xffffffffu, w0, 16 + j), wy1 = __shfl_sync(0xffffffffu, w1, 16 + j);
-                if (!active) continue;
-                float acc = 0.0f;
-                if (patch_ok) {
-                    const float* s = patch + (y0 - py0) * PD + (x0 - px0);
-                    acc = __fmul_rn(s[0], __fmul_rn(wx0, wy0));
-                    acc = __fmaf_rn(s[1], __fmul_rn(wx1, wy0), acc);
-                    acc = __fmaf_rn(s[PD], __fmul_rn(wx0, wy1), acc);
-                    acc = __fmaf_rn(s[PD + 1], __fmul_rn(wx1, wy1), acc);
-                }
-                otile[k][qx] = acc;
-            }
+            // ---- 3. (2r+1)^2 samples, 3 per lane
+            ofb::warp_window_samples(
+                win, patch, P.radius, lane,
+                [](int, int, float, float, float, float) { return 0.0f; },
+                [&](int k, int, int, float v) { otile[k][qx] = v; });
             __syncwarp();
         }
         // ---- one tile row of queries is done: 32-byte runs per channel

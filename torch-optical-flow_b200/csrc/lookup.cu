@@ -6,66 +6,54 @@
 // grid_sample, 5 concatenations); here one kernel reads the coordinates and the pyramid and
 // writes the (B, L*(2r+1)^2, h, w) fp32 output.
 //
-// Bit-exactness contract (SURVEY.md 8c): the fp32 coordinate sequence is replayed operation
-// by operation with round-to-nearest intrinsics so nvcc cannot contract it:
-//     c  = coord / 2^l                       (corr.py:68, exact)
-//     x  = c + (i - r)                       (corr.py:70; window TRANSPOSED: i moves x, j moves y)
-//     g  = 2*x/(W_l-1) - 1                   (utils.py:70-71)
-//     ix = ((g + 1)/2) * (W_l-1)             (ATen GridSampler.h:30, align_corners=True)
-//     x0 = floor(ix); valid = -1 < g < 1     (utils.py:77)
+// The tap coordinates follow the bit-exact sequence of ofb::lookup_tap (common.cuh, SURVEY.md 8c).
 //
 // Work decomposition: a CTA owns 32 consecutive queries; each of its 8 warps walks 4 of them.
 // Per (query, level) the warp
-//   1. computes the 2*(2r+1) tap coordinates, one per lane (lanes 0..8: x taps, 16..24: y taps),
+//   1. computes the 2*(2r+1) tap coordinates, one per lane (ofb::warp_window),
 //   2. loads the <=12x12 patch of the query's level slice that covers all taps into a private
 //      shared-memory patch (4-byte words; out-of-image elements become zeros = zeros padding),
-//   3. produces the (2r+1)^2 samples, 3 per lane, fetching the per-axis floor index / weight of
-//      its cell from the owning lanes with warp shuffles.
+//   3. produces the (2r+1)^2 samples, 3 per lane (ofb::warp_window_samples).
 // Results are staged in a [channel][query] shared tile so the global writes are 128-byte rows.
 // HBM roofline per query and iteration (SURVEY.md 8d): L*(2r+2)^2*esize + 8 read, 4*L*(2r+1)^2 written.
 #include <climits>
-#include <cstdlib>
-#include <type_traits>
 
 #include "common.cuh"
 
 namespace {
 
+using ofb::PD;
+using ofb::MAX_D;
 constexpr int QT = 32;        // queries per CTA
 constexpr int NW = 8;         // warps per CTA
-constexpr int PD = 12;        // patch rows / cols
 constexpr int OT_PITCH = QT + 1;
-constexpr int MAX_D = 9;      // 2*radius+1, radius <= 4
 
-struct LookupParams {
-    const void* base[OFB_MAX_LEVELS];
-    long long q_stride[OFB_MAX_LEVELS];
-    int pitch[OFB_MAX_LEVELS];
-    int lh[OFB_MAX_LEVELS];
-    int lw[OFB_MAX_LEVELS];
+struct LookupParams : ofb::PyramidLevels {
     int levels, radius, B, h, w;
     int blocked;   // 8x4-blocked layouts (register-tile kernel only, 16-bit pyramids)
     long long blk_stride;   // elements between consecutive blocks: 32, or 32 * Q (query-minor)
 };
 
-template <typename T> struct Elem;
-template <> struct Elem<float> {
-    static __device__ __forceinline__ float get(const float* row, int x) { return __ldg(row + x); }
-};
-template <> struct Elem<__nv_bfloat16> {
-    static __device__ __forceinline__ float get(const __nv_bfloat16* row, int x) {
-        return __bfloat162float(__ldg(row + x));
-    }
-};
-template <> struct Elem<__half> {
-    static __device__ __forceinline__ float get(const __half* row, int x) { return __half2float(__ldg(row + x)); }
-};
-
-// patch load: fp32 -> one element per word; bf16 / fp16 -> two elements per 4-byte word
+// patch load: bf16 / fp16 -> two elements per 4-byte word (px0 and pitch are even, the slice base is 4-byte aligned)
 template <typename T>
 __device__ __forceinline__ void load_patch(float* patch, const T* slice, int pitch, int Hl, int Wl, int px0, int py0,
-                                           int rows, int lane);
+                                           int rows, int lane) {
+#pragma unroll
+    for (int e = lane; e < PD * (PD / 2); e += 32) {
+        const int r = e / (PD / 2), cw = e - r * (PD / 2);
+        const int y = py0 + r, x = px0 + 2 * cw;
+        float v0 = 0.0f, v1 = 0.0f;
+        if (r < rows && y >= 0 && y < Hl && x >= 0 && x < Wl) {
+            const unsigned wd = __ldg(reinterpret_cast<const unsigned*>(slice + (size_t)y * pitch + x));
+            v0 = ofb::widen16<T>(wd, 0);
+            if (x + 1 < Wl) v1 = ofb::widen16<T>(wd, 1);
+        }
+        patch[r * PD + 2 * cw] = v0;
+        patch[r * PD + 2 * cw + 1] = v1;
+    }
+}
 
+// fp32 -> one element per word
 template <>
 __device__ __forceinline__ void load_patch<float>(float* patch, const float* slice, int pitch, int Hl, int Wl, int px0,
                                                   int py0, int rows, int lane) {
@@ -76,44 +64,6 @@ __device__ __forceinline__ void load_patch<float>(float* patch, const float* sli
         float v = 0.0f;
         if (r < rows && y >= 0 && y < Hl && x >= 0 && x < Wl) v = __ldg(slice + (size_t)y * pitch + x);
         patch[e] = v;
-    }
-}
-
-template <>
-__device__ __forceinline__ void load_patch<__nv_bfloat16>(float* patch, const __nv_bfloat16* slice, int pitch, int Hl,
-                                                          int Wl, int px0, int py0, int rows, int lane) {
-    // px0 is even, pitch is even, the slice base is 4-byte aligned
-#pragma unroll
-    for (int e = lane; e < PD * (PD / 2); e += 32) {
-        const int r = e / (PD / 2), cw = e - r * (PD / 2);
-        const int y = py0 + r, x = px0 + 2 * cw;
-        float v0 = 0.0f, v1 = 0.0f;
-        if (r < rows && y >= 0 && y < Hl && x >= 0 && x < Wl) {
-            const unsigned wd = __ldg(reinterpret_cast<const unsigned*>(slice + (size_t)y * pitch + x));
-            v0 = __uint_as_float(wd << 16);
-            if (x + 1 < Wl) v1 = __uint_as_float(wd & 0xffff0000u);
-        }
-        patch[r * PD + 2 * cw] = v0;
-        patch[r * PD + 2 * cw + 1] = v1;
-    }
-}
-
-template <>
-__device__ __forceinline__ void load_patch<__half>(float* patch, const __half* slice, int pitch, int Hl, int Wl, int px0,
-                                                   int py0, int rows, int lane) {
-    // px0 is even, pitch is even, the slice base is 4-byte aligned
-#pragma unroll
-    for (int e = lane; e < PD * (PD / 2); e += 32) {
-        const int r = e / (PD / 2), cw = e - r * (PD / 2);
-        const int y = py0 + r, x = px0 + 2 * cw;
-        float v0 = 0.0f, v1 = 0.0f;
-        if (r < rows && y >= 0 && y < Hl && x >= 0 && x < Wl) {
-            const float2 v = __half22float2(__ldg(reinterpret_cast<const __half2*>(slice + (size_t)y * pitch + x)));
-            v0 = v.x;
-            if (x + 1 < Wl) v1 = v.y;
-        }
-        patch[r * PD + 2 * cw] = v0;
-        patch[r * PD + 2 * cw + 1] = v1;
     }
 }
 
@@ -129,7 +79,6 @@ __global__ void __launch_bounds__(NW * 32) lookup_kernel(const LookupParams P, c
     float* patch = patches + warp * PD * PD;
     const long long HW = (long long)P.h * P.w, Q = (long long)P.B * HW;
     const long long q0 = (long long)blockIdx.x * QT;
-    constexpr bool kBf16 = sizeof(T) == 2;
 
     for (int qi = warp; qi < QT; qi += NW) {
         const long long q = q0 + qi;
@@ -141,61 +90,32 @@ __global__ void __launch_bounds__(NW * 32) lookup_kernel(const LookupParams P, c
             const int Wl = P.lw[l], Hl = P.lh[l], pitch = P.pitch[l];
             const T* slice = reinterpret_cast<const T*>(P.base[l]) + q * P.q_stride[l];
             const float inv = 1.0f / (float)(1 << l);          // exact power of two
-            // ---- 1. tap coordinates: lane t (x taps) and lane 16+t (y taps)
+            // ---- 1. tap coordinates; 16-bit patches start on an even column (word loads)
+            const ofb::WarpWindow win = ofb::warp_window<sizeof(T) == 2>(cx0, cy0, inv, P.radius, Wl, Hl, lane);
             const int t = lane & 15, isy = lane >> 4;
-            const float cen = __fmul_rn(isy ? cy0 : cx0, inv);
-            const int size = isy ? Hl : Wl;
-            const float pos = __fadd_rn(cen, (float)(t - P.radius));
-            const float sm1 = (float)(size - 1);
-            const float g = __fsub_rn(__fdiv_rn(__fmul_rn(2.0f, pos), sm1), 1.0f);
-            const float ic = __fmul_rn(__fdiv_rn(__fadd_rn(g, 1.0f), 2.0f), sm1);
-            const float fl = floorf(ic);
-            float w1 = __fsub_rn(ic, fl), w0 = __fsub_rn(__fadd_rn(fl, 1.0f), ic);
-            // int conversion guarded: non-finite / far-away coordinates map to "everything out of range"
-            int i0 = (fl >= -8.0f && fl <= 70000.0f) ? (int)fl : -1000000;
-            if (i0 == -1000000) { w0 = 0.0f; w1 = 0.0f; }
-            const int gv = (g > -1.0f) && (g < 1.0f);
             if (idx_out && t < D)
-                idx_out[((q * P.levels + l) * 2 + isy) * D + t] = (int32_t)fl;
-            const int x_first = __shfl_sync(0xffffffffu, i0, 0), x_last = __shfl_sync(0xffffffffu, i0, D - 1);
-            const int y_first = __shfl_sync(0xffffffffu, i0, 16), y_last = __shfl_sync(0xffffffffu, i0, 16 + D - 1);
-            const int px0 = kBf16 ? (x_first & ~1) : x_first;
-            const int py0 = y_first;
-            const int cols = x_last + 2 - px0, rows = y_last + 2 - py0;
-            const bool patch_ok = cols <= PD && rows <= PD && cols > 0 && rows > 0;   // warp-uniform
+                idx_out[((q * P.levels + l) * 2 + isy) * D + t] = (int32_t)win.fl;
+            const unsigned vmask = __ballot_sync(0xffffffffu, win.valid);   // bit lane: that tap's utils.py:77 predicate
             // ---- 2. stage the patch
-            if (patch_ok) load_patch<T>(patch, slice, pitch, Hl, Wl, px0, py0, rows, lane);
+            if (win.patch_ok) load_patch<T>(patch, slice, pitch, Hl, Wl, win.px0, win.py0, win.rows, lane);
             __syncwarp();
-            // ---- 3. (2r+1)^2 samples, 3 per lane
-#pragma unroll
-            for (int kk = 0; kk < (MAX_D * MAX_D + 31) / 32; ++kk) {
-                const int k = kk * 32 + lane;
-                const bool active = k < DD;
-                const int i = active ? k / D : 0, j = active ? k - (k / D) * D : 0;
-                const int x0 = __shfl_sync(0xffffffffu, i0, i), y0 = __shfl_sync(0xffffffffu, i0, 16 + j);
-                const float wx0 = __shfl_sync(0xffffffffu, w0, i), wx1 = __shfl_sync(0xffffffffu, w1, i);
-                const float wy0 = __shfl_sync(0xffffffffu, w0, 16 + j), wy1 = __shfl_sync(0xffffffffu, w1, 16 + j);
-                const int vx = __shfl_sync(0xffffffffu, gv, i), vy = __shfl_sync(0xffffffffu, gv, 16 + j);
-                if (!active) continue;
-                float v00, v01, v10, v11;
-                if (patch_ok) {
-                    const float* s = patch + (y0 - py0) * PD + (x0 - px0);
-                    v00 = s[0]; v01 = s[1]; v10 = s[PD]; v11 = s[PD + 1];
-                } else {   // generic path: taps straight from global memory
+            // ---- 3. (2r+1)^2 samples; a window the patch does not cover reads its taps straight from global memory
+            ofb::warp_window_samples(
+                win, patch, P.radius, lane,
+                [&](int x0, int y0, float wx0, float wx1, float wy0, float wy1) {
                     const bool inx0 = x0 >= 0 && x0 < Wl, inx1 = x0 + 1 >= 0 && x0 + 1 < Wl;
                     const bool iny0 = y0 >= 0 && y0 < Hl, iny1 = y0 + 1 >= 0 && y0 + 1 < Hl;
-                    v00 = (iny0 && inx0) ? Elem<T>::get(slice + (size_t)y0 * pitch, x0) : 0.0f;
-                    v01 = (iny0 && inx1) ? Elem<T>::get(slice + (size_t)y0 * pitch, x0 + 1) : 0.0f;
-                    v10 = (iny1 && inx0) ? Elem<T>::get(slice + (size_t)(y0 + 1) * pitch, x0) : 0.0f;
-                    v11 = (iny1 && inx1) ? Elem<T>::get(slice + (size_t)(y0 + 1) * pitch, x0 + 1) : 0.0f;
-                }
-                float acc = __fmul_rn(v00, __fmul_rn(wx0, wy0));
-                acc = __fmaf_rn(v01, __fmul_rn(wx1, wy0), acc);
-                acc = __fmaf_rn(v10, __fmul_rn(wx0, wy1), acc);
-                acc = __fmaf_rn(v11, __fmul_rn(wx1, wy1), acc);
-                otile[(l * DD + k) * OT_PITCH + qi] = acc;
-                if (valid_out) valid_out[(q * P.levels + l) * DD + k] = (uint8_t)(vx & vy);
-            }
+                    const float v00 = (iny0 && inx0) ? ofb::ld_f32(slice + (size_t)y0 * pitch + x0) : 0.0f;
+                    const float v01 = (iny0 && inx1) ? ofb::ld_f32(slice + (size_t)y0 * pitch + x0 + 1) : 0.0f;
+                    const float v10 = (iny1 && inx0) ? ofb::ld_f32(slice + (size_t)(y0 + 1) * pitch + x0) : 0.0f;
+                    const float v11 = (iny1 && inx1) ? ofb::ld_f32(slice + (size_t)(y0 + 1) * pitch + x0 + 1) : 0.0f;
+                    return ofb::bilinear(v00, v01, v10, v11, wx0, wx1, wy0, wy1);
+                },
+                [&](int k, int i, int j, float v) {
+                    otile[(l * DD + k) * OT_PITCH + qi] = v;
+                    if (valid_out)
+                        valid_out[(q * P.levels + l) * DD + k] = (uint8_t)((vmask >> i) & (vmask >> (16 + j)) & 1u);
+                });
             __syncwarp();
         }
     }
@@ -214,7 +134,7 @@ __global__ void __launch_bounds__(NW * 32) lookup_kernel(const LookupParams P, c
 //
 // thread = (query, level): lane <-> query (coordinates in, channel rows out are 128-byte coalesced),
 // warp <-> pyramid level.  Each thread
-//   1. evaluates its 2*(2R+1) tap coordinates with the bit-exact sequence above;
+//   1. evaluates its 2*(2R+1) tap coordinates with ofb::lookup_tap;
 //   2. anchors an 11 x 11 element window at (xs, ys) = min over taps of (floor index - tap number).
 //      Within the guarded coordinate range every tap's floor index is tap + anchor + {0, 1} (the fp32
 //      round trip can move a tap sitting on an integer to the pixel below), so tap i reads window
@@ -245,23 +165,16 @@ __device__ __forceinline__ TapSet<R> make_taps(float center, int size, int32_t* 
     int i0[D];
     ts.dead = false;
     ts.vmask = 0;
-    const float sm1 = (float)(size - 1);
     int anchor = INT_MAX;
 #pragma unroll
     for (int t = 0; t < D; ++t) {
-        const float pos = __fadd_rn(center, (float)(t - R));
-        const float g = __fsub_rn(__fdiv_rn(__fmul_rn(2.0f, pos), sm1), 1.0f);
-        const float ic = __fmul_rn(__fmul_rn(__fadd_rn(g, 1.0f), 0.5f), sm1);   // x / 2 == x * 0.5 exactly
-        const float fl = floorf(ic);
-        ts.w1[t] = __fsub_rn(ic, fl);
-        ts.w0[t] = __fsub_rn(__fadd_rn(fl, 1.0f), ic);
-        // guard for the int conversion; a tap outside it implies the whole window is outside the image
-        // (level sizes are <= 65536), and inside it fp32 resolves the coordinate to better than 1/64
-        const bool ok = fl >= -32768.0f && fl <= 70000.0f;
-        ts.dead |= !ok;
-        i0[t] = ok ? (int)fl : 0;
-        if (idx_dst) idx_dst[t] = (int32_t)fl;
-        ts.vmask |= ((g > -1.0f) && (g < 1.0f)) ? (1u << t) : 0u;
+        const ofb::LookupTap tp = ofb::lookup_tap(center, t, R, size);
+        ts.w1[t] = tp.w1;
+        ts.w0[t] = tp.w0;
+        ts.dead |= !tp.in_guard;
+        i0[t] = tp.in_guard ? (int)tp.fl : 0;
+        if (idx_dst) idx_dst[t] = (int32_t)tp.fl;
+        ts.vmask |= tp.valid ? (1u << t) : 0u;
         anchor = min(anchor, i0[t] - t);
     }
     ts.anchor = anchor;
@@ -400,15 +313,8 @@ __global__ void __launch_bounds__(128) lookup_tile_kernel(const LookupParams P, 
 #pragma unroll
         for (int k = 0; k < NW; ++k) v[k] = __funnelshift_r(t2[k], t2[k + 1], hs);
         float px[WIN];
-        if constexpr (std::is_same<T, __half>::value) {
 #pragma unroll
-            for (int e = 0; e < WIN; ++e)
-                px[e] = __half2float(__ushort_as_half((unsigned short)((e & 1) ? (v[e >> 1] >> 16) : (v[e >> 1] & 0xffffu))));
-        } else {
-#pragma unroll
-            for (int e = 0; e < WIN; ++e)
-                px[e] = __uint_as_float((e & 1) ? (v[e >> 1] & 0xffff0000u) : (v[e >> 1] << 16));
-        }
+        for (int e = 0; e < WIN; ++e) px[e] = ofb::widen16<T>(v[e >> 1], e & 1);
         // ---- horizontal filter
         float hrow[D];
 #pragma unroll
@@ -467,14 +373,13 @@ __global__ void __launch_bounds__(256) bilinear_sampler_kernel(const float* __re
     }
 }
 
+// window rows per cp.async commit group: 3 for radius 4 (measured ~2 % faster than one group for the whole window)
 template <typename T>
-int launch_tile(const LookupParams& P, const float* coords, float* out, int32_t* idx, uint8_t* valid, int radius, int gr,
+int launch_tile(const LookupParams& P, const float* coords, float* out, int32_t* idx, uint8_t* valid, int radius,
                 int blocks, int threads, size_t wsm, cudaStream_t st) {
     OFB_CUDA(ofb_smem_once<lookup_tile_kernel<4, 3, T>>(11 * 128 * 40));
-    OFB_CUDA(ofb_smem_once<lookup_tile_kernel<4, 16, T>>(11 * 128 * 40));
     OFB_CUDA(ofb_smem_once<lookup_tile_kernel<3, 16, T>>(9 * 128 * 40));
-    if (radius == 4 && gr == 3) lookup_tile_kernel<4, 3, T><<<blocks, threads, wsm, st>>>(P, coords, out, idx, valid);
-    else if (radius == 4) lookup_tile_kernel<4, 16, T><<<blocks, threads, wsm, st>>>(P, coords, out, idx, valid);
+    if (radius == 4) lookup_tile_kernel<4, 3, T><<<blocks, threads, wsm, st>>>(P, coords, out, idx, valid);
     else lookup_tile_kernel<3, 16, T><<<blocks, threads, wsm, st>>>(P, coords, out, idx, valid);
     OFB_LAUNCH_CHECK();
     return OFB_OK;
@@ -486,30 +391,19 @@ OFB_API int ofb_corr_lookup(const ofb_pyramid* pyr, const float* coords, float* 
                             uint8_t* valid_or_null, int B, int h, int w, int radius, void* stream) {
     if (B == 0) return OFB_OK;   // nothing to do: empty tensors have no storage, their pointers may be null
     if (!pyr || !coords || !out || B < 0 || h <= 0 || w <= 0) return OFB_EINVAL;
-    if (pyr->levels < 1 || pyr->levels > OFB_MAX_LEVELS) return OFB_EINVAL;
     if (radius < 0 || 2 * radius + 1 > MAX_D) return OFB_EUNSUPPORTED;
     if (pyr->dtype != OFB_DTYPE_F32 && pyr->dtype != OFB_DTYPE_BF16 && pyr->dtype != OFB_DTYPE_F16) return OFB_EINVAL;
+    if (pyr->layout < OFB_LAYOUT_ROWS || pyr->layout > OFB_LAYOUT_QMINOR8X4) return OFB_EINVAL;
     const bool half16 = pyr->dtype != OFB_DTYPE_F32;      // 16-bit storage: bf16 or fp16
-    if (B == 0) return OFB_OK;
     LookupParams P;
+    if (const int rc = ofb::unpack_levels(*pyr, P)) return rc;
     P.levels = pyr->levels; P.radius = radius; P.B = B; P.h = h; P.w = w;
     P.blocked = pyr->layout != OFB_LAYOUT_ROWS;
     P.blk_stride = pyr->layout == OFB_LAYOUT_QMINOR8X4 ? 32LL * B * h * w : 32LL;
-    if (pyr->layout < OFB_LAYOUT_ROWS || pyr->layout > OFB_LAYOUT_QMINOR8X4) return OFB_EINVAL;
-    for (int l = 0; l < OFB_MAX_LEVELS; ++l) {
-        const bool on = l < pyr->levels;
-        P.base[l] = on ? pyr->base[l] : nullptr;
-        P.q_stride[l] = on ? pyr->q_stride[l] : 0;
-        P.pitch[l] = on ? pyr->row_pitch[l] : 0;
-        P.lh[l] = on ? pyr->lvl_h[l] : 0;
-        P.lw[l] = on ? pyr->lvl_w[l] : 0;
-        if (on) {
-            if (!P.base[l] || P.lh[l] <= 0 || P.lw[l] <= 0 || P.pitch[l] < P.lw[l]) return OFB_EINVAL;
-            if (P.lh[l] > 65536 || P.lw[l] > 65536) return OFB_EUNSUPPORTED;
-            if (half16 &&
-                ((P.pitch[l] & 1) || (P.q_stride[l] & 1) || (reinterpret_cast<uintptr_t>(P.base[l]) & 3)))
-                return OFB_EALIGN;
-        }
+    for (int l = 0; l < P.levels; ++l) {
+        if (P.lh[l] > 65536 || P.lw[l] > 65536) return OFB_EUNSUPPORTED;
+        if (half16 && ((P.pitch[l] & 1) || (P.q_stride[l] & 1) || (reinterpret_cast<uintptr_t>(P.base[l]) & 3)))
+            return OFB_EALIGN;
     }
     const int D = 2 * radius + 1, CH = pyr->levels * D * D;
     const size_t smem = ((size_t)CH * OT_PITCH + (size_t)NW * PD * PD) * sizeof(float);
@@ -518,22 +412,15 @@ OFB_API int ofb_corr_lookup(const ofb_pyramid* pyr, const float* coords, float* 
     if (blocks > 0x7fffffffLL) return OFB_EUNSUPPORTED;
     cudaStream_t st = (cudaStream_t)stream;
     // product path: 16-bit pyramid with padded rows (pitch multiple of 8, 16-byte aligned slices)
-    bool tile_ok = half16 && (radius == 4 || radius == 3) && !getenv("OFB_LOOKUP_V1");
+    bool tile_ok = half16 && (radius == 4 || radius == 3);
     for (int l = 0; l < pyr->levels && tile_ok; ++l)
         tile_ok = (P.pitch[l] % 8 == 0) && (P.q_stride[l] % 8 == 0) && ((reinterpret_cast<uintptr_t>(P.base[l]) & 15) == 0);
     if (tile_ok) {
         const int threads = 32 * pyr->levels;
         const size_t wsm = (size_t)(2 * radius + 3) * threads * 40;               // window slots: rows x (16 + 16 + 8) B
-        // window rows per cp.async commit group: 3 (measured ~2 % faster than one group for the whole window);
-        // OFB_LOOKUP_GR=16 for A/B
-        static const int gr = [] {
-            const char* e = getenv("OFB_LOOKUP_GR");
-            return (e && atoi(e) == 16) ? 16 : 3;
-        }();
-        if (pyr->dtype == OFB_DTYPE_F16) return launch_tile<__half>(P, coords, out, idx_or_null, valid_or_null, radius, gr,
+        if (pyr->dtype == OFB_DTYPE_F16) return launch_tile<__half>(P, coords, out, idx_or_null, valid_or_null, radius,
                                                                     (int)blocks, threads, wsm, st);
-        return launch_tile<__nv_bfloat16>(P, coords, out, idx_or_null, valid_or_null, radius, gr, (int)blocks, threads, wsm,
-                                          st);
+        return launch_tile<__nv_bfloat16>(P, coords, out, idx_or_null, valid_or_null, radius, (int)blocks, threads, wsm, st);
     }
     if (P.blocked) return OFB_EUNSUPPORTED;   // the generic kernels read rows
     if (pyr->dtype == OFB_DTYPE_BF16) {

@@ -16,41 +16,24 @@
 //       dP[r][c] += T[r][c] * w0y[r] + T[r-1][c] * w1y[r-1]           (y pass)
 //     i.e. (2r+2)^2 accumulations in 2r+2 short rows instead of 4 (2r+1)^2 scattered ones;
 //   * anything else: the direct 4-tap scatter.
-// The tap positions and weights replay the forward kernel's fp32 sequence (lookup.cu header).
+// The tap positions and weights are the forward kernels' (ofb::lookup_tap, common.cuh).
 #include "common.cuh"
 
 namespace {
 
-struct BwdParams {
-    float* base[OFB_MAX_LEVELS];
-    long long q_stride[OFB_MAX_LEVELS];
-    int pitch[OFB_MAX_LEVELS];
-    int lh[OFB_MAX_LEVELS];
-    int lw[OFB_MAX_LEVELS];
+struct BwdParams : ofb::PyramidLevels {
     int levels, B, h, w;
 };
-
-constexpr int FAR = -1000000;
 
 struct Tap {
     int i0;
     float w0, w1;
 };
 
-// one axis, one window offset: the reference's normalise / un-normalise round trip (utils.py:70-71, ATen
-// GridSampler.h:30), as in the forward kernel
+// one axis, one window offset; a tap outside the guard gets index TAP_FAR and zero weights
 __device__ __forceinline__ Tap make_tap(float cen, int t, int radius, int size) {
-    const float pos = __fadd_rn(cen, (float)(t - radius));
-    const float sm1 = (float)(size - 1);
-    const float g = __fsub_rn(__fdiv_rn(__fmul_rn(2.0f, pos), sm1), 1.0f);
-    const float ic = __fmul_rn(__fdiv_rn(__fadd_rn(g, 1.0f), 2.0f), sm1);
-    const float fl = floorf(ic);
-    Tap tp;
-    tp.w1 = __fsub_rn(ic, fl);
-    tp.w0 = __fsub_rn(__fadd_rn(fl, 1.0f), ic);
-    tp.i0 = (fl >= -32768.0f && fl <= 70000.0f) ? (int)fl : FAR;
-    if (tp.i0 == FAR) { tp.w0 = 0.0f; tp.w1 = 0.0f; }
-    return tp;
+    const ofb::LookupTap tp = ofb::lookup_tap(cen, t, radius, size);
+    return tp.in_guard ? Tap{(int)tp.fl, tp.w0, tp.w1} : Tap{ofb::TAP_FAR, 0.0f, 0.0f};
 }
 
 template <int R>
@@ -63,7 +46,7 @@ __global__ void __launch_bounds__(128) lookup_bwd_kernel(const __grid_constant__
     if (q >= Q) return;
     const long long b = q / HW, p = q - b * HW;
     const int Wl = P.lw[l], Hl = P.lh[l], pitch = P.pitch[l];
-    float* slice = P.base[l] + q * P.q_stride[l];
+    float* slice = static_cast<float*>(P.base[l]) + q * P.q_stride[l];
     const float inv = 1.0f / (float)(1 << l);
     const float cx = __fmul_rn(__ldg(coords + (b * 2 + 0) * HW + p), inv);
     const float cy = __fmul_rn(__ldg(coords + (b * 2 + 1) * HW + p), inv);
@@ -77,7 +60,7 @@ __global__ void __launch_bounds__(128) lookup_bwd_kernel(const __grid_constant__
         const Tap tx = make_tap(cx, t, R, Wl), ty = make_tap(cy, t, R, Hl);
         wx0[t] = tx.w0; wx1[t] = tx.w1; wy0[t] = ty.w0; wy1[t] = ty.w1;
         if (t == 0) { ax = tx.i0; ay = ty.i0; }
-        regular = regular && tx.i0 != FAR && ty.i0 != FAR && tx.i0 == ax + t && ty.i0 == ay + t;
+        regular = regular && tx.i0 != ofb::TAP_FAR && ty.i0 != ofb::TAP_FAR && tx.i0 == ax + t && ty.i0 == ay + t;
     }
 
     if (regular) {
@@ -120,11 +103,11 @@ __global__ void __launch_bounds__(128) lookup_bwd_kernel(const __grid_constant__
 #pragma unroll 1
     for (int j = 0; j < D; ++j) {
         const Tap ty = make_tap(cy, j, R, Hl);
-        if (ty.i0 == FAR) continue;
+        if (ty.i0 == ofb::TAP_FAR) continue;
 #pragma unroll 1
         for (int i = 0; i < D; ++i) {
             const Tap tx = make_tap(cx, i, R, Wl);
-            if (tx.i0 == FAR) continue;
+            if (tx.i0 == ofb::TAP_FAR) continue;
             const float g = __ldg(g0 + (long long)(i * D + j) * HW);
             const bool inx0 = tx.i0 >= 0 && tx.i0 < Wl, inx1 = tx.i0 + 1 >= 0 && tx.i0 + 1 < Wl;
             const bool iny0 = ty.i0 >= 0 && ty.i0 < Hl, iny1 = ty.i0 + 1 >= 0 && ty.i0 + 1 < Hl;
@@ -144,21 +127,11 @@ OFB_API int ofb_corr_lookup_backward_f32(const ofb_pyramid* d_pyr, const float* 
                                          int w, int radius, void* stream) {
     if (B == 0) return OFB_OK;   // nothing to do: empty tensors have no storage, their pointers may be null
     if (!d_pyr || !coords || !d_out || B < 0 || h <= 0 || w <= 0) return OFB_EINVAL;
-    if (d_pyr->levels < 1 || d_pyr->levels > OFB_MAX_LEVELS) return OFB_EINVAL;
     if (d_pyr->dtype != OFB_DTYPE_F32 || d_pyr->layout != OFB_LAYOUT_ROWS) return OFB_EUNSUPPORTED;
     if (radius < 0 || radius > 4) return OFB_EUNSUPPORTED;
-    if (B == 0) return OFB_OK;
     BwdParams P;
+    if (const int rc = ofb::unpack_levels(*d_pyr, P)) return rc;
     P.levels = d_pyr->levels; P.B = B; P.h = h; P.w = w;
-    for (int l = 0; l < OFB_MAX_LEVELS; ++l) {
-        const bool on = l < d_pyr->levels;
-        P.base[l] = on ? static_cast<float*>(d_pyr->base[l]) : nullptr;
-        P.q_stride[l] = on ? d_pyr->q_stride[l] : 0;
-        P.pitch[l] = on ? d_pyr->row_pitch[l] : 0;
-        P.lh[l] = on ? d_pyr->lvl_h[l] : 0;
-        P.lw[l] = on ? d_pyr->lvl_w[l] : 0;
-        if (on && (!P.base[l] || P.lh[l] <= 0 || P.lw[l] <= 0 || P.pitch[l] < P.lw[l])) return OFB_EINVAL;
-    }
     const long long Q = (long long)B * h * w;
     const long long blocks = (Q + 127) / 128;
     if (blocks > 0x7fffffffLL) return OFB_EUNSUPPORTED;
