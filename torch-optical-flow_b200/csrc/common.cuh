@@ -5,6 +5,8 @@
 #include <cuda_fp16.h>
 #include <stdint.h>
 
+#include <type_traits>
+
 #include "../../include/ofb200.h"
 
 #define OFB_API extern "C" __attribute__((visibility("default")))
@@ -44,6 +46,23 @@ static inline int ofb_num_sms() {
     return sms[dev];
 }
 
+// Returns f(pad, ac) with both as std::integral_constant, so f can name a kernel template instance: pad is one of the
+// OFB_PAD_* modes and ac is 0 or 1, anything else is OFB_EINVAL.
+template <typename F>
+static inline int ofb_dispatch_pad_ac(int pad, int ac, F f) {
+    auto with_pad = [&](auto p) -> int {
+        if (ac == 0) return f(p, std::false_type{});
+        if (ac == 1) return f(p, std::true_type{});
+        return OFB_EINVAL;
+    };
+    switch (pad) {
+        case OFB_PAD_ZEROS: return with_pad(std::integral_constant<int, OFB_PAD_ZEROS>{});
+        case OFB_PAD_BORDER: return with_pad(std::integral_constant<int, OFB_PAD_BORDER>{});
+        case OFB_PAD_REFLECTION: return with_pad(std::integral_constant<int, OFB_PAD_REFLECTION>{});
+        default: return OFB_EINVAL;
+    }
+}
+
 // Raises Kernel's dynamic shared-memory limit to `bytes`, the first time it is called on each device.
 template <auto Kernel>
 static inline cudaError_t ofb_smem_once(int bytes) {
@@ -75,14 +94,25 @@ __device__ __forceinline__ float unnormalize(float g, int size) {
     return __fmaf_rn(__fadd_rn(g, 1.0f), 0.5f * (float)size, -0.5f);
 }
 __device__ __forceinline__ float clip_coord(float x, int size) { return fminf((float)(size - 1), fmaxf(x, 0.0f)); }
-__device__ __forceinline__ float reflect_coord(float in, int twice_low, int twice_high) {
-    if (twice_low == twice_high) return 0.0f;
-    float mn = (float)twice_low / 2.0f;
-    float span = (float)(twice_high - twice_low) / 2.0f;
-    in = fabsf(in - mn);
-    float extra = fmodf(in, span);
-    int flips = (int)floorf(in / span);
-    return (flips % 2 == 0) ? (extra + mn) : (span - extra + mn);
+// reflect_coordinates(_set_grad) (GridSampler.h:88-107,110-140); *dsign receives d(result)/d(in): +-1, or 0 for a
+// one-pixel span
+__device__ __forceinline__ float reflect_coord(float in, int twice_low, int twice_high, float* dsign = nullptr) {
+    if (twice_low == twice_high) {
+        if (dsign) *dsign = 0.0f;
+        return 0.0f;
+    }
+    const float mn = (float)twice_low / 2.0f;
+    const float span = (float)(twice_high - twice_low) / 2.0f;
+    const float d = in - mn;
+    in = fabsf(d);
+    const float extra = fmodf(in, span);
+    const bool odd = ((int)floorf(in / span)) % 2 != 0;
+    if (dsign) *dsign = (d < 0.0f) != odd ? -1.0f : 1.0f;
+    return odd ? (span - extra + mn) : (extra + mn);
+}
+template <bool AC>
+__device__ __forceinline__ float reflect_index(float x, int size, float* dsign = nullptr) {
+    return AC ? reflect_coord(x, 0, 2 * (size - 1), dsign) : reflect_coord(x, -1, 2 * size - 1, dsign);
 }
 template <int PAD, bool AC>
 __device__ __forceinline__ float source_index(float g, int size) {
@@ -90,10 +120,108 @@ __device__ __forceinline__ float source_index(float g, int size) {
     if (PAD == OFB_PAD_BORDER) {
         x = clip_coord(x, size);
     } else if (PAD == OFB_PAD_REFLECTION) {
-        x = AC ? reflect_coord(x, 0, 2 * (size - 1)) : reflect_coord(x, -1, 2 * size - 1);
-        x = clip_coord(x, size);
+        x = clip_coord(reflect_index<AC>(x, size), size);
     }
     return x;
+}
+
+// ---- the warp's sampling contract (K1 forward and backward, bilinear_sampler)
+//
+// Every grid_sample-style kernel takes its source coordinate from warp_source, its taps from bilinear_taps and, when
+// it gathers from global memory, its sample from gather4.  Non-finite and far coordinates:
+//   * zeros padding: a non-finite source coordinate samples 0, as does a finite one a pixel or more outside the frame;
+//     that is what the oracle gives.  ATen's bilinear grid_sample returns NaN for a NaN or +-inf coordinate (its
+//     weights are NaN and it multiplies them by the zero padding); it returns 0 for a finite far one.  bilinear_taps
+//     leaves such a coordinate no tap in bounds, so gather4 returns 0; a kernel that multiplies zero-filled taps by the
+//     weights instead (the NHWC float4 path, the TMA window) must keep it off that path.
+//   * border padding: clip_coord maps NaN and -inf to 0 and +inf to size - 1.
+//   * reflection: reflect_coord turns every non-finite coordinate into NaN and the clip maps it to 0.  ATen's CPU
+//     kernel agrees on both.
+// The mask (warp_source's valid) is false for every non-finite coordinate.
+
+// flow multipliers and linspace steps.  x, y: 1 for a normalised flow (the reference's contract); 2/(W-1), 2/(H-1)
+// fuse optical_flow.normalize (operator.py:117-130) into the warp -- one separately rounded multiply, as there.
+// step_x, step_y: linspace(-1, 1, W / H) steps, divided once on the host (linspace_step, the same IEEE fp32 division).
+struct FlowMul {
+    float x, y;
+    float step_x, step_y;
+};
+
+struct SrcPos {
+    float ix, iy;   // source position in pixels, after padding
+    bool valid;     // the grid coordinate lies strictly inside (-1, 1) on both axes
+};
+
+// Grid coordinate of output index i of n along one axis, with flow component f: linspace(-1, 1, n)[i] + f * mul
+// (operator.py:49-56)
+__device__ __forceinline__ float warp_grid_coord(float f, int i, int n, float step, float mul) {
+    return __fadd_rn(linspace_m1_p1(i, n, step), __fmul_rn(f, mul));
+}
+
+// Output pixel (i, j) with flow (fx, fy): its grid coordinate, then grid_sample's un-normalise and padding
+template <int PAD, bool AC>
+__device__ __forceinline__ SrcPos warp_source(float fx, float fy, int i, int j, int H, int W, const FlowMul& fm) {
+    const float gx = warp_grid_coord(fx, j, W, fm.step_x, fm.x);
+    const float gy = warp_grid_coord(fy, i, H, fm.step_y, fm.y);
+    SrcPos s;
+    s.ix = source_index<PAD, AC>(gx, W);
+    s.iy = source_index<PAD, AC>(gy, H);
+    s.valid = (gx > -1.0f) && (gy > -1.0f) && (gx < 1.0f) && (gy < 1.0f);
+    return s;
+}
+
+// A floor or rounded index as an int, clamped to [-2, size + 1] first: the one guard of the int conversion.  Indices
+// outside the frame stay outside it (with their + 1 neighbour), and NaN becomes -2 (fmaxf(NaN, -2) = -2).
+__device__ __forceinline__ int tap_index(float f, int size) { return (int)fminf(fmaxf(f, -2.0f), (float)size + 1.0f); }
+
+struct BilinearTaps {
+    int x0, y0;                  // upper-left tap (the + 1 taps are right of and below it)
+    float wx0, wx1, wy0, wy1;    // per-axis weights of columns x0, x0 + 1 and rows y0, y0 + 1
+    float w00, w01, w10, w11;    // tap weights, w<row><column>
+    unsigned inb;                // in-bounds mask: bit 0 (x0, y0), 1 (x0 + 1, y0), 2 (x0, y0 + 1), 3 (x0 + 1, y0 + 1)
+};
+
+// BilinearTaps::inb of upper-left tap (x0, y0); PAD as bilinear_taps
+template <int PAD>
+__device__ __forceinline__ unsigned tap_mask(int x0, int y0, int H, int W) {
+    bool inx0 = true, iny0 = true;
+    if (PAD == OFB_PAD_ZEROS) { inx0 = x0 >= 0 && x0 < W; iny0 = y0 >= 0 && y0 < H; }
+    const bool inx1 = (PAD != OFB_PAD_ZEROS || x0 + 1 >= 0) && x0 + 1 < W;
+    const bool iny1 = (PAD != OFB_PAD_ZEROS || y0 + 1 >= 0) && y0 + 1 < H;
+    return ((iny0 && inx0) ? 1u : 0u) | ((iny0 && inx1) ? 2u : 0u) | ((iny1 && inx0) ? 4u : 0u) |
+           ((iny1 && inx1) ? 8u : 0u);
+}
+// Taps of source position (ix, iy) in an H x W frame (GridSampler.h:330-380).  PAD != zeros promises that ix, iy were
+// clipped into [0, size - 1] by source_index: the upper-left tap is then inside, only the + 1 taps can fall off the
+// far edge (with weight 0), and no guard is needed.  The zeros form takes any coordinate: a non-finite one has NaN
+// weights and no tap in bounds.
+template <int PAD>
+__device__ __forceinline__ BilinearTaps bilinear_taps(float ix, float iy, int H, int W) {
+    const float x0f = floorf(ix), y0f = floorf(iy);
+    BilinearTaps t;
+    t.wx1 = ix - x0f; t.wx0 = (x0f + 1.0f) - ix;
+    t.wy1 = iy - y0f; t.wy0 = (y0f + 1.0f) - iy;
+    t.w00 = t.wx0 * t.wy0; t.w01 = t.wx1 * t.wy0; t.w10 = t.wx0 * t.wy1; t.w11 = t.wx1 * t.wy1;
+    t.x0 = PAD != OFB_PAD_ZEROS ? (int)x0f : tap_index(x0f, W);
+    t.y0 = PAD != OFB_PAD_ZEROS ? (int)y0f : tap_index(y0f, H);
+    t.inb = tap_mask<PAD>(t.x0, t.y0, H, W);
+    return t;
+}
+
+// The bilinear sample at p (the upper-left tap) from global memory, dx / dy elements to the next column / row: the
+// in-bounds taps of mask m (bits as BilinearTaps::inb; higher bits are ignored), accumulated in tap order with one
+// rounding each.  Taps outside m are not read and add nothing, whatever their weight.
+__device__ __forceinline__ float gather4(const float* p, size_t dx, size_t dy, unsigned m, float w00, float w01,
+                                         float w10, float w11) {
+    float acc = 0.0f;
+    if (m & 1u) acc = __fmaf_rn(__ldg(p), w00, acc);
+    if (m & 2u) acc = __fmaf_rn(__ldg(p + dx), w01, acc);
+    if (m & 4u) acc = __fmaf_rn(__ldg(p + dy), w10, acc);
+    if (m & 8u) acc = __fmaf_rn(__ldg(p + dy + dx), w11, acc);
+    return acc;
+}
+__device__ __forceinline__ float gather4(const float* p, size_t dx, size_t dy, const BilinearTaps& t) {
+    return gather4(p, dx, dy, t.inb, t.w00, t.w01, t.w10, t.w11);
 }
 
 // One tap of the correlation lookup's window (CorrBlock.__call__ + bilinear_sampler, methods/raft/model/corr.py:56-77,

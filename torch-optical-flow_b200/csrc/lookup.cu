@@ -355,21 +355,10 @@ __global__ void __launch_bounds__(256) bilinear_sampler_kernel(const float* __re
         const float gy = __fsub_rn(__fdiv_rn(__fmul_rn(2.0f, c.y), (float)(H - 1)), 1.0f);
         const float ix = ofb::unnormalize<true>(gx, W), iy = ofb::unnormalize<true>(gy, H);
         if (mask) mask[t] = ((gx > -1.0f) && (gy > -1.0f) && (gx < 1.0f) && (gy < 1.0f)) ? 1.0f : 0.0f;
-        const float x0f = floorf(ix), y0f = floorf(iy);
-        const bool fin = x0f >= -8.0f && x0f <= 1.0e6f && y0f >= -8.0f && y0f <= 1.0e6f;
-        const int x0 = fin ? (int)x0f : -100, y0 = fin ? (int)y0f : -100;
-        const float wx1 = ix - x0f, wx0 = (x0f + 1.0f) - ix, wy1 = iy - y0f, wy0 = (y0f + 1.0f) - iy;
-        const bool inx0 = x0 >= 0 && x0 < W, inx1 = x0 + 1 >= 0 && x0 + 1 < W;
-        const bool iny0 = y0 >= 0 && y0 < H, iny1 = y0 + 1 >= 0 && y0 + 1 < H;
-        for (int ch = 0; ch < C; ++ch) {
-            const float* plane = img + ((size_t)n * C + ch) * H * W;
-            float acc = 0.0f;
-            if (iny0 && inx0) acc = __fmaf_rn(__ldg(plane + (size_t)y0 * W + x0), wx0 * wy0, acc);
-            if (iny0 && inx1) acc = __fmaf_rn(__ldg(plane + (size_t)y0 * W + x0 + 1), wx1 * wy0, acc);
-            if (iny1 && inx0) acc = __fmaf_rn(__ldg(plane + (size_t)(y0 + 1) * W + x0), wx0 * wy1, acc);
-            if (iny1 && inx1) acc = __fmaf_rn(__ldg(plane + (size_t)(y0 + 1) * W + x0 + 1), wx1 * wy1, acc);
-            out[((size_t)n * C + ch) * HWo + p] = acc;
-        }
+        const ofb::BilinearTaps tp = ofb::bilinear_taps<OFB_PAD_ZEROS>(ix, iy, H, W);
+        const size_t o00 = (size_t)tp.y0 * W + tp.x0;
+        for (int ch = 0; ch < C; ++ch)
+            out[((size_t)n * C + ch) * HWo + p] = ofb::gather4(img + ((size_t)n * C + ch) * H * W + o00, 1, W, tp);
     }
 }
 

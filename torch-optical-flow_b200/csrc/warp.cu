@@ -22,46 +22,6 @@ namespace {
 
 using namespace ofb;
 
-struct SrcPos {
-    float ix, iy;
-    bool valid;
-};
-
-// flow multipliers: 1 for a normalised flow (the reference's contract); 2/(W-1), 2/(H-1) fuse
-// optical_flow.normalize (operator.py:117-130) into the warp -- one separately rounded multiply, as there
-struct FlowMul {
-    float x, y;
-    float step_x, step_y;   // linspace(-1, 1, W / H) steps, divided once on the host (same IEEE fp32 division)
-};
-
-template <int PAD, bool AC>
-__device__ __forceinline__ SrcPos source_from_flow(float fx, float fy, int i, int j, int H, int W, float step_x,
-                                                   float step_y, FlowMul fm) {
-    const float gx = __fadd_rn(linspace_m1_p1(j, W, step_x), __fmul_rn(fx, fm.x));
-    const float gy = __fadd_rn(linspace_m1_p1(i, H, step_y), __fmul_rn(fy, fm.y));
-    SrcPos s;
-    s.ix = source_index<PAD, AC>(gx, W);
-    s.iy = source_index<PAD, AC>(gy, H);
-    s.valid = (gx > -1.0f) && (gy > -1.0f) && (gx < 1.0f) && (gy < 1.0f);
-    return s;
-}
-
-template <int PAD, bool AC>
-__device__ __forceinline__ SrcPos source_position(const float* __restrict__ flow, int b, int i, int j, int H, int W,
-                                                  float step_x, float step_y, FlowMul fm = FlowMul{1.0f, 1.0f}) {
-    const size_t HW = (size_t)H * W;
-    const size_t p = (size_t)i * W + j;
-    float fx = __fmul_rn(__ldg(flow + ((size_t)b * 2 + 0) * HW + p), fm.x);
-    float fy = __fmul_rn(__ldg(flow + ((size_t)b * 2 + 1) * HW + p), fm.y);
-    float gx = __fadd_rn(linspace_m1_p1(j, W, step_x), fx);
-    float gy = __fadd_rn(linspace_m1_p1(i, H, step_y), fy);
-    SrcPos s;
-    s.ix = source_index<PAD, AC>(gx, W);
-    s.iy = source_index<PAD, AC>(gy, H);
-    s.valid = (gx > -1.0f) && (gy > -1.0f) && (gx < 1.0f) && (gy < 1.0f);
-    return s;
-}
-
 // ------------------------------------------------------------------------------ direct kernel
 template <int MODE, int PAD, bool AC, bool NHWC>
 __global__ void __launch_bounds__(256) warp_direct_kernel(const float* __restrict__ frame, const float* __restrict__ flow,
@@ -69,16 +29,16 @@ __global__ void __launch_bounds__(256) warp_direct_kernel(const float* __restric
                                                           int C, int H, int W, FlowMul fm) {
     const size_t HW = (size_t)H * W;
     const size_t total = (size_t)B * HW;
-    const float step_x = linspace_step(W), step_y = linspace_step(H);
     for (size_t q = (size_t)blockIdx.x * blockDim.x + threadIdx.x; q < total; q += (size_t)gridDim.x * blockDim.x) {
         const int b = (int)(q / HW);
         const size_t p = q - (size_t)b * HW;
         const int i = (int)(p / W), j = (int)(p - (size_t)i * W);
-        SrcPos s = source_position<PAD, AC>(flow, b, i, j, H, W, step_x, step_y, fm);
+        const float* fxp = flow + (size_t)b * 2 * HW + p;
+        const SrcPos s = warp_source<PAD, AC>(__ldg(fxp), __ldg(fxp + HW), i, j, H, W, fm);
         if (valid) valid[q] = s.valid ? 1 : 0;
         if (MODE == OFB_MODE_NEAREST) {
-            int x = (int)rintf(s.ix), y = (int)rintf(s.iy);
-            bool in = x >= 0 && x < W && y >= 0 && y < H;
+            const int x = tap_index(rintf(s.ix), W), y = tap_index(rintf(s.iy), H);
+            const bool in = x >= 0 && x < W && y >= 0 && y < H;
             for (int c = 0; c < C; ++c) {
                 float v = 0.0f;
                 if (in) v = NHWC ? __ldg(frame + ((size_t)b * HW + (size_t)y * W + x) * C + c)
@@ -87,56 +47,39 @@ __global__ void __launch_bounds__(256) warp_direct_kernel(const float* __restric
             }
             continue;
         }
-        const float x0f = floorf(s.ix), y0f = floorf(s.iy);
-        const int x0 = (int)x0f, y0 = (int)y0f, x1 = x0 + 1, y1 = y0 + 1;
-        const float wx1 = s.ix - x0f, wx0 = (x0f + 1.0f) - s.ix;
-        const float wy1 = s.iy - y0f, wy0 = (y0f + 1.0f) - s.iy;
-        const float w00 = wx0 * wy0, w01 = wx1 * wy0, w10 = wx0 * wy1, w11 = wx1 * wy1;
-        const bool inx0 = x0 >= 0 && x0 < W, inx1 = x1 >= 0 && x1 < W;
-        const bool iny0 = y0 >= 0 && y0 < H, iny1 = y1 >= 0 && y1 < H;
+        const BilinearTaps t = bilinear_taps<PAD>(s.ix, s.iy, H, W);
+        if (NHWC && !t.inb) {
+            // no tap in the frame: 0, which the float4 path would not give for the NaN weights of a non-finite position
+            for (int c = 0; c < C; ++c) out[((size_t)b * C + c) * HW + p] = 0.0f;
+            continue;
+        }
         if (NHWC) {
-            const float* base = frame + (size_t)b * HW * C;
-            const float* p00 = base + ((size_t)y0 * W + x0) * C;
-            const float* p01 = p00 + C;
-            const float* p10 = p00 + (size_t)W * C;
-            const float* p11 = p10 + C;
+            const float* p00 = frame + ((size_t)b * HW + (size_t)t.y0 * W + t.x0) * C;
+            const size_t row = (size_t)W * C;
             if ((C & 3) == 0) {
+                const float *p01 = p00 + C, *p10 = p00 + row, *p11 = p10 + C;
                 for (int c = 0; c < C; c += 4) {
                     float4 a = make_float4(0, 0, 0, 0), bb = a, cc = a, dd = a;
-                    if (iny0 && inx0) a = __ldg(reinterpret_cast<const float4*>(p00 + c));
-                    if (iny0 && inx1) bb = __ldg(reinterpret_cast<const float4*>(p01 + c));
-                    if (iny1 && inx0) cc = __ldg(reinterpret_cast<const float4*>(p10 + c));
-                    if (iny1 && inx1) dd = __ldg(reinterpret_cast<const float4*>(p11 + c));
-                    float r0 = __fmaf_rn(dd.x, w11, __fmaf_rn(cc.x, w10, __fmaf_rn(bb.x, w01, a.x * w00)));
-                    float r1 = __fmaf_rn(dd.y, w11, __fmaf_rn(cc.y, w10, __fmaf_rn(bb.y, w01, a.y * w00)));
-                    float r2 = __fmaf_rn(dd.z, w11, __fmaf_rn(cc.z, w10, __fmaf_rn(bb.z, w01, a.z * w00)));
-                    float r3 = __fmaf_rn(dd.w, w11, __fmaf_rn(cc.w, w10, __fmaf_rn(bb.w, w01, a.w * w00)));
+                    if (t.inb & 1u) a = __ldg(reinterpret_cast<const float4*>(p00 + c));
+                    if (t.inb & 2u) bb = __ldg(reinterpret_cast<const float4*>(p01 + c));
+                    if (t.inb & 4u) cc = __ldg(reinterpret_cast<const float4*>(p10 + c));
+                    if (t.inb & 8u) dd = __ldg(reinterpret_cast<const float4*>(p11 + c));
+                    float r0 = __fmaf_rn(dd.x, t.w11, __fmaf_rn(cc.x, t.w10, __fmaf_rn(bb.x, t.w01, a.x * t.w00)));
+                    float r1 = __fmaf_rn(dd.y, t.w11, __fmaf_rn(cc.y, t.w10, __fmaf_rn(bb.y, t.w01, a.y * t.w00)));
+                    float r2 = __fmaf_rn(dd.z, t.w11, __fmaf_rn(cc.z, t.w10, __fmaf_rn(bb.z, t.w01, a.z * t.w00)));
+                    float r3 = __fmaf_rn(dd.w, t.w11, __fmaf_rn(cc.w, t.w10, __fmaf_rn(bb.w, t.w01, a.w * t.w00)));
                     out[((size_t)b * C + c + 0) * HW + p] = r0;
                     out[((size_t)b * C + c + 1) * HW + p] = r1;
                     out[((size_t)b * C + c + 2) * HW + p] = r2;
                     out[((size_t)b * C + c + 3) * HW + p] = r3;
                 }
             } else {
-                for (int c = 0; c < C; ++c) {
-                    float acc = 0.0f;
-                    if (iny0 && inx0) acc = __fmaf_rn(__ldg(p00 + c), w00, acc);
-                    if (iny0 && inx1) acc = __fmaf_rn(__ldg(p01 + c), w01, acc);
-                    if (iny1 && inx0) acc = __fmaf_rn(__ldg(p10 + c), w10, acc);
-                    if (iny1 && inx1) acc = __fmaf_rn(__ldg(p11 + c), w11, acc);
-                    out[((size_t)b * C + c) * HW + p] = acc;
-                }
+                for (int c = 0; c < C; ++c) out[((size_t)b * C + c) * HW + p] = gather4(p00 + c, C, row, t);
             }
         } else {
-            const size_t o00 = (size_t)y0 * W + x0;
-            for (int c = 0; c < C; ++c) {
-                const float* plane = frame + ((size_t)b * C + c) * HW;
-                float acc = 0.0f;
-                if (iny0 && inx0) acc = __fmaf_rn(__ldg(plane + o00), w00, acc);
-                if (iny0 && inx1) acc = __fmaf_rn(__ldg(plane + o00 + 1), w01, acc);
-                if (iny1 && inx0) acc = __fmaf_rn(__ldg(plane + o00 + W), w10, acc);
-                if (iny1 && inx1) acc = __fmaf_rn(__ldg(plane + o00 + W + 1), w11, acc);
-                out[((size_t)b * C + c) * HW + p] = acc;
-            }
+            const size_t o00 = (size_t)t.y0 * W + t.x0;
+            for (int c = 0; c < C; ++c)
+                out[((size_t)b * C + c) * HW + p] = gather4(frame + ((size_t)b * C + c) * HW + o00, 1, W, t);
         }
     }
 }
@@ -154,17 +97,18 @@ __device__ __forceinline__ void cp_async16(void* smem, const void* gmem) {
 }
 __device__ __forceinline__ void cp_async_wait_all() { asm volatile("cp.async.wait_all;\n" ::: "memory"); }
 
+// Takes its taps in the guarded (zeros) form under every padding, valid for clipped coordinates too.  With that and
+// the 2 CTAs per SM its shared memory allows at CG_MAX channels, every instance compiles to 96 registers, no spills.
 template <int PAD, bool AC>
-__global__ void __launch_bounds__(NT) warp_staged_kernel(const float* __restrict__ frame, const float* __restrict__ flow,
-                                                         float* __restrict__ out, uint8_t* __restrict__ valid, int B,
-                                                         int C, int H, int W, int vec4, FlowMul fm) {
+__global__ void __launch_bounds__(NT, 2) warp_staged_kernel(const float* __restrict__ frame, const float* __restrict__ flow,
+                                                            float* __restrict__ out, uint8_t* __restrict__ valid, int B,
+                                                            int C, int H, int W, int vec4, FlowMul fm) {
     extern __shared__ __align__(16) float win[];  // [cg][WIN_H][pitch]
     __shared__ int s_box[4];                      // min x, max x, min y, max y of the taps
     const int b = blockIdx.z;
     const int tile_x = blockIdx.x * TW, tile_y = blockIdx.y * TH;
     const int tx = threadIdx.x % TW, ty = threadIdx.x / TW;  // ty in [0, NT/TW)
     const size_t HW = (size_t)H * W;
-    const float step_x = linspace_step(W), step_y = linspace_step(H);
 
     if (threadIdx.x == 0) { s_box[0] = INT_MAX; s_box[1] = INT_MIN; s_box[2] = INT_MAX; s_box[3] = INT_MIN; }
     __syncthreads();
@@ -176,14 +120,13 @@ __global__ void __launch_bounds__(NT) warp_staged_kernel(const float* __restrict
         const int i = tile_y + ty + k * (NT / TW), j = tile_x + tx;
         ix[k] = 0.0f; iy[k] = 0.0f;
         if (i < H && j < W) {
-            SrcPos s = source_position<PAD, AC>(flow, b, i, j, H, W, step_x, step_y, fm);
+            const float* fxp = flow + (size_t)b * 2 * HW + (size_t)i * W + j;
+            const SrcPos s = warp_source<PAD, AC>(__ldg(fxp), __ldg(fxp + HW), i, j, H, W, fm);
             ix[k] = s.ix; iy[k] = s.iy;
             if (valid) valid[(size_t)b * HW + (size_t)i * W + j] = s.valid ? 1 : 0;
-            // clamp before the int conversion: zeros padding can leave coordinates far outside
-            int x0 = (int)floorf(fminf(fmaxf(s.ix, -2.0f), (float)W + 1.0f));
-            int y0 = (int)floorf(fminf(fmaxf(s.iy, -2.0f), (float)H + 1.0f));
-            bx0 = min(bx0, x0); bx1 = max(bx1, x0 + 1);
-            by0 = min(by0, y0); by1 = max(by1, y0 + 1);
+            const BilinearTaps t = bilinear_taps<OFB_PAD_ZEROS>(s.ix, s.iy, H, W);
+            bx0 = min(bx0, t.x0); bx1 = max(bx1, t.x0 + 1);
+            by0 = min(by0, t.y0); by1 = max(by1, t.y0 + 1);
         }
     }
     bx0 = warp_min(bx0); bx1 = warp_max(bx1); by0 = warp_min(by0); by1 = warp_max(by1);
@@ -229,36 +172,24 @@ __global__ void __launch_bounds__(NT) warp_staged_kernel(const float* __restrict
         for (int k = 0; k < PPT; ++k) {
             const int i = tile_y + ty + k * (NT / TW), j = tile_x + tx;
             if (i >= H || j >= W) continue;
-            const float x0f = floorf(ix[k]), y0f = floorf(iy[k]);
-            const float wx1 = ix[k] - x0f, wx0 = (x0f + 1.0f) - ix[k];
-            const float wy1 = iy[k] - y0f, wy0 = (y0f + 1.0f) - iy[k];
-            const float w00 = wx0 * wy0, w01 = wx1 * wy0, w10 = wx0 * wy1, w11 = wx1 * wy1;
-            const int x0 = (int)fminf(fmaxf(x0f, -2.0f), (float)W + 1.0f);
-            const int y0 = (int)fminf(fmaxf(y0f, -2.0f), (float)H + 1.0f);
-            const int x1 = x0 + 1, y1 = y0 + 1;
-            const bool fast = x0 >= wx_lo && x1 <= wx_hi && y0 >= wy_lo && y1 <= wy_hi;
+            const BilinearTaps t = bilinear_taps<OFB_PAD_ZEROS>(ix[k], iy[k], H, W);
+            const bool fast = t.x0 >= wx_lo && t.x0 + 1 <= wx_hi && t.y0 >= wy_lo && t.y0 + 1 <= wy_hi;
             const size_t p = (size_t)i * W + j;
             if (fast) {
-                const float* s00 = win + (y0 - wy_lo) * pitch + (x0 - wx_lo);
+                const float* s00 = win + (t.y0 - wy_lo) * pitch + (t.x0 - wx_lo);
                 for (int c = 0; c < cg; ++c) {
                     const float* s = s00 + c * plane_sz;
-                    float acc = s[0] * w00;
-                    acc = __fmaf_rn(s[1], w01, acc);
-                    acc = __fmaf_rn(s[pitch], w10, acc);
-                    acc = __fmaf_rn(s[pitch + 1], w11, acc);
+                    float acc = s[0] * t.w00;
+                    acc = __fmaf_rn(s[1], t.w01, acc);
+                    acc = __fmaf_rn(s[pitch], t.w10, acc);
+                    acc = __fmaf_rn(s[pitch + 1], t.w11, acc);
                     out[((size_t)b * C + c0 + c) * HW + p] = acc;
                 }
             } else {
-                const bool inx0 = x0 >= 0 && x0 < W, inx1 = x1 >= 0 && x1 < W;
-                const bool iny0 = y0 >= 0 && y0 < H, iny1 = y1 >= 0 && y1 < H;
+                const size_t o00 = (size_t)t.y0 * W + t.x0;
                 for (int c = 0; c < cg; ++c) {
                     const float* plane = frame + ((size_t)b * C + c0 + c) * HW;
-                    float acc = 0.0f;
-                    if (iny0 && inx0) acc = __fmaf_rn(__ldg(plane + (size_t)y0 * W + x0), w00, acc);
-                    if (iny0 && inx1) acc = __fmaf_rn(__ldg(plane + (size_t)y0 * W + x1), w01, acc);
-                    if (iny1 && inx0) acc = __fmaf_rn(__ldg(plane + (size_t)y1 * W + x0), w10, acc);
-                    if (iny1 && inx1) acc = __fmaf_rn(__ldg(plane + (size_t)y1 * W + x1), w11, acc);
-                    out[((size_t)b * C + c0 + c) * HW + p] = acc;
+                    out[((size_t)b * C + c0 + c) * HW + p] = gather4(plane + o00, 1, W, t);
                 }
             }
         }
@@ -282,7 +213,6 @@ __global__ void __launch_bounds__(128) warp_rows_kernel(const float* __restrict_
     const int i0 = blockIdx.y * RPT;
     if (j >= W) return;
     const int HW = H * W;                                     // launch guard: H*W < 2^30
-    const float step_x = fm.step_x, step_y = fm.step_y;
     const float* fxp = flow + (size_t)(b * 2) * HW;
     const float* fyp = fxp + HW;
     int o00[RPT];
@@ -294,29 +224,12 @@ __global__ void __launch_bounds__(128) warp_rows_kernel(const float* __restrict_
         o00[k] = 0; w00[k] = w01[k] = w10[k] = w11[k] = 0.0f;
         if (i >= H) continue;
         const int off = i * W + j;
-        const SrcPos s = source_from_flow<PAD, AC>(__ldg(fxp + off), __ldg(fyp + off), i, j, H, W, step_x, step_y, fm);
+        const SrcPos s = warp_source<PAD, AC>(__ldg(fxp + off), __ldg(fyp + off), i, j, H, W, fm);
         if (valid) valid[(size_t)b * HW + off] = s.valid ? 1 : 0;
-        const float x0f = floorf(s.ix), y0f = floorf(s.iy);
-        const float wx1 = s.ix - x0f, wx0 = (x0f + 1.0f) - s.ix;
-        const float wy1 = s.iy - y0f, wy0 = (y0f + 1.0f) - s.iy;
-        w00[k] = wx0 * wy0; w01[k] = wx1 * wy0; w10[k] = wx0 * wy1; w11[k] = wx1 * wy1;
-        int x0, y0;
-        bool inx0, inx1, iny0, iny1;
-        if (PAD != OFB_PAD_ZEROS) {
-            // border / reflection clip the coordinate into [0, size-1] (NaN clips to 0): the upper-left tap is
-            // always inside, only the +1 taps can fall off the far edge (their weight is 0 there)
-            x0 = (int)x0f; y0 = (int)y0f;
-            inx0 = true; iny0 = true; inx1 = x0 + 1 < W; iny1 = y0 + 1 < H;
-        } else {
-            // clamp before the int conversion: zeros padding can leave coordinates far outside; NaN samples nothing
-            x0 = (int)fminf(fmaxf(x0f, -2.0f), (float)W + 1.0f); y0 = (int)fminf(fmaxf(y0f, -2.0f), (float)H + 1.0f);
-            const bool fin = x0f == x0f && y0f == y0f;
-            inx0 = fin && x0 >= 0 && x0 < W; inx1 = fin && x0 + 1 >= 0 && x0 + 1 < W;
-            iny0 = y0 >= 0 && y0 < H; iny1 = y0 + 1 >= 0 && y0 + 1 < H;
-        }
-        inb |= (((iny0 && inx0) ? 1u : 0u) | ((iny0 && inx1) ? 2u : 0u) | ((iny1 && inx0) ? 4u : 0u) |
-                ((iny1 && inx1) ? 8u : 0u)) << (4 * k);
-        o00[k] = y0 * W + x0;
+        const BilinearTaps t = bilinear_taps<PAD>(s.ix, s.iy, H, W);
+        w00[k] = t.w00; w01[k] = t.w01; w10[k] = t.w10; w11[k] = t.w11;
+        inb |= t.inb << (4 * k);
+        o00[k] = t.y0 * W + t.x0;
     }
     // interior pixels (all 4 x RPT taps inside the frame -- everything but the last row / column and, under zeros
     // padding, samples that leave the frame): no predicates, no per-tap address arithmetic.  The kernel is bound
@@ -350,14 +263,7 @@ __global__ void __launch_bounds__(128) warp_rows_kernel(const float* __restrict_
 #pragma unroll
         for (int k = 0; k < RPT; ++k) {
             if (i0 + k >= H) continue;
-            const unsigned m = inb >> (4 * k);
-            const float* p = plane + o00[k];
-            float acc = 0.0f;
-            if (m & 1u) acc = __fmaf_rn(__ldg(p), w00[k], acc);
-            if (m & 2u) acc = __fmaf_rn(__ldg(p + 1), w01[k], acc);
-            if (m & 4u) acc = __fmaf_rn(__ldg(p + W), w10[k], acc);
-            if (m & 8u) acc = __fmaf_rn(__ldg(p + W + 1), w11[k], acc);
-            op[k * W] = acc;
+            op[k * W] = gather4(plane + o00[k], 1, W, inb >> (4 * k), w00[k], w01[k], w10[k], w11[k]);
         }
     }
 }
@@ -423,43 +329,11 @@ int launch_staged(const float* frame, const float* flow, float* out, uint8_t* va
     return OFB_OK;
 }
 
-template <int MODE>
-int dispatch_direct(int pad, int ac, const float* frame, const float* flow, float* out, uint8_t* valid, int B, int C,
-                    int H, int W, int cl, FlowMul fm, cudaStream_t st) {
-#define OFB_CASE(P, A)                                                                                 \
-    if (pad == P && ac == (A ? 1 : 0))                                                                  \
-        return launch_direct<MODE, P, A>(frame, flow, out, valid, B, C, H, W, cl, fm, st);
-    OFB_CASE(OFB_PAD_ZEROS, false)
-    OFB_CASE(OFB_PAD_ZEROS, true)
-    OFB_CASE(OFB_PAD_BORDER, false)
-    OFB_CASE(OFB_PAD_BORDER, true)
-    OFB_CASE(OFB_PAD_REFLECTION, false)
-    OFB_CASE(OFB_PAD_REFLECTION, true)
-#undef OFB_CASE
-    return OFB_EINVAL;
-}
-
-int dispatch_staged(int pad, int ac, int rows, const float* frame, const float* flow, float* out, uint8_t* valid, int B,
-                    int C, int H, int W, FlowMul fm, cudaStream_t st) {
-#define OFB_CASE(P, A)                                                                                   \
-    if (pad == P && ac == (A ? 1 : 0))                                                                    \
-        return rows ? launch_rows<P, A>(frame, flow, out, valid, B, C, H, W, fm, st)                      \
-                    : launch_staged<P, A>(frame, flow, out, valid, B, C, H, W, fm, st);
-    OFB_CASE(OFB_PAD_ZEROS, false)
-    OFB_CASE(OFB_PAD_ZEROS, true)
-    OFB_CASE(OFB_PAD_BORDER, false)
-    OFB_CASE(OFB_PAD_BORDER, true)
-    OFB_CASE(OFB_PAD_REFLECTION, false)
-    OFB_CASE(OFB_PAD_REFLECTION, true)
-#undef OFB_CASE
-    return OFB_EINVAL;
-}
-
 }  // namespace
 
 // warp_tma.cu
 int ofb_warp_tma_launch(const float* frame, const float* flow, float* out, uint8_t* valid, int B, int C, int H, int W,
-                        int pad, int ac, float fmx, float fmy, cudaStream_t st);
+                        int pad, int ac, const ofb::FlowMul& fm, cudaStream_t st);
 
 OFB_API int ofb_warp_f32(const float* frame, const float* flow, float* out, uint8_t* valid_or_null, int B, int C, int H,
                          int W, int mode, int padding_mode, int align_corners, int channels_last, int variant,
@@ -487,14 +361,15 @@ OFB_API int ofb_warp_f32(const float* frame, const float* flow, float* out, uint
     }();
     int v = variant != 0 ? variant : (auto_v == 4 && can_tma ? 4 : (can_rows ? 3 : 1));
     if (v == 4)
-        return ofb_warp_tma_launch(frame, flow, out, valid_or_null, B, C, H, W, padding_mode, align_corners, fm.x, fm.y, st);
-    if (v == 2 || v == 3)
-        return dispatch_staged(padding_mode, align_corners, v == 3, frame, flow, out, valid_or_null, B, C, H, W, fm, st);
-    if (mode == OFB_MODE_BILINEAR)
-        return dispatch_direct<OFB_MODE_BILINEAR>(padding_mode, align_corners, frame, flow, out, valid_or_null, B, C, H,
-                                                  W, channels_last, fm, st);
-    return dispatch_direct<OFB_MODE_NEAREST>(padding_mode, align_corners, frame, flow, out, valid_or_null, B, C, H, W,
-                                             channels_last, fm, st);
+        return ofb_warp_tma_launch(frame, flow, out, valid_or_null, B, C, H, W, padding_mode, align_corners, fm, st);
+    return ofb_dispatch_pad_ac(padding_mode, align_corners, [&](auto P, auto A) {
+        if (v == 3) return launch_rows<P, A>(frame, flow, out, valid_or_null, B, C, H, W, fm, st);
+        if (v == 2) return launch_staged<P, A>(frame, flow, out, valid_or_null, B, C, H, W, fm, st);
+        const int cl = channels_last;
+        if (mode == OFB_MODE_BILINEAR)
+            return launch_direct<OFB_MODE_BILINEAR, P, A>(frame, flow, out, valid_or_null, B, C, H, W, cl, fm, st);
+        return launch_direct<OFB_MODE_NEAREST, P, A>(frame, flow, out, valid_or_null, B, C, H, W, cl, fm, st);
+    });
 }
 
 OFB_API int ofb_warp_grid_f32(const float* flow_bhw2, float* grid_bhw2, int B, int H, int W, void* stream) {

@@ -16,36 +16,16 @@ namespace {
 
 using namespace ofb;
 
-struct Steps {
-    float mul_x, mul_y;     // flow multipliers (1, 1 or the fused normalize factors)
-    float step_x, step_y;   // linspace steps, divided on the host
-};
-
-// source index and d(index)/d(grid coordinate)
+// source index and d(index)/d(grid coordinate).  Its clip is not source_index's: ATen's backward keeps NaN here,
+// where the forward's clip_coord maps it to 0.
 template <int PAD, bool AC>
 __device__ __forceinline__ float source_index_grad(float g, int size, float& grad) {
-    float x;
-    if (AC) {
-        grad = (float)(size - 1) / 2.0f;
-        x = __fmul_rn(__fdiv_rn(__fadd_rn(g, 1.0f), 2.0f), (float)(size - 1));
-    } else {
-        grad = (float)size / 2.0f;
-        x = __fmaf_rn(__fadd_rn(g, 1.0f), 0.5f * (float)size, -0.5f);
-    }
+    grad = AC ? (float)(size - 1) / 2.0f : (float)size / 2.0f;
+    float x = unnormalize<AC>(g, size);
     if (PAD == OFB_PAD_REFLECTION) {
-        const int twice_low = AC ? 0 : -1, twice_high = AC ? 2 * (size - 1) : 2 * size - 1;
-        if (twice_low == twice_high) {
-            grad = 0.0f;
-            x = 0.0f;
-        } else {
-            const float mn = (float)twice_low / 2.0f, span = (float)(twice_high - twice_low) / 2.0f;
-            float in = x - mn, sign = 1.0f;
-            if (in < 0.0f) { sign = -1.0f; in = -in; }
-            const float extra = fmodf(in, span);
-            const int flips = (int)floorf(in / span);
-            if (flips % 2 == 0) { x = extra + mn; } else { x = span - extra + mn; sign = -sign; }
-            grad *= sign;
-        }
+        float dsign;
+        x = reflect_index<AC>(x, size, &dsign);
+        grad *= dsign;
     }
     if (PAD != OFB_PAD_ZEROS) {
         // borders count as out of bounds for the gradient (GridSampler.h:68-69); NaN falls to the last branch as there
@@ -58,38 +38,32 @@ __device__ __forceinline__ float source_index_grad(float g, int size, float& gra
 template <int PAD, bool AC>
 __global__ void __launch_bounds__(128) warp_bwd_kernel(const float* __restrict__ frame, const float* __restrict__ flow,
                                                        const float* __restrict__ d_out, float* __restrict__ d_frame,
-                                                       float* __restrict__ d_flow, int C, int H, int W, Steps st) {
+                                                       float* __restrict__ d_flow, int C, int H, int W, FlowMul fm) {
     const int j = blockIdx.x * blockDim.x + threadIdx.x, i = blockIdx.y, b = blockIdx.z;
     if (j >= W) return;
     const int HW = H * W;                                  // launch guard: H*W < 2^30
     const int off = i * W + j;
     const float* fxp = flow + (size_t)(b * 2) * HW;
-    const float gx = __fadd_rn(linspace_m1_p1(j, W, st.step_x), __fmul_rn(__ldg(fxp + off), st.mul_x));
-    const float gy = __fadd_rn(linspace_m1_p1(i, H, st.step_y), __fmul_rn(__ldg(fxp + HW + off), st.mul_y));
+    const float gx = warp_grid_coord(__ldg(fxp + off), j, W, fm.step_x, fm.x);
+    const float gy = warp_grid_coord(__ldg(fxp + HW + off), i, H, fm.step_y, fm.y);
     float gmx, gmy;
     const float ix = source_index_grad<PAD, AC>(gx, W, gmx);
     const float iy = source_index_grad<PAD, AC>(gy, H, gmy);
-    const float x0f = floorf(ix), y0f = floorf(iy);
-    const float wx1 = ix - x0f, wx0 = (x0f + 1.0f) - ix;
-    const float wy1 = iy - y0f, wy0 = (y0f + 1.0f) - iy;
-    // clamp before the int conversion: zeros padding can leave coordinates far outside; NaN samples nothing
-    const int x0 = (int)fminf(fmaxf(x0f, -2.0f), (float)W + 1.0f), y0 = (int)fminf(fmaxf(y0f, -2.0f), (float)H + 1.0f);
-    const bool fin = x0f == x0f && y0f == y0f;
-    const bool inx0 = fin && x0 >= 0 && x0 < W, inx1 = fin && x0 + 1 >= 0 && x0 + 1 < W;
-    const bool iny0 = y0 >= 0 && y0 < H, iny1 = y0 + 1 >= 0 && y0 + 1 < H;
-    const bool i00 = iny0 && inx0, i01 = iny0 && inx1, i10 = iny1 && inx0, i11 = iny1 && inx1;
-    const float w00 = wx0 * wy0, w01 = wx1 * wy0, w10 = wx0 * wy1, w11 = wx1 * wy1;
-    const int o = y0 * W + x0;
+    // the zeros form whatever the padding: the clip above can leave NaN, which has no tap in bounds
+    const BilinearTaps t = bilinear_taps<OFB_PAD_ZEROS>(ix, iy, H, W);
+    const float wx0 = t.wx0, wx1 = t.wx1, wy0 = t.wy0, wy1 = t.wy1;
+    const bool i00 = t.inb & 1u, i01 = t.inb & 2u, i10 = t.inb & 4u, i11 = t.inb & 8u;
+    const int o = t.y0 * W + t.x0;
     float gix = 0.0f, giy = 0.0f;
     for (int c = 0; c < C; ++c) {
         const size_t plane = (size_t)(b * C + c) * HW;
         const float g = __ldg(d_out + plane + off);
         if (d_frame) {
             float* p = d_frame + plane + o;
-            if (i00) atomicAdd(p, w00 * g);
-            if (i01) atomicAdd(p + 1, w01 * g);
-            if (i10) atomicAdd(p + W, w10 * g);
-            if (i11) atomicAdd(p + W + 1, w11 * g);
+            if (i00) atomicAdd(p, t.w00 * g);
+            if (i01) atomicAdd(p + 1, t.w01 * g);
+            if (i10) atomicAdd(p + W, t.w10 * g);
+            if (i11) atomicAdd(p + W + 1, t.w11 * g);
         }
         if (d_flow) {
             const float* p = frame + plane + o;
@@ -101,16 +75,16 @@ __global__ void __launch_bounds__(128) warp_bwd_kernel(const float* __restrict__
     }
     if (d_flow) {
         float* dp = d_flow + (size_t)(b * 2) * HW + off;
-        dp[0] = st.mul_x * (gmx * gix);
-        dp[HW] = st.mul_y * (gmy * giy);
+        dp[0] = fm.x * (gmx * gix);
+        dp[HW] = fm.y * (gmy * giy);
     }
 }
 
 template <int PAD, bool AC>
 int launch(const float* frame, const float* flow, const float* d_out, float* d_frame, float* d_flow, int B, int C, int H,
-           int W, Steps st, cudaStream_t stream) {
+           int W, const FlowMul& fm, cudaStream_t stream) {
     const dim3 grid((W + 127) / 128, H, B);
-    warp_bwd_kernel<PAD, AC><<<grid, 128, 0, stream>>>(frame, flow, d_out, d_frame, d_flow, C, H, W, st);
+    warp_bwd_kernel<PAD, AC><<<grid, 128, 0, stream>>>(frame, flow, d_out, d_frame, d_flow, C, H, W, fm);
     OFB_LAUNCH_CHECK();
     return OFB_OK;
 }
@@ -126,17 +100,8 @@ OFB_API int ofb_warp_backward_f32(const float* frame, const float* flow, const f
     if ((size_t)B * H * W == 0 || (!d_frame_or_null && !d_flow_or_null)) return OFB_OK;
     if (B > 65535 || H > 65535 || (long long)H * W >= (1LL << 30) || (long long)B * (C > 2 ? C : 2) * H * W >= (1LL << 40))
         return OFB_EUNSUPPORTED;
-    const Steps st{flow_mul_x, flow_mul_y, ofb::linspace_step(W), ofb::linspace_step(H)};
-    cudaStream_t s = (cudaStream_t)stream;
-#define OFB_CASE(P, A)                            \
-    if (padding_mode == P && (align_corners != 0) == A) \
-        return launch<P, A>(frame, flow, d_out, d_frame_or_null, d_flow_or_null, B, C, H, W, st, s);
-    OFB_CASE(OFB_PAD_ZEROS, false)
-    OFB_CASE(OFB_PAD_ZEROS, true)
-    OFB_CASE(OFB_PAD_BORDER, false)
-    OFB_CASE(OFB_PAD_BORDER, true)
-    OFB_CASE(OFB_PAD_REFLECTION, false)
-    OFB_CASE(OFB_PAD_REFLECTION, true)
-#undef OFB_CASE
-    return OFB_EINVAL;
+    const ofb::FlowMul fm{flow_mul_x, flow_mul_y, ofb::linspace_step(W), ofb::linspace_step(H)};
+    return ofb_dispatch_pad_ac(padding_mode, align_corners != 0, [&](auto P, auto A) {
+        return launch<P, A>(frame, flow, d_out, d_frame_or_null, d_flow_or_null, B, C, H, W, fm, (cudaStream_t)stream);
+    });
 }

@@ -28,10 +28,6 @@ constexpr int PLANE = PLANE_BYTES / 4;
 constexpr int CGRP = 4;                                  // channels staged per pipeline slot
 constexpr int STAGES = 2;
 
-struct FlowMul2 {
-    float x, y;
-};
-
 struct TileCoord {
     int b, tile_x, tile_y;
 };
@@ -53,12 +49,11 @@ __global__ void __launch_bounds__(NT + 32, 3) warp_tma_kernel(const __grid_const
                                                               const float* __restrict__ frame,
                                                               const float* __restrict__ flow, float* __restrict__ out,
                                                               uint8_t* __restrict__ valid, int C, int H, int W, int ntx,
-                                                              int nty, int ntiles, FlowMul2 fm) {
+                                                              int nty, int ntiles, FlowMul fm) {
     extern __shared__ __align__(128) float win[];    // [STAGES][cgmax][PLANE]
     __shared__ __align__(8) unsigned long long s_full[STAGES], s_empty[STAGES];
     __shared__ int s_org[STAGES][2];
     const int HW = H * W;                                  // launch guard: H*W < 2^30
-    const float step_x = linspace_step(W), step_y = linspace_step(H);
     const int cgmax = min(CGRP, C);
     const int ngrp = (C + CGRP - 1) / CGRP;
     const uint32_t stage_bytes = (uint32_t)cgmax * PLANE_BYTES;
@@ -80,13 +75,11 @@ __global__ void __launch_bounds__(NT + 32, 3) warp_tma_kernel(const __grid_const
             // the tile's displacement: where the centre pixel samples from, relative to itself
             const int ic = min(tc.tile_y + TH / 2, H - 1), jc = min(tc.tile_x + TW / 2, W - 1);
             const float* fxp = flow + (size_t)(tc.b * 2) * HW;
-            const float fx = __ldg(fxp + ic * W + jc), fy = __ldg(fxp + HW + ic * W + jc);
-            const float gx = __fadd_rn(linspace_m1_p1(jc, W, step_x), __fmul_rn(fx, fm.x));
-            const float gy = __fadd_rn(linspace_m1_p1(ic, H, step_y), __fmul_rn(fy, fm.y));
-            const float sx = source_index<PAD, AC>(gx, W), sy = source_index<PAD, AC>(gy, H);
+            const SrcPos sc =
+                warp_source<PAD, AC>(__ldg(fxp + ic * W + jc), __ldg(fxp + HW + ic * W + jc), ic, jc, H, W, fm);
             // NaN -> 0 displacement; far-out coordinates are clamped (their pixels take the fallback anyway)
-            const int dx = (int)floorf(fminf(fmaxf(sx - (float)jc, -1.0e6f), 1.0e6f));
-            const int dy = (int)floorf(fminf(fmaxf(sy - (float)ic, -1.0e6f), 1.0e6f));
+            const int dx = (int)floorf(fminf(fmaxf(sc.ix - (float)jc, -1.0e6f), 1.0e6f));
+            const int dy = (int)floorf(fminf(fmaxf(sc.iy - (float)ic, -1.0e6f), 1.0e6f));
             // measured on sm_100a: an un-swizzled fp32 box whose first in-bounds element is not 16-byte aligned
             // in global memory faults (illegal instruction), so the window starts on a multiple of 4 columns --
             // WIN_W carries the 3 spare columns
@@ -132,27 +125,19 @@ __global__ void __launch_bounds__(NT + 32, 3) warp_tma_kernel(const __grid_const
         // coordinate pipeline of this thread's 4 pixels (does not depend on the window)
         float w00[RPT], w01[RPT], w10[RPT], w11[RPT];
         int x0[RPT], y0[RPT];
-        unsigned fin = 0;                                  // bit k: fast-path eligible; bit 4+k: not NaN
+        unsigned fin = 0;                                  // bit k: pixel k's source position is finite
 #pragma unroll
         for (int k = 0; k < RPT; ++k) {
             const int i = i0 + k;
             w00[k] = w01[k] = w10[k] = w11[k] = 0.0f; x0[k] = y0[k] = 0;
             if (i >= H || j >= W) continue;
-            const float gx = __fadd_rn(linspace_m1_p1(j, W, step_x), __fmul_rn(nfx[k], fm.x));
-            const float gy = __fadd_rn(linspace_m1_p1(i, H, step_y), __fmul_rn(nfy[k], fm.y));
-            const float ix = source_index<PAD, AC>(gx, W), iy = source_index<PAD, AC>(gy, H);
-            if (valid)
-                valid[(size_t)b * HW + i * W + j] = ((gx > -1.0f) && (gy > -1.0f) && (gx < 1.0f) && (gy < 1.0f)) ? 1 : 0;
-            const float x0f = floorf(ix), y0f = floorf(iy);
-            const float wx1 = ix - x0f, wx0 = (x0f + 1.0f) - ix;
-            const float wy1 = iy - y0f, wy0 = (y0f + 1.0f) - iy;
-            w00[k] = wx0 * wy0; w01[k] = wx1 * wy0; w10[k] = wx0 * wy1; w11[k] = wx1 * wy1;
-            // clamp before the int conversion (zeros padding can leave coordinates far outside)
-            x0[k] = (int)fminf(fmaxf(x0f, -2.0f), (float)W + 1.0f);
-            y0[k] = (int)fminf(fmaxf(y0f, -2.0f), (float)H + 1.0f);
-            // finite weights only: a zero-filled tap times a NaN weight would not be the 0 the reference samples
-            if (fabsf(ix) < 1.0e9f && fabsf(iy) < 1.0e9f) fin |= 1u << k;
-            if (x0f == x0f && y0f == y0f) fin |= 16u << k;
+            const SrcPos s = warp_source<PAD, AC>(nfx[k], nfy[k], i, j, H, W, fm);
+            if (valid) valid[(size_t)b * HW + i * W + j] = s.valid ? 1 : 0;
+            const BilinearTaps tp = bilinear_taps<PAD>(s.ix, s.iy, H, W);
+            w00[k] = tp.w00; w01[k] = tp.w01; w10[k] = tp.w10; w11[k] = tp.w11;
+            x0[k] = tp.x0; y0[k] = tp.y0;
+            // a non-finite position has NaN weights, which the window's zero-filled taps must not meet
+            if (fabsf(s.ix) < 1.0e9f && fabsf(s.iy) < 1.0e9f) fin |= 1u << k;
         }
         load_flow(t + gridDim.x);                          // in flight during the gather below
 
@@ -178,20 +163,10 @@ __global__ void __launch_bounds__(NT + 32, 3) warp_tma_kernel(const __grid_const
                         op[(size_t)c * HW] = acc;
                     }
                 } else {
-                    const bool nn = (fin >> (4 + k)) & 1u;
-                    const int x1 = x0[k] + 1, y1 = y0[k] + 1;
-                    const bool inx0 = nn && x0[k] >= 0 && x0[k] < W, inx1 = nn && x1 >= 0 && x1 < W;
-                    const bool iny0 = y0[k] >= 0 && y0[k] < H, iny1 = y1 >= 0 && y1 < H;
                     const int o = y0[k] * W + x0[k];
-                    for (int c = 0; c < cg; ++c) {
-                        const float* p = frame + (size_t)(b * C + c0 + c) * HW + o;
-                        float acc = 0.0f;
-                        if (iny0 && inx0) acc = __fmaf_rn(__ldg(p), w00[k], acc);
-                        if (iny0 && inx1) acc = __fmaf_rn(__ldg(p + 1), w01[k], acc);
-                        if (iny1 && inx0) acc = __fmaf_rn(__ldg(p + W), w10[k], acc);
-                        if (iny1 && inx1) acc = __fmaf_rn(__ldg(p + W + 1), w11[k], acc);
-                        op[(size_t)c * HW] = acc;
-                    }
+                    for (int c = 0; c < cg; ++c)
+                        op[(size_t)c * HW] = gather4(frame + (size_t)(b * C + c0 + c) * HW + o, 1, W,
+                                                     tap_mask<PAD>(x0[k], y0[k], H, W), w00[k], w01[k], w10[k], w11[k]);
                 }
             }
             __syncwarp();
@@ -203,7 +178,7 @@ __global__ void __launch_bounds__(NT + 32, 3) warp_tma_kernel(const __grid_const
 
 template <int PAD, bool AC>
 int launch(const CUtensorMap& map, const float* frame, const float* flow, float* out, uint8_t* valid, int B, int C,
-           int H, int W, FlowMul2 fm, cudaStream_t st) {
+           int H, int W, const FlowMul& fm, cudaStream_t st) {
     OFB_CUDA(ofb_smem_once<warp_tma_kernel<PAD, AC>>(STAGES * CGRP * PLANE_BYTES));
     const int cg = C < CGRP ? C : CGRP;
     const size_t smem = (size_t)STAGES * cg * PLANE_BYTES;
@@ -223,7 +198,7 @@ int launch(const CUtensorMap& map, const float* frame, const float* flow, float*
 // frame must be 16-byte aligned with W % 4 == 0 (TMA global strides are multiples of 16 bytes); the caller
 // (warp.cu) checks that and the 32-bit offset limits.
 int ofb_warp_tma_launch(const float* frame, const float* flow, float* out, uint8_t* valid, int B, int C, int H, int W,
-                        int pad, int ac, float fmx, float fmy, cudaStream_t st) {
+                        int pad, int ac, const ofb::FlowMul& fm, cudaStream_t st) {
     CUtensorMap map;
     const cuuint64_t gdim[3] = {(cuuint64_t)W, (cuuint64_t)H, (cuuint64_t)B * C};
     const cuuint64_t gstr[2] = {(cuuint64_t)W * 4, (cuuint64_t)W * H * 4};
@@ -231,15 +206,7 @@ int ofb_warp_tma_launch(const float* frame, const float* flow, float* out, uint8
     if (!encode_tiled(&map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 3, frame, gdim, gstr, box, CU_TENSOR_MAP_SWIZZLE_NONE,
                       CU_TENSOR_MAP_L2_PROMOTION_L2_128B))
         return OFB_EDRIVER;
-    const FlowMul2 fm{fmx, fmy};
-#define OFB_CASE(P, A) \
-    if (pad == P && ac == (A ? 1 : 0)) return launch<P, A>(map, frame, flow, out, valid, B, C, H, W, fm, st);
-    OFB_CASE(OFB_PAD_ZEROS, false)
-    OFB_CASE(OFB_PAD_ZEROS, true)
-    OFB_CASE(OFB_PAD_BORDER, false)
-    OFB_CASE(OFB_PAD_BORDER, true)
-    OFB_CASE(OFB_PAD_REFLECTION, false)
-    OFB_CASE(OFB_PAD_REFLECTION, true)
-#undef OFB_CASE
-    return OFB_EINVAL;
+    return ofb_dispatch_pad_ac(pad, ac, [&](auto P, auto A) {
+        return launch<P, A>(map, frame, flow, out, valid, B, C, H, W, fm, st);
+    });
 }
