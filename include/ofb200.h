@@ -300,6 +300,18 @@ int ofb_corr_lookup(const ofb_pyramid* pyr_host, const float* coords, float* out
 int ofb_corr_lookup_backward_f32(const ofb_pyramid* d_pyr, const float* coords, const float* d_out,
                                  int B, int h, int w, int radius, void* stream);
 
+/* Backward of ofb_corr_lookup with respect to the coordinates: what autograd computes for coords through
+ * CorrBlock.__call__ (methods/raft/model/corr.py:56-77) and bilinear_sampler = grid_sample(align_corners=True, zeros
+ * padding) (methods/raft/model/utils.py:64-80), ATen's d grid with the normalise / un-normalise chain factors applied
+ * as exactly 1.  pyr: the STORED pyramid the forward read (every dtype and layout ofb_corr_lookup accepts, same argument
+ * checks); d_out (B, L*(2r+1)^2, h, w) fp32; d_coords (B,2,h,w) fp32 is OVERWRITTEN.  Taps on the floors and weights of
+ * the forward (integer coordinates: the one-sided derivative the reference's fp32 floor picks).  Taps outside the
+ * image read 0; a level with a tap outside the floor guard, a non-finite or far coordinate, or a width or height of 1,
+ * contributes 0 (ATen: NaN for NaN coordinates).  Row padding is never read into the result.  Deterministic: the same
+ * bits on every run. */
+int ofb_corr_lookup_coords_backward(const ofb_pyramid* pyr, const float* coords, const float* d_out, float* d_coords,
+                                    int B, int h, int w, int radius, void* stream);
+
 /* The two GEMMs behind d CorrBlock / d fmap (autograd through corr.py:45-54,79-87), on the tensor cores:
  *   D[b] (M x N, fp32, row pitch ldd) = alpha * A[b] (M x K) . B[b]^T (N x K)  (+ D[b] when accumulate != 0)
  * A, B bf16, K-major (row pitches lda, ldb and batch strides in elements, multiples of 8); N a multiple of 32,

@@ -5,6 +5,7 @@
 #include <cuda_fp16.h>
 #include <stdint.h>
 
+#include <climits>
 #include <type_traits>
 
 #include "../../include/ofb200.h"
@@ -232,8 +233,12 @@ __device__ __forceinline__ float gather4(const float* p, size_t dx, size_t dy, c
 //     g  = 2*x/(size-1) - 1                  (utils.py:70-71)
 //     ix = ((g + 1) * 0.5) * (size-1)        (ATen GridSampler.h:30, align_corners=True; (g+1)/2 == (g+1)*0.5 exactly)
 //     fl = floor(ix); valid = -1 < g < 1     (utils.py:77)
-// Every lookup kernel (forward, backward, on-demand) takes its taps from here; each decides what an out-of-guard tap
-// contributes.
+// Every lookup kernel (forward, backward, coordinate backward, on-demand) takes its taps from here; each decides what an
+// out-of-guard tap contributes.
+// The coordinate backward (lookup_coords_bwd.cu) differentiates the samples of these taps as ATen's GridSampler backward
+// does (zeros padding): a tap outside the image reads the value 0; a level with a tap outside the guard -- a non-finite
+// or far coordinate, or a level of width or height 1 (size - 1 = 0) -- contributes exactly 0 (ATen: NaN for a NaN
+// coordinate); elements between w_l and the row pitch never reach the result.
 struct LookupTap {
     float fl;          // floor of the un-normalised coordinate (what the idx output reports)
     float w0, w1;      // bilinear weights of columns fl and fl + 1
@@ -295,6 +300,50 @@ __device__ __forceinline__ WarpWindow warp_window(float cx0, float cy0, float in
     return w;
 }
 
+// One axis of a (query, level) window for the kernels that stream it row by row (the register-tile forward lookup and
+// the coordinate backward).  Within the guarded coordinate range every tap's floor index is t + anchor + {0, 1} (the
+// fp32 round trip can move a tap sitting on an integer to the pixel below), so tap t reads window positions t + d[t]
+// and t + d[t] + 1 of a D + 2 element window starting at the anchor.
+template <int R>
+struct TapSet {
+    static constexpr int D = 2 * R + 1;
+    float w0[D], w1[D];
+    int anchor;          // min over taps of (floor index - tap number); tap t reads anchor + t + d[t]
+    unsigned dmask;      // bit t = d[t]
+    unsigned vmask;      // bit t = utils.py:77 predicate
+    bool dead;           // some tap outside the guarded range: every in-range tap is outside the image
+};
+
+template <int R>
+__device__ __forceinline__ TapSet<R> make_taps(float center, int size, int32_t* idx_dst) {
+    constexpr int D = 2 * R + 1;
+    TapSet<R> ts;
+    int i0[D];
+    ts.dead = false;
+    ts.vmask = 0;
+    int anchor = INT_MAX;
+#pragma unroll
+    for (int t = 0; t < D; ++t) {
+        const LookupTap tp = lookup_tap(center, t, R, size);
+        ts.w1[t] = tp.w1;
+        ts.w0[t] = tp.w0;
+        ts.dead |= !tp.in_guard;
+        i0[t] = tp.in_guard ? (int)tp.fl : 0;
+        if (idx_dst) idx_dst[t] = (int32_t)tp.fl;
+        ts.vmask |= tp.valid ? (1u << t) : 0u;
+        anchor = min(anchor, i0[t] - t);
+    }
+    ts.anchor = anchor;
+    ts.dmask = 0;
+#pragma unroll
+    for (int t = 0; t < D; ++t) {
+        const int d = i0[t] - t - anchor;           // 0 or 1 unless dead
+        ts.dmask |= (d != 0) ? (1u << t) : 0u;
+        ts.dead |= (d > 1);
+    }
+    return ts;
+}
+
 __device__ __forceinline__ float bilinear(float v00, float v01, float v10, float v11, float wx0, float wx1, float wy0,
                                           float wy1) {
     float acc = __fmul_rn(v00, __fmul_rn(wx0, wy0));
@@ -348,6 +397,55 @@ template <> __device__ __forceinline__ float widen16<__nv_bfloat16>(unsigned wd,
 template <> __device__ __forceinline__ float widen16<__half>(unsigned wd, int hi) {
     return __half2float(__ushort_as_half((unsigned short)(hi ? (wd >> 16) : (wd & 0xffffu))));
 }
+
+// One window row of a 16-bit pyramid from its aligned chunk loads: w[0..7] are the 8-element (16-byte) chunks at
+// xa and xa + 8, w[8..9] the first 4 elements at xa + 16, as packed pairs.  px receives elements s .. s + WIN - 1
+// (s = xs - xa in 0..7, passed as q1 = bit 1, q2 = bit 2 and hs = 16 * bit 0) widened to fp32: word shifts by 1 and
+// 2, then a half-word funnel shift.
+template <typename T, int WIN>
+__device__ __forceinline__ void realign_row(const uint32_t (&w)[10], unsigned q1, unsigned q2, unsigned hs,
+                                            float (&px)[WIN]) {
+    constexpr int NW = (WIN + 1) / 2;                           // packed words per realigned row (6 for WIN = 11)
+    uint32_t t1[9], t2[NW + 1], v[NW];
+#pragma unroll
+    for (int k = 0; k < 9; ++k) t1[k] = q1 ? w[k + 1] : w[k];
+#pragma unroll
+    for (int k = 0; k <= NW; ++k) t2[k] = q2 ? t1[k + 2] : t1[k];
+#pragma unroll
+    for (int k = 0; k < NW; ++k) v[k] = __funnelshift_r(t2[k], t2[k + 1], hs);
+#pragma unroll
+    for (int e = 0; e < WIN; ++e) px[e] = widen16<T>(v[e >> 1], e & 1);
+}
+
+// The aligned 8-element (16-byte) chunks holding window columns xs .. xs + cols - 1 of a 16-bit level whose row pitch
+// is a multiple of 8 (the register-tile forward lookup and the coordinate backward read window rows this way): chunks
+// at xa, xa + 8 and xa + 16, of the last only the first 4 elements (s + cols - 1 <= 17).  ck0 .. ck2: the chunk lies
+// inside the row (ck2 only when it holds a window column); q1, q2, hs: realign_row's shift of s.
+struct RowChunks {
+    int xa, s;
+    unsigned q1, q2, hs;
+    bool ck0, ck1, ck2;
+};
+__device__ __forceinline__ RowChunks row_chunks(int xs, int cols, int pitch) {
+    RowChunks c;
+    c.xa = xs & ~7;
+    c.s = xs - c.xa;                                            // s in 0..7
+    c.q1 = (unsigned)(c.s >> 1) & 1u;
+    c.q2 = (unsigned)(c.s >> 2) & 1u;
+    c.hs = (unsigned)(c.s & 1) * 16u;
+    c.ck0 = c.xa >= 0 && c.xa + 8 <= pitch;
+    c.ck1 = c.xa + 8 >= 0 && c.xa + 16 <= pitch;
+    c.ck2 = (c.s + cols > 16) && c.xa + 16 >= 0 && c.xa + 24 <= pitch;
+    return c;
+}
+// Chunk xa of window row y: one row of an 8x4 block (P.blocked; the next chunk is P.blk_stride elements further) or 8
+// consecutive elements of a padded row (the next chunk 8 further, OFB_CHUNK_STEP).  P: the kernel's parameter block.
+// Macros rather than functions: the register-tile forward's code must stay what it was (as inline functions they change
+// its instruction schedule).
+#define OFB_CHUNK_ROW(slice, y, xa, pitch, P)                                                       \
+    ((P).blocked ? (slice) + ((long long)((y) >> 2) * ((pitch) >> 3) + ((xa) >> 3)) * (P).blk_stride + ((y) & 3) * 8 \
+                 : (slice) + (long long)(y) * (pitch) + (xa))
+#define OFB_CHUNK_STEP(P) ((P).blocked ? (P).blk_stride : 8)
 
 __device__ __forceinline__ float warp_sum(float v) {
 #pragma unroll

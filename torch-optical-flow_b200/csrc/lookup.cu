@@ -16,8 +16,6 @@
 //   3. produces the (2r+1)^2 samples, 3 per lane (ofb::warp_window_samples).
 // Results are staged in a [channel][query] shared tile so the global writes are 128-byte rows.
 // HBM roofline per query and iteration (SURVEY.md 8d): L*(2r+2)^2*esize + 8 read, 4*L*(2r+1)^2 written.
-#include <climits>
-
 #include "common.cuh"
 
 namespace {
@@ -148,45 +146,8 @@ __global__ void __launch_bounds__(NW * 32) lookup_kernel(const LookupParams P, c
 // No shared memory, no shuffles, ~56 warp instructions per (query, level) against ~230 before.
 // Contract with the builder: elements between w_l and the row pitch hold FINITE values (the tcgen05
 // builder writes zeros there); they are multiplied by zero weights.
-template <int R>
-struct TapSet {
-    static constexpr int D = 2 * R + 1;
-    float w0[D], w1[D];
-    int anchor;          // min over taps of (floor index - tap number); tap t reads anchor + t + d[t]
-    unsigned dmask;      // bit t = d[t]
-    unsigned vmask;      // bit t = utils.py:77 predicate
-    bool dead;           // some tap outside the guarded range: every in-range tap is outside the image
-};
-
-template <int R>
-__device__ __forceinline__ TapSet<R> make_taps(float center, int size, int32_t* idx_dst) {
-    constexpr int D = 2 * R + 1;
-    TapSet<R> ts;
-    int i0[D];
-    ts.dead = false;
-    ts.vmask = 0;
-    int anchor = INT_MAX;
-#pragma unroll
-    for (int t = 0; t < D; ++t) {
-        const ofb::LookupTap tp = ofb::lookup_tap(center, t, R, size);
-        ts.w1[t] = tp.w1;
-        ts.w0[t] = tp.w0;
-        ts.dead |= !tp.in_guard;
-        i0[t] = tp.in_guard ? (int)tp.fl : 0;
-        if (idx_dst) idx_dst[t] = (int32_t)tp.fl;
-        ts.vmask |= tp.valid ? (1u << t) : 0u;
-        anchor = min(anchor, i0[t] - t);
-    }
-    ts.anchor = anchor;
-    ts.dmask = 0;
-#pragma unroll
-    for (int t = 0; t < D; ++t) {
-        const int d = i0[t] - t - anchor;           // 0 or 1 unless dead
-        ts.dmask |= (d != 0) ? (1u << t) : 0u;
-        ts.dead |= (d > 1);
-    }
-    return ts;
-}
+using ofb::TapSet;
+using ofb::make_taps;
 
 // T: the pyramid's 16-bit type.  Only the widening of the realigned words depends on it: the coordinates, floor
 // indices, validity masks and filter weights are the same code for both types.
@@ -195,7 +156,6 @@ __global__ void __launch_bounds__(128) lookup_tile_kernel(const LookupParams P, 
                                                            float* __restrict__ out, int32_t* __restrict__ idx_out,
                                                            uint8_t* __restrict__ valid_out) {
     constexpr int D = 2 * R + 1, DD = D * D, WIN = D + 2;       // window rows / columns
-    constexpr int NW = (WIN + 1) / 2;                           // packed words per realigned row (6 for R = 4)
     const int l = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const long long HW = (long long)P.h * P.w, Q = (long long)P.B * HW;
     const long long q = (long long)blockIdx.x * 32 + lane;
@@ -232,14 +192,10 @@ __global__ void __launch_bounds__(128) lookup_tile_kernel(const LookupParams P, 
         fw[i][0] = a0; fw[i][1] = a1; fw[i][2] = a2;
     }
 
-    // chunk geometry: 8-element (16-byte) aligned chunks covering columns xs .. xs + WIN - 1
-    const int xa = xs & ~7, s = xs - xa;                        // s in 0..7
-    const unsigned q1 = (unsigned)(s >> 1) & 1u, q2 = (unsigned)(s >> 2) & 1u, hs = (unsigned)(s & 1) * 16u;
-    const bool ck0 = xa >= 0 && xa + 8 <= pitch;
-    const bool ck1 = xa + 8 >= 0 && xa + 16 <= pitch;
     // the last window column / row only carries weight when some tap slid by one (dmask != 0)
     const int wcols = tx.dmask ? WIN : WIN - 1, wrows = ty.dmask ? WIN : WIN - 1;
-    const bool ck2 = (s + wcols > 16) && xa + 16 >= 0 && xa + 24 <= pitch;
+    // chunk geometry: 8-element (16-byte) aligned chunks covering columns xs .. xs + wcols - 1
+    const ofb::RowChunks ck = ofb::row_chunks(xs, wcols, pitch);
     const T* slice = reinterpret_cast<const T*>(P.base[l]) + q * P.q_stride[l];
     float* outp = out + (b * (long long)(P.levels * DD) + (long long)l * DD) * HW + p;
 
@@ -261,24 +217,21 @@ __global__ void __launch_bounds__(128) lookup_tile_kernel(const LookupParams P, 
     const uint32_t my_slot2 = smem0 + (uint32_t)(WIN * 2) * slot_stride + threadIdx.x * 8u;
     const uint32_t slot2_stride = blockDim.x * 8u;
     {
-        const long long cstep = P.blocked ? P.blk_stride : 8;
+        const long long cstep = OFB_CHUNK_STEP(P);
 #pragma unroll
         for (int r = 0; r < WIN; ++r) {
             const int y = ys + r;
             const bool rok = !dead && r < wrows && y >= 0 && y < Hl;
-            // an aligned 8-element chunk is one row of an 8x4 block (blocked) or 8 consecutive row elements
-            const T* row = P.blocked
-                ? slice + ((long long)(y >> 2) * (pitch >> 3) + (xa >> 3)) * P.blk_stride + (y & 3) * 8
-                : slice + (long long)y * pitch + xa;
+            const T* row = OFB_CHUNK_ROW(slice, y, ck.xa, pitch, P);
 #pragma unroll
             for (int c = 0; c < 2; ++c) {
-                const bool ok = rok && (c == 0 ? ck0 : ck1);
+                const bool ok = rok && (c == 0 ? ck.ck0 : ck.ck1);
                 const void* src = ok ? (const void*)(row + c * cstep) : (const void*)slice;
                 asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(my_slot + (uint32_t)(r * 2 + c) * slot_stride),
                              "l"(src), "r"(ok ? 16 : 0) : "memory");
             }
             {
-                const bool ok = rok && ck2;
+                const bool ok = rok && ck.ck2;
                 const void* src = ok ? (const void*)(row + 2 * cstep) : (const void*)slice;
                 asm volatile("cp.async.ca.shared.global [%0], [%1], 8, %2;" ::"r"(my_slot2 + (uint32_t)r * slot2_stride),
                              "l"(src), "r"(ok ? 8 : 0) : "memory");
@@ -304,17 +257,8 @@ __global__ void __launch_bounds__(128) lookup_tile_kernel(const LookupParams P, 
                          : "=r"(w[4 * c]), "=r"(w[4 * c + 1]), "=r"(w[4 * c + 2]), "=r"(w[4 * c + 3])
                          : "r"(my_slot + (uint32_t)(r * 2 + c) * slot_stride));
         asm volatile("ld.shared.v2.b32 {%0, %1}, [%2];" : "=r"(w[8]), "=r"(w[9]) : "r"(my_slot2 + (uint32_t)r * slot2_stride));
-        // ---- realign: drop s leading elements (word shifts by 1 and 2, then a half-word funnel shift)
-        uint32_t t1[9], t2[NW + 1], v[NW];
-#pragma unroll
-        for (int k = 0; k < 9; ++k) t1[k] = q1 ? w[k + 1] : w[k];
-#pragma unroll
-        for (int k = 0; k <= NW; ++k) t2[k] = q2 ? t1[k + 2] : t1[k];
-#pragma unroll
-        for (int k = 0; k < NW; ++k) v[k] = __funnelshift_r(t2[k], t2[k + 1], hs);
         float px[WIN];
-#pragma unroll
-        for (int e = 0; e < WIN; ++e) px[e] = ofb::widen16<T>(v[e >> 1], e & 1);
+        ofb::realign_row<T>(w, ck.q1, ck.q2, ck.hs, px);
         // ---- horizontal filter
         float hrow[D];
 #pragma unroll

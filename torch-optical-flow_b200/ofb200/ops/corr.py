@@ -7,8 +7,11 @@ Differences a caller can observe, all deliberate (DESIGN.md):
     pass `pyramid_dtype=torch.float16` for the precision the reference's shipped configs store it in
     (`precision: 16`: an fp16 pyramid, the same bytes and tensor-core path as bf16, 3 more significand
     bits, but correlations beyond +-65504 become inf), or `torch.float32` for an fp32 pyramid (CUDA-core builder).
-  * differentiable with respect to the feature maps (K3 backward kernel + two library GEMMs per level); the
-    lookup coordinates get no gradient (the reference's RAFT detaches them, raft.py:127).
+  * differentiable with respect to the feature maps (K3 backward kernel + two library GEMMs per level) and, as
+    bilinear_sampler's grid_sample is in the reference (utils.py:64-80), with respect to the lookup coordinates (one
+    K3 coordinate-backward launch per lookup, only when the coordinates require grad; RAFT itself detaches them,
+    raft.py:127).  A coordinate whose window leaves the floor guard, or is non-finite, gets gradient 0 at that level
+    (the reference: NaN for NaN).  Forward-only, as before: `return_index=True` lookups and `on_demand=True` blocks.
 """
 import ctypes
 import math
@@ -238,26 +241,42 @@ class _PyramidHandle(torch.autograd.Function):
 
 
 class _LookupFn(torch.autograd.Function):
-    """One CorrBlock.__call__: forward = the K3 kernel, backward = scatter into the block's gradient pyramid."""
+    """One CorrBlock.__call__: forward = the K3 kernel; backward = the coordinate gradient (when `coords_d` requires
+    grad) and the scatter into the block's gradient pyramid (when there is a handle, i.e. the feature maps require
+    grad).  The context never keeps the CorrBlock (see _GradState).  Only a lookup whose coordinates require grad keeps
+    the stored pyramid's buffers, which its backward reads: with detached coordinates the multi-GB pyramid is freed as
+    soon as the block is dropped, while the graph lives on."""
 
     @staticmethod
     def forward(ctx, block, coords_d, handle):
         ctx.state = block._grad
+        if ctx.needs_input_grad[1]:
+            ctx.pyr, ctx.buffers = block._pyr, block._buffers
+        ctx.shape, ctx.dev, ctx.radius = block._shape, block._dev, block.radius
         ctx.save_for_backward(coords_d)
-        return block._lookup(coords_d, None, None, None)
+        return block._lookup(coords_d.detach(), None, None, None)
 
     @staticmethod
     def backward(ctx, grad_out):
         st = ctx.state
         (coords_d,) = ctx.saved_tensors
-        b, c, h, w = st.shape
-        with torch.cuda.device(st.dev):
-            desc = st.grad_pyramid()
-            rc = ofb200.load().ofb_corr_lookup_backward_f32(
-                ctypes.byref(desc), ofb200.ptr(coords_d), ofb200.ptr(grad_out.contiguous()), b, h, w, st.radius,
-                ofb200.stream_ptr())
-            ofb200.check(rc, "ofb_corr_lookup_backward_f32")
-        return None, None, torch.zeros(1, dtype=torch.float32, device=st.dev)
+        b, c, h, w = ctx.shape
+        g = grad_out.contiguous()
+        d_coords = None
+        with torch.cuda.device(ctx.dev):
+            if ctx.needs_input_grad[1]:
+                d_coords = torch.empty((b, 2, h, w), dtype=torch.float32, device=ctx.dev)
+                rc = ofb200.load().ofb_corr_lookup_coords_backward(
+                    ctypes.byref(ctx.pyr), ofb200.ptr(coords_d), ofb200.ptr(g), ofb200.ptr(d_coords), b, h, w, ctx.radius,
+                    ofb200.stream_ptr())
+                ofb200.check(rc, "ofb_corr_lookup_coords_backward")
+            if st is not None:
+                desc = st.grad_pyramid()
+                rc = ofb200.load().ofb_corr_lookup_backward_f32(
+                    ctypes.byref(desc), ofb200.ptr(coords_d), ofb200.ptr(g), b, h, w, st.radius, ofb200.stream_ptr())
+                ofb200.check(rc, "ofb_corr_lookup_backward_f32")
+        handle_grad = torch.zeros(1, dtype=torch.float32, device=ctx.dev) if st is not None else None
+        return None, d_coords, handle_grad
 
 
 class CorrBlock:
@@ -423,16 +442,23 @@ class CorrBlock:
     def __call__(self, coords: Tensor, return_index: bool = False, out: Optional[Tensor] = None):
         """Index the pyramid (reference corr.py:56-77): coords (B, 2, h, w) -> (B, L*(2r+1)^2, h, w) fp32.
 
-        `return_index=True` (extension) also returns the floor indices (B*h*w, L, 2, 2r+1) int32 and
-        the validity mask (B*h*w, L, (2r+1)^2) uint8 the kernel used.  `out` (extension) is an
-        optional preallocated contiguous fp32 CUDA tensor of the output shape."""
+        Differentiable with respect to `coords` when they require grad (host coordinates get a host gradient) and to
+        the feature maps when those did at construction.  `return_index=True` (extension) also returns the floor
+        indices (B*h*w, L, 2, 2r+1) int32 and the validity mask (B*h*w, L, (2r+1)^2) uint8 the kernel used; such a
+        call, and every lookup of an `on_demand=True` block, is forward-only: its output carries no gradient.  `out`
+        (extension) is an optional preallocated contiguous fp32 CUDA tensor of the output shape; on the
+        differentiable path it receives the values and the returned tensor carries the graph."""
         b, c, h, w = self._shape
         if tuple(coords.shape) != (b, 2, h, w):
             raise RuntimeError(f"CorrBlock: coords must be {(b, 2, h, w)}, got {tuple(coords.shape)}")
         if coords.dtype != torch.float32:
             raise NotImplementedError("CorrBlock: coords must be fp32")
         on_host = not coords.is_cuda
-        coords_d = ofb200.to_device(coords).detach().contiguous()
+        diff_coords = (torch.is_grad_enabled() and coords.requires_grad and not return_index
+                       and self._on_demand is None)
+        coords_d = ofb200.to_device(coords).contiguous()           # differentiable: a host leaf gets a host gradient
+        if not diff_coords:
+            coords_d = coords_d.detach()
         d = 2 * self.radius + 1
         lvls = self.num_levels
         oshape = (b, lvls * d * d, h, w)
@@ -440,7 +466,7 @@ class CorrBlock:
                                 or not out.is_contiguous()):
             raise RuntimeError(f"CorrBlock: out must be a contiguous fp32 CUDA tensor of shape {oshape}")
         idx = valid = None
-        if self._handle is not None and torch.is_grad_enabled() and not return_index:
+        if diff_coords or (self._handle is not None and torch.is_grad_enabled() and not return_index):
             res = _LookupFn.apply(self, coords_d, self._handle)
             if out is not None:
                 out.copy_(res.detach())                       # the preallocated buffer is filled, the graph keeps `res`
