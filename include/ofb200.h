@@ -186,6 +186,11 @@ int ofb_sequence_loss_backward_f32(const float* const* preds, float* const* d_pr
  * The tensor-core builder needs mode 1, 2 or 3 and writes whole 8-element pieces, i.e. zeros into the
  * padding columns; the 16-bit lookup kernel relies on padding columns holding finite values.
  * The blocked layouts are 16-bit layouts: bf16 or fp16 pyramids, not fp32 ones.
+ * Every entry point that takes an ofb_pyramid checks it in one place (ofb::check_pyramid, csrc/common.cuh) and
+ * returns OFB_EINVAL when levels is outside 1..OFB_MAX_LEVELS, dtype or layout is not one of the values below, a
+ * level has a null base, a non-positive size or row_pitch < lvl_w, or a query-minor level has q_stride != 32; each
+ * then adds only its own requirements.  ofb_corr_lookup and ofb_corr_lookup_coords_backward pick their reader in one
+ * place too (ofb::lookup_reader), so they accept the same pyramids.
  * ------------------------------------------------------------------------------------- */
 #define OFB_LAYOUT_ROWS 0
 #define OFB_LAYOUT_BLOCK8X4 1
@@ -303,7 +308,7 @@ int ofb_corr_lookup_backward_f32(const ofb_pyramid* d_pyr, const float* coords, 
 /* Backward of ofb_corr_lookup with respect to the coordinates: what autograd computes for coords through
  * CorrBlock.__call__ (methods/raft/model/corr.py:56-77) and bilinear_sampler = grid_sample(align_corners=True, zeros
  * padding) (methods/raft/model/utils.py:64-80), ATen's d grid with the normalise / un-normalise chain factors applied
- * as exactly 1.  pyr: the STORED pyramid the forward read (every dtype and layout ofb_corr_lookup accepts, same argument
+ * as exactly 1.  pyr: the STORED pyramid the forward read (exactly the pyramids ofb_corr_lookup accepts, same argument
  * checks); d_out (B, L*(2r+1)^2, h, w) fp32; d_coords (B,2,h,w) fp32 is OVERWRITTEN.  Taps on the floors and weights of
  * the forward (integer coordinates: the one-sided derivative the reference's fp32 floor picks).  Taps outside the
  * image read 0; a level with a tap outside the floor guard, a non-finite or far coordinate, or a width or height of 1,

@@ -273,6 +273,7 @@ def _fp16_pyramid(levels, layout, pad_value=6.0e4):
     """Device fp16 pyramid of the given fp32 levels (fp16-representable) in `layout`; padding holds a large finite value
     (the lookup contract), so a padding element that leaked into a sample would show."""
     import ofb200
+    from ofb200.ops.corr import level_buffer
 
     q = levels[0].shape[0]
     pyr = ofb200.Pyramid()
@@ -282,18 +283,10 @@ def _fp16_pyramid(levels, layout, pad_value=6.0e4):
     bufs = []
     for l, lv in enumerate(levels):
         hl, wl = lv.shape[-2:]
-        if layout == "rows":
-            pitch, rows = (wl + 15) & ~15, hl
-        else:
-            pitch, rows = (wl + 7) & ~7, (hl + 3) & ~3
+        pitch, rows = ((wl + 15) & ~15, hl) if layout == "rows" else ((wl + 7) & ~7, (hl + 3) & ~3)
         img = torch.full((q, rows, pitch), pad_value, dtype=torch.float16, device="cuda")
         img[:, :hl, :wl] = T(lv[:, 0]).half()
-        if layout == "qminor":
-            buf = img.view(q, rows // 4, 4, pitch // 8, 8).permute(1, 3, 0, 2, 4).contiguous()
-        elif layout == "blocked":
-            buf = img.view(q, rows // 4, 4, pitch // 8, 8).permute(0, 1, 3, 2, 4).contiguous()
-        else:
-            buf = img
+        buf = level_buffer(img, pyr.layout)
         bufs.append(buf)
         pyr.base[l] = buf.data_ptr()
         pyr.q_stride[l] = 32 if layout == "qminor" else rows * pitch

@@ -1067,43 +1067,27 @@ def test_epe_vs_oracle(shape):
 def _pyramid_from_numpy(levels, dtype, blocked=False):
     """Wrap oracle-built fp32 levels into a CorrBlock-like object that owns padded device buffers
     (padded rows, or the 8x4-blocked layout of include/ofb200.h)."""
-    import ctypes
-
     import ofb200
+    from ofb200.ops.corr import level_buffer
 
-    q, _, h0, w0 = levels[0].shape
+    q = levels[0].shape[0]
     pyr = ofb200.Pyramid()
     pyr.levels = len(levels)
     pyr.dtype = ofb200.DTYPE_BF16 if dtype == torch.bfloat16 else ofb200.DTYPE_F32
     pyr.layout = (ofb200.LAYOUT_QMINOR8X4 if blocked == "qminor" else ofb200.LAYOUT_BLOCK8X4) if blocked else ofb200.LAYOUT_ROWS
+    # fp32 rows kernel: pads must never be read (NaN).  bf16 register-tile kernel: pads may be read but must
+    # not reach the output -- the contract is "finite", so poison them with a huge finite value
+    poison = float("nan") if dtype == torch.float32 and not blocked else 3.0e38
     bufs = []
     for l, lv in enumerate(levels):
         hl, wl = lv.shape[-2:]
-        pitch = (wl + 15) & ~15
-        if blocked:
-            pitch = (wl + 7) & ~7
-            rows = (hl + 3) & ~3
-            img = torch.full((q, rows, pitch), 3.0e38, dtype=dtype, device="cuda")
-            img[:, :hl, :wl] = T(lv[:, 0]).to(dtype)
-            if blocked == "qminor":
-                buf = img.view(q, rows // 4, 4, pitch // 8, 8).permute(1, 3, 0, 2, 4).contiguous()   # (by, bx, q, y, x)
-            else:
-                buf = img.view(q, rows // 4, 4, pitch // 8, 8).permute(0, 1, 3, 2, 4).contiguous()   # (q, by, bx, y, x)
-            bufs.append(buf)
-            pyr.base[l] = buf.data_ptr()
-            pyr.q_stride[l] = 32 if blocked == "qminor" else rows * pitch
-            pyr.row_pitch[l] = pitch
-            pyr.lvl_h[l] = hl
-            pyr.lvl_w[l] = wl
-            continue
-        # fp32 kernel: pads must never be read (NaN).  bf16 register-tile kernel: pads may be read but must
-        # not reach the output -- the contract is "finite", so poison them with a huge finite value
-        poison = float("nan") if dtype == torch.float32 else 3.0e38
-        buf = torch.full((q, hl, pitch), poison, dtype=dtype, device="cuda")
-        buf[:, :, :wl] = T(lv[:, 0]).to(dtype)
+        pitch, rows = ((wl + 7) & ~7, (hl + 3) & ~3) if blocked else ((wl + 15) & ~15, hl)
+        img = torch.full((q, rows, pitch), poison, dtype=dtype, device="cuda")
+        img[:, :hl, :wl] = T(lv[:, 0]).to(dtype)
+        buf = level_buffer(img, pyr.layout)
         bufs.append(buf)
         pyr.base[l] = buf.data_ptr()
-        pyr.q_stride[l] = hl * pitch
+        pyr.q_stride[l] = 32 if blocked == "qminor" else rows * pitch
         pyr.row_pitch[l] = pitch
         pyr.lvl_h[l] = hl
         pyr.lvl_w[l] = wl

@@ -339,6 +339,67 @@ def test_lookup_backward_validates_arguments_without_launch(lib):
     assert call(p) == OFB_EINVAL
 
 
+def test_pyramid_descriptor_checks_agree_without_launch(lib):
+    """A descriptor that breaks a rule every user relies on is OFB_EINVAL at all five pyramid entry points; and the
+    forward lookup and its coordinate backward give the same code for every layout, dtype, radius 0-4 and descriptor
+    variant.  B * h * w = 2^36 queries is too many for either launch, so a descriptor both readers accept is refused
+    only there (OFB_EUNSUPPORTED) and nothing is launched."""
+    import ofb200
+
+    fake = ctypes.c_void_p(1 << 20)                      # never dereferenced: every call below returns before a launch
+
+    def pyr(mode, dtype, base=1 << 20):
+        p = ofb200.Pyramid()
+        elems = (ctypes.c_int64 * ofb200.MAX_LEVELS)()
+        assert lib.ofb_pyramid_layout(16, 24, 4, mode, ctypes.byref(p), ctypes.byref(elems)) == 0
+        for l in range(4):
+            p.base[l] = base
+        p.dtype = dtype
+        return p
+
+    def entry_points(p):
+        r = ctypes.byref(p)
+        return [lib.ofb_corr_lookup(r, fake, fake, None, None, 1, 16, 24, 4, None),
+                lib.ofb_corr_lookup_coords_backward(r, fake, fake, fake, 1, 16, 24, 4, None),
+                lib.ofb_corr_lookup_backward_f32(r, fake, fake, 1, 16, 24, 4, None),
+                lib.ofb_corr_pyramid_bf16(fake, fake, fake, r, 1, 64, 16, 24, 1.0, 0, None),
+                lib.ofb_corr_pyramid_simt_f32(fake, fake, r, 1, 64, 16, 24, 1.0, None)]
+
+    def edit(**kw):
+        def apply(p):
+            for k, v in kw.items():
+                if isinstance(v, tuple):
+                    getattr(p, k)[v[0]] = v[1]
+                else:
+                    setattr(p, k, v)
+            return p
+        return apply
+
+    before = lib.ofb_launch_count()
+    broken = [edit(levels=0), edit(levels=5), edit(dtype=3), edit(dtype=-1), edit(layout=3), edit(layout=-1),
+              edit(base=(2, None)), edit(lvl_h=(1, 0)), edit(lvl_w=(3, 0)), edit(row_pitch=(2, 5)),
+              edit(q_stride=(1, 64))]
+    for dtype in (ofb200.DTYPE_F32, ofb200.DTYPE_BF16):
+        for k, fault in enumerate(broken):
+            p = fault(pyr(3, dtype))                         # query-minor 8x4 blocks: q_stride = 32 until broken
+            assert entry_points(p) == [OFB_EINVAL] * 5, (dtype, k)
+
+    variants = [edit(), edit(base=(1, (1 << 20) + 2)), edit(base=(2, (1 << 20) + 4)), edit(row_pitch=(1, 13)),
+                edit(row_pitch=(1, 14)), edit(lvl_w=(0, 70000), row_pitch=(0, 70000)), edit(q_stride=(3, 64))]
+    seen = set()
+    for mode in range(4):
+        for dtype in (ofb200.DTYPE_F32, ofb200.DTYPE_BF16, ofb200.DTYPE_F16):
+            for radius in range(5):
+                for k, variant in enumerate(variants):
+                    r = ctypes.byref(variant(pyr(mode, dtype)))
+                    fwd = lib.ofb_corr_lookup(r, fake, fake, None, None, 65536, 1024, 1024, radius, None)
+                    bwd = lib.ofb_corr_lookup_coords_backward(r, fake, fake, fake, 65536, 1024, 1024, radius, None)
+                    assert fwd == bwd, (mode, dtype, radius, k, fwd, bwd)
+                    seen.add(fwd)
+    assert seen == {OFB_EINVAL, OFB_EUNSUPPORTED, OFB_EALIGN}
+    assert lib.ofb_launch_count() == before
+
+
 def test_ondemand_lookup_validates_arguments_without_launch(lib):
     fake = 1 << 20
 
@@ -519,6 +580,7 @@ def lookup_pyramid(levels, dtype, layout, b, h, w):
     """Device pyramid of the (Q, 1, h_l, w_l) float32 levels (already rounded to dtype) in one of FWD_LAYOUTS, padding
     poisoned.  Returns the descriptor and the buffers that back it."""
     import ofb200
+    from ofb200.ops.corr import level_buffer
 
     q = levels[0].shape[0]
     pyr = ofb200.Pyramid()
@@ -536,12 +598,7 @@ def lookup_pyramid(levels, dtype, layout, b, h, w):
             pitch, rows = (wl + 7) & ~7, (hl + 3) & ~3
         img = torch.full((q, rows, pitch), poison(dtype), dtype=dtype, device="cuda")
         img[:, :hl, :wl] = T(lv[:, 0]).to(dtype)
-        if layout == "qminor8x4":
-            buf = img.view(q, rows // 4, 4, pitch // 8, 8).permute(1, 3, 0, 2, 4).contiguous()
-        elif layout == "block8x4":
-            buf = img.view(q, rows // 4, 4, pitch // 8, 8).permute(0, 1, 3, 2, 4).contiguous()
-        else:
-            buf = img
+        buf = level_buffer(img, pyr.layout)
         bufs.append(buf)
         pyr.base[l] = buf.data_ptr()
         pyr.q_stride[l] = 32 if layout == "qminor8x4" else rows * pitch

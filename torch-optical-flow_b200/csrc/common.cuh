@@ -438,14 +438,6 @@ __device__ __forceinline__ RowChunks row_chunks(int xs, int cols, int pitch) {
     c.ck2 = (c.s + cols > 16) && c.xa + 16 >= 0 && c.xa + 24 <= pitch;
     return c;
 }
-// Chunk xa of window row y: one row of an 8x4 block (P.blocked; the next chunk is P.blk_stride elements further) or 8
-// consecutive elements of a padded row (the next chunk 8 further, OFB_CHUNK_STEP).  P: the kernel's parameter block.
-// Macros rather than functions: the register-tile forward's code must stay what it was (as inline functions they change
-// its instruction schedule).
-#define OFB_CHUNK_ROW(slice, y, xa, pitch, P)                                                       \
-    ((P).blocked ? (slice) + ((long long)((y) >> 2) * ((pitch) >> 3) + ((xa) >> 3)) * (P).blk_stride + ((y) & 3) * 8 \
-                 : (slice) + (long long)(y) * (pitch) + (xa))
-#define OFB_CHUNK_STEP(P) ((P).blocked ? (P).blk_stride : 8)
 
 __device__ __forceinline__ float warp_sum(float v) {
 #pragma unroll
@@ -468,28 +460,71 @@ __device__ __forceinline__ int warp_max(int v) {
     return v;
 }
 
-// An ofb_pyramid's level geometry as the lookup kernels receive it (strides in elements, unused levels zeroed)
-struct PyramidLevels {
+// ---- the correlation pyramid's layout contract (include/ofb200.h): the one check, addressing rule and reader choice
+// An ofb_pyramid as the kernels receive it (strides in elements, unused levels zeroed); kernel parameter blocks derive
+// from it and add their scalars.
+struct PyramidView {
     void* base[OFB_MAX_LEVELS];
     long long q_stride[OFB_MAX_LEVELS];
     int pitch[OFB_MAX_LEVELS];
     int lh[OFB_MAX_LEVELS];
     int lw[OFB_MAX_LEVELS];
+    int levels, dtype;
+    int blocked;            // 8x4-blocked layouts (OFB_LAYOUT_BLOCK8X4, OFB_LAYOUT_QMINOR8X4)
+    long long blk_stride;   // elements between consecutive 8x4 blocks: 32, or 32 * Q (query-minor)
 };
 
-// Copies pyr's levels into lv and checks them: 1 .. OFB_MAX_LEVELS levels, each with a base pointer, a positive size
-// and a row pitch no smaller than its width.
-inline int unpack_levels(const ofb_pyramid& pyr, PyramidLevels& lv) {
-    if (pyr.levels < 1 || pyr.levels > OFB_MAX_LEVELS) return OFB_EINVAL;
+// The 8-element piece at (y, x), x % 8 == 0, of a level of view V with row pitch `pitch`: one row of an 8x4 block
+// (V.blocked) or 8 consecutive elements of a row; OFB_PIECE_OFFSET is its offset in the (query, level) slice, OFB_PIECE
+// its address, the next piece along x OFB_PIECE_STEP(V) elements further.  Macros, and OFB_PIECE adds the _TERMS to the
+// pointer one by one: as an inline function or slice + OFB_PIECE_OFFSET, the register-tile forward's schedule changes.
+#define OFB_BLOCK_TERMS(V, y, x, pitch) ((long long)((y) >> 2) * ((pitch) >> 3) + ((x) >> 3)) * (V).blk_stride + ((y) & 3) * 8
+#define OFB_ROW_TERMS(y, x, pitch) (long long)(y) * (pitch) + (x)
+#define OFB_PIECE_OFFSET(V, y, x, pitch) ((V).blocked ? (OFB_BLOCK_TERMS(V, y, x, pitch)) : (OFB_ROW_TERMS(y, x, pitch)))
+#define OFB_PIECE(slice, V, y, x, pitch) \
+    ((V).blocked ? (slice) + OFB_BLOCK_TERMS(V, y, x, pitch) : (slice) + OFB_ROW_TERMS(y, x, pitch))
+#define OFB_PIECE_STEP(V) ((V).blocked ? (V).blk_stride : 8)
+
+// Fills v from pyr (Q = B * h * w queries) and checks the rules every user relies on, else OFB_EINVAL: 1 ..
+// OFB_MAX_LEVELS levels, a known dtype and layout, per level a base, a positive size, pitch >= width, and q_stride = 32
+// in the query-minor layout.  Each entry point then checks only its own requirements.
+inline int check_pyramid(const ofb_pyramid* pyr, long long Q, PyramidView& v) {
+    if (pyr->levels < 1 || pyr->levels > OFB_MAX_LEVELS) return OFB_EINVAL;
+    if (pyr->dtype != OFB_DTYPE_F32 && pyr->dtype != OFB_DTYPE_BF16 && pyr->dtype != OFB_DTYPE_F16) return OFB_EINVAL;
+    if (pyr->layout < OFB_LAYOUT_ROWS || pyr->layout > OFB_LAYOUT_QMINOR8X4) return OFB_EINVAL;
+    const bool qminor = pyr->layout == OFB_LAYOUT_QMINOR8X4;
+    v.levels = pyr->levels; v.dtype = pyr->dtype;
+    v.blocked = pyr->layout != OFB_LAYOUT_ROWS;
+    v.blk_stride = qminor ? 32 * Q : 32;
     for (int l = 0; l < OFB_MAX_LEVELS; ++l) {
-        const bool on = l < pyr.levels;
-        lv.base[l] = on ? pyr.base[l] : nullptr;
-        lv.q_stride[l] = on ? pyr.q_stride[l] : 0;
-        lv.pitch[l] = on ? pyr.row_pitch[l] : 0;
-        lv.lh[l] = on ? pyr.lvl_h[l] : 0;
-        lv.lw[l] = on ? pyr.lvl_w[l] : 0;
-        if (on && (!lv.base[l] || lv.lh[l] <= 0 || lv.lw[l] <= 0 || lv.pitch[l] < lv.lw[l])) return OFB_EINVAL;
+        const bool on = l < pyr->levels;
+        v.base[l] = on ? pyr->base[l] : nullptr;
+        v.q_stride[l] = on ? pyr->q_stride[l] : 0;
+        v.pitch[l] = on ? pyr->row_pitch[l] : 0;
+        v.lh[l] = on ? pyr->lvl_h[l] : 0;
+        v.lw[l] = on ? pyr->lvl_w[l] : 0;
+        if (on && (!v.base[l] || v.lh[l] <= 0 || v.lw[l] <= 0 || v.pitch[l] < v.lw[l] || (qminor && v.q_stride[l] != 32)))
+            return OFB_EINVAL;
     }
+    return OFB_OK;
+}
+
+// The radii the register-tile forward lookup is built for
+constexpr bool tile_radius(int radius) { return radius == 3 || radius == 4; }
+
+// How ofb_corr_lookup and ofb_corr_lookup_coords_backward read v at `radius` (both decide here, so they accept the same
+// pyramids).  *chunked: 16-bit rows or 8x4 blocks in 16-byte aligned 8-element chunks, read whole by the register-tile
+// forward at tile_radius and by the coordinate backward; other rows are read element-wise.  OFB_EUNSUPPORTED: a level
+// above 65536, or blocks the register-tile forward does not read; OFB_EALIGN: 16-bit levels not in 4-byte words.
+inline int lookup_reader(const PyramidView& v, int radius, bool& chunked) {
+    const bool half16 = chunked = v.dtype != OFB_DTYPE_F32;
+    for (int l = 0; l < v.levels; ++l) {
+        const uintptr_t base = reinterpret_cast<uintptr_t>(v.base[l]);
+        if (v.lh[l] > 65536 || v.lw[l] > 65536) return OFB_EUNSUPPORTED;
+        if (half16 && ((v.pitch[l] & 1) || (v.q_stride[l] & 1) || (base & 3))) return OFB_EALIGN;
+        chunked = chunked && v.pitch[l] % 8 == 0 && v.q_stride[l] % 8 == 0 && (base & 15) == 0;
+    }
+    if (v.blocked && !(chunked && tile_radius(radius))) return OFB_EUNSUPPORTED;
     return OFB_OK;
 }
 

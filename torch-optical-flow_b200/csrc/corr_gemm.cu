@@ -93,18 +93,22 @@ static_assert(Ring<1, 0>::SMEM_ALLOC <= 232448 && Ring<2, 0>::SMEM_ALLOC <= 2324
               Ring<2, 2>::SMEM_ALLOC <= 232448 && Ring<2, 2>::STAGES <= MAX_STAGES && Ring<1, 2, 1>::SMEM_ALLOC <= 232448 &&
               Ring<2, 2, 1>::SMEM_ALLOC <= 232448, "shared memory budget");
 
+// One level of a run's output, copied from the PyramidView (level_out): fields side by side keep the kernel's code
 template <typename T> struct LevelOut {
     T* base;                     // 16-bit storage: __nv_bfloat16 or __half
     long long q_stride;
     int pitch, h, w;
-    int blocked;                 // 8x4 blocks (OFB_LAYOUT_BLOCK8X4 / QMINOR8X4): a 16-byte piece is one block row
-    long long blk_stride;        // elements between consecutive blocks: 32, or 32 * Q for the query-minor layout
+    int blocked;                 // PyramidView::blocked
+    long long blk_stride;        // PyramidView::blk_stride
 };
+template <typename T>
+LevelOut<T> level_out(const PyramidView& v, int l) {
+    return {static_cast<T*>(v.base[l]), v.q_stride[l], v.pitch[l], v.lh[l], v.lw[l], v.blocked, v.blk_stride};
+}
 // element offset (without the query term q * q_stride) of the 8-element piece starting at (y, x), x % 8 == 0
 template <typename T>
 __device__ __forceinline__ long long piece_offset(const LevelOut<T>& L, int y, int x) {
-    if (L.blocked) return ((long long)(y >> 2) * (L.pitch >> 3) + (x >> 3)) * L.blk_stride + (y & 3) * 8;
-    return (long long)y * L.pitch + x;
+    return OFB_PIECE_OFFSET(L, y, x, L.pitch);
 }
 
 template <typename T> struct GemmParams {
@@ -747,11 +751,11 @@ int launch_gemm(const CUtensorMap& ma, const CUtensorMap& mb, const GemmParams<T
     return OFB_OK;
 }
 
-// One GEMM run: queries (B, Nq, C) x targets (B, th*tw, C) -> level la_idx (th x tw per query) and, when
-// lb_idx >= 0, its 2x2 mean.  T: the operands' and the pyramid's 16-bit type.
+// One GEMM run: queries (B, Nq, C) x targets (B, th*tw, C) -> level la of view v (th x tw per query) and, when
+// has_b, its 2x2 mean, level la + 1.  layout: v's OFB_LAYOUT_*.  T: the operands' and the pyramid's 16-bit type.
 template <typename T>
-int run_gemm(const void* f1_km, const void* f2_km, const ofb_pyramid* pyr, int la_idx, int lb_idx, int B, int C, int Nq,
-             int th, int tw, float scale, int cg_mode, unsigned long long* prof, int prof_slot, cudaStream_t st) {
+int run_gemm(const void* f1_km, const void* f2_km, const PyramidView& v, int layout, int la, bool has_b, int B, int C,
+             int Nq, int th, int tw, float scale, int cg_mode, unsigned long long* prof, int prof_slot, cudaStream_t st) {
     // cg_mode: 1 = one CTA per tile, 2 = CTA pair sharing one 256-row accumulator tile (cta_group::2),
     //          3 = cluster of two independent cta_group::1 CTAs with the fmap2 ring multicast into both
     const bool mc = cg_mode == 3;
@@ -762,8 +766,7 @@ int run_gemm(const void* f1_km, const void* f2_km, const ofb_pyramid* pyr, int l
     P.scale = scale; P.apply_scale = (scale != 1.0f) ? 1 : 0;
     // chunk shape follows the output layout (a chunk must be whole 64/128-byte runs of it); tile shape =
     // the arrangement of 4 chunks that covers the image with the fewest tiles (ties: the widest)
-    const bool blk = pyr->layout != OFB_LAYOUT_ROWS;
-    const long long blk_stride = pyr->layout == OFB_LAYOUT_QMINOR8X4 ? 32LL * B * Nq : 32LL;
+    const bool blk = v.blocked;
     P.CW = blk ? 16 : 32; P.CR = blk ? 4 : 2;
     long long best = -1;
     for (int xb = 1; xb <= 4; xb *= 2) {
@@ -800,15 +803,9 @@ int run_gemm(const void* f1_km, const void* f2_km, const ofb_pyramid* pyr, int l
     const long long n_items = (long long)B * P.mblk * P.n_chunks;
     if (n_items > 0x7fffffffLL) return OFB_EUNSUPPORTED;
     P.n_items = (int)n_items;
-    P.la.base = reinterpret_cast<T*>(pyr->base[la_idx]);
-    P.la.q_stride = pyr->q_stride[la_idx]; P.la.pitch = pyr->row_pitch[la_idx];
-    P.la.h = pyr->lvl_h[la_idx]; P.la.w = pyr->lvl_w[la_idx]; P.la.blocked = blk; P.la.blk_stride = blk_stride;
-    P.has_b = lb_idx >= 0 ? 1 : 0;
-    if (P.has_b) {
-        P.lb.base = reinterpret_cast<T*>(pyr->base[lb_idx]);
-        P.lb.q_stride = pyr->q_stride[lb_idx]; P.lb.pitch = pyr->row_pitch[lb_idx];
-        P.lb.h = pyr->lvl_h[lb_idx]; P.lb.w = pyr->lvl_w[lb_idx]; P.lb.blocked = blk; P.lb.blk_stride = blk_stride;
-    }
+    P.la = level_out<T>(v, la);
+    P.has_b = has_b ? 1 : 0;
+    if (has_b) P.lb = level_out<T>(v, la + 1);
     P.prof = prof ? prof + (size_t)prof_slot * PROF_SLOT : nullptr;
     P.dbg = 0;
     if (prof) {
@@ -838,10 +835,10 @@ int run_gemm(const void* f1_km, const void* f2_km, const ofb_pyramid* pyr, int l
     if constexpr (std::is_same<T, __half>::value) {
         // fp16 is built with the direct epilogue only and has no diagnostics variant: OFB_K2_EPI is ignored here
         if (prof) return OFB_EUNSUPPORTED;
-        if (mc) return pyr->layout == OFB_LAYOUT_QMINOR8X4 ? launch_gemm<T, 1, false, 2, 0, true>(ma, mb, P, grid, st)
-                                                           : OFB_EUNSUPPORTED;
+        if (mc) return layout == OFB_LAYOUT_QMINOR8X4 ? launch_gemm<T, 1, false, 2, 0, true>(ma, mb, P, grid, st)
+                                                      : OFB_EUNSUPPORTED;
 #define OFB_GEMM_CASE_F16(CGV, LAYV) \
-        if (cg == CGV && pyr->layout == LAYV) return launch_gemm<T, CGV, false, LAYV, EPI_DIRECT, false>(ma, mb, P, grid, st);
+        if (cg == CGV && layout == LAYV) return launch_gemm<T, CGV, false, LAYV, EPI_DIRECT, false>(ma, mb, P, grid, st);
         OFB_GEMM_CASE_F16(1, 0) OFB_GEMM_CASE_F16(1, 1) OFB_GEMM_CASE_F16(1, 2)
         OFB_GEMM_CASE_F16(2, 0) OFB_GEMM_CASE_F16(2, 1) OFB_GEMM_CASE_F16(2, 2)
 #undef OFB_GEMM_CASE_F16
@@ -850,9 +847,9 @@ int run_gemm(const void* f1_km, const void* f2_km, const ofb_pyramid* pyr, int l
         // epilogue store mode of the query-minor layout (OFB_K2_EPI=direct|bulk overrides; other layouts stage through smem)
         int epi = EPI_DIRECT;
         if (const char* e = getenv("OFB_K2_EPI")) epi = (e[0] == 'd' || e[0] == '0') ? EPI_DIRECT : (e[0] == 'p' || e[0] == '2') ? EPI_PIPE : EPI_BULK;
-        if (pyr->layout != OFB_LAYOUT_QMINOR8X4) epi = EPI_DIRECT;
+        if (layout != OFB_LAYOUT_QMINOR8X4) epi = EPI_DIRECT;
 #define OFB_GEMM_CASE(CGV, PROFV, LAYV, EPIV) \
-        if (cg == CGV && !mc && (prof != nullptr) == PROFV && pyr->layout == LAYV && epi == EPIV) \
+        if (cg == CGV && !mc && (prof != nullptr) == PROFV && layout == LAYV && epi == EPIV) \
             return launch_gemm<T, CGV, PROFV, LAYV, EPIV, false>(ma, mb, P, grid, st);
         OFB_GEMM_CASE(1, false, 0, 0) OFB_GEMM_CASE(1, false, 1, 0) OFB_GEMM_CASE(1, false, 2, 0) OFB_GEMM_CASE(1, false, 2, 1)
         OFB_GEMM_CASE(2, false, 0, 0) OFB_GEMM_CASE(2, false, 1, 0) OFB_GEMM_CASE(2, false, 2, 0) OFB_GEMM_CASE(2, false, 2, 1)
@@ -860,7 +857,7 @@ int run_gemm(const void* f1_km, const void* f2_km, const ofb_pyramid* pyr, int l
         OFB_GEMM_CASE(2, true, 0, 0) OFB_GEMM_CASE(2, true, 1, 0) OFB_GEMM_CASE(2, true, 2, 0) OFB_GEMM_CASE(2, true, 2, 1)
         OFB_GEMM_CASE(1, false, 2, 2) OFB_GEMM_CASE(2, false, 2, 2) OFB_GEMM_CASE(1, true, 2, 2) OFB_GEMM_CASE(2, true, 2, 2)
         // multicast clusters: the product layout (query-minor) only
-        if (mc && pyr->layout == OFB_LAYOUT_QMINOR8X4) {
+        if (mc && layout == OFB_LAYOUT_QMINOR8X4) {
             if (!prof && epi == EPI_DIRECT) return launch_gemm<T, 1, false, 2, 0, true>(ma, mb, P, grid, st);
             if (!prof && epi == EPI_BULK) return launch_gemm<T, 1, false, 2, 1, true>(ma, mb, P, grid, st);
             if (prof && epi == EPI_DIRECT) return launch_gemm<T, 1, true, 2, 0, true>(ma, mb, P, grid, st);
@@ -880,39 +877,37 @@ int corr_pyramid_impl(int dtype, const void* f1_km, const void* f2_km, const voi
     if (B == 0) return OFB_OK;   // nothing to do: empty tensors have no storage, their pointers may be null
     if (!f1_km || !f2_km || !pyr || B < 0 || C <= 0 || h <= 0 || w <= 0) return OFB_EINVAL;
     if (cta_group < 0 || cta_group > 3) return OFB_EINVAL;
-    if (pyr->levels < 1 || pyr->levels > OFB_MAX_LEVELS) return OFB_EINVAL;
-    if (pyr->dtype != dtype) return OFB_EUNSUPPORTED;                   // fp32 pyramids: ofb_corr_pyramid_simt_f32
+    PyramidView v;
+    if (const int rc = check_pyramid(pyr, (long long)B * h * w, v)) return rc;
+    if (v.dtype != dtype) return OFB_EUNSUPPORTED;                     // fp32 pyramids: ofb_corr_pyramid_simt_f32
     if (C % BLOCK_K != 0 || C > MAX_KB * BLOCK_K) return OFB_EUNSUPPORTED;
-    if (pyr->levels > 2 && !f2q_km) return OFB_EINVAL;                  // levels 2, 3 come from the 4x4-averaged fmap2
-    if (B == 0) return OFB_OK;
+    if (v.levels > 2 && !f2q_km) return OFB_EINVAL;                    // levels 2, 3 come from the 4x4-averaged fmap2
     const uintptr_t al = reinterpret_cast<uintptr_t>(f1_km) | reinterpret_cast<uintptr_t>(f2_km) |
                          reinterpret_cast<uintptr_t>(f2q_km);
     if (al & 15) return OFB_EALIGN;
-    for (int l = 0; l < pyr->levels; ++l) {
-        if (!pyr->base[l] || pyr->lvl_h[l] != (h >> l) || pyr->lvl_w[l] != (w >> l)) return OFB_EINVAL;
-        if (pyr->lvl_h[l] <= 0 || pyr->lvl_w[l] <= 0 || pyr->row_pitch[l] < pyr->lvl_w[l]) return OFB_EINVAL;
-        // 16-byte store pieces: rows and query slices start on 8-element boundaries
-        const uintptr_t amask = pyr->layout == OFB_LAYOUT_QMINOR8X4 ? 31 : 15;   // query-minor: 32-byte sector stores
-        if ((pyr->row_pitch[l] & 7) || (pyr->q_stride[l] & 7) || (reinterpret_cast<uintptr_t>(pyr->base[l]) & amask))
+    for (int l = 0; l < v.levels; ++l)      // level l of the (h, w) feature maps: (h >> l) x (w >> l)
+        if (v.lh[l] != (h >> l) || v.lw[l] != (w >> l)) return OFB_EINVAL;
+    const bool qminor = pyr->layout == OFB_LAYOUT_QMINOR8X4;
+    for (int l = 0; l < v.levels; ++l) {
+        // 16-byte store pieces: rows and query slices start on 8-element boundaries; query-minor: 32-byte sector stores
+        if ((v.pitch[l] & 7) || (v.q_stride[l] & 7) || (reinterpret_cast<uintptr_t>(v.base[l]) & (qminor ? 31 : 15)))
             return OFB_EALIGN;
-        const int rows = pyr->layout != OFB_LAYOUT_ROWS ? ((pyr->lvl_h[l] + 3) & ~3) : pyr->lvl_h[l];
-        if (pyr->layout == OFB_LAYOUT_QMINOR8X4 ? pyr->q_stride[l] != 32 : pyr->q_stride[l] < (int64_t)pyr->row_pitch[l] * rows)
-            return OFB_EINVAL;
+        const int rows = v.blocked ? ((v.lh[l] + 3) & ~3) : v.lh[l];
+        if (!qminor && v.q_stride[l] < (long long)v.pitch[l] * rows) return OFB_EINVAL;
     }
-    if (pyr->layout < OFB_LAYOUT_ROWS || pyr->layout > OFB_LAYOUT_QMINOR8X4) return OFB_EINVAL;
     // auto (round-2 measurements, profiles/r02_k2_*.jsonl): the builder runs into the 1 kW power cap, so what pays is
     // energy per tile.  Clusters of two independent cta_group::1 CTAs with the fmap2 ring multicast into both (mode 3)
     // halve the L2 -> SM operand traffic and are 3-5 % faster than one CTA per tile at every BASELINE shape in sustained
     // runs; the CTA pair (cta_group::2) is slower (its MMAs run below the single-CTA rate and the pair's epilogues are
     // coupled through one accumulator barrier).  Mode 3 is built for the product layout only.
     int cg = cta_group;
-    if (cg == 0) cg = (pyr->layout == OFB_LAYOUT_QMINOR8X4 && h * w > BLOCK_M) ? 3 : 1;
-    if (cg == 3 && pyr->layout != OFB_LAYOUT_QMINOR8X4) return OFB_EUNSUPPORTED;
+    if (cg == 0) cg = (qminor && h * w > BLOCK_M) ? 3 : 1;
+    if (cg == 3 && !qminor) return OFB_EUNSUPPORTED;
     cudaStream_t st = (cudaStream_t)stream;
     const auto run = dtype == OFB_DTYPE_F16 ? run_gemm<__half> : run_gemm<__nv_bfloat16>;
-    const int rc = run(f1_km, f2_km, pyr, 0, pyr->levels > 1 ? 1 : -1, B, C, h * w, h, w, scale, cg, prof, 0, st);
-    if (rc != OFB_OK || pyr->levels <= 2) return rc;
-    return run(f1_km, f2q_km, pyr, 2, pyr->levels > 3 ? 3 : -1, B, C, h * w, h >> 2, w >> 2, scale, cg, prof, 1, st);
+    const int rc = run(f1_km, f2_km, v, pyr->layout, 0, v.levels > 1, B, C, h * w, h, w, scale, cg, prof, 0, st);
+    if (rc != OFB_OK || v.levels <= 2) return rc;
+    return run(f1_km, f2q_km, v, pyr->layout, 2, v.levels > 3, B, C, h * w, h >> 2, w >> 2, scale, cg, prof, 1, st);
 }
 
 }  // namespace

@@ -146,23 +146,22 @@ __global__ void __launch_bounds__(256) pool2_kernel(const T* __restrict__ src, T
 }
 
 template <typename T>
-int build_simt(const float* f1, const float* f2, const ofb_pyramid* pyr, int B, int C, int h, int w, float scale,
+int build_simt(const float* f1, const float* f2, const ofb::PyramidView& v, int B, int C, int h, int w, float scale,
                cudaStream_t st) {
     const int N = h * w;
     dim3 grid((N + GT - 1) / GT, (N + GT - 1) / GT, B);
-    corr_l0_kernel<T><<<grid, GT * GT / 4, 0, st>>>(f1, f2, reinterpret_cast<T*>(pyr->base[0]), pyr->q_stride[0],
-                                                    pyr->row_pitch[0], C, h, w, scale);
+    corr_l0_kernel<T><<<grid, GT * GT / 4, 0, st>>>(f1, f2, reinterpret_cast<T*>(v.base[0]), v.q_stride[0], v.pitch[0], C, h,
+                                                    w, scale);
     OFB_LAUNCH_CHECK();
-    for (int l = 1; l < pyr->levels; ++l) {
-        const long long total = (long long)B * N * pyr->lvl_h[l] * pyr->lvl_w[l];
+    for (int l = 1; l < v.levels; ++l) {
+        const long long total = (long long)B * N * v.lh[l] * v.lw[l];
         if (total == 0) continue;
         long long blocks = (total + 255) / 256;
         const int cap = ofb_num_sms() * 32;
         if (blocks > cap) blocks = cap;
-        pool2_kernel<T><<<(int)blocks, 256, 0, st>>>(reinterpret_cast<const T*>(pyr->base[l - 1]),
-                                                     reinterpret_cast<T*>(pyr->base[l]), (long long)B * N,
-                                                     pyr->q_stride[l - 1], pyr->row_pitch[l - 1], pyr->q_stride[l],
-                                                     pyr->row_pitch[l], pyr->lvl_h[l], pyr->lvl_w[l]);
+        pool2_kernel<T><<<(int)blocks, 256, 0, st>>>(reinterpret_cast<const T*>(v.base[l - 1]), reinterpret_cast<T*>(v.base[l]),
+                                                     (long long)B * N, v.q_stride[l - 1], v.pitch[l - 1], v.q_stride[l],
+                                                     v.pitch[l], v.lh[l], v.lw[l]);
         OFB_LAUNCH_CHECK();
     }
     return OFB_OK;
@@ -248,16 +247,14 @@ OFB_API int ofb_corr_pyramid_simt_f32(const float* fmap1, const float* fmap2, co
                                       int h, int w, float scale, void* stream) {
     if (B == 0) return OFB_OK;   // nothing to do: empty tensors have no storage, their pointers may be null
     if (!fmap1 || !fmap2 || !pyr || B < 0 || C <= 0 || h <= 0 || w <= 0) return OFB_EINVAL;
-    if (pyr->levels < 1 || pyr->levels > OFB_MAX_LEVELS) return OFB_EINVAL;
-    if (pyr->layout != OFB_LAYOUT_ROWS) return OFB_EUNSUPPORTED;      // the CUDA-core builder writes rows
-    for (int l = 0; l < pyr->levels; ++l)
-        if (!pyr->base[l] || pyr->lvl_h[l] != (h >> l) || pyr->lvl_w[l] != (w >> l) || pyr->row_pitch[l] < pyr->lvl_w[l])
-            return OFB_EINVAL;
-    if (B == 0) return OFB_OK;
+    ofb::PyramidView v;
+    if (const int rc = ofb::check_pyramid(pyr, (long long)B * h * w, v)) return rc;
+    if (v.blocked) return OFB_EUNSUPPORTED;                           // the CUDA-core builder writes rows
+    for (int l = 0; l < v.levels; ++l)      // level l of the (h, w) feature maps: (h >> l) x (w >> l)
+        if (v.lh[l] != (h >> l) || v.lw[l] != (w >> l)) return OFB_EINVAL;
     if (B > 65535 || (h * w + GT - 1) / GT > 65535) return OFB_EUNSUPPORTED;
     cudaStream_t st = (cudaStream_t)stream;
-    if (pyr->dtype == OFB_DTYPE_F32) return build_simt<float>(fmap1, fmap2, pyr, B, C, h, w, scale, st);
-    if (pyr->dtype == OFB_DTYPE_BF16) return build_simt<__nv_bfloat16>(fmap1, fmap2, pyr, B, C, h, w, scale, st);
-    if (pyr->dtype == OFB_DTYPE_F16) return build_simt<__half>(fmap1, fmap2, pyr, B, C, h, w, scale, st);
-    return OFB_EINVAL;
+    if (v.dtype == OFB_DTYPE_F32) return build_simt<float>(fmap1, fmap2, v, B, C, h, w, scale, st);
+    if (v.dtype == OFB_DTYPE_BF16) return build_simt<__nv_bfloat16>(fmap1, fmap2, v, B, C, h, w, scale, st);
+    return build_simt<__half>(fmap1, fmap2, v, B, C, h, w, scale, st);
 }

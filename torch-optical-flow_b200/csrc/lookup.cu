@@ -26,10 +26,8 @@ constexpr int QT = 32;        // queries per CTA
 constexpr int NW = 8;         // warps per CTA
 constexpr int OT_PITCH = QT + 1;
 
-struct LookupParams : ofb::PyramidLevels {
-    int levels, radius, B, h, w;
-    int blocked;   // 8x4-blocked layouts (register-tile kernel only, 16-bit pyramids)
-    long long blk_stride;   // elements between consecutive blocks: 32, or 32 * Q (query-minor)
+struct LookupParams : ofb::PyramidView {
+    int B, h, w, radius;   // in this order: (B, h) is one 8-byte constant load of the register-tile kernel
 };
 
 // patch load: bf16 / fp16 -> two elements per 4-byte word (px0 and pitch are even, the slice base is 4-byte aligned)
@@ -217,12 +215,12 @@ __global__ void __launch_bounds__(128) lookup_tile_kernel(const LookupParams P, 
     const uint32_t my_slot2 = smem0 + (uint32_t)(WIN * 2) * slot_stride + threadIdx.x * 8u;
     const uint32_t slot2_stride = blockDim.x * 8u;
     {
-        const long long cstep = OFB_CHUNK_STEP(P);
+        const long long cstep = OFB_PIECE_STEP(P);
 #pragma unroll
         for (int r = 0; r < WIN; ++r) {
             const int y = ys + r;
             const bool rok = !dead && r < wrows && y >= 0 && y < Hl;
-            const T* row = OFB_CHUNK_ROW(slice, y, ck.xa, pitch, P);
+            const T* row = OFB_PIECE(slice, P, y, ck.xa, pitch);
 #pragma unroll
             for (int c = 0; c < 2; ++c) {
                 const bool ok = rok && (c == 0 ? ck.ck0 : ck.ck1);
@@ -325,41 +323,29 @@ OFB_API int ofb_corr_lookup(const ofb_pyramid* pyr, const float* coords, float* 
     if (B == 0) return OFB_OK;   // nothing to do: empty tensors have no storage, their pointers may be null
     if (!pyr || !coords || !out || B < 0 || h <= 0 || w <= 0) return OFB_EINVAL;
     if (radius < 0 || 2 * radius + 1 > MAX_D) return OFB_EUNSUPPORTED;
-    if (pyr->dtype != OFB_DTYPE_F32 && pyr->dtype != OFB_DTYPE_BF16 && pyr->dtype != OFB_DTYPE_F16) return OFB_EINVAL;
-    if (pyr->layout < OFB_LAYOUT_ROWS || pyr->layout > OFB_LAYOUT_QMINOR8X4) return OFB_EINVAL;
-    const bool half16 = pyr->dtype != OFB_DTYPE_F32;      // 16-bit storage: bf16 or fp16
-    LookupParams P;
-    if (const int rc = ofb::unpack_levels(*pyr, P)) return rc;
-    P.levels = pyr->levels; P.radius = radius; P.B = B; P.h = h; P.w = w;
-    P.blocked = pyr->layout != OFB_LAYOUT_ROWS;
-    P.blk_stride = pyr->layout == OFB_LAYOUT_QMINOR8X4 ? 32LL * B * h * w : 32LL;
-    for (int l = 0; l < P.levels; ++l) {
-        if (P.lh[l] > 65536 || P.lw[l] > 65536) return OFB_EUNSUPPORTED;
-        if (half16 && ((P.pitch[l] & 1) || (P.q_stride[l] & 1) || (reinterpret_cast<uintptr_t>(P.base[l]) & 3)))
-            return OFB_EALIGN;
-    }
-    const int D = 2 * radius + 1, CH = pyr->levels * D * D;
-    const size_t smem = ((size_t)CH * OT_PITCH + (size_t)NW * PD * PD) * sizeof(float);
     const long long Q = (long long)B * h * w;
+    LookupParams P;
+    if (const int rc = ofb::check_pyramid(pyr, Q, P)) return rc;
+    bool chunked;
+    if (const int rc = ofb::lookup_reader(P, radius, chunked)) return rc;
+    P.radius = radius; P.B = B; P.h = h; P.w = w;
     const long long blocks = (Q + QT - 1) / QT;
     if (blocks > 0x7fffffffLL) return OFB_EUNSUPPORTED;
     cudaStream_t st = (cudaStream_t)stream;
-    // product path: 16-bit pyramid with padded rows (pitch multiple of 8, 16-byte aligned slices)
-    bool tile_ok = half16 && (radius == 4 || radius == 3);
-    for (int l = 0; l < pyr->levels && tile_ok; ++l)
-        tile_ok = (P.pitch[l] % 8 == 0) && (P.q_stride[l] % 8 == 0) && ((reinterpret_cast<uintptr_t>(P.base[l]) & 15) == 0);
-    if (tile_ok) {
-        const int threads = 32 * pyr->levels;
+    // product path: 16-bit chunks (padded rows or 8x4 blocks) at radius 3 and 4 -- the only way blocked pyramids are read
+    if (chunked && ofb::tile_radius(radius)) {
+        const int threads = 32 * P.levels;
         const size_t wsm = (size_t)(2 * radius + 3) * threads * 40;               // window slots: rows x (16 + 16 + 8) B
-        if (pyr->dtype == OFB_DTYPE_F16) return launch_tile<__half>(P, coords, out, idx_or_null, valid_or_null, radius,
-                                                                    (int)blocks, threads, wsm, st);
+        if (P.dtype == OFB_DTYPE_F16) return launch_tile<__half>(P, coords, out, idx_or_null, valid_or_null, radius,
+                                                                 (int)blocks, threads, wsm, st);
         return launch_tile<__nv_bfloat16>(P, coords, out, idx_or_null, valid_or_null, radius, (int)blocks, threads, wsm, st);
     }
-    if (P.blocked) return OFB_EUNSUPPORTED;   // the generic kernels read rows
-    if (pyr->dtype == OFB_DTYPE_BF16) {
+    const int D = 2 * radius + 1, CH = P.levels * D * D;
+    const size_t smem = ((size_t)CH * OT_PITCH + (size_t)NW * PD * PD) * sizeof(float);
+    if (P.dtype == OFB_DTYPE_BF16) {
         OFB_CUDA(cudaFuncSetAttribute(lookup_kernel<__nv_bfloat16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         lookup_kernel<__nv_bfloat16><<<(int)blocks, NW * 32, smem, st>>>(P, coords, out, idx_or_null, valid_or_null);
-    } else if (pyr->dtype == OFB_DTYPE_F16) {
+    } else if (P.dtype == OFB_DTYPE_F16) {
         OFB_CUDA(cudaFuncSetAttribute(lookup_kernel<__half>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
         lookup_kernel<__half><<<(int)blocks, NW * 32, smem, st>>>(P, coords, out, idx_or_null, valid_or_null);
     } else {

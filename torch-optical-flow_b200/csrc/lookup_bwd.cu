@@ -21,8 +21,8 @@
 
 namespace {
 
-struct BwdParams : ofb::PyramidLevels {
-    int levels, B, h, w;
+struct BwdParams : ofb::PyramidView {
+    int h, w, B;   // in this order: (h, w) is one 8-byte constant load
 };
 
 struct Tap {
@@ -127,15 +127,15 @@ OFB_API int ofb_corr_lookup_backward_f32(const ofb_pyramid* d_pyr, const float* 
                                          int w, int radius, void* stream) {
     if (B == 0) return OFB_OK;   // nothing to do: empty tensors have no storage, their pointers may be null
     if (!d_pyr || !coords || !d_out || B < 0 || h <= 0 || w <= 0) return OFB_EINVAL;
-    if (d_pyr->dtype != OFB_DTYPE_F32 || d_pyr->layout != OFB_LAYOUT_ROWS) return OFB_EUNSUPPORTED;
     if (radius < 0 || radius > 4) return OFB_EUNSUPPORTED;
-    BwdParams P;
-    if (const int rc = ofb::unpack_levels(*d_pyr, P)) return rc;
-    P.levels = d_pyr->levels; P.B = B; P.h = h; P.w = w;
     const long long Q = (long long)B * h * w;
+    BwdParams P;
+    if (const int rc = ofb::check_pyramid(d_pyr, Q, P)) return rc;
+    if (P.dtype != OFB_DTYPE_F32 || P.blocked) return OFB_EUNSUPPORTED;     // the gradient pyramid: fp32 rows
+    P.B = B; P.h = h; P.w = w;
     const long long blocks = (Q + 127) / 128;
     if (blocks > 0x7fffffffLL) return OFB_EUNSUPPORTED;
-    const dim3 grid((unsigned)blocks, (unsigned)d_pyr->levels);
+    const dim3 grid((unsigned)blocks, (unsigned)P.levels);
     cudaStream_t st = (cudaStream_t)stream;
     switch (radius) {
         case 0: lookup_bwd_kernel<0><<<grid, 128, 0, st>>>(P, coords, d_out); break;

@@ -26,10 +26,8 @@ namespace {
 
 using ofb::MAX_D;
 
-struct CoordsBwdParams : ofb::PyramidLevels {
-    int levels, B, h, w;
-    int blocked;            // 8x4-blocked layouts
-    long long blk_stride;   // elements between consecutive blocks: 32, or 32 * Q (query-minor)
+struct CoordsBwdParams : ofb::PyramidView {
+    int h, w, B;   // in this order: (h, w) is one 8-byte constant load
 };
 
 // Window row y, columns xs .. xs + WIN - 1 of a (query, level) slice -> px, 0 outside the image.  CHUNKED: 16-bit
@@ -44,8 +42,8 @@ __device__ __forceinline__ void load_row(float (&px)[WIN], const T* slice, const
 #pragma unroll
         for (int k = 0; k < 10; ++k) w[k] = 0u;
         if (rok) {
-            const long long cstep = OFB_CHUNK_STEP(P);
-            const T* row = OFB_CHUNK_ROW(slice, y, ck.xa, pitch, P);
+            const long long cstep = OFB_PIECE_STEP(P);
+            const T* row = OFB_PIECE(slice, P, y, ck.xa, pitch);
             if (ck.ck0) {
                 const uint4 v = __ldg(reinterpret_cast<const uint4*>(row));
                 w[0] = v.x; w[1] = v.y; w[2] = v.z; w[3] = v.w;
@@ -200,30 +198,18 @@ OFB_API int ofb_corr_lookup_coords_backward(const ofb_pyramid* pyr, const float*
     if (B == 0) return OFB_OK;   // nothing to do: empty tensors have no storage, their pointers may be null
     if (!pyr || !coords || !d_out || !d_coords || B < 0 || h <= 0 || w <= 0) return OFB_EINVAL;
     if (radius < 0 || 2 * radius + 1 > MAX_D) return OFB_EUNSUPPORTED;
-    if (pyr->dtype != OFB_DTYPE_F32 && pyr->dtype != OFB_DTYPE_BF16 && pyr->dtype != OFB_DTYPE_F16) return OFB_EINVAL;
-    if (pyr->layout < OFB_LAYOUT_ROWS || pyr->layout > OFB_LAYOUT_QMINOR8X4) return OFB_EINVAL;
-    const bool half16 = pyr->dtype != OFB_DTYPE_F32;
+    const long long Q = (long long)B * h * w;
     CoordsBwdParams P;
-    if (const int rc = ofb::unpack_levels(*pyr, P)) return rc;
-    P.levels = pyr->levels; P.B = B; P.h = h; P.w = w;
-    P.blocked = pyr->layout != OFB_LAYOUT_ROWS;
-    P.blk_stride = pyr->layout == OFB_LAYOUT_QMINOR8X4 ? 32LL * B * h * w : 32LL;
-    bool chunked = half16;
-    for (int l = 0; l < P.levels; ++l) {
-        if (P.lh[l] > 65536 || P.lw[l] > 65536) return OFB_EUNSUPPORTED;
-        if (half16 && ((P.pitch[l] & 1) || (P.q_stride[l] & 1) || (reinterpret_cast<uintptr_t>(P.base[l]) & 3)))
-            return OFB_EALIGN;
-        chunked = chunked && (P.pitch[l] % 8 == 0) && (P.q_stride[l] % 8 == 0) &&
-                  ((reinterpret_cast<uintptr_t>(P.base[l]) & 15) == 0);
-    }
-    // the pyramids ofb_corr_lookup accepts: the blocked layouts only where its register-tile kernel reads them
-    if (P.blocked && !(chunked && (radius == 3 || radius == 4))) return OFB_EUNSUPPORTED;
-    const long long blocks = ((long long)B * h * w + 31) / 32;
+    if (const int rc = ofb::check_pyramid(pyr, Q, P)) return rc;
+    bool chunked;
+    if (const int rc = ofb::lookup_reader(P, radius, chunked)) return rc;
+    P.B = B; P.h = h; P.w = w;
+    const long long blocks = (Q + 31) / 32;
     if (blocks > 0x7fffffffLL) return OFB_EUNSUPPORTED;
     cudaStream_t st = (cudaStream_t)stream;
-    if (pyr->dtype == OFB_DTYPE_F32)
+    if (P.dtype == OFB_DTYPE_F32)
         return launch_radius<float, false>(P, coords, d_out, d_coords, radius, (int)blocks, st);
-    if (pyr->dtype == OFB_DTYPE_F16)
+    if (P.dtype == OFB_DTYPE_F16)
         return chunked ? launch_radius<__half, true>(P, coords, d_out, d_coords, radius, (int)blocks, st)
                        : launch_radius<__half, false>(P, coords, d_out, d_coords, radius, (int)blocks, st);
     return chunked ? launch_radius<__nv_bfloat16, true>(P, coords, d_out, d_coords, radius, (int)blocks, st)

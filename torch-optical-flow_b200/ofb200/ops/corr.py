@@ -97,6 +97,28 @@ def build_pyramid(ops, pyr, b: int, c: int, h: int, w: int, dtype: torch.dtype =
               int(cta_group), ofb200.stream_ptr())
 
 
+def level_images(buf: Tensor, layout: int, q: int, pitch: int) -> Tensor:
+    """One pyramid level's buffer in `layout` (OFB_LAYOUT_*, include/ofb200.h) -> its (q, rows, pitch) images, rows =
+    buf.numel() // (q * pitch): a view of the buffer for rows, a copy that unfolds the 8x4 blocks otherwise.  The inverse
+    of level_buffer."""
+    rows = buf.numel() // (q * pitch)
+    if layout == ofb200.LAYOUT_ROWS:
+        return buf.view(q, rows, pitch)
+    if layout == ofb200.LAYOUT_QMINOR8X4:
+        return buf.view(rows // 4, pitch // 8, q, 4, 8).permute(2, 0, 3, 1, 4).reshape(q, rows, pitch)   # (by, bx, q, y, x)
+    return buf.view(q, rows // 4, pitch // 8, 4, 8).permute(0, 1, 3, 2, 4).reshape(q, rows, pitch)       # (q, by, bx, y, x)
+
+
+def level_buffer(img: Tensor, layout: int) -> Tensor:
+    """(q, rows, pitch) images -> one pyramid level's contiguous buffer in `layout` (8x4 blocks: rows a multiple of 4,
+    pitch a multiple of 8).  The inverse of level_images."""
+    q, rows, pitch = img.shape
+    if layout == ofb200.LAYOUT_ROWS:
+        return img.contiguous()
+    order = (1, 3, 0, 2, 4) if layout == ofb200.LAYOUT_QMINOR8X4 else (0, 1, 3, 2, 4)   # (by, bx, q, y, x) / (q, by, bx, y, x)
+    return img.reshape(q, rows // 4, 4, pitch // 8, 8).permute(*order).contiguous()
+
+
 class _GradState:
     """What the backward nodes of one CorrBlock share: the dense fp32 gradient pyramid the lookups' backwards
     accumulate into, and the few scalars needed to allocate and consume it.  The autograd contexts hold THIS object,
@@ -413,8 +435,8 @@ class CorrBlock:
     def corr_pyramid(self) -> List[Tensor]:
         """The levels with the reference's shapes (B*h*w, 1, h_l, w_l) (reference corr.py:48-54).
 
-        Row layout: strided views of the padded buffers.  8x4-blocked layout (tcgen05 builder): the
-        blocks are unfolded into a copy on first access -- the lookup never needs this, only callers
+        Row layout: strided views of the padded buffers.  8x4-blocked layouts (tcgen05 builder): the
+        blocks are unfolded into a copy on first access (level_images) -- the lookup never needs this, only callers
         that inspect the volume do."""
         if self._on_demand is not None:
             raise NotImplementedError("CorrBlock(on_demand=True) does not materialise the correlation pyramid")
@@ -423,19 +445,9 @@ class CorrBlock:
             n = h * w
             views = []
             for lvl, buf in enumerate(self._buffers):
-                qs, pitch = int(self._pyr.q_stride[lvl]), int(self._pyr.row_pitch[lvl])
                 hl, wl = int(self._pyr.lvl_h[lvl]), int(self._pyr.lvl_w[lvl])
-                if self._pyr.layout == ofb200.LAYOUT_QMINOR8X4:
-                    rows = buf.numel() // (b * n * pitch)
-                    blocks = buf.view(rows // 4, pitch // 8, b * n, 4, 8)                  # (by, bx, q, y, x)
-                    img = blocks.permute(2, 0, 3, 1, 4).reshape(b * n, rows, pitch)
-                    views.append(img[:, :hl, :wl].unsqueeze(1))
-                elif self._pyr.layout == ofb200.LAYOUT_BLOCK8X4:
-                    blocks = buf.view(b * n, qs // (4 * pitch), pitch // 8, 4, 8)          # (q, by, bx, y, x)
-                    img = blocks.permute(0, 1, 3, 2, 4).reshape(b * n, qs // pitch, pitch)
-                    views.append(img[:, :hl, :wl].unsqueeze(1))
-                else:
-                    views.append(torch.as_strided(buf, (b * n, 1, hl, wl), (qs, qs, pitch, 1)))
+                img = level_images(buf, self._pyr.layout, b * n, int(self._pyr.row_pitch[lvl]))
+                views.append(img[:, :hl, :wl].unsqueeze(1))
             self._views = views
         return self._views
 
