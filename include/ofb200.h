@@ -45,7 +45,7 @@ extern "C" {
 #define OFB_DTYPE_F32 0
 #define OFB_DTYPE_BF16 1
 #define OFB_DTYPE_F16 2 /* feature maps and operands of ofb_corr_prep_from / _to, correlation pyramids, mask of
-                           ofb_convex_upsample, ofb_scale_flow */
+                           ofb_convex_upsample, ofb_scale_flow, the lookup's output and its gradient */
 #define OFB_DTYPE_F64 3 /* ofb_scale_flow only */
 
 #define OFB_MAX_LEVELS 4
@@ -263,11 +263,16 @@ int ofb_corr_pyramid_f16(const void* f1_km, const void* f2_km, const void* f2q_k
  * coordinate sequence as ofb_corr_lookup.
  *   f1_km            (B, h*w, C) bf16 K-major, already multiplied by 1/sqrt(C)      (ofb_corr_prep_from, pool 1)
  *   f2_km_levels[l]  (B, (h>>l)*(w>>l), C) bf16 K-major, fmap2 averaged over complete 2^l x 2^l blocks (pool 1, 2, 4, 8)
- *   coords (B,2,h,w) fp32 -> out (B, levels*(2r+1)^2, h, w) fp32.  C in {64, 128, 256}.
+ *   coords (B,2,h,w) fp32 -> out (B, levels*(2r+1)^2, h, w) fp32 (ofb_corr_lookup_ondemand_to: fp16 / bf16).
+ *   C in {64, 128, 256}.
  * Memory: the operand maps (22 MB per 1088x1920 pair) instead of the 2.83 GB pyramid; it is slower than build + lookup
  * (DESIGN.md section 4) -- a capacity feature. */
 int ofb_corr_lookup_ondemand(const void* f1_km, const void* const* f2_km_levels_host, const float* coords, float* out,
                              int B, int C, int h, int w, int levels, int radius, void* stream);
+/* The same lookup with the output's dtype chosen, as ofb_corr_lookup_to: out_dtype OFB_DTYPE_F32 (= ofb_corr_lookup_ondemand),
+ * F16 or BF16; anything else is OFB_EINVAL. */
+int ofb_corr_lookup_ondemand_to(const void* f1_km, const void* const* f2_km_levels_host, const float* coords, void* out,
+                                int out_dtype, int B, int C, int h, int w, int levels, int radius, void* stream);
 
 /* Diagnostics build of the same kernel: additionally fills prof_dev[2][148][16] (device, uint64; one
  * slot per GEMM run) with per-CTA cycle counters -- [0] TMA warp waiting for a free fmap2 stage,
@@ -286,7 +291,7 @@ int ofb_corr_pyramid_simt_f32(const float* fmap1, const float* fmap2, const ofb_
  * level and window cell (i,j): bilinear sample (zeros outside, align_corners=True after the
  * reference's normalise/un-normalise round trip) of the query's level slice at
  * (x/2^l + i - r, y/2^l + j - r); out channel = l*(2r+1)^2 + i*(2r+1) + j.
- *   coords (B,2,h,w) fp32 (ch0 = x, ch1 = y);  out (B, L*(2r+1)^2, h, w) fp32
+ *   coords (B,2,h,w) fp32 (ch0 = x, ch1 = y);  out (B, L*(2r+1)^2, h, w) fp32 (ofb_corr_lookup_to: fp16 / bf16)
  *   idx_or_null   (B*h*w, L, 2, 2r+1) int32 floor indices (x taps then y taps)
  *   valid_or_null (B*h*w, L, (2r+1)^2) u8   utils.py:77 predicate per sample
  * pyr: dtype F32, BF16 or F16.  Floor indices and validity masks do not depend on the dtype.  16-bit pyramids with
@@ -297,6 +302,14 @@ int ofb_corr_pyramid_simt_f32(const float* fmap1, const float* fmap2, const ofb_
 int ofb_corr_lookup(const ofb_pyramid* pyr_host, const float* coords, float* out,
                     int32_t* idx_or_null, uint8_t* valid_or_null, int B, int h, int w, int radius,
                     void* stream);
+/* ofb_corr_lookup with the output's dtype chosen: out_dtype OFB_DTYPE_F32 (= ofb_corr_lookup), F16 or BF16; anything
+ * else is OFB_EINVAL.  Each sample is accumulated in fp32 exactly as for an fp32 output and rounded once to nearest
+ * even: the same bits as the fp32 output cast to that dtype (fp16: beyond +-65504 is inf).  Under the reference's
+ * `precision: 16` the lookup's only consumer, BasicMotionEncoder.convc1 (methods/raft/model/update.py:114), receives
+ * the output autocast to half precision; writing it in that precision saves the cast and half the output bytes.
+ * Indices and masks are unchanged. */
+int ofb_corr_lookup_to(const ofb_pyramid* pyr_host, const float* coords, void* out, int out_dtype,
+                       int32_t* idx_or_null, uint8_t* valid_or_null, int B, int h, int w, int radius, void* stream);
 
 /* Backward of ofb_corr_lookup with respect to the pyramid (autograd through corr.py:56-77 /
  * utils.py:64-80; the coordinates get no gradient -- RAFT detaches them, raft.py:127).
@@ -304,6 +317,11 @@ int ofb_corr_lookup(const ofb_pyramid* pyr_host, const float* coords, float* out
  * first of the refinement iterations, then call once per lookup.  d_out (B, L*(2r+1)^2, h, w). */
 int ofb_corr_lookup_backward_f32(const ofb_pyramid* d_pyr, const float* coords, const float* d_out,
                                  int B, int h, int w, int radius, void* stream);
+/* The same backward reading d_out in d_out_dtype OFB_DTYPE_F32 (= ofb_corr_lookup_backward_f32), F16 or BF16 (the
+ * gradient of an ofb_corr_lookup_to output); anything else is OFB_EINVAL.  Each element is widened exactly to fp32;
+ * the arithmetic, its order and the fp32 gradient pyramid are those of the fp32 form. */
+int ofb_corr_lookup_backward(const ofb_pyramid* d_pyr, const float* coords, const void* d_out, int d_out_dtype,
+                             int B, int h, int w, int radius, void* stream);
 
 /* Backward of ofb_corr_lookup with respect to the coordinates: what autograd computes for coords through
  * CorrBlock.__call__ (methods/raft/model/corr.py:56-77) and bilinear_sampler = grid_sample(align_corners=True, zeros
@@ -316,6 +334,11 @@ int ofb_corr_lookup_backward_f32(const ofb_pyramid* d_pyr, const float* coords, 
  * bits on every run. */
 int ofb_corr_lookup_coords_backward(const ofb_pyramid* pyr, const float* coords, const float* d_out, float* d_coords,
                                     int B, int h, int w, int radius, void* stream);
+/* The same backward reading d_out in d_out_dtype OFB_DTYPE_F32 (= ofb_corr_lookup_coords_backward), F16 or BF16,
+ * widened exactly to fp32 on load; anything else is OFB_EINVAL.  d_coords stays fp32. */
+int ofb_corr_lookup_coords_backward_from(const ofb_pyramid* pyr, const float* coords, const void* d_out,
+                                         int d_out_dtype, float* d_coords, int B, int h, int w, int radius,
+                                         void* stream);
 
 /* The two GEMMs behind d CorrBlock / d fmap (autograd through corr.py:45-54,79-87), on the tensor cores:
  *   D[b] (M x N, fp32, row pitch ldd) = alpha * A[b] (M x K) . B[b]^T (N x K)  (+ D[b] when accumulate != 0)

@@ -64,6 +64,22 @@ static inline int ofb_dispatch_pad_ac(int pad, int ac, F f) {
     }
 }
 
+// The floating-point element types of correlation pyramids and of the lookup's output and its gradient
+static inline bool ofb_float_dtype(int dtype) {
+    return dtype == OFB_DTYPE_F32 || dtype == OFB_DTYPE_F16 || dtype == OFB_DTYPE_BF16;
+}
+// Returns f(T{}) for the element type of dtype OFB_DTYPE_F32 / F16 / BF16 (float, __half, __nv_bfloat16), so f can name
+// a kernel template instance; any other dtype is OFB_EINVAL.
+template <typename F>
+static inline int ofb_dispatch_dtype(int dtype, F f) {
+    switch (dtype) {
+        case OFB_DTYPE_F32: return f(float{});
+        case OFB_DTYPE_F16: return f(__half{});
+        case OFB_DTYPE_BF16: return f(__nv_bfloat16{});
+        default: return OFB_EINVAL;
+    }
+}
+
 // Raises Kernel's dynamic shared-memory limit to `bytes`, the first time it is called on each device.
 template <auto Kernel>
 static inline cudaError_t ofb_smem_once(int bytes) {
@@ -397,6 +413,12 @@ template <> __device__ __forceinline__ float widen16<__nv_bfloat16>(unsigned wd,
 template <> __device__ __forceinline__ float widen16<__half>(unsigned wd, int hi) {
     return __half2float(__ushort_as_half((unsigned short)(hi ? (wd >> 16) : (wd & 0xffffu))));
 }
+// fp32 -> an output element, rounded to nearest even: the bits ATen's out_fp32.to(dtype) gives (fp16: beyond +-65504
+// is inf).  Its inverse for a 16-bit gradient read back is ld_f32, an exact widening.
+template <typename T> __device__ __forceinline__ T narrow(float v);
+template <> __device__ __forceinline__ float narrow<float>(float v) { return v; }
+template <> __device__ __forceinline__ __half narrow<__half>(float v) { return __float2half_rn(v); }
+template <> __device__ __forceinline__ __nv_bfloat16 narrow<__nv_bfloat16>(float v) { return __float2bfloat16_rn(v); }
 
 // One window row of a 16-bit pyramid from its aligned chunk loads: w[0..7] are the 8-element (16-byte) chunks at
 // xa and xa + 8, w[8..9] the first 4 elements at xa + 16, as packed pairs.  px receives elements s .. s + WIN - 1
@@ -490,7 +512,7 @@ struct PyramidView {
 // in the query-minor layout.  Each entry point then checks only its own requirements.
 inline int check_pyramid(const ofb_pyramid* pyr, long long Q, PyramidView& v) {
     if (pyr->levels < 1 || pyr->levels > OFB_MAX_LEVELS) return OFB_EINVAL;
-    if (pyr->dtype != OFB_DTYPE_F32 && pyr->dtype != OFB_DTYPE_BF16 && pyr->dtype != OFB_DTYPE_F16) return OFB_EINVAL;
+    if (!ofb_float_dtype(pyr->dtype)) return OFB_EINVAL;
     if (pyr->layout < OFB_LAYOUT_ROWS || pyr->layout > OFB_LAYOUT_QMINOR8X4) return OFB_EINVAL;
     const bool qminor = pyr->layout == OFB_LAYOUT_QMINOR8X4;
     v.levels = pyr->levels; v.dtype = pyr->dtype;

@@ -23,7 +23,8 @@
 //      one 16-byte load + 8 FMAs per position and lane, then ONE transposing butterfly (31 shuffles) turns the 32 lanes'
 //      partial sums of 32 positions into one finished value per lane,
 //   3. samples the (2r+1)^2 outputs from the patch, 3 per lane,
-// and stages 8 queries' outputs so that the global writes are 32-byte runs.
+// and stages 8 queries' outputs so that the global writes are runs of 8 elements (32 bytes in fp32; the output may also
+// be fp16 or bf16, each fp32 sample rounded once, as ofb_corr_lookup_to does).
 #include <cstdlib>
 
 #include "common.cuh"
@@ -82,9 +83,9 @@ __device__ __forceinline__ float transpose_reduce(float (&v)[32], int lane) {
     return v[0];
 }
 
-template <int CPL>
+template <int CPL, typename O>
 __global__ void __launch_bounds__(128) ondemand_lookup_kernel(const OdParams P, const float* __restrict__ coords,
-                                                              float* __restrict__ out) {
+                                                              O* __restrict__ out) {
     __shared__ float patch_s[TQY][PD * PD];
     __shared__ float otile_s[TQY][MAX_DD][TQ + 1];
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -165,10 +166,10 @@ __global__ void __launch_bounds__(128) ondemand_lookup_kernel(const OdParams P, 
             __syncwarp();
         }
         // ---- one tile row of queries is done: 32-byte runs per channel
-        float* dst = out + ((long long)b * CH + (long long)l * DD) * HW + (long long)y * P.w + x_tile;
+        O* dst = out + ((long long)b * CH + (long long)l * DD) * HW + (long long)y * P.w + x_tile;
         for (int idx = lane; idx < DD * TQ; idx += 32) {
             const int k = idx >> 3, qx = idx & 7;
-            if (qx < nqx) dst[(long long)k * HW + qx] = otile[k][qx];
+            if (qx < nqx) dst[(long long)k * HW + qx] = ofb::narrow<O>(otile[k][qx]);
         }
         __syncwarp();
     }
@@ -177,8 +178,10 @@ __global__ void __launch_bounds__(128) ondemand_lookup_kernel(const OdParams P, 
 
 }  // namespace
 
-OFB_API int ofb_corr_lookup_ondemand(const void* f1_km, const void* const* f2_km_levels, const float* coords, float* out,
-                                     int B, int C, int h, int w, int levels, int radius, void* stream) {
+OFB_API int ofb_corr_lookup_ondemand_to(const void* f1_km, const void* const* f2_km_levels, const float* coords,
+                                        void* out, int out_dtype, int B, int C, int h, int w, int levels, int radius,
+                                        void* stream) {
+    if (!ofb_float_dtype(out_dtype)) return OFB_EINVAL;
     if (B == 0) return OFB_OK;   // nothing to do: empty tensors have no storage, their pointers may be null
     if (!f1_km || !f2_km_levels || !coords || !out || B < 0 || C <= 0 || h <= 0 || w <= 0) return OFB_EINVAL;
     if (levels < 1 || levels > OFB_MAX_LEVELS) return OFB_EINVAL;
@@ -206,9 +209,19 @@ OFB_API int ofb_corr_lookup_ondemand(const void* f1_km, const void* const* f2_km
     if (blocks > P.n_items) blocks = P.n_items;
     cudaStream_t st = (cudaStream_t)stream;
     const int threads = 32 * TQY;
-    if (C == 256) ondemand_lookup_kernel<8><<<(int)blocks, threads, 0, st>>>(P, coords, out);
-    else if (C == 128) ondemand_lookup_kernel<4><<<(int)blocks, threads, 0, st>>>(P, coords, out);
-    else ondemand_lookup_kernel<2><<<(int)blocks, threads, 0, st>>>(P, coords, out);
-    OFB_LAUNCH_CHECK();
-    return OFB_OK;
+    return ofb_dispatch_dtype(out_dtype, [&](auto o) {
+        using O = decltype(o);
+        O* dst = static_cast<O*>(out);
+        if (C == 256) ondemand_lookup_kernel<8, O><<<(int)blocks, threads, 0, st>>>(P, coords, dst);
+        else if (C == 128) ondemand_lookup_kernel<4, O><<<(int)blocks, threads, 0, st>>>(P, coords, dst);
+        else ondemand_lookup_kernel<2, O><<<(int)blocks, threads, 0, st>>>(P, coords, dst);
+        OFB_LAUNCH_CHECK();
+        return OFB_OK;
+    });
+}
+
+OFB_API int ofb_corr_lookup_ondemand(const void* f1_km, const void* const* f2_km_levels, const float* coords, float* out,
+                                     int B, int C, int h, int w, int levels, int radius, void* stream) {
+    return ofb_corr_lookup_ondemand_to(f1_km, f2_km_levels, coords, out, OFB_DTYPE_F32, B, C, h, w, levels, radius,
+                                       stream);
 }

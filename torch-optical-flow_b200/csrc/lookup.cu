@@ -4,7 +4,8 @@
 // methods/raft/model/utils.py:64-80).  The reference runs ~70 small ATen launches per
 // refinement iteration (delta grid + H2D copy, 3 materialised (N,9,9,2) coordinate tensors,
 // grid_sample, 5 concatenations); here one kernel reads the coordinates and the pyramid and
-// writes the (B, L*(2r+1)^2, h, w) fp32 output.
+// writes the (B, L*(2r+1)^2, h, w) output in fp32, or rounded once to fp16 / bf16 (ofb::narrow) for a caller that
+// consumes it in half precision.
 //
 // The tap coordinates follow the bit-exact sequence of ofb::lookup_tap (common.cuh, SURVEY.md 8c).
 //
@@ -63,9 +64,10 @@ __device__ __forceinline__ void load_patch<float>(float* patch, const float* sli
     }
 }
 
-template <typename T>
+// T: the pyramid's element type; O: the output's (float, __half or __nv_bfloat16): samples are accumulated in fp32
+template <typename T, typename O>
 __global__ void __launch_bounds__(NW * 32) lookup_kernel(const LookupParams P, const float* __restrict__ coords,
-                                                         float* __restrict__ out, int32_t* __restrict__ idx_out,
+                                                         O* __restrict__ out, int32_t* __restrict__ idx_out,
                                                          uint8_t* __restrict__ valid_out) {
     extern __shared__ float smem[];
     const int D = 2 * P.radius + 1, DD = D * D, CH = P.levels * DD;
@@ -120,8 +122,8 @@ __global__ void __launch_bounds__(NW * 32) lookup_kernel(const LookupParams P, c
     const long long q = q0 + lane;
     if (q < Q) {
         const long long b = q / HW, p = q - b * HW;
-        float* dst = out + b * CH * HW + p;
-        for (int ch = warp; ch < CH; ch += NW) dst[(long long)ch * HW] = otile[ch * OT_PITCH + lane];
+        O* dst = out + b * CH * HW + p;
+        for (int ch = warp; ch < CH; ch += NW) dst[(long long)ch * HW] = ofb::narrow<O>(otile[ch * OT_PITCH + lane]);
     }
 }
 
@@ -140,7 +142,8 @@ __global__ void __launch_bounds__(NW * 32) lookup_kernel(const LookupParams P, c
 //      realigned in registers with two select stages (word shift) and a funnel shift (half-word),
 //      widened to fp32 (bf16: a shift or mask of the word; fp16: a conversion of each half),
 //      horizontal filter -> 9 values, vertical filter accumulated into three live output rows;
-//   4. writes each finished output row straight to its 9 channels.
+//   4. writes each finished output row straight to its 9 channels (a warp stores one contiguous row per channel: 128
+//      bytes in fp32, 64 in fp16 / bf16).
 // No shared memory, no shuffles, ~56 warp instructions per (query, level) against ~230 before.
 // Contract with the builder: elements between w_l and the row pitch hold FINITE values (the tcgen05
 // builder writes zeros there); they are multiplied by zero weights.
@@ -148,10 +151,10 @@ using ofb::TapSet;
 using ofb::make_taps;
 
 // T: the pyramid's 16-bit type.  Only the widening of the realigned words depends on it: the coordinates, floor
-// indices, validity masks and filter weights are the same code for both types.
-template <int R, int GR, typename T>
+// indices, validity masks and filter weights are the same code for both types.  O: the output's type, as lookup_kernel.
+template <int R, int GR, typename T, typename O>
 __global__ void __launch_bounds__(128) lookup_tile_kernel(const LookupParams P, const float* __restrict__ coords,
-                                                           float* __restrict__ out, int32_t* __restrict__ idx_out,
+                                                           O* __restrict__ out, int32_t* __restrict__ idx_out,
                                                            uint8_t* __restrict__ valid_out) {
     constexpr int D = 2 * R + 1, DD = D * D, WIN = D + 2;       // window rows / columns
     const int l = threadIdx.x >> 5, lane = threadIdx.x & 31;
@@ -195,7 +198,7 @@ __global__ void __launch_bounds__(128) lookup_tile_kernel(const LookupParams P, 
     // chunk geometry: 8-element (16-byte) aligned chunks covering columns xs .. xs + wcols - 1
     const ofb::RowChunks ck = ofb::row_chunks(xs, wcols, pitch);
     const T* slice = reinterpret_cast<const T*>(P.base[l]) + q * P.q_stride[l];
-    float* outp = out + (b * (long long)(P.levels * DD) + (long long)l * DD) * HW + p;
+    O* outp = out + (b * (long long)(P.levels * DD) + (long long)l * DD) * HW + p;
 
     float acc[3][D];                                            // output rows j = r, r-1, r-2 in flight
 #pragma unroll
@@ -278,7 +281,7 @@ __global__ void __launch_bounds__(128) lookup_tile_kernel(const LookupParams P, 
             const int j = r - 2;
 #pragma unroll
             for (int i = 0; i < D; ++i) {
-                outp[(long long)(i * D + j) * HW] = acc[j % 3][i];
+                outp[(long long)(i * D + j) * HW] = ofb::narrow<O>(acc[j % 3][i]);
                 acc[j % 3][i] = 0.0f;
             }
         }
@@ -305,21 +308,51 @@ __global__ void __launch_bounds__(256) bilinear_sampler_kernel(const float* __re
 }
 
 // window rows per cp.async commit group: 3 for radius 4 (measured ~2 % faster than one group for the whole window)
-template <typename T>
-int launch_tile(const LookupParams& P, const float* coords, float* out, int32_t* idx, uint8_t* valid, int radius,
+template <typename T, typename O>
+int launch_tile(const LookupParams& P, const float* coords, O* out, int32_t* idx, uint8_t* valid, int radius,
                 int blocks, int threads, size_t wsm, cudaStream_t st) {
-    OFB_CUDA(ofb_smem_once<lookup_tile_kernel<4, 3, T>>(11 * 128 * 40));
-    OFB_CUDA(ofb_smem_once<lookup_tile_kernel<3, 16, T>>(9 * 128 * 40));
-    if (radius == 4) lookup_tile_kernel<4, 3, T><<<blocks, threads, wsm, st>>>(P, coords, out, idx, valid);
-    else lookup_tile_kernel<3, 16, T><<<blocks, threads, wsm, st>>>(P, coords, out, idx, valid);
+    OFB_CUDA(ofb_smem_once<lookup_tile_kernel<4, 3, T, O>>(11 * 128 * 40));
+    OFB_CUDA(ofb_smem_once<lookup_tile_kernel<3, 16, T, O>>(9 * 128 * 40));
+    if (radius == 4) lookup_tile_kernel<4, 3, T, O><<<blocks, threads, wsm, st>>>(P, coords, out, idx, valid);
+    else lookup_tile_kernel<3, 16, T, O><<<blocks, threads, wsm, st>>>(P, coords, out, idx, valid);
+    OFB_LAUNCH_CHECK();
+    return OFB_OK;
+}
+
+template <typename O>
+int launch_lookup(const LookupParams& P, bool chunked, const float* coords, O* out, int32_t* idx, uint8_t* valid,
+                  long long blocks, cudaStream_t st) {
+    const int radius = P.radius;
+    // product path: 16-bit chunks (padded rows or 8x4 blocks) at radius 3 and 4 -- the only way blocked pyramids are read
+    if (chunked && ofb::tile_radius(radius)) {
+        const int threads = 32 * P.levels;
+        const size_t wsm = (size_t)(2 * radius + 3) * threads * 40;               // window slots: rows x (16 + 16 + 8) B
+        if (P.dtype == OFB_DTYPE_F16)
+            return launch_tile<__half, O>(P, coords, out, idx, valid, radius, (int)blocks, threads, wsm, st);
+        return launch_tile<__nv_bfloat16, O>(P, coords, out, idx, valid, radius, (int)blocks, threads, wsm, st);
+    }
+    const int D = 2 * radius + 1, CH = P.levels * D * D;
+    const size_t smem = ((size_t)CH * OT_PITCH + (size_t)NW * PD * PD) * sizeof(float);
+    if (P.dtype == OFB_DTYPE_BF16) {
+        OFB_CUDA(cudaFuncSetAttribute(lookup_kernel<__nv_bfloat16, O>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        lookup_kernel<__nv_bfloat16, O><<<(int)blocks, NW * 32, smem, st>>>(P, coords, out, idx, valid);
+    } else if (P.dtype == OFB_DTYPE_F16) {
+        OFB_CUDA(cudaFuncSetAttribute(lookup_kernel<__half, O>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        lookup_kernel<__half, O><<<(int)blocks, NW * 32, smem, st>>>(P, coords, out, idx, valid);
+    } else {
+        OFB_CUDA(cudaFuncSetAttribute(lookup_kernel<float, O>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+        lookup_kernel<float, O><<<(int)blocks, NW * 32, smem, st>>>(P, coords, out, idx, valid);
+    }
     OFB_LAUNCH_CHECK();
     return OFB_OK;
 }
 
 }  // namespace
 
-OFB_API int ofb_corr_lookup(const ofb_pyramid* pyr, const float* coords, float* out, int32_t* idx_or_null,
-                            uint8_t* valid_or_null, int B, int h, int w, int radius, void* stream) {
+OFB_API int ofb_corr_lookup_to(const ofb_pyramid* pyr, const float* coords, void* out, int out_dtype,
+                               int32_t* idx_or_null, uint8_t* valid_or_null, int B, int h, int w, int radius,
+                               void* stream) {
+    if (!ofb_float_dtype(out_dtype)) return OFB_EINVAL;
     if (B == 0) return OFB_OK;   // nothing to do: empty tensors have no storage, their pointers may be null
     if (!pyr || !coords || !out || B < 0 || h <= 0 || w <= 0) return OFB_EINVAL;
     if (radius < 0 || 2 * radius + 1 > MAX_D) return OFB_EUNSUPPORTED;
@@ -331,29 +364,16 @@ OFB_API int ofb_corr_lookup(const ofb_pyramid* pyr, const float* coords, float* 
     P.radius = radius; P.B = B; P.h = h; P.w = w;
     const long long blocks = (Q + QT - 1) / QT;
     if (blocks > 0x7fffffffLL) return OFB_EUNSUPPORTED;
-    cudaStream_t st = (cudaStream_t)stream;
-    // product path: 16-bit chunks (padded rows or 8x4 blocks) at radius 3 and 4 -- the only way blocked pyramids are read
-    if (chunked && ofb::tile_radius(radius)) {
-        const int threads = 32 * P.levels;
-        const size_t wsm = (size_t)(2 * radius + 3) * threads * 40;               // window slots: rows x (16 + 16 + 8) B
-        if (P.dtype == OFB_DTYPE_F16) return launch_tile<__half>(P, coords, out, idx_or_null, valid_or_null, radius,
-                                                                 (int)blocks, threads, wsm, st);
-        return launch_tile<__nv_bfloat16>(P, coords, out, idx_or_null, valid_or_null, radius, (int)blocks, threads, wsm, st);
-    }
-    const int D = 2 * radius + 1, CH = P.levels * D * D;
-    const size_t smem = ((size_t)CH * OT_PITCH + (size_t)NW * PD * PD) * sizeof(float);
-    if (P.dtype == OFB_DTYPE_BF16) {
-        OFB_CUDA(cudaFuncSetAttribute(lookup_kernel<__nv_bfloat16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        lookup_kernel<__nv_bfloat16><<<(int)blocks, NW * 32, smem, st>>>(P, coords, out, idx_or_null, valid_or_null);
-    } else if (P.dtype == OFB_DTYPE_F16) {
-        OFB_CUDA(cudaFuncSetAttribute(lookup_kernel<__half>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        lookup_kernel<__half><<<(int)blocks, NW * 32, smem, st>>>(P, coords, out, idx_or_null, valid_or_null);
-    } else {
-        OFB_CUDA(cudaFuncSetAttribute(lookup_kernel<float>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-        lookup_kernel<float><<<(int)blocks, NW * 32, smem, st>>>(P, coords, out, idx_or_null, valid_or_null);
-    }
-    OFB_LAUNCH_CHECK();
-    return OFB_OK;
+    return ofb_dispatch_dtype(out_dtype, [&](auto o) {
+        using O = decltype(o);
+        return launch_lookup(P, chunked, coords, static_cast<O*>(out), idx_or_null, valid_or_null, blocks,
+                             (cudaStream_t)stream);
+    });
+}
+
+OFB_API int ofb_corr_lookup(const ofb_pyramid* pyr, const float* coords, float* out, int32_t* idx_or_null,
+                            uint8_t* valid_or_null, int B, int h, int w, int radius, void* stream) {
+    return ofb_corr_lookup_to(pyr, coords, out, OFB_DTYPE_F32, idx_or_null, valid_or_null, B, h, w, radius, stream);
 }
 
 OFB_API int ofb_bilinear_sampler_f32(const float* img, const float* coords, float* out, float* mask_or_null, int N, int C,

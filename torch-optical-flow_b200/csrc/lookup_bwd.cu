@@ -5,7 +5,9 @@
 // to the sampled image scatters weight * grad into the four taps of every sample.  RAFT detaches the coordinates
 // (raft.py:127), so only d / d pyramid is produced.
 //
-// thread = (query, level), lane <-> query (d_out reads are 128-byte rows).  A (query, level) slice is touched by
+// d_out is read in fp32, fp16 or bf16 (the dtype of the forward's output) and widened exactly on load; everything after
+// the load is the same fp32 arithmetic for all three.
+// thread = (query, level), lane <-> query (d_out reads are 128-byte rows in fp32).  A (query, level) slice is touched by
 // exactly one thread per launch, so the accumulation into the fp32 gradient pyramid needs no atomicity; it is
 // still issued as red.global.add.f32 (result unused): one fire-and-forget operation per element instead of a load
 // + store round trip (measured 0.75 -> 0.40 ms per iteration at C4).  The 12 refinement iterations accumulate
@@ -36,9 +38,9 @@ __device__ __forceinline__ Tap make_tap(float cen, int t, int radius, int size) 
     return tp.in_guard ? Tap{(int)tp.fl, tp.w0, tp.w1} : Tap{ofb::TAP_FAR, 0.0f, 0.0f};
 }
 
-template <int R>
+template <int R, typename G>
 __global__ void __launch_bounds__(128) lookup_bwd_kernel(const __grid_constant__ BwdParams P, const float* __restrict__ coords,
-                                                         const float* __restrict__ d_out) {
+                                                         const G* __restrict__ d_out) {
     constexpr int D = 2 * R + 1, DD = D * D;
     const long long HW = (long long)P.h * P.w, Q = (long long)P.B * HW;
     const long long q = (long long)blockIdx.x * blockDim.x + threadIdx.x;
@@ -50,7 +52,7 @@ __global__ void __launch_bounds__(128) lookup_bwd_kernel(const __grid_constant__
     const float inv = 1.0f / (float)(1 << l);
     const float cx = __fmul_rn(__ldg(coords + (b * 2 + 0) * HW + p), inv);
     const float cy = __fmul_rn(__ldg(coords + (b * 2 + 1) * HW + p), inv);
-    const float* g0 = d_out + (b * (long long)(P.levels * DD) + (long long)l * DD) * HW + p;   // channel c at g0[c * HW]
+    const G* g0 = d_out + (b * (long long)(P.levels * DD) + (long long)l * DD) * HW + p;   // channel c at g0[c * HW]
 
     float wx0[D], wx1[D], wy0[D], wy1[D];
     int ax = 0, ay = 0;
@@ -75,7 +77,7 @@ __global__ void __launch_bounds__(128) lookup_bwd_kernel(const __grid_constant__
             if (j < D) {
                 float g[D];
 #pragma unroll
-                for (int i = 0; i < D; ++i) g[i] = __ldg(g0 + (long long)(i * D + j) * HW);
+                for (int i = 0; i < D; ++i) g[i] = ofb::ld_f32(g0 + (long long)(i * D + j) * HW);
 #pragma unroll
                 for (int c = 0; c < D; ++c) {
                     tcur[c] = __fmaf_rn(g[c], wx0[c], tcur[c]);
@@ -108,7 +110,7 @@ __global__ void __launch_bounds__(128) lookup_bwd_kernel(const __grid_constant__
         for (int i = 0; i < D; ++i) {
             const Tap tx = make_tap(cx, i, R, Wl);
             if (tx.i0 == ofb::TAP_FAR) continue;
-            const float g = __ldg(g0 + (long long)(i * D + j) * HW);
+            const float g = ofb::ld_f32(g0 + (long long)(i * D + j) * HW);
             const bool inx0 = tx.i0 >= 0 && tx.i0 < Wl, inx1 = tx.i0 + 1 >= 0 && tx.i0 + 1 < Wl;
             const bool iny0 = ty.i0 >= 0 && ty.i0 < Hl, iny1 = ty.i0 + 1 >= 0 && ty.i0 + 1 < Hl;
             float* r0 = slice + (long long)ty.i0 * pitch + tx.i0;
@@ -121,10 +123,22 @@ __global__ void __launch_bounds__(128) lookup_bwd_kernel(const __grid_constant__
     }
 }
 
+template <typename G>
+void launch_radius(const BwdParams& P, const float* coords, const G* d_out, int radius, dim3 grid, cudaStream_t st) {
+    switch (radius) {
+        case 0: lookup_bwd_kernel<0, G><<<grid, 128, 0, st>>>(P, coords, d_out); break;
+        case 1: lookup_bwd_kernel<1, G><<<grid, 128, 0, st>>>(P, coords, d_out); break;
+        case 2: lookup_bwd_kernel<2, G><<<grid, 128, 0, st>>>(P, coords, d_out); break;
+        case 3: lookup_bwd_kernel<3, G><<<grid, 128, 0, st>>>(P, coords, d_out); break;
+        default: lookup_bwd_kernel<4, G><<<grid, 128, 0, st>>>(P, coords, d_out); break;
+    }
+}
+
 }  // namespace
 
-OFB_API int ofb_corr_lookup_backward_f32(const ofb_pyramid* d_pyr, const float* coords, const float* d_out, int B, int h,
-                                         int w, int radius, void* stream) {
+OFB_API int ofb_corr_lookup_backward(const ofb_pyramid* d_pyr, const float* coords, const void* d_out, int d_out_dtype,
+                                     int B, int h, int w, int radius, void* stream) {
+    if (!ofb_float_dtype(d_out_dtype)) return OFB_EINVAL;
     if (B == 0) return OFB_OK;   // nothing to do: empty tensors have no storage, their pointers may be null
     if (!d_pyr || !coords || !d_out || B < 0 || h <= 0 || w <= 0) return OFB_EINVAL;
     if (radius < 0 || radius > 4) return OFB_EUNSUPPORTED;
@@ -136,14 +150,15 @@ OFB_API int ofb_corr_lookup_backward_f32(const ofb_pyramid* d_pyr, const float* 
     const long long blocks = (Q + 127) / 128;
     if (blocks > 0x7fffffffLL) return OFB_EUNSUPPORTED;
     const dim3 grid((unsigned)blocks, (unsigned)P.levels);
-    cudaStream_t st = (cudaStream_t)stream;
-    switch (radius) {
-        case 0: lookup_bwd_kernel<0><<<grid, 128, 0, st>>>(P, coords, d_out); break;
-        case 1: lookup_bwd_kernel<1><<<grid, 128, 0, st>>>(P, coords, d_out); break;
-        case 2: lookup_bwd_kernel<2><<<grid, 128, 0, st>>>(P, coords, d_out); break;
-        case 3: lookup_bwd_kernel<3><<<grid, 128, 0, st>>>(P, coords, d_out); break;
-        default: lookup_bwd_kernel<4><<<grid, 128, 0, st>>>(P, coords, d_out); break;
-    }
-    OFB_LAUNCH_CHECK();
-    return OFB_OK;
+    return ofb_dispatch_dtype(d_out_dtype, [&](auto g) {
+        using G = decltype(g);
+        launch_radius(P, coords, static_cast<const G*>(d_out), radius, grid, (cudaStream_t)stream);
+        OFB_LAUNCH_CHECK();
+        return OFB_OK;
+    });
+}
+
+OFB_API int ofb_corr_lookup_backward_f32(const ofb_pyramid* d_pyr, const float* coords, const float* d_out, int B, int h,
+                                         int w, int radius, void* stream) {
+    return ofb_corr_lookup_backward(d_pyr, coords, d_out, OFB_DTYPE_F32, B, h, w, radius, stream);
 }

@@ -19,7 +19,8 @@
 // with a_i, b_i the two columns of x tap i, and (wy_rj, sy_rj) = (wy0_j, -1) when r is the upper row of sample j,
 // (wy1_j, +1) when it is its lower row (a row serves at most three samples: j = r, r - 1, r - 2).  The levels are
 // summed in shared memory in level order and d coords is written once, without atomics: the same bits on every run.
-// HBM roofline per query: L*(2r+2)^2*esize window + 4*L*(2r+1)^2 d_out + 8 coordinates read, 8 written.
+// d_out is read in fp32, fp16 or bf16 (the dtype of the forward's output) and widened exactly on load.
+// HBM roofline per query: L*(2r+2)^2*esize window + L*(2r+1)^2*(d_out esize) + 8 coordinates read, 8 written.
 #include "common.cuh"
 
 namespace {
@@ -69,10 +70,10 @@ __device__ __forceinline__ void load_row(float (&px)[WIN], const T* slice, const
     }
 }
 
-template <int R, typename T, bool CHUNKED>
+template <int R, typename T, bool CHUNKED, typename G>
 __global__ void __launch_bounds__(128, 4) lookup_coords_bwd_kernel(const __grid_constant__ CoordsBwdParams P,
                                                                 const float* __restrict__ coords,
-                                                                const float* __restrict__ d_out,
+                                                                const G* __restrict__ d_out,
                                                                 float* __restrict__ d_coords) {
     constexpr int D = 2 * R + 1, DD = D * D, WIN = D + 2;
     constexpr int GROUPS_UNROLLED = CHUNKED ? (WIN + 2) / 3 : 1;
@@ -95,7 +96,7 @@ __global__ void __launch_bounds__(128, 4) lookup_coords_bwd_kernel(const __grid_
             const int xs = tx.anchor, ys = ty.anchor;
             const T* slice = reinterpret_cast<const T*>(P.base[l]) + q * P.q_stride[l];
             // d_out of window cell (i, j) at g0[(i*D + j) * HW]
-            const float* g0 = d_out + (b * (long long)(P.levels * DD) + (long long)l * DD) * HW + p;
+            const G* g0 = d_out + (b * (long long)(P.levels * DD) + (long long)l * DD) * HW + p;
             // window rows some sample reads (tap j: rows j + d[j] and j + d[j] + 1); the others are never loaded, so
             // an inf stored there is not multiplied by an exact-zero coefficient
             unsigned used_rows = 0;
@@ -130,7 +131,7 @@ __global__ void __launch_bounds__(128, 4) lookup_coords_bwd_kernel(const __grid_
                     }
                     if (r < D) {
 #pragma unroll
-                        for (int i = 0; i < D; ++i) g[c][i] = __ldg(g0 + (long long)(i * D + r) * HW);
+                        for (int i = 0; i < D; ++i) g[c][i] = ofb::ld_f32(g0 + (long long)(i * D + r) * HW);
                     }
                     // row r is the upper row of sample j = r - k when k = d[j], its lower row when k = d[j] + 1
                     float row_x = 0.0f, row_y = 0.0f;
@@ -171,16 +172,16 @@ __global__ void __launch_bounds__(128, 4) lookup_coords_bwd_kernel(const __grid_
     }
 }
 
-template <int R, typename T, bool CHUNKED>
-int launch(const CoordsBwdParams& P, const float* coords, const float* d_out, float* d_coords, int blocks,
+template <int R, typename T, bool CHUNKED, typename G>
+int launch(const CoordsBwdParams& P, const float* coords, const G* d_out, float* d_coords, int blocks,
            cudaStream_t st) {
-    lookup_coords_bwd_kernel<R, T, CHUNKED><<<blocks, 32 * P.levels, 0, st>>>(P, coords, d_out, d_coords);
+    lookup_coords_bwd_kernel<R, T, CHUNKED, G><<<blocks, 32 * P.levels, 0, st>>>(P, coords, d_out, d_coords);
     OFB_LAUNCH_CHECK();
     return OFB_OK;
 }
 
-template <typename T, bool CHUNKED>
-int launch_radius(const CoordsBwdParams& P, const float* coords, const float* d_out, float* d_coords, int radius,
+template <typename T, bool CHUNKED, typename G>
+int launch_radius(const CoordsBwdParams& P, const float* coords, const G* d_out, float* d_coords, int radius,
                   int blocks, cudaStream_t st) {
     switch (radius) {
         case 0: return launch<0, T, CHUNKED>(P, coords, d_out, d_coords, blocks, st);
@@ -191,10 +192,24 @@ int launch_radius(const CoordsBwdParams& P, const float* coords, const float* d_
     }
 }
 
+template <typename G>
+int launch_pyramid(const CoordsBwdParams& P, bool chunked, const float* coords, const G* d_out, float* d_coords,
+                   int radius, int blocks, cudaStream_t st) {
+    if (P.dtype == OFB_DTYPE_F32)
+        return launch_radius<float, false>(P, coords, d_out, d_coords, radius, blocks, st);
+    if (P.dtype == OFB_DTYPE_F16)
+        return chunked ? launch_radius<__half, true>(P, coords, d_out, d_coords, radius, blocks, st)
+                       : launch_radius<__half, false>(P, coords, d_out, d_coords, radius, blocks, st);
+    return chunked ? launch_radius<__nv_bfloat16, true>(P, coords, d_out, d_coords, radius, blocks, st)
+                   : launch_radius<__nv_bfloat16, false>(P, coords, d_out, d_coords, radius, blocks, st);
+}
+
 }  // namespace
 
-OFB_API int ofb_corr_lookup_coords_backward(const ofb_pyramid* pyr, const float* coords, const float* d_out,
-                                            float* d_coords, int B, int h, int w, int radius, void* stream) {
+OFB_API int ofb_corr_lookup_coords_backward_from(const ofb_pyramid* pyr, const float* coords, const void* d_out,
+                                                 int d_out_dtype, float* d_coords, int B, int h, int w, int radius,
+                                                 void* stream) {
+    if (!ofb_float_dtype(d_out_dtype)) return OFB_EINVAL;
     if (B == 0) return OFB_OK;   // nothing to do: empty tensors have no storage, their pointers may be null
     if (!pyr || !coords || !d_out || !d_coords || B < 0 || h <= 0 || w <= 0) return OFB_EINVAL;
     if (radius < 0 || 2 * radius + 1 > MAX_D) return OFB_EUNSUPPORTED;
@@ -206,12 +221,14 @@ OFB_API int ofb_corr_lookup_coords_backward(const ofb_pyramid* pyr, const float*
     P.B = B; P.h = h; P.w = w;
     const long long blocks = (Q + 31) / 32;
     if (blocks > 0x7fffffffLL) return OFB_EUNSUPPORTED;
-    cudaStream_t st = (cudaStream_t)stream;
-    if (P.dtype == OFB_DTYPE_F32)
-        return launch_radius<float, false>(P, coords, d_out, d_coords, radius, (int)blocks, st);
-    if (P.dtype == OFB_DTYPE_F16)
-        return chunked ? launch_radius<__half, true>(P, coords, d_out, d_coords, radius, (int)blocks, st)
-                       : launch_radius<__half, false>(P, coords, d_out, d_coords, radius, (int)blocks, st);
-    return chunked ? launch_radius<__nv_bfloat16, true>(P, coords, d_out, d_coords, radius, (int)blocks, st)
-                   : launch_radius<__nv_bfloat16, false>(P, coords, d_out, d_coords, radius, (int)blocks, st);
+    return ofb_dispatch_dtype(d_out_dtype, [&](auto g) {
+        using G = decltype(g);
+        return launch_pyramid(P, chunked, coords, static_cast<const G*>(d_out), d_coords, radius, (int)blocks,
+                              (cudaStream_t)stream);
+    });
+}
+
+OFB_API int ofb_corr_lookup_coords_backward(const ofb_pyramid* pyr, const float* coords, const float* d_out,
+                                            float* d_coords, int B, int h, int w, int radius, void* stream) {
+    return ofb_corr_lookup_coords_backward_from(pyr, coords, d_out, OFB_DTYPE_F32, d_coords, B, h, w, radius, stream);
 }

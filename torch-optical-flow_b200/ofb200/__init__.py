@@ -78,9 +78,13 @@ SIGNATURES = {
     "ofb_pool_cast_bf16": (_i, [_vp, _i, _vp, _i, _i, _i, _i, _i, _i, _vp]),
     "ofb_pool_adjoint_f32": (_i, [ctypes.POINTER(_vp), _vp, _i, _i, _i, _i, _i, _vp]),
     "ofb_corr_lookup_backward_f32": (_i, [ctypes.POINTER(Pyramid), _vp, _vp, _i, _i, _i, _i, _vp]),
+    "ofb_corr_lookup_backward": (_i, [ctypes.POINTER(Pyramid), _vp, _vp, _i, _i, _i, _i, _i, _vp]),
     "ofb_corr_lookup_coords_backward": (_i, [ctypes.POINTER(Pyramid), _vp, _vp, _vp, _i, _i, _i, _i, _vp]),
+    "ofb_corr_lookup_coords_backward_from": (_i, [ctypes.POINTER(Pyramid), _vp, _vp, _i, _vp, _i, _i, _i, _i, _vp]),
     "ofb_corr_lookup": (_i, [ctypes.POINTER(Pyramid), _vp, _vp, _vp, _vp, _i, _i, _i, _i, _vp]),
+    "ofb_corr_lookup_to": (_i, [ctypes.POINTER(Pyramid), _vp, _vp, _i, _vp, _vp, _i, _i, _i, _i, _vp]),
     "ofb_corr_lookup_ondemand": (_i, [_vp, ctypes.POINTER(_vp), _vp, _vp, _i, _i, _i, _i, _i, _i, _vp]),
+    "ofb_corr_lookup_ondemand_to": (_i, [_vp, ctypes.POINTER(_vp), _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _vp]),
     "ofb_bilinear_sampler_f32": (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _vp]),
 }
 

@@ -12,6 +12,11 @@ Differences a caller can observe, all deliberate (DESIGN.md):
     K3 coordinate-backward launch per lookup, only when the coordinates require grad; RAFT itself detaches them,
     raft.py:127).  A coordinate whose window leaves the floor guard, or is non-finite, gets gradient 0 at that level
     (the reference: NaN for NaN).  Forward-only, as before: `return_index=True` lookups and `on_demand=True` blocks.
+  * the lookup's output is fp32, as the reference's (corr.py:77), unless `lookup_dtype` (or OFB200_LOOKUP_DTYPE) asks
+    for fp16 or bf16: each fp32 sample rounded once, the same bits as the fp32 output cast to that dtype.  "autocast"
+    picks the dtype CUDA autocast would cast the output to before its only consumer, BasicMotionEncoder.convc1
+    (update.py:114), so that cast and its backward disappear while convc1 receives the same bits; the gradient is then
+    read back in that dtype, widened exactly.
 """
 import ctypes
 import math
@@ -31,6 +36,19 @@ def _default_pyramid_dtype() -> torch.dtype:
     if name in ("fp16", "f16", "float16", "half"):
         return torch.float16
     return torch.bfloat16
+
+
+_LOOKUP_DTYPES = {"fp32": torch.float32, "f32": torch.float32, "float32": torch.float32, "fp16": torch.float16,
+                  "f16": torch.float16, "float16": torch.float16, "half": torch.float16, "bf16": torch.bfloat16,
+                  "bfloat16": torch.bfloat16, "autocast": "autocast"}
+
+
+def _default_lookup_dtype():
+    """OFB200_LOOKUP_DTYPE=fp32|fp16|bf16|autocast; unset means fp32."""
+    name = os.environ.get("OFB200_LOOKUP_DTYPE", "").lower() or "fp32"
+    if name not in _LOOKUP_DTYPES:
+        raise ValueError(f"OFB200_LOOKUP_DTYPE must be fp32, fp16, bf16 or autocast, got {name!r}")
+    return _LOOKUP_DTYPES[name]
 
 
 # optional ofb200.runner.KernelTimers: when set (bench.py), the prep launches and the pyramid kernel get their own
@@ -267,16 +285,16 @@ class _LookupFn(torch.autograd.Function):
     grad) and the scatter into the block's gradient pyramid (when there is a handle, i.e. the feature maps require
     grad).  The context never keeps the CorrBlock (see _GradState).  Only a lookup whose coordinates require grad keeps
     the stored pyramid's buffers, which its backward reads: with detached coordinates the multi-GB pyramid is freed as
-    soon as the block is dropped, while the graph lives on."""
+    soon as the block is dropped, while the graph lives on.  The output gradient is read in its own dtype."""
 
     @staticmethod
-    def forward(ctx, block, coords_d, handle):
+    def forward(ctx, block, coords_d, handle, out_dtype):
         ctx.state = block._grad
         if ctx.needs_input_grad[1]:
             ctx.pyr, ctx.buffers = block._pyr, block._buffers
         ctx.shape, ctx.dev, ctx.radius = block._shape, block._dev, block.radius
         ctx.save_for_backward(coords_d)
-        return block._lookup(coords_d.detach(), None, None, None)
+        return block._lookup(coords_d.detach(), None, None, None, out_dtype)
 
     @staticmethod
     def backward(ctx, grad_out):
@@ -284,21 +302,22 @@ class _LookupFn(torch.autograd.Function):
         (coords_d,) = ctx.saved_tensors
         b, c, h, w = ctx.shape
         g = grad_out.contiguous()
+        g_dt = _IN_DTYPES[g.dtype]
         d_coords = None
         with torch.cuda.device(ctx.dev):
             if ctx.needs_input_grad[1]:
                 d_coords = torch.empty((b, 2, h, w), dtype=torch.float32, device=ctx.dev)
-                rc = ofb200.load().ofb_corr_lookup_coords_backward(
-                    ctypes.byref(ctx.pyr), ofb200.ptr(coords_d), ofb200.ptr(g), ofb200.ptr(d_coords), b, h, w, ctx.radius,
-                    ofb200.stream_ptr())
-                ofb200.check(rc, "ofb_corr_lookup_coords_backward")
+                rc = ofb200.load().ofb_corr_lookup_coords_backward_from(
+                    ctypes.byref(ctx.pyr), ofb200.ptr(coords_d), ofb200.ptr(g), g_dt, ofb200.ptr(d_coords), b, h, w,
+                    ctx.radius, ofb200.stream_ptr())
+                ofb200.check(rc, "ofb_corr_lookup_coords_backward_from")
             if st is not None:
                 desc = st.grad_pyramid()
-                rc = ofb200.load().ofb_corr_lookup_backward_f32(
-                    ctypes.byref(desc), ofb200.ptr(coords_d), ofb200.ptr(g), b, h, w, st.radius, ofb200.stream_ptr())
-                ofb200.check(rc, "ofb_corr_lookup_backward_f32")
+                rc = ofb200.load().ofb_corr_lookup_backward(
+                    ctypes.byref(desc), ofb200.ptr(coords_d), ofb200.ptr(g), g_dt, b, h, w, st.radius, ofb200.stream_ptr())
+                ofb200.check(rc, "ofb_corr_lookup_backward")
         handle_grad = torch.zeros(1, dtype=torch.float32, device=ctx.dev) if st is not None else None
-        return None, d_coords, handle_grad
+        return None, d_coords, handle_grad, None
 
 
 class CorrBlock:
@@ -313,6 +332,7 @@ class CorrBlock:
         builder: str = "auto",
         cta_group: int = 0,
         on_demand: Optional[bool] = None,
+        lookup_dtype=None,
     ) -> None:
         """fmap1, fmap2 (B, C, h, w) in fp32 / bf16 / fp16 (reference corr.py:38-54).
 
@@ -321,9 +341,18 @@ class CorrBlock:
         OFB200_PYRAMID_DTYPE=bf16|fp16|fp32 sets the default; ignored with `on_demand`), `builder`, `cta_group` (K2
         launch mode), and `on_demand=True` (or OFB200_CORR_ON_DEMAND=1): nothing is materialised -- every lookup
         evaluates the correlation values of its own windows from the operand maps (ofb_corr_lookup_ondemand; 22 MB
-        instead of 2.83 GB per 1080p pair, slower per lookup; forward-only)."""
+        instead of 2.83 GB per 1080p pair, slower per lookup; forward-only).  `lookup_dtype`: the dtype of every lookup's
+        output -- torch.float32 (default, the reference's), torch.float16, torch.bfloat16, or "autocast", resolved at
+        each call to torch.get_autocast_dtype("cuda") while CUDA autocast is enabled and to fp32 otherwise;
+        OFB200_LOOKUP_DTYPE=fp32|fp16|bf16|autocast sets the default."""
         self.num_levels = num_levels
         self.radius = radius
+        if lookup_dtype is None:
+            lookup_dtype = _default_lookup_dtype()
+        if not (lookup_dtype == "autocast" or lookup_dtype in _IN_DTYPES):
+            raise NotImplementedError('CorrBlock: lookup_dtype must be torch.float32, torch.float16, torch.bfloat16 or '
+                                      '"autocast"')
+        self.lookup_dtype = lookup_dtype
         if fmap1.shape != fmap2.shape or fmap1.dim() != 4:
             raise RuntimeError("CorrBlock: fmap1 and fmap2 must both be (B, C, h, w)")
         if not (1 <= num_levels <= ofb200.MAX_LEVELS):
@@ -451,14 +480,26 @@ class CorrBlock:
             self._views = views
         return self._views
 
+    def out_dtype(self) -> torch.dtype:
+        """The dtype a lookup made now returns: `lookup_dtype`, with "autocast" resolved."""
+        if self.lookup_dtype != "autocast":
+            return self.lookup_dtype
+        if not torch.is_autocast_enabled("cuda"):
+            return torch.float32
+        dt = torch.get_autocast_dtype("cuda")
+        if dt not in _IN_DTYPES:
+            raise NotImplementedError(f"CorrBlock: no lookup output in the autocast dtype {dt}")
+        return dt
+
     def __call__(self, coords: Tensor, return_index: bool = False, out: Optional[Tensor] = None):
-        """Index the pyramid (reference corr.py:56-77): coords (B, 2, h, w) -> (B, L*(2r+1)^2, h, w) fp32.
+        """Index the pyramid (reference corr.py:56-77): coords (B, 2, h, w) -> (B, L*(2r+1)^2, h, w) in out_dtype()
+        (fp32 unless `lookup_dtype` says otherwise).
 
         Differentiable with respect to `coords` when they require grad (host coordinates get a host gradient) and to
         the feature maps when those did at construction.  `return_index=True` (extension) also returns the floor
         indices (B*h*w, L, 2, 2r+1) int32 and the validity mask (B*h*w, L, (2r+1)^2) uint8 the kernel used; such a
         call, and every lookup of an `on_demand=True` block, is forward-only: its output carries no gradient.  `out`
-        (extension) is an optional preallocated contiguous fp32 CUDA tensor of the output shape; on the
+        (extension) is an optional preallocated contiguous CUDA tensor of the output shape and dtype; on the
         differentiable path it receives the values and the returned tensor carries the graph."""
         b, c, h, w = self._shape
         if tuple(coords.shape) != (b, 2, h, w):
@@ -474,12 +515,13 @@ class CorrBlock:
         d = 2 * self.radius + 1
         lvls = self.num_levels
         oshape = (b, lvls * d * d, h, w)
-        if out is not None and (tuple(out.shape) != oshape or out.dtype != torch.float32 or not out.is_cuda
+        out_dtype = self.out_dtype()
+        if out is not None and (tuple(out.shape) != oshape or out.dtype != out_dtype or not out.is_cuda
                                 or not out.is_contiguous()):
-            raise RuntimeError(f"CorrBlock: out must be a contiguous fp32 CUDA tensor of shape {oshape}")
+            raise RuntimeError(f"CorrBlock: out must be a contiguous {out_dtype} CUDA tensor of shape {oshape}")
         idx = valid = None
         if diff_coords or (self._handle is not None and torch.is_grad_enabled() and not return_index):
-            res = _LookupFn.apply(self, coords_d, self._handle)
+            res = _LookupFn.apply(self, coords_d, self._handle, out_dtype)
             if out is not None:
                 out.copy_(res.detach())                       # the preallocated buffer is filled, the graph keeps `res`
             out = res
@@ -488,33 +530,36 @@ class CorrBlock:
                 if return_index:
                     idx = torch.empty((b * h * w, lvls, 2, d), dtype=torch.int32, device=self._dev)
                     valid = torch.empty((b * h * w, lvls, d * d), dtype=torch.uint8, device=self._dev)
-            out = self._lookup(coords_d, out, idx, valid)
+            out = self._lookup(coords_d, out, idx, valid, out_dtype)
         if on_host:
             out = out.cpu()
             idx = idx.cpu() if idx is not None else None
             valid = valid.cpu() if valid is not None else None
         return (out, idx, valid) if return_index else out
 
-    def _lookup(self, coords_d: Tensor, out: Optional[Tensor], idx: Optional[Tensor], valid: Optional[Tensor]) -> Tensor:
+    def _lookup(self, coords_d: Tensor, out: Optional[Tensor], idx: Optional[Tensor], valid: Optional[Tensor],
+                out_dtype: torch.dtype = torch.float32) -> Tensor:
         b, c, h, w = self._shape
         d = 2 * self.radius + 1
+        out_dt = _IN_DTYPES[out_dtype]
         with torch.cuda.device(self._dev):
             if out is None:
-                out = torch.empty((b, self.num_levels * d * d, h, w), dtype=torch.float32, device=self._dev)
+                out = torch.empty((b, self.num_levels * d * d, h, w), dtype=out_dtype, device=self._dev)
             if self._on_demand is not None:
                 if idx is not None or valid is not None:
                     raise NotImplementedError("CorrBlock(on_demand=True): return_index is not available")
                 a_km, levels = self._on_demand
                 ptrs = (ctypes.c_void_p * ofb200.MAX_LEVELS)(*[t.data_ptr() for t in levels])
-                rc = ofb200.load().ofb_corr_lookup_ondemand(ofb200.ptr(a_km), ptrs, ofb200.ptr(coords_d), ofb200.ptr(out),
-                                                            b, c, h, w, self.num_levels, self.radius, ofb200.stream_ptr())
-                ofb200.check(rc, "ofb_corr_lookup_ondemand")
+                rc = ofb200.load().ofb_corr_lookup_ondemand_to(ofb200.ptr(a_km), ptrs, ofb200.ptr(coords_d), ofb200.ptr(out),
+                                                               out_dt, b, c, h, w, self.num_levels, self.radius,
+                                                               ofb200.stream_ptr())
+                ofb200.check(rc, "ofb_corr_lookup_ondemand_to")
                 return out
-            rc = ofb200.load().ofb_corr_lookup(
-                ctypes.byref(self._pyr), ofb200.ptr(coords_d), ofb200.ptr(out), ofb200.ptr(idx), ofb200.ptr(valid),
+            rc = ofb200.load().ofb_corr_lookup_to(
+                ctypes.byref(self._pyr), ofb200.ptr(coords_d), ofb200.ptr(out), out_dt, ofb200.ptr(idx), ofb200.ptr(valid),
                 b, h, w, self.radius, ofb200.stream_ptr(),
             )
-        ofb200.check(rc, "ofb_corr_lookup")
+        ofb200.check(rc, "ofb_corr_lookup_to")
         return out
 
     @staticmethod
