@@ -45,7 +45,7 @@ extern "C" {
 #define OFB_DTYPE_F32 0
 #define OFB_DTYPE_BF16 1
 #define OFB_DTYPE_F16 2 /* feature maps and operands of ofb_corr_prep_from / _to, correlation pyramids, mask of
-                           ofb_convex_upsample, ofb_scale_flow, the lookup's output and its gradient */
+                           ofb_convex_upsample and its gradient, ofb_scale_flow, the lookup's output and its gradient */
 #define OFB_DTYPE_F64 3 /* ofb_scale_flow only */
 
 #define OFB_MAX_LEVELS 4
@@ -128,6 +128,14 @@ int ofb_convex_upsample(const float* flow, const void* mask, int mask_dtype, flo
 int ofb_convex_upsample_backward_f32(const float* flow, const float* mask, const float* d_out,
                                      float* d_flow_or_null, float* d_mask_or_null, int N, int h, int w,
                                      void* stream);
+/* The same backward with the mask in its own precision, mask_dtype OFB_DTYPE_F32 (= ofb_convex_upsample_backward_f32),
+ * BF16 or F16; anything else is OFB_EINVAL.  d_mask_or_null is written in that dtype: each logit is widened exactly, the
+ * gradient computed in fp32 with the arithmetic of the fp32 form and rounded once to nearest even -- the bits of the
+ * fp32 gradient cast to the mask's dtype, which is what autocast's cast hands the mask head under `precision: 16`
+ * (fp16: beyond +-65504 is inf).  flow, d_out and d_flow_or_null stay fp32.  A mask or d_mask not aligned to its
+ * element size is OFB_EALIGN. */
+int ofb_convex_upsample_backward(const float* flow, const void* mask, int mask_dtype, const float* d_out,
+                                 float* d_flow_or_null, void* d_mask_or_null, int N, int h, int w, void* stream);
 
 /* ---------------------------------------------------------------------------------------
  * K4c  end-point-error reduction.  Replaces AverageEndPointError.update

@@ -92,10 +92,14 @@ __global__ void __launch_bounds__(NT) convex_upsample_kernel(const float* __rest
 // neighbourhood) and g = d_out at the fine pixel:
 //   a_k = g_x v_k,x + g_y v_k,y ;  d_mask_k = p_k (a_k - sum_m p_m a_m)
 //   d_flow[c, y+ky-1, x+kx-1] += 8 * sum_{i,j} p_k g_c        (18 red.global.add.f32 per thread; d_flow is small)
+// The mask and d_mask share the element type TM, as in the forward: a 16-bit logit is widened exactly, d_mask is
+// computed in fp32 and rounded once (ofb::narrow), the bits of the fp32 gradient cast to the mask's dtype -- what
+// autocast's cast backward hands the mask head.  d_out, flow and d_flow stay fp32 (the upsampled flow is fp32).
+template <typename TM>
 __global__ void __launch_bounds__(NT) convex_upsample_bwd_kernel(const float* __restrict__ flow,
-                                                                 const float* __restrict__ mask,
+                                                                 const TM* __restrict__ mask,
                                                                  const float* __restrict__ d_out,
-                                                                 float* __restrict__ d_flow, float* __restrict__ d_mask,
+                                                                 float* __restrict__ d_flow, TM* __restrict__ d_mask,
                                                                  int N, int h, int w) {
     const int hw = h * w;
     const int lane_p = threadIdx.x % PX;
@@ -136,7 +140,7 @@ __global__ void __launch_bounds__(NT) convex_upsample_bwd_kernel(const float* __
     for (int j = 0; j < 8; ++j) {
         float m[9];
 #pragma unroll
-        for (int k = 0; k < 9; ++k) m[k] = __ldg(mask + moff + (size_t)(k * 64 + j) * hw);
+        for (int k = 0; k < 9; ++k) m[k] = ofb::ld_f32(mask + moff + (size_t)(k * 64 + j) * hw);
         float mx = m[0];
 #pragma unroll
         for (int k = 1; k < 9; ++k) mx = fmaxf(mx, m[k]);
@@ -155,7 +159,7 @@ __global__ void __launch_bounds__(NT) convex_upsample_bwd_kernel(const float* __
         }
         if (d_mask) {
 #pragma unroll
-            for (int k = 0; k < 9; ++k) d_mask[moff + (size_t)(k * 64 + j) * hw] = m[k] * (a[k] - dot);
+            for (int k = 0; k < 9; ++k) d_mask[moff + (size_t)(k * 64 + j) * hw] = ofb::narrow<TM>(m[k] * (a[k] - dot));
         }
     }
     if (d_flow) {
@@ -201,17 +205,28 @@ OFB_API int ofb_convex_upsample_f32(const float* flow, const float* mask, float*
     return ofb_convex_upsample(flow, mask, OFB_DTYPE_F32, out, N, h, w, stream);
 }
 
-OFB_API int ofb_convex_upsample_backward_f32(const float* flow, const float* mask, const float* d_out,
-                                             float* d_flow_or_null, float* d_mask_or_null, int N, int h, int w,
-                                             void* stream) {
+OFB_API int ofb_convex_upsample_backward(const float* flow, const void* mask, int mask_dtype, const float* d_out,
+                                         float* d_flow_or_null, void* d_mask_or_null, int N, int h, int w, void* stream) {
+    if (!ofb_float_dtype(mask_dtype)) return OFB_EINVAL;
     if (N == 0 || h == 0 || w == 0) return OFB_OK;   // nothing to do: empty tensors have no storage, their pointers may be null
     if (!flow || !mask || !d_out || N < 0 || h < 0 || w < 0) return OFB_EINVAL;
     if ((size_t)N * h * w == 0 || (!d_flow_or_null && !d_mask_or_null)) return OFB_OK;
     if (N > 65535) return OFB_EUNSUPPORTED;
     if (reinterpret_cast<uintptr_t>(d_out) & 15) return OFB_EALIGN;
+    const uintptr_t elem = mask_dtype == OFB_DTYPE_F32 ? 3 : 1;
+    if ((reinterpret_cast<uintptr_t>(mask) | reinterpret_cast<uintptr_t>(d_mask_or_null)) & elem) return OFB_EALIGN;
     dim3 grid((h * w + PX - 1) / PX, N);
-    convex_upsample_bwd_kernel<<<grid, NT, 0, (cudaStream_t)stream>>>(flow, mask, d_out, d_flow_or_null, d_mask_or_null,
-                                                                     N, h, w);
-    OFB_LAUNCH_CHECK();
-    return OFB_OK;
+    return ofb_dispatch_dtype(mask_dtype, [&](auto t) {
+        using TM = decltype(t);
+        convex_upsample_bwd_kernel<TM><<<grid, NT, 0, (cudaStream_t)stream>>>(
+            flow, static_cast<const TM*>(mask), d_out, d_flow_or_null, static_cast<TM*>(d_mask_or_null), N, h, w);
+        OFB_LAUNCH_CHECK();
+        return OFB_OK;
+    });
+}
+
+OFB_API int ofb_convex_upsample_backward_f32(const float* flow, const float* mask, const float* d_out,
+                                             float* d_flow_or_null, float* d_mask_or_null, int N, int h, int w,
+                                             void* stream) {
+    return ofb_convex_upsample_backward(flow, mask, OFB_DTYPE_F32, d_out, d_flow_or_null, d_mask_or_null, N, h, w, stream);
 }

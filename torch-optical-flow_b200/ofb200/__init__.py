@@ -64,6 +64,7 @@ SIGNATURES = {
     "ofb_sequence_loss_backward_f32": (_i, [ctypes.POINTER(_vp), ctypes.POINTER(_vp), _i, _vp, _vp, _vp, _i, _i, _i,
                                             ctypes.c_double, _f, _vp]),
     "ofb_convex_upsample_backward_f32": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, _vp]),
+    "ofb_convex_upsample_backward": (_i, [_vp, _vp, _i, _vp, _vp, _vp, _i, _i, _i, _vp]),
     "ofb_sequence_loss_f32": (_i, [ctypes.POINTER(_vp), _i, _vp, _vp, _vp, _i, _i, _i, ctypes.c_double, _f, _vp]),
     "ofb_pyramid_layout": (_i, [_i, _i, _i, _i, ctypes.POINTER(Pyramid), ctypes.POINTER(_i64 * MAX_LEVELS)]),
     "ofb_corr_prep_bf16": (_i, [_vp, _vp, _i, _i, _i, _i, _i, _f, _vp]),

@@ -21,8 +21,9 @@ def upsample_flow(flow: Tensor, mask: Tensor) -> Tensor:
     """Upsample flow field [H/8, W/8, 2] -> [H, W, 2] using convex combination (reference raft.py:73-85).
 
     flow (N, 2, h, w) fp32, mask (N, 576, h, w) -> (N, 2, 8h, 8w) fp32.  The mask may be fp32, bf16 or fp16 (the mask
-    head's output under `precision: 16`) and is read as it is; a half-precision mask that requires grad is cast to fp32
-    first (the backward kernel writes an fp32 gradient)."""
+    head's output under `precision: 16`) and is read as it is, in both directions: the backward keeps the caller's mask
+    and writes its gradient in the mask's dtype, the bits of the fp32 gradient cast to it (what autocast's cast around
+    the reference's fp32 softmax, raft.py:78, hands the mask head)."""
     n, _, h, w = flow.shape
     if flow.shape[1] != 2 or tuple(mask.shape) != (n, 576, h, w):
         raise RuntimeError(f"upsample_flow: expected flow (N,2,h,w) and mask (N,576,h,w), got "
@@ -30,8 +31,6 @@ def upsample_flow(flow: Tensor, mask: Tensor) -> Tensor:
     _check_f32(flow)
     if mask.dtype not in _MASK_DTYPES:
         raise NotImplementedError(f"upsample_flow: mask must be fp32, bf16 or fp16, got {mask.dtype}")
-    if mask.dtype != torch.float32 and torch.is_grad_enabled() and mask.requires_grad:
-        mask = mask.float()
 
     def run(flow_d: Tensor, mask_d: Tensor):
         flow_d, mask_d = flow_d.contiguous(), aligned16(mask_d)
@@ -46,15 +45,14 @@ def upsample_flow(flow: Tensor, mask: Tensor) -> Tensor:
         """d up / d flow and d up / d mask: autograd through softmax, unfold and the weighted sum (raft.py:77-85)."""
         flow_d, mask_d = saved
         with torch.cuda.device(flow_d.device):
-            mask_f = mask_d if mask_d.dtype == torch.float32 else mask_d.float()      # the backward kernel reads fp32
-            flow_c, mask_c, grad_c = flow_d.contiguous(), aligned16(mask_f), aligned16(grad_out)
+            flow_c, mask_c, grad_c = flow_d.contiguous(), aligned16(mask_d), aligned16(grad_out)
             d_flow = torch.zeros((n, 2, h, w), dtype=torch.float32, device=flow_c.device) if needs[0] else None
-            d_mask = torch.empty((n, 576, h, w), dtype=torch.float32, device=flow_c.device) if needs[1] else None
-            rc = ofb200.load().ofb_convex_upsample_backward_f32(
-                ofb200.ptr(flow_c), ofb200.ptr(mask_c), ofb200.ptr(grad_c), ofb200.ptr(d_flow), ofb200.ptr(d_mask),
-                n, h, w, ofb200.stream_ptr(),
+            d_mask = torch.empty((n, 576, h, w), dtype=mask_c.dtype, device=flow_c.device) if needs[1] else None
+            rc = ofb200.load().ofb_convex_upsample_backward(
+                ofb200.ptr(flow_c), ofb200.ptr(mask_c), _MASK_DTYPES[mask_c.dtype], ofb200.ptr(grad_c), ofb200.ptr(d_flow),
+                ofb200.ptr(d_mask), n, h, w, ofb200.stream_ptr(),
             )
-            ofb200.check(rc, "ofb_convex_upsample_backward_f32")
+            ofb200.check(rc, "ofb_convex_upsample_backward")
         return d_flow, d_mask
 
     return _run(run, "upsample_flow", flow, mask, bwd=backward)
