@@ -45,7 +45,8 @@ extern "C" {
 #define OFB_DTYPE_F32 0
 #define OFB_DTYPE_BF16 1
 #define OFB_DTYPE_F16 2 /* feature maps and operands of ofb_corr_prep_from / _to, correlation pyramids, mask of
-                           ofb_convex_upsample and its gradient, ofb_scale_flow, the lookup's output and its gradient */
+                           ofb_convex_upsample and its gradient, ofb_scale_flow, the lookup's output and its gradient,
+                           the frame and flow of ofb_warp / ofb_warp_backward and the flow's gradient */
 #define OFB_DTYPE_F64 3 /* ofb_scale_flow only */
 
 #define OFB_MAX_LEVELS 4
@@ -74,6 +75,16 @@ int64_t ofb_launch_count(void);
 int ofb_warp_f32(const float* frame, const float* flow, float* out, uint8_t* valid_or_null,
                  int B, int C, int H, int W, int mode, int padding_mode, int align_corners,
                  int channels_last, int variant, float flow_mul_x, float flow_mul_y, void* stream);
+/* The same warp with the frame and the flow each in fp32, bf16 or fp16 (frame_dtype, flow_dtype: OFB_DTYPE_F32, BF16
+ * or F16; anything else is OFB_EINVAL, checked before any other argument).  Replaces operator.py:8-56 as
+ * ofb_warp_f32 does, on the inputs autocast hands grid_sample: each 16-bit element is widened exactly and the fp32
+ * kernel's arithmetic runs on it, so out (always fp32) and valid_or_null are, bit for bit, those of ofb_warp_f32 on
+ * the fp32 copies of frame and flow.  With fp32 for both it is ofb_warp_f32.  A 16-bit frame or flow not 2-byte
+ * aligned is OFB_EALIGN; variants 2 and 4 read fp32 frames and flows only (otherwise OFB_EUNSUPPORTED) and auto never
+ * picks them for 16-bit inputs. */
+int ofb_warp(const void* frame, int frame_dtype, const void* flow, int flow_dtype, float* out,
+             uint8_t* valid_or_null, int B, int C, int H, int W, int mode, int padding_mode, int align_corners,
+             int channels_last, int variant, float flow_mul_x, float flow_mul_y, void* stream);
 
 /* Backward of ofb_warp_f32 (bilinear, NCHW): what autograd computes for the reference's warp
  * (operator.py:28-33: grid_sample's backward, then d grid / d flow = 1 through warp_grid :56 and the
@@ -84,6 +95,15 @@ int ofb_warp_backward_f32(const float* frame, const float* flow, const float* d_
                           float* d_frame_or_null, float* d_flow_or_null, int B, int C, int H, int W,
                           int padding_mode, int align_corners, float flow_mul_x, float flow_mul_y,
                           void* stream);
+/* The backward of ofb_warp (operator.py:8-56), frame and flow each in fp32, bf16 or fp16 as there (OFB_EINVAL for any
+ * other dtype, before any other argument; OFB_EALIGN for a 16-bit frame, flow or d_flow not 2-byte aligned).  d_out
+ * and d_frame_f32_or_null stay fp32: d_frame is accumulated in fp32 whatever the frame's dtype, and rounding it to that
+ * dtype once afterwards gives what autocast's cast backward hands the frame.  d_flow_or_null is written in flow_dtype,
+ * the fp32 gradient rounded once to nearest even (fp16: beyond +-65504 is inf).  With fp32 for both it is
+ * ofb_warp_backward_f32. */
+int ofb_warp_backward(const void* frame, int frame_dtype, const void* flow, int flow_dtype, const float* d_out,
+                      float* d_frame_f32_or_null, void* d_flow_or_null, int B, int C, int H, int W,
+                      int padding_mode, int align_corners, float flow_mul_x, float flow_mul_y, void* stream);
 
 /* warp_grid alone (operator.py:36-56): flow (B,H,W,2) -> grid (B,H,W,2). */
 int ofb_warp_grid_f32(const float* flow_bhw2, float* grid_bhw2, int B, int H, int W, void* stream);

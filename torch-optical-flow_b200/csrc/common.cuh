@@ -225,19 +225,31 @@ __device__ __forceinline__ BilinearTaps bilinear_taps(float ix, float iy, int H,
     return t;
 }
 
+// input element -> fp32: frames, flows, feature maps and mask logits arrive in fp32, or in half precision from an
+// autocast caller
+__device__ __forceinline__ float ld_f32(const float* p) { return __ldg(p); }
+__device__ __forceinline__ float ld_f32(const __nv_bfloat16* p) {
+    return __uint_as_float((unsigned)__ldg(reinterpret_cast<const unsigned short*>(p)) << 16);
+}
+__device__ __forceinline__ float ld_f32(const __half* p) {
+    return __half2float(__ushort_as_half(__ldg(reinterpret_cast<const unsigned short*>(p))));
+}
+
 // The bilinear sample at p (the upper-left tap) from global memory, dx / dy elements to the next column / row: the
-// in-bounds taps of mask m (bits as BilinearTaps::inb; higher bits are ignored), accumulated in tap order with one
-// rounding each.  Taps outside m are not read and add nothing, whatever their weight.
-__device__ __forceinline__ float gather4(const float* p, size_t dx, size_t dy, unsigned m, float w00, float w01,
-                                         float w10, float w11) {
+// in-bounds taps of mask m (bits as BilinearTaps::inb; higher bits are ignored), each widened exactly to fp32 and
+// accumulated in tap order with one rounding each.  Taps outside m are not read and add nothing, whatever their weight.
+template <typename T>
+__device__ __forceinline__ float gather4(const T* p, size_t dx, size_t dy, unsigned m, float w00, float w01, float w10,
+                                         float w11) {
     float acc = 0.0f;
-    if (m & 1u) acc = __fmaf_rn(__ldg(p), w00, acc);
-    if (m & 2u) acc = __fmaf_rn(__ldg(p + dx), w01, acc);
-    if (m & 4u) acc = __fmaf_rn(__ldg(p + dy), w10, acc);
-    if (m & 8u) acc = __fmaf_rn(__ldg(p + dy + dx), w11, acc);
+    if (m & 1u) acc = __fmaf_rn(ld_f32(p), w00, acc);
+    if (m & 2u) acc = __fmaf_rn(ld_f32(p + dx), w01, acc);
+    if (m & 4u) acc = __fmaf_rn(ld_f32(p + dy), w10, acc);
+    if (m & 8u) acc = __fmaf_rn(ld_f32(p + dy + dx), w11, acc);
     return acc;
 }
-__device__ __forceinline__ float gather4(const float* p, size_t dx, size_t dy, const BilinearTaps& t) {
+template <typename T>
+__device__ __forceinline__ float gather4(const T* p, size_t dx, size_t dy, const BilinearTaps& t) {
     return gather4(p, dx, dy, t.inb, t.w00, t.w01, t.w10, t.w11);
 }
 
@@ -397,14 +409,6 @@ __device__ __forceinline__ void warp_window_samples(const WarpWindow& w, const f
 
 __device__ __forceinline__ float ld_nc(const float* p) { return __ldg(p); }
 
-// input element -> fp32: feature maps and mask logits arrive in fp32, or in half precision from an autocast caller
-__device__ __forceinline__ float ld_f32(const float* p) { return __ldg(p); }
-__device__ __forceinline__ float ld_f32(const __nv_bfloat16* p) {
-    return __uint_as_float((unsigned)__ldg(reinterpret_cast<const unsigned short*>(p)) << 16);
-}
-__device__ __forceinline__ float ld_f32(const __half* p) {
-    return __half2float(__ushort_as_half(__ldg(reinterpret_cast<const unsigned short*>(p))));
-}
 // half-word `hi` (0: low, 1: high) of a 4-byte word of two bf16 / fp16 elements -> fp32
 template <typename T> __device__ __forceinline__ float widen16(unsigned wd, int hi);
 template <> __device__ __forceinline__ float widen16<__nv_bfloat16>(unsigned wd, int hi) {

@@ -5,7 +5,7 @@
 //   out[b,c,i,j] = grid_sample(frame[b,c], (gx,gy), mode, padding_mode, align_corners)
 // Neither the base grid nor grid+flow is ever materialised.
 //
-// Bilinear NCHW kernels (variant argument of ofb_warp_f32; all produce the same bits):
+// Bilinear NCHW kernels (variant argument of ofb_warp / ofb_warp_f32; all produce the same bits):
 //   * rows (default): lane <-> column, a thread owns 2 consecutive rows of its column, coordinates / weights /
 //     tap offsets computed once per pixel and reused per channel; interior pixels take a predicate-free channel
 //     loop with every gather in flight before the first FMA.  32 registers -> 64 resident warps per SM: the
@@ -13,7 +13,8 @@
 //   * direct: one thread per output pixel, grid-stride; also serves nearest mode and NHWC frames.
 //   * staged: one CTA per 64x16 output tile, bounding box of the taps copied to shared memory with cp.async.
 //   * TMA window (warp_tma.cu): persistent CTAs, the tile's neighbourhood arrives as 3-D TMA boxes.
-// HBM roofline (SURVEY.md 8d): 4*(C + 2 + C) bytes per pixel (+1 for the u8 mask).
+// HBM roofline (SURVEY.md 8d): 4*(C + 2 + C) bytes per pixel (+1 for the u8 mask); 2 per frame or flow element instead
+// of 4 for a 16-bit one (the direct and row kernels read frames and flows in fp32, fp16 or bf16; the output is fp32).
 #include <cstdlib>
 
 #include "common.cuh"
@@ -23,8 +24,12 @@ namespace {
 using namespace ofb;
 
 // ------------------------------------------------------------------------------ direct kernel
-template <int MODE, int PAD, bool AC, bool NHWC>
-__global__ void __launch_bounds__(256) warp_direct_kernel(const float* __restrict__ frame, const float* __restrict__ flow,
+// TI, TV: element types of the frame and the flow (float, __half, __nv_bfloat16), each widened exactly on load; the
+// arithmetic is the fp32 kernel's.  A 16-bit NHWC frame takes the scalar gather4 path: a float4-style 8-byte load of 4
+// halves would add a second vector path (and its alignment rule) to a kernel that is not the default, for a warp that
+// is bound by issue and latency rather than bytes (DESIGN.md section 4).
+template <int MODE, int PAD, bool AC, bool NHWC, typename TI = float, typename TV = float>
+__global__ void __launch_bounds__(256) warp_direct_kernel(const TI* __restrict__ frame, const TV* __restrict__ flow,
                                                           float* __restrict__ out, uint8_t* __restrict__ valid, int B,
                                                           int C, int H, int W, FlowMul fm) {
     const size_t HW = (size_t)H * W;
@@ -33,17 +38,28 @@ __global__ void __launch_bounds__(256) warp_direct_kernel(const float* __restric
         const int b = (int)(q / HW);
         const size_t p = q - (size_t)b * HW;
         const int i = (int)(p / W), j = (int)(p - (size_t)i * W);
-        const float* fxp = flow + (size_t)b * 2 * HW + p;
-        const SrcPos s = warp_source<PAD, AC>(__ldg(fxp), __ldg(fxp + HW), i, j, H, W, fm);
+        const TV* fxp = flow + (size_t)b * 2 * HW + p;
+        const SrcPos s = warp_source<PAD, AC>(ld_f32(fxp), ld_f32(fxp + HW), i, j, H, W, fm);
         if (valid) valid[q] = s.valid ? 1 : 0;
         if (MODE == OFB_MODE_NEAREST) {
             const int x = tap_index(rintf(s.ix), W), y = tap_index(rintf(s.iy), H);
             const bool in = x >= 0 && x < W && y >= 0 && y < H;
-            for (int c = 0; c < C; ++c) {
-                float v = 0.0f;
-                if (in) v = NHWC ? __ldg(frame + ((size_t)b * HW + (size_t)y * W + x) * C + c)
-                                 : __ldg(frame + ((size_t)b * C + c) * HW + (size_t)y * W + x);
-                out[((size_t)b * C + c) * HW + p] = v;
+            if constexpr (std::is_same<TI, float>::value) {
+                for (int c = 0; c < C; ++c) {
+                    float v = 0.0f;
+                    if (in) v = NHWC ? ld_f32(frame + ((size_t)b * HW + (size_t)y * W + x) * C + c)
+                                     : ld_f32(frame + ((size_t)b * C + c) * HW + (size_t)y * W + x);
+                    out[((size_t)b * C + c) * HW + p] = v;
+                }
+            } else {
+                // the same loop, kept rolled: unrolled, ptxas spills a register in the fp16-frame border instances
+#pragma unroll 1
+                for (int c = 0; c < C; ++c) {
+                    float v = 0.0f;
+                    if (in) v = NHWC ? ld_f32(frame + ((size_t)b * HW + (size_t)y * W + x) * C + c)
+                                     : ld_f32(frame + ((size_t)b * C + c) * HW + (size_t)y * W + x);
+                    out[((size_t)b * C + c) * HW + p] = v;
+                }
             }
             continue;
         }
@@ -54,10 +70,10 @@ __global__ void __launch_bounds__(256) warp_direct_kernel(const float* __restric
             continue;
         }
         if (NHWC) {
-            const float* p00 = frame + ((size_t)b * HW + (size_t)t.y0 * W + t.x0) * C;
+            const TI* p00 = frame + ((size_t)b * HW + (size_t)t.y0 * W + t.x0) * C;
             const size_t row = (size_t)W * C;
-            if ((C & 3) == 0) {
-                const float *p01 = p00 + C, *p10 = p00 + row, *p11 = p10 + C;
+            if (std::is_same<TI, float>::value && (C & 3) == 0) {
+                const TI *p01 = p00 + C, *p10 = p00 + row, *p11 = p10 + C;
                 for (int c = 0; c < C; c += 4) {
                     float4 a = make_float4(0, 0, 0, 0), bb = a, cc = a, dd = a;
                     if (t.inb & 1u) a = __ldg(reinterpret_cast<const float4*>(p00 + c));
@@ -205,16 +221,17 @@ __global__ void __launch_bounds__(NT, 2) warp_staged_kernel(const float* __restr
 // and reused for every channel.
 constexpr int RPT_DEFAULT = 2;   // rows per thread: 32 registers, 64 resident warps per SM (see the sweep in DESIGN.md)
 
-template <int PAD, bool AC, int RPT>
-__global__ void __launch_bounds__(128) warp_rows_kernel(const float* __restrict__ frame, const float* __restrict__ flow,
+// TI, TV: element types of the frame and the flow, as in the direct kernel.
+template <int PAD, bool AC, int RPT, typename TI = float, typename TV = float>
+__global__ void __launch_bounds__(128) warp_rows_kernel(const TI* __restrict__ frame, const TV* __restrict__ flow,
                                                         float* __restrict__ out, uint8_t* __restrict__ valid, int C,
                                                         int H, int W, FlowMul fm) {
     const int j = blockIdx.x * blockDim.x + threadIdx.x, b = blockIdx.z;
     const int i0 = blockIdx.y * RPT;
     if (j >= W) return;
     const int HW = H * W;                                     // launch guard: H*W < 2^30
-    const float* fxp = flow + (size_t)(b * 2) * HW;
-    const float* fyp = fxp + HW;
+    const TV* fxp = flow + (size_t)(b * 2) * HW;
+    const TV* fyp = fxp + HW;
     int o00[RPT];
     float w00[RPT], w01[RPT], w10[RPT], w11[RPT];
     unsigned inb = 0;
@@ -224,7 +241,7 @@ __global__ void __launch_bounds__(128) warp_rows_kernel(const float* __restrict_
         o00[k] = 0; w00[k] = w01[k] = w10[k] = w11[k] = 0.0f;
         if (i >= H) continue;
         const int off = i * W + j;
-        const SrcPos s = warp_source<PAD, AC>(__ldg(fxp + off), __ldg(fyp + off), i, j, H, W, fm);
+        const SrcPos s = warp_source<PAD, AC>(ld_f32(fxp + off), ld_f32(fyp + off), i, j, H, W, fm);
         if (valid) valid[(size_t)b * HW + off] = s.valid ? 1 : 0;
         const BilinearTaps t = bilinear_taps<PAD>(s.ix, s.iy, H, W);
         w00[k] = t.w00; w01[k] = t.w01; w10[k] = t.w10; w11[k] = t.w11;
@@ -235,16 +252,16 @@ __global__ void __launch_bounds__(128) warp_rows_kernel(const float* __restrict_
     // padding, samples that leave the frame): no predicates, no per-tap address arithmetic.  The kernel is bound
     // by instruction issue, not by HBM, so the channel loop is kept to 4 loads + 4 FMAs + 1 store per pixel.
     if (inb == (RPT == 8 ? 0xFFFFFFFFu : (1u << (4 * RPT)) - 1u)) {
-        const float* plane = frame + (size_t)(b * C) * HW;
+        const TI* plane = frame + (size_t)(b * C) * HW;
         float* op = out + (size_t)(b * C) * HW + i0 * W + j;
 #pragma unroll 1
         for (int c = 0; c < C; ++c, plane += HW, op += HW) {
             float v[RPT][4];                              // all 4 x RPT gathers in flight before the first FMA
 #pragma unroll
             for (int k = 0; k < RPT; ++k) {
-                const float* p = plane + o00[k];
-                const float* q = p + W;
-                v[k][0] = __ldg(p); v[k][1] = __ldg(p + 1); v[k][2] = __ldg(q); v[k][3] = __ldg(q + 1);
+                const TI* p = plane + o00[k];
+                const TI* q = p + W;
+                v[k][0] = ld_f32(p); v[k][1] = ld_f32(p + 1); v[k][2] = ld_f32(q); v[k][3] = ld_f32(q + 1);
             }
 #pragma unroll
             for (int k = 0; k < RPT; ++k) {
@@ -258,7 +275,7 @@ __global__ void __launch_bounds__(128) warp_rows_kernel(const float* __restrict_
         return;
     }
     for (int c = 0; c < C; ++c) {
-        const float* plane = frame + (size_t)(b * C + c) * HW;
+        const TI* plane = frame + (size_t)(b * C + c) * HW;
         float* op = out + (size_t)(b * C + c) * HW + i0 * W + j;
 #pragma unroll
         for (int k = 0; k < RPT; ++k) {
@@ -282,36 +299,49 @@ __global__ void __launch_bounds__(256) warp_grid_kernel(const float* __restrict_
     }
 }
 
-template <int MODE, int PAD, bool AC>
-int launch_direct(const float* frame, const float* flow, float* out, uint8_t* valid, int B, int C, int H, int W,
+template <int MODE, int PAD, bool AC, typename TI, typename TV>
+int launch_direct(const TI* frame, const TV* flow, float* out, uint8_t* valid, int B, int C, int H, int W,
                   int channels_last, FlowMul fm, cudaStream_t st) {
     const size_t total = (size_t)B * H * W;
     int blocks = (int)((total + 255) / 256);
     const int cap = ofb_num_sms() * 32;
     if (blocks > cap) blocks = cap;
     if (channels_last)
-        warp_direct_kernel<MODE, PAD, AC, true><<<blocks, 256, 0, st>>>(frame, flow, out, valid, B, C, H, W, fm);
+        warp_direct_kernel<MODE, PAD, AC, true, TI, TV><<<blocks, 256, 0, st>>>(frame, flow, out, valid, B, C, H, W, fm);
     else
-        warp_direct_kernel<MODE, PAD, AC, false><<<blocks, 256, 0, st>>>(frame, flow, out, valid, B, C, H, W, fm);
+        warp_direct_kernel<MODE, PAD, AC, false, TI, TV><<<blocks, 256, 0, st>>>(frame, flow, out, valid, B, C, H, W, fm);
     OFB_LAUNCH_CHECK();
     return OFB_OK;
 }
 
-template <int PAD, bool AC>
-int launch_rows(const float* frame, const float* flow, float* out, uint8_t* valid, int B, int C, int H, int W,
-                FlowMul fm, cudaStream_t st) {
+// Rows per thread of the fp32 row kernel: RPT_DEFAULT, or the OFB_WARP_RPT tuning override
+int warp_rpt() {
     static const int rpt = [] {
-        const char* e = getenv("OFB_WARP_RPT");           // tuning override
+        const char* e = getenv("OFB_WARP_RPT");
         const int r = e ? atoi(e) : RPT_DEFAULT;
         return (r == 1 || r == 2 || r == 4 || r == 8) ? r : RPT_DEFAULT;
     }();
+    return rpt;
+}
+
+// A 16-bit frame or flow runs the row kernel at RPT_DEFAULT only: the override is an fp32 tuning knob, and the
+// 16-bit instances stay one per (frame, flow, padding, align_corners).
+template <int PAD, bool AC, typename TI, typename TV>
+int launch_rows(const TI* frame, const TV* flow, float* out, uint8_t* valid, int B, int C, int H, int W,
+                FlowMul fm, cudaStream_t st) {
+    constexpr bool f32 = std::is_same<TI, float>::value && std::is_same<TV, float>::value;
+    const int rpt = f32 ? warp_rpt() : RPT_DEFAULT;
     const dim3 block(128);
     const dim3 grid((W + 127) / 128, (H + rpt - 1) / rpt, B);
     if (grid.y > 65535) return OFB_EUNSUPPORTED;
-    if (rpt == 1) warp_rows_kernel<PAD, AC, 1><<<grid, block, 0, st>>>(frame, flow, out, valid, C, H, W, fm);
-    else if (rpt == 2) warp_rows_kernel<PAD, AC, 2><<<grid, block, 0, st>>>(frame, flow, out, valid, C, H, W, fm);
-    else if (rpt == 8) warp_rows_kernel<PAD, AC, 8><<<grid, block, 0, st>>>(frame, flow, out, valid, C, H, W, fm);
-    else warp_rows_kernel<PAD, AC, 4><<<grid, block, 0, st>>>(frame, flow, out, valid, C, H, W, fm);
+    if constexpr (f32) {
+        if (rpt == 1) warp_rows_kernel<PAD, AC, 1><<<grid, block, 0, st>>>(frame, flow, out, valid, C, H, W, fm);
+        else if (rpt == 2) warp_rows_kernel<PAD, AC, 2><<<grid, block, 0, st>>>(frame, flow, out, valid, C, H, W, fm);
+        else if (rpt == 8) warp_rows_kernel<PAD, AC, 8><<<grid, block, 0, st>>>(frame, flow, out, valid, C, H, W, fm);
+        else warp_rows_kernel<PAD, AC, 4><<<grid, block, 0, st>>>(frame, flow, out, valid, C, H, W, fm);
+    } else {
+        warp_rows_kernel<PAD, AC, RPT_DEFAULT, TI, TV><<<grid, block, 0, st>>>(frame, flow, out, valid, C, H, W, fm);
+    }
     OFB_LAUNCH_CHECK();
     return OFB_OK;
 }
@@ -335,14 +365,19 @@ int launch_staged(const float* frame, const float* flow, float* out, uint8_t* va
 int ofb_warp_tma_launch(const float* frame, const float* flow, float* out, uint8_t* valid, int B, int C, int H, int W,
                         int pad, int ac, const ofb::FlowMul& fm, cudaStream_t st);
 
-OFB_API int ofb_warp_f32(const float* frame, const float* flow, float* out, uint8_t* valid_or_null, int B, int C, int H,
-                         int W, int mode, int padding_mode, int align_corners, int channels_last, int variant,
-                         float flow_mul_x, float flow_mul_y, void* stream) {
+OFB_API int ofb_warp(const void* frame, int frame_dtype, const void* flow, int flow_dtype, float* out,
+                     uint8_t* valid_or_null, int B, int C, int H, int W, int mode, int padding_mode, int align_corners,
+                     int channels_last, int variant, float flow_mul_x, float flow_mul_y, void* stream) {
+    if (!ofb_float_dtype(frame_dtype) || !ofb_float_dtype(flow_dtype)) return OFB_EINVAL;
     if (B == 0 || C == 0 || H == 0 || W == 0) return OFB_OK;   // nothing to do: empty tensors have no storage, their pointers may be null
     if (!frame || !flow || !out || B < 0 || C < 0 || H < 0 || W < 0) return OFB_EINVAL;
     if (mode != OFB_MODE_BILINEAR && mode != OFB_MODE_NEAREST) return OFB_EINVAL;
     if (padding_mode < 0 || padding_mode > 2 || variant < 0 || variant > 4) return OFB_EINVAL;
     if ((size_t)B * C * H * W == 0) return OFB_OK;
+    const bool f32 = frame_dtype == OFB_DTYPE_F32 && flow_dtype == OFB_DTYPE_F32;
+    if ((frame_dtype != OFB_DTYPE_F32 && (reinterpret_cast<uintptr_t>(frame) & 1)) ||
+        (flow_dtype != OFB_DTYPE_F32 && (reinterpret_cast<uintptr_t>(flow) & 1)))
+        return OFB_EALIGN;
     if (B > 65535) return OFB_EUNSUPPORTED;
     cudaStream_t st = (cudaStream_t)stream;
     const FlowMul fm{flow_mul_x, flow_mul_y, ofb::linspace_step(W), ofb::linspace_step(H)};
@@ -351,7 +386,9 @@ OFB_API int ofb_warp_f32(const float* frame, const float* flow, float* out, uint
     // TMA needs 16-byte global strides
     const bool can_tma = can_rows && W % 4 == 0 && (reinterpret_cast<uintptr_t>(frame) & 15) == 0 &&
                          (long long)B * C < (1LL << 31);
-    if ((variant == 2 && !nchw_bilinear) || (variant == 3 && !can_rows) || (variant == 4 && !can_tma))
+    // the staged and TMA kernels read fp32 frames and flows only
+    if (((variant == 2 || variant == 4) && !f32) || (variant == 2 && !nchw_bilinear) || (variant == 3 && !can_rows) ||
+        (variant == 4 && !can_tma))
         return OFB_EUNSUPPORTED;
     // auto: the row kernel; 1 = direct gather (also nearest / NHWC), 2 = cp.async-staged, 3 = row kernel,
     // 4 = TMA-staged window (warp_tma.cu)
@@ -359,17 +396,37 @@ OFB_API int ofb_warp_f32(const float* frame, const float* flow, float* out, uint
         const char* e = getenv("OFB_WARP_VARIANT");       // tuning override for variant 0
         return e ? atoi(e) : 0;
     }();
-    int v = variant != 0 ? variant : (auto_v == 4 && can_tma ? 4 : (can_rows ? 3 : 1));
+    int v = variant != 0 ? variant : (auto_v == 4 && can_tma && f32 ? 4 : (can_rows ? 3 : 1));
     if (v == 4)
-        return ofb_warp_tma_launch(frame, flow, out, valid_or_null, B, C, H, W, padding_mode, align_corners, fm, st);
-    return ofb_dispatch_pad_ac(padding_mode, align_corners, [&](auto P, auto A) {
-        if (v == 3) return launch_rows<P, A>(frame, flow, out, valid_or_null, B, C, H, W, fm, st);
-        if (v == 2) return launch_staged<P, A>(frame, flow, out, valid_or_null, B, C, H, W, fm, st);
-        const int cl = channels_last;
-        if (mode == OFB_MODE_BILINEAR)
-            return launch_direct<OFB_MODE_BILINEAR, P, A>(frame, flow, out, valid_or_null, B, C, H, W, cl, fm, st);
-        return launch_direct<OFB_MODE_NEAREST, P, A>(frame, flow, out, valid_or_null, B, C, H, W, cl, fm, st);
+        return ofb_warp_tma_launch(static_cast<const float*>(frame), static_cast<const float*>(flow), out,
+                                   valid_or_null, B, C, H, W, padding_mode, align_corners, fm, st);
+    if (v == 2)
+        return ofb_dispatch_pad_ac(padding_mode, align_corners, [&](auto P, auto A) {
+            return launch_staged<P, A>(static_cast<const float*>(frame), static_cast<const float*>(flow), out,
+                                       valid_or_null, B, C, H, W, fm, st);
+        });
+    return ofb_dispatch_dtype(frame_dtype, [&](auto ti) {
+        return ofb_dispatch_dtype(flow_dtype, [&](auto tv) {
+            using TI = decltype(ti);
+            using TV = decltype(tv);
+            const TI* fr = static_cast<const TI*>(frame);
+            const TV* fl = static_cast<const TV*>(flow);
+            return ofb_dispatch_pad_ac(padding_mode, align_corners, [&](auto P, auto A) {
+                if (v == 3) return launch_rows<P, A>(fr, fl, out, valid_or_null, B, C, H, W, fm, st);
+                const int cl = channels_last;
+                if (mode == OFB_MODE_BILINEAR)
+                    return launch_direct<OFB_MODE_BILINEAR, P, A>(fr, fl, out, valid_or_null, B, C, H, W, cl, fm, st);
+                return launch_direct<OFB_MODE_NEAREST, P, A>(fr, fl, out, valid_or_null, B, C, H, W, cl, fm, st);
+            });
+        });
     });
+}
+
+OFB_API int ofb_warp_f32(const float* frame, const float* flow, float* out, uint8_t* valid_or_null, int B, int C, int H,
+                         int W, int mode, int padding_mode, int align_corners, int channels_last, int variant,
+                         float flow_mul_x, float flow_mul_y, void* stream) {
+    return ofb_warp(frame, OFB_DTYPE_F32, flow, OFB_DTYPE_F32, out, valid_or_null, B, C, H, W, mode, padding_mode,
+                    align_corners, channels_last, variant, flow_mul_x, flow_mul_y, stream);
 }
 
 OFB_API int ofb_warp_grid_f32(const float* flow_bhw2, float* grid_bhw2, int B, int H, int W, void* stream) {

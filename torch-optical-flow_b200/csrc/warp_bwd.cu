@@ -35,17 +35,20 @@ __device__ __forceinline__ float source_index_grad(float g, int size, float& gra
     return x;
 }
 
-template <int PAD, bool AC>
-__global__ void __launch_bounds__(128) warp_bwd_kernel(const float* __restrict__ frame, const float* __restrict__ flow,
+// TI, TV: element types of the frame and the flow (float, __half, __nv_bfloat16), widened exactly on load; d_out and
+// d_frame are fp32 whatever TI (a 16-bit d_frame is the fp32 sum rounded once, after the kernel: half-precision atomics
+// would round after every addition).  d_flow is one store per pixel in TV, the fp32 gradient rounded once.
+template <int PAD, bool AC, typename TI = float, typename TV = float>
+__global__ void __launch_bounds__(128) warp_bwd_kernel(const TI* __restrict__ frame, const TV* __restrict__ flow,
                                                        const float* __restrict__ d_out, float* __restrict__ d_frame,
-                                                       float* __restrict__ d_flow, int C, int H, int W, FlowMul fm) {
+                                                       TV* __restrict__ d_flow, int C, int H, int W, FlowMul fm) {
     const int j = blockIdx.x * blockDim.x + threadIdx.x, i = blockIdx.y, b = blockIdx.z;
     if (j >= W) return;
     const int HW = H * W;                                  // launch guard: H*W < 2^30
     const int off = i * W + j;
-    const float* fxp = flow + (size_t)(b * 2) * HW;
-    const float gx = warp_grid_coord(__ldg(fxp + off), j, W, fm.step_x, fm.x);
-    const float gy = warp_grid_coord(__ldg(fxp + HW + off), i, H, fm.step_y, fm.y);
+    const TV* fxp = flow + (size_t)(b * 2) * HW;
+    const float gx = warp_grid_coord(ld_f32(fxp + off), j, W, fm.step_x, fm.x);
+    const float gy = warp_grid_coord(ld_f32(fxp + HW + off), i, H, fm.step_y, fm.y);
     float gmx, gmy;
     const float ix = source_index_grad<PAD, AC>(gx, W, gmx);
     const float iy = source_index_grad<PAD, AC>(gy, H, gmy);
@@ -66,42 +69,61 @@ __global__ void __launch_bounds__(128) warp_bwd_kernel(const float* __restrict__
             if (i11) atomicAdd(p + W + 1, t.w11 * g);
         }
         if (d_flow) {
-            const float* p = frame + plane + o;
-            if (i00) { const float v = __ldg(p); gix -= v * wy0 * g; giy -= v * wx0 * g; }
-            if (i01) { const float v = __ldg(p + 1); gix += v * wy0 * g; giy -= v * wx1 * g; }
-            if (i10) { const float v = __ldg(p + W); gix -= v * wy1 * g; giy += v * wx0 * g; }
-            if (i11) { const float v = __ldg(p + W + 1); gix += v * wy1 * g; giy += v * wx1 * g; }
+            const TI* p = frame + plane + o;
+            if (i00) { const float v = ld_f32(p); gix -= v * wy0 * g; giy -= v * wx0 * g; }
+            if (i01) { const float v = ld_f32(p + 1); gix += v * wy0 * g; giy -= v * wx1 * g; }
+            if (i10) { const float v = ld_f32(p + W); gix -= v * wy1 * g; giy += v * wx0 * g; }
+            if (i11) { const float v = ld_f32(p + W + 1); gix += v * wy1 * g; giy += v * wx1 * g; }
         }
     }
     if (d_flow) {
-        float* dp = d_flow + (size_t)(b * 2) * HW + off;
-        dp[0] = fm.x * (gmx * gix);
-        dp[HW] = fm.y * (gmy * giy);
+        TV* dp = d_flow + (size_t)(b * 2) * HW + off;
+        dp[0] = narrow<TV>(fm.x * (gmx * gix));
+        dp[HW] = narrow<TV>(fm.y * (gmy * giy));
     }
 }
 
-template <int PAD, bool AC>
-int launch(const float* frame, const float* flow, const float* d_out, float* d_frame, float* d_flow, int B, int C, int H,
-           int W, const FlowMul& fm, cudaStream_t stream) {
+template <int PAD, bool AC, typename TI, typename TV>
+int launch(const TI* frame, const TV* flow, const float* d_out, float* d_frame, TV* d_flow, int B, int C, int H, int W,
+           const FlowMul& fm, cudaStream_t stream) {
     const dim3 grid((W + 127) / 128, H, B);
-    warp_bwd_kernel<PAD, AC><<<grid, 128, 0, stream>>>(frame, flow, d_out, d_frame, d_flow, C, H, W, fm);
+    warp_bwd_kernel<PAD, AC, TI, TV><<<grid, 128, 0, stream>>>(frame, flow, d_out, d_frame, d_flow, C, H, W, fm);
     OFB_LAUNCH_CHECK();
     return OFB_OK;
 }
 
 }  // namespace
 
-OFB_API int ofb_warp_backward_f32(const float* frame, const float* flow, const float* d_out, float* d_frame_or_null,
-                                  float* d_flow_or_null, int B, int C, int H, int W, int padding_mode, int align_corners,
-                                  float flow_mul_x, float flow_mul_y, void* stream) {
+OFB_API int ofb_warp_backward(const void* frame, int frame_dtype, const void* flow, int flow_dtype, const float* d_out,
+                              float* d_frame_f32_or_null, void* d_flow_or_null, int B, int C, int H, int W,
+                              int padding_mode, int align_corners, float flow_mul_x, float flow_mul_y, void* stream) {
+    if (!ofb_float_dtype(frame_dtype) || !ofb_float_dtype(flow_dtype)) return OFB_EINVAL;
     if (B == 0 || H == 0 || W == 0) return OFB_OK;   // nothing to do: empty tensors have no storage, their pointers may be null
     if (!frame || !flow || !d_out || B < 0 || C < 0 || H < 0 || W < 0) return OFB_EINVAL;
     if (padding_mode < 0 || padding_mode > 2) return OFB_EINVAL;
-    if ((size_t)B * H * W == 0 || (!d_frame_or_null && !d_flow_or_null)) return OFB_OK;
+    if ((size_t)B * H * W == 0 || (!d_frame_f32_or_null && !d_flow_or_null)) return OFB_OK;
+    if ((frame_dtype != OFB_DTYPE_F32 && (reinterpret_cast<uintptr_t>(frame) & 1)) ||
+        (flow_dtype != OFB_DTYPE_F32 && ((reinterpret_cast<uintptr_t>(flow) | reinterpret_cast<uintptr_t>(d_flow_or_null)) & 1)))
+        return OFB_EALIGN;
     if (B > 65535 || H > 65535 || (long long)H * W >= (1LL << 30) || (long long)B * (C > 2 ? C : 2) * H * W >= (1LL << 40))
         return OFB_EUNSUPPORTED;
     const ofb::FlowMul fm{flow_mul_x, flow_mul_y, ofb::linspace_step(W), ofb::linspace_step(H)};
-    return ofb_dispatch_pad_ac(padding_mode, align_corners != 0, [&](auto P, auto A) {
-        return launch<P, A>(frame, flow, d_out, d_frame_or_null, d_flow_or_null, B, C, H, W, fm, (cudaStream_t)stream);
+    return ofb_dispatch_dtype(frame_dtype, [&](auto ti) {
+        return ofb_dispatch_dtype(flow_dtype, [&](auto tv) {
+            using TI = decltype(ti);
+            using TV = decltype(tv);
+            return ofb_dispatch_pad_ac(padding_mode, align_corners != 0, [&](auto P, auto A) {
+                return launch<P, A>(static_cast<const TI*>(frame), static_cast<const TV*>(flow), d_out,
+                                    d_frame_f32_or_null, static_cast<TV*>(d_flow_or_null), B, C, H, W, fm,
+                                    (cudaStream_t)stream);
+            });
+        });
     });
+}
+
+OFB_API int ofb_warp_backward_f32(const float* frame, const float* flow, const float* d_out, float* d_frame_or_null,
+                                  float* d_flow_or_null, int B, int C, int H, int W, int padding_mode, int align_corners,
+                                  float flow_mul_x, float flow_mul_y, void* stream) {
+    return ofb_warp_backward(frame, OFB_DTYPE_F32, flow, OFB_DTYPE_F32, d_out, d_frame_or_null, d_flow_or_null, B, C, H,
+                             W, padding_mode, align_corners, flow_mul_x, flow_mul_y, stream);
 }

@@ -51,6 +51,8 @@ SIGNATURES = {
     "ofb_launch_count": (_i64, []),
     "ofb_warp_f32": (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _i, _f, _f, _vp]),
     "ofb_warp_backward_f32": (_i, [_vp, _vp, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _f, _f, _vp]),
+    "ofb_warp": (_i, [_vp, _i, _vp, _i, _vp, _vp, _i, _i, _i, _i, _i, _i, _i, _i, _i, _f, _f, _vp]),
+    "ofb_warp_backward": (_i, [_vp, _i, _vp, _i, _vp, _vp, _vp, _i, _i, _i, _i, _i, _i, _f, _f, _vp]),
     "ofb_warp_grid_f32": (_i, [_vp, _vp, _i, _i, _i, _vp]),
     "ofb_scale_flow_f32": (_i, [_vp, _vp, _i, _i64, _f, _f, _vp]),
     "ofb_scale_flow": (_i, [_vp, _vp, _i, _i, _i64, ctypes.c_double, ctypes.c_double, _vp]),

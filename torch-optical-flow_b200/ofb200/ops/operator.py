@@ -2,7 +2,8 @@
 (reference optical_flow/operator/operator.py), computed by the K1 / K4a kernels of libofb200.
 
 Tensors may live on the host or on the GPU: host tensors are staged through the device and the
-result is returned on the host (the reference's tests/operator build CPU tensors).  fp32 only.
+result is returned on the host (the reference's tests/operator build CPU tensors).  fp32 only, except `scale` /
+`normalize` / `denormalize` (dtype-preserving) and `warp` (fp32, fp16 or bf16 frames and flows).
 """
 from typing import Optional, Tuple, Union
 
@@ -23,6 +24,9 @@ def _check_f32(*tensors: Tensor) -> None:
     for t in tensors:
         if t.dtype != torch.float32:
             raise NotImplementedError(f"ofb200 kernels are fp32 only, got {t.dtype}")
+
+
+_WARP_DTYPES = {torch.float32: ofb200.DTYPE_F32, torch.float16: ofb200.DTYPE_F16, torch.bfloat16: ofb200.DTYPE_BF16}
 
 
 def _run(fn, name: str, *tensors: Tensor, bwd=None) -> Tensor:
@@ -60,10 +64,19 @@ def warp(
             evaluated on the warp grid: True where the source position lies strictly inside the frame
         variant: kernel selection, 0 = auto, 1 = direct gather, 2 = cp.async-staged, 3 = row kernel, 4 = TMA-staged
         pixel_flow: extension (default off): `flow` is in pixel units and :func:`normalize` is fused into
-            the kernel -- ``warp(f, flow, pixel_flow=True)`` equals ``warp(f, normalize(flow))`` bit for bit
+            the kernel -- ``warp(f, flow, pixel_flow=True)`` equals ``warp(f, normalize(flow))`` bit for bit for an
+            fp32 flow, and ``warp(f.float(), normalize(flow.float()))`` for a half one.  It does not equal
+            ``warp(f, normalize(flow))`` for a half flow: `normalize` keeps the flow's dtype and rounds the product
+            to it, the fused multiply is one fp32 rounding.
+
+    The frame and the flow may each be fp32, fp16 or bf16.  Half-precision inputs are read directly, each element
+    widened exactly, so the result is always fp32 and bit for bit ``warp(frame.float(), flow.float(), ...)``: what
+    the reference returns under CUDA autocast, where grid_sample runs in fp32.  Outside autocast ATen raises for a
+    half frame; this computes the same fp32 result instead.  The gradients arrive in the inputs' dtypes, the fp32
+    gradients rounded once (what autocast's cast, or type promotion's, hands them).
 
     Returns:
-        The warped image (B, C, H, W), contiguous; with ``return_mask`` a tuple (warped, mask).
+        The warped image (B, C, H, W), contiguous fp32; with ``return_mask`` a tuple (warped, mask).
     """
     if mode not in ofb200.MODE:
         if mode == "bicubic":
@@ -76,7 +89,9 @@ def warp(
     b, c, h, w = frame.shape
     if tuple(flow.shape) != (b, 2, h, w):
         raise RuntimeError(f"warp: flow shape {tuple(flow.shape)} does not match frame {tuple(frame.shape)}")
-    _check_f32(frame, flow)
+    for t in (frame, flow):
+        if t.dtype not in _WARP_DTYPES:
+            raise NotImplementedError(f"ofb200 warp kernels are fp32, fp16 or bf16 only, got {t.dtype}")
     mul_x, mul_y = (2.0 / max(w - 1, 1), 2.0 / max(h - 1, 1)) if pixel_flow else (1.0, 1.0)
 
     def run(frame_d: Tensor, flow_d: Tensor):
@@ -89,17 +104,18 @@ def warp(
         flow_d = flow_d.contiguous()
         out = torch.empty((b, c, h, w), dtype=torch.float32, device=frame_d.device)
         mask = torch.empty((b, h, w), dtype=torch.uint8, device=frame_d.device) if return_mask else None
-        rc = lib.ofb_warp_f32(
-            ofb200.ptr(frame_d), ofb200.ptr(flow_d), ofb200.ptr(out), ofb200.ptr(mask), b, c, h, w,
-            ofb200.MODE[mode], ofb200.PAD[padding_mode], int(bool(align_corners)), int(channels_last),
-            int(variant), mul_x, mul_y, ofb200.stream_ptr(),
+        rc = lib.ofb_warp(
+            ofb200.ptr(frame_d), _WARP_DTYPES[frame_d.dtype], ofb200.ptr(flow_d), _WARP_DTYPES[flow_d.dtype],
+            ofb200.ptr(out), ofb200.ptr(mask), b, c, h, w, ofb200.MODE[mode], ofb200.PAD[padding_mode],
+            int(bool(align_corners)), int(channels_last), int(variant), mul_x, mul_y, ofb200.stream_ptr(),
         )
-        ofb200.check(rc, "ofb_warp_f32")
+        ofb200.check(rc, "ofb_warp")
         return (out, mask.view(torch.bool)) if return_mask else out     # the kernel writes 0 / 1 bytes: zero-copy view
 
     def backward(saved, grad_out: Tensor, needs):
         """d warp / d frame (scatter-add of the bilinear weights) and d warp / d flow, as F.grid_sample's backward
-        through warp_grid (reference operator.py:28-33,56)."""
+        through warp_grid (reference operator.py:28-33,56).  d_frame is accumulated in fp32 and rounded once to the
+        frame's dtype; d_flow is written in the flow's dtype."""
         if mode != "bilinear":
             raise NotImplementedError("warp: backward exists for mode='bilinear' only")
         frame_d, flow_d = saved
@@ -107,13 +123,14 @@ def warp(
             frame_c, flow_c = frame_d.contiguous(), flow_d.contiguous()
             grad_c = grad_out.contiguous()
             d_frame = torch.zeros((b, c, h, w), dtype=torch.float32, device=frame_c.device) if needs[0] else None
-            d_flow = torch.empty((b, 2, h, w), dtype=torch.float32, device=frame_c.device) if needs[1] else None
-            rc = ofb200.load().ofb_warp_backward_f32(
-                ofb200.ptr(frame_c), ofb200.ptr(flow_c), ofb200.ptr(grad_c), ofb200.ptr(d_frame), ofb200.ptr(d_flow),
-                b, c, h, w, ofb200.PAD[padding_mode], int(bool(align_corners)), mul_x, mul_y, ofb200.stream_ptr(),
+            d_flow = torch.empty((b, 2, h, w), dtype=flow_c.dtype, device=frame_c.device) if needs[1] else None
+            rc = ofb200.load().ofb_warp_backward(
+                ofb200.ptr(frame_c), _WARP_DTYPES[frame_c.dtype], ofb200.ptr(flow_c), _WARP_DTYPES[flow_c.dtype],
+                ofb200.ptr(grad_c), ofb200.ptr(d_frame), ofb200.ptr(d_flow), b, c, h, w, ofb200.PAD[padding_mode],
+                int(bool(align_corners)), mul_x, mul_y, ofb200.stream_ptr(),
             )
-            ofb200.check(rc, "ofb_warp_backward_f32")
-        return d_frame, d_flow
+            ofb200.check(rc, "ofb_warp_backward")
+        return (d_frame.to(frame_c.dtype) if d_frame is not None else None), d_flow
 
     return _run(run, "warp", frame, flow, bwd=backward)
 
