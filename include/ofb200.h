@@ -169,6 +169,15 @@ int ofb_convex_upsample_backward(const float* flow, const void* mask, int mask_d
 int ofb_epe_reduce_f32(const float* pred, const float* target, const float* valid_or_null,
                        double* acc, int B, int H, int W, void* stream);
 int ofb_epe_map_f32(const float* pred, const float* target, float* out, int B, int H, int W, void* stream);
+/* Backward of end_point_error (optical_flow/metrics/epe.py:41-61), as ATen's norm / mean backward:
+ *   g_p      = d_epe[p]                   (map: d_epe is (B,H,W))
+ *            = d_epe[0] / (float)(B*H*W)  (mean, d_epe_is_scalar != 0: ONE device scalar, never read on the host)
+ *   d_pred   = g_p * ((pred - target) / n_p), 0 where n_p == 0;  n_p = the end-point error ofb_epe_map_f32 computes
+ *   d_target = -d_pred
+ * pred, target, d_pred, d_target (B,2,H,W) fp32.  Either output may be NULL (not written); both NULL is a no-op.
+ * Outputs are overwritten, not accumulated. */
+int ofb_epe_backward_f32(const float* pred, const float* target, const float* d_epe, int d_epe_is_scalar,
+                         float* d_pred_or_null, float* d_target_or_null, int B, int H, int W, void* stream);
 /* OutlierRatio.update (optical_flow/metrics/f1.py:33-48): acc[0] += number of selected pixels with
  * epe > abs_threshold and epe / |target| > rel_threshold, acc[1] += number of selected pixels. */
 int ofb_outlier_reduce_f32(const float* pred, const float* target, const float* valid_or_null,

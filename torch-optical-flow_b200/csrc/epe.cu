@@ -7,6 +7,8 @@
 // The cross-rank reduction (dist_reduce_fx="sum", epe.py:22-23) is a single all-reduce of
 // that 16-byte buffer, issued by the host (see optical_flow/metrics/epe.py in this repo).
 // HBM roofline: 16 bytes per pixel (+4 with a validity map).
+// end_point_error's backward (epe_bwd_kernel) is one more streaming pass of the same shape: 16 bytes read per pixel
+// (+4 for a map gradient), 8 written per requested gradient.
 #include "common.cuh"
 
 namespace {
@@ -84,6 +86,68 @@ __global__ void __launch_bounds__(NT) epe_map_kernel(const float* __restrict__ p
         const int64_t b = t / HW, q = t - b * HW;
         out[t] = epe1(__ldg(pred + (b * 2 + 0) * HW + q), __ldg(pred + (b * 2 + 1) * HW + q),
                       __ldg(target + (b * 2 + 0) * HW + q), __ldg(target + (b * 2 + 1) * HW + q));
+    }
+}
+
+// d end_point_error / d pred of one pixel, ATen's norm backward op for op: g * ((p - t) / n).masked_fill(n == 0, 0)
+// with n the forward's own end-point error.  Not (p - t) * (g / n): that rounds differently.
+__device__ __forceinline__ float2 epe_grad1(float px, float py, float tx, float ty, float g) {
+    const float n = epe1(px, py, tx, ty);
+    const float qx = n == 0.0f ? 0.0f : __fdiv_rn(__fsub_rn(px, tx), n);
+    const float qy = n == 0.0f ? 0.0f : __fdiv_rn(__fsub_rn(py, ty), n);
+    return make_float2(__fmul_rn(g, qx), __fmul_rn(g, qy));
+}
+
+// One streaming pass, lane <-> pixel (VEC: 4 consecutive pixels, float4 loads and stores), both gradients written;
+// d_target = -d_pred (the subtraction's backward).  d_epe is the (B,H,W) map, or with `scalar` the mean's one
+// upstream gradient, divided by B*H*W on the device as ATen's mean backward divides it.
+template <bool VEC>
+__global__ void __launch_bounds__(NT) epe_bwd_kernel(const float* __restrict__ pred, const float* __restrict__ target,
+                                                     const float* __restrict__ d_epe, int scalar,
+                                                     float* __restrict__ d_pred, float* __restrict__ d_target, int B,
+                                                     int64_t HW) {
+    constexpr int V = VEC ? 4 : 1;
+    const int64_t per_b = HW / V;
+    const int64_t total = (int64_t)B * per_b;
+    const float g0 = scalar ? __fdiv_rn(__ldg(d_epe), (float)((int64_t)B * HW)) : 0.0f;
+    for (int64_t t = (int64_t)blockIdx.x * NT + threadIdx.x; t < total; t += (int64_t)gridDim.x * NT) {
+        const int64_t b = t / per_b, q = (t - b * per_b) * V;
+        const int64_t ox = (b * 2 + 0) * HW + q, oy = (b * 2 + 1) * HW + q;
+        float px[V], py[V], tx[V], ty[V], g[V], dx[V], dy[V];
+        if constexpr (VEC) {
+            const float4 a = __ldg(reinterpret_cast<const float4*>(pred + ox));
+            const float4 c = __ldg(reinterpret_cast<const float4*>(pred + oy));
+            const float4 e = __ldg(reinterpret_cast<const float4*>(target + ox));
+            const float4 f = __ldg(reinterpret_cast<const float4*>(target + oy));
+            const float4 h = scalar ? make_float4(g0, g0, g0, g0) : __ldg(reinterpret_cast<const float4*>(d_epe + b * HW + q));
+            px[0] = a.x; px[1] = a.y; px[2] = a.z; px[3] = a.w;
+            py[0] = c.x; py[1] = c.y; py[2] = c.z; py[3] = c.w;
+            tx[0] = e.x; tx[1] = e.y; tx[2] = e.z; tx[3] = e.w;
+            ty[0] = f.x; ty[1] = f.y; ty[2] = f.z; ty[3] = f.w;
+            g[0] = h.x; g[1] = h.y; g[2] = h.z; g[3] = h.w;
+        } else {
+            px[0] = __ldg(pred + ox); py[0] = __ldg(pred + oy);
+            tx[0] = __ldg(target + ox); ty[0] = __ldg(target + oy);
+            g[0] = scalar ? g0 : __ldg(d_epe + t);
+        }
+#pragma unroll
+        for (int k = 0; k < V; ++k) {
+            const float2 d = epe_grad1(px[k], py[k], tx[k], ty[k], g[k]);
+            dx[k] = d.x; dy[k] = d.y;
+        }
+        if constexpr (VEC) {
+            if (d_pred) {
+                *reinterpret_cast<float4*>(d_pred + ox) = make_float4(dx[0], dx[1], dx[2], dx[3]);
+                *reinterpret_cast<float4*>(d_pred + oy) = make_float4(dy[0], dy[1], dy[2], dy[3]);
+            }
+            if (d_target) {
+                *reinterpret_cast<float4*>(d_target + ox) = make_float4(-dx[0], -dx[1], -dx[2], -dx[3]);
+                *reinterpret_cast<float4*>(d_target + oy) = make_float4(-dy[0], -dy[1], -dy[2], -dy[3]);
+            }
+        } else {
+            if (d_pred) { d_pred[ox] = dx[0]; d_pred[oy] = dy[0]; }
+            if (d_target) { d_target[ox] = -dx[0]; d_target[oy] = -dy[0]; }
+        }
     }
 }
 
@@ -253,6 +317,31 @@ OFB_API int ofb_epe_map_f32(const float* pred, const float* target, float* out, 
     const int cap = ofb_num_sms() * 32;
     if (blocks > cap) blocks = cap;
     epe_map_kernel<<<(int)blocks, NT, 0, (cudaStream_t)stream>>>(pred, target, out, B, HW);
+    OFB_LAUNCH_CHECK();
+    return OFB_OK;
+}
+
+OFB_API int ofb_epe_backward_f32(const float* pred, const float* target, const float* d_epe, int d_epe_is_scalar,
+                                 float* d_pred_or_null, float* d_target_or_null, int B, int H, int W, void* stream) {
+    if (B == 0 || H == 0 || W == 0) return OFB_OK;   // nothing to do: empty tensors have no storage, their pointers may be null
+    if (!pred || !target || !d_epe || B < 0 || H < 0 || W < 0) return OFB_EINVAL;
+    if (!d_pred_or_null && !d_target_or_null) return OFB_OK;
+    const int64_t HW = (int64_t)H * W;
+    const int scalar = d_epe_is_scalar != 0;
+    const uintptr_t al = reinterpret_cast<uintptr_t>(pred) | reinterpret_cast<uintptr_t>(target) |
+                         reinterpret_cast<uintptr_t>(d_pred_or_null) | reinterpret_cast<uintptr_t>(d_target_or_null) |
+                         (scalar ? 0 : reinterpret_cast<uintptr_t>(d_epe));
+    const bool vec = (HW % 4 == 0) && ((al & 15) == 0);
+    const int64_t work = vec ? (int64_t)B * (HW / 4) : (int64_t)B * HW;
+    int64_t blocks = (work + NT - 1) / NT;
+    const int cap = ofb_num_sms() * 8;   // 8 x 256 threads fill an SM; each thread strides over the rest
+    if (blocks > cap) blocks = cap;
+    if (vec)
+        epe_bwd_kernel<true><<<(int)blocks, NT, 0, (cudaStream_t)stream>>>(pred, target, d_epe, scalar, d_pred_or_null,
+                                                                          d_target_or_null, B, HW);
+    else
+        epe_bwd_kernel<false><<<(int)blocks, NT, 0, (cudaStream_t)stream>>>(pred, target, d_epe, scalar, d_pred_or_null,
+                                                                           d_target_or_null, B, HW);
     OFB_LAUNCH_CHECK();
     return OFB_OK;
 }

@@ -62,6 +62,7 @@ SIGNATURES = {
     "ofb_convex_upsample": (_i, [_vp, _vp, _i, _vp, _i, _i, _i, _vp]),
     "ofb_epe_reduce_f32": (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _vp]),
     "ofb_epe_map_f32": (_i, [_vp, _vp, _vp, _i, _i, _i, _vp]),
+    "ofb_epe_backward_f32": (_i, [_vp, _vp, _vp, _i, _vp, _vp, _i, _i, _i, _vp]),
     "ofb_outlier_reduce_f32": (_i, [_vp, _vp, _vp, _vp, _i, _i, _i, _f, _f, _vp]),
     "ofb_sequence_loss_backward_f32": (_i, [ctypes.POINTER(_vp), ctypes.POINTER(_vp), _i, _vp, _vp, _vp, _i, _i, _i,
                                             ctypes.c_double, _f, _vp]),

@@ -8,12 +8,15 @@ import torch
 from torch import Tensor
 
 import ofb200
+from ofb200.ops.operator import aligned16
 
 
-def _prep(pred: Tensor, target: Tensor, dim: int):
+def _prep(pred: Tensor, target: Tensor, dim: int, keep_graph: bool = False):
     """Device, fp32, contiguous, viewed as (L, 2, T, 1): `dim` may be any dimension holding the two flow components
     (reference epe.py:41-61 takes any dim); the dimensions before it fold into L, those after it into T -- a free view
-    of a contiguous tensor, (B, 2, H, W) with dim=1 being the usual case."""
+    of a contiguous tensor, (B, 2, H, W) with dim=1 being the usual case.  Detached unless `keep_graph`: then the
+    staging, the copy and the view stay on the autograd path and carry gradients back to the inputs' shapes,
+    strides and devices."""
     if pred.shape != target.shape:
         raise RuntimeError(f"pred {tuple(pred.shape)} and target {tuple(target.shape)} differ in shape")
     nd = pred.dim()
@@ -32,7 +35,12 @@ def _prep(pred: Tensor, target: Tensor, dim: int):
     for n in pred.shape[d + 1:]:
         trail *= int(n)
     view = (lead, 2, trail, 1)
-    return (ofb200.to_device(pred).detach().contiguous().view(view), ofb200.to_device(target).detach().contiguous().view(view))
+
+    def flat(t: Tensor) -> Tensor:
+        t = ofb200.to_device(t)
+        return (t if keep_graph else t.detach()).contiguous().view(view)
+
+    return flat(pred), flat(target)
 
 
 def _prep_valid(valid: Optional[Tensor], b: int, h: int, w: int) -> Optional[Tensor]:
@@ -141,21 +149,43 @@ class AverageEndPointError(SumCountMetric):
 
 
 def end_point_error(pred: Tensor, target: Tensor, dim: int = 1, reduce: bool = True) -> Tensor:
-    """End-to-end Point Error (reference epe.py:41-61): mean EPE, or the (B, H, W) map with reduce=False."""
+    """End-to-end Point Error (reference epe.py:41-61): mean EPE, or the (B, H, W) map with reduce=False.
+
+    Differentiable with respect to `pred` and `target` as the reference's `torch.norm(pred - target, p=2, dim=dim)`
+    [`.mean()`] is: d pred = g * ((pred - target) / epe), 0 where epe == 0, and d target = -d pred, with g the map's
+    gradient or the mean's divided by the number of pixels (`ofb_epe_backward_f32`)."""
     on_host = not pred.is_cuda
-    pred_d, target_d = _prep(pred, target, dim)
+    grad = torch.is_grad_enabled() and (pred.requires_grad or target.requires_grad)
+    pred_d, target_d = _prep(pred, target, dim, keep_graph=grad)
     b, _, h, w = pred_d.shape
     map_shape = tuple(pred.shape[:dim % pred.dim()]) + tuple(pred.shape[dim % pred.dim() + 1:])
-    if reduce:
-        acc = torch.zeros(2, dtype=torch.float64, device=pred_d.device)
-        _accumulate(acc, pred_d, target_d, None)
-        out = (acc[0] / acc[1]).to(torch.float32)
-    else:
-        out = torch.empty((b, h, w), dtype=torch.float32, device=pred_d.device)
-        with torch.cuda.device(pred_d.device):
-            rc = ofb200.load().ofb_epe_map_f32(
-                ofb200.ptr(pred_d), ofb200.ptr(target_d), ofb200.ptr(out), b, h, w, ofb200.stream_ptr()
-            )
+
+    def run(p: Tensor, t: Tensor) -> Tensor:
+        if reduce:
+            acc = torch.zeros(2, dtype=torch.float64, device=p.device)
+            _accumulate(acc, p, t, None)
+            return (acc[0] / acc[1]).to(torch.float32)
+        out = torch.empty((b, h, w), dtype=torch.float32, device=p.device)
+        rc = ofb200.load().ofb_epe_map_f32(ofb200.ptr(p), ofb200.ptr(t), ofb200.ptr(out), b, h, w, ofb200.stream_ptr())
         ofb200.check(rc, "ofb_epe_map_f32")
+        return out
+
+    def backward(saved, grad_out: Tensor, needs):
+        """Both gradients from one kernel launch; the mean's upstream gradient stays on the device."""
+        p, t = saved
+        with torch.cuda.device(p.device):
+            g = grad_out.contiguous() if reduce else aligned16(grad_out)
+            d_p = torch.empty_like(p) if needs[0] else None
+            d_t = torch.empty_like(t) if needs[1] else None
+            rc = ofb200.load().ofb_epe_backward_f32(
+                ofb200.ptr(p), ofb200.ptr(t), ofb200.ptr(g), int(reduce), ofb200.ptr(d_p), ofb200.ptr(d_t), b, h, w,
+                ofb200.stream_ptr(),
+            )
+            ofb200.check(rc, "ofb_epe_backward_f32")
+        return d_p, d_t
+
+    with torch.cuda.device(pred_d.device):
+        out = ofb200.differentiable(run, backward, "end_point_error", pred_d, target_d)
+    if not reduce:
         out = out.view(map_shape)
     return out.cpu() if on_host else out

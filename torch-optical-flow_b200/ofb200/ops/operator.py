@@ -138,7 +138,8 @@ def warp(
 def warp_grid(flow: Tensor) -> Tensor:
     """Warping grid of a normalised flow map, (B, H, W, 2) -> (B, H, W, 2) (reference operator.py:36-56).
 
-    `warp` never materialises this grid; the function exists for API parity.
+    `warp` never materialises this grid; the function exists for API parity.  Differentiable: the grid is the base
+    grid plus the flow, so the flow's gradient is the grid's gradient itself.
     """
     b, h, w, _ = flow.shape
     _check_f32(flow)
@@ -150,7 +151,10 @@ def warp_grid(flow: Tensor) -> Tensor:
         ofb200.check(rc, "ofb_warp_grid_f32")
         return grid
 
-    return _run(run, "warp_grid", flow)
+    def backward(saved, grad_out: Tensor, needs):
+        return (grad_out,)
+
+    return _run(run, "warp_grid", flow, bwd=backward)
 
 
 _SCALE_DTYPES = {torch.float32: ofb200.DTYPE_F32, torch.float64: ofb200.DTYPE_F64, torch.float16: ofb200.DTYPE_F16,
