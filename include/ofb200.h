@@ -89,8 +89,10 @@ int ofb_warp(const void* frame, int frame_dtype, const void* flow, int flow_dtyp
 /* Backward of ofb_warp_f32 (bilinear, NCHW): what autograd computes for the reference's warp
  * (operator.py:28-33: grid_sample's backward, then d grid / d flow = 1 through warp_grid :56 and the
  * permute :28).  d_out (B,C,H,W).  d_frame_or_null (B,C,H,W) is ACCUMULATED into (zero it first):
- * each in-bounds tap receives weight * d_out.  d_flow_or_null (B,2,H,W) is overwritten, in the
- * units of `flow` (the flow_mul factors are applied).  Either output may be NULL. */
+ * each in-bounds tap receives weight * d_out, by atomic adds in no fixed order, so its last bits may
+ * differ between runs (as grid_sample's).  d_flow_or_null (B,2,H,W) is overwritten, in the units of
+ * `flow` (the flow_mul factors are applied), one store per element: deterministic, the same bits on
+ * every run.  Either output may be NULL. */
 int ofb_warp_backward_f32(const float* frame, const float* flow, const float* d_out,
                           float* d_frame_or_null, float* d_flow_or_null, int B, int C, int H, int W,
                           int padding_mode, int align_corners, float flow_mul_x, float flow_mul_y,
@@ -127,8 +129,9 @@ int ofb_scale_flow(const void* flow, void* out, int dtype, int B, int64_t HW, do
 int ofb_resize_bilinear_f32(const float* in, float* out, int N, int C, int H, int W, int Ho, int Wo,
                             int align_corners, float mul_x, float mul_y, void* stream);
 /* Its adjoint (autograd through F.interpolate + scale, operator.py:112-113; through upflow8,
- * utils.py:91): d_out (N,C,Ho,Wo) is scattered into d_in (N,C,H,W), which is ACCUMULATED into
- * (zero it first). */
+ * utils.py:91): d_out (N,C,Ho,Wo) is gathered into d_in (N,C,H,W), which is ACCUMULATED into
+ * (zero it first): one add per element, of a sum over the outputs in a fixed order.  Deterministic:
+ * the same bits on every run. */
 int ofb_resize_bilinear_backward_f32(const float* d_out, float* d_in, int N, int C, int H, int W,
                                      int Ho, int Wo, int align_corners, float mul_x, float mul_y,
                                      void* stream);
@@ -144,7 +147,8 @@ int ofb_convex_upsample_f32(const float* flow, const float* mask, float* out, in
 int ofb_convex_upsample(const float* flow, const void* mask, int mask_dtype, float* out, int N, int h, int w, void* stream);
 /* Backward of the convex upsampling (autograd through raft.py:77-85): d_out (N,2,8h,8w), 16-byte
  * aligned.  d_mask_or_null (N,576,h,w) is overwritten; d_flow_or_null (N,2,h,w) is ACCUMULATED
- * into (zero it first).  Either may be NULL. */
+ * into (zero it first): one add per element, of a sum formed in a fixed order.  Either may be NULL.
+ * Deterministic: the same bits on every run. */
 int ofb_convex_upsample_backward_f32(const float* flow, const float* mask, const float* d_out,
                                      float* d_flow_or_null, float* d_mask_or_null, int N, int h, int w,
                                      void* stream);

@@ -67,26 +67,64 @@ __global__ void __launch_bounds__(256) resize_kernel(const float* __restrict__ i
     }
 }
 
+// Candidate outputs whose taps may touch source index `src` along one axis: every dst with src_index(dst) in
+// {src - 1, src}, i.e. a source coordinate r in [src - 1, src + 1), from the inverse of the forward's mapping, widened
+// by 2 for its rounding and clamped to [0, out_size).  Only a superset: the caller re-checks each candidate's taps.
+__device__ __forceinline__ void dst_range(float ratio, int src, int in_size, int out_size, bool ac, int& lo, int& hi) {
+    if (out_size == in_size) { lo = hi = src; return; }
+    if (ratio == 0.0f) { lo = 0; hi = out_size - 1; return; }   // align_corners with one output: every dst reads 0
+    float a, b;
+    if (ac) {
+        a = (float)(src - 1) / ratio;
+        b = (float)(src + 1) / ratio;
+    } else {
+        a = ((float)(src - 1) + 0.5f) / ratio - 0.5f;
+        b = ((float)(src + 1) + 0.5f) / ratio - 0.5f;
+    }
+    a = src <= 1 ? 0.0f : fmaxf(floorf(a) - 2.0f, 0.0f);   // r < 0 is clamped to 0: taps 0 and 1 (weight 0)
+    b = fminf(ceilf(b) + 2.0f, (float)(out_size - 1));
+    lo = (int)a;
+    hi = (int)b;
+}
+
 // Adjoint of resize_kernel (what autograd computes through F.interpolate + scale, operator.py:112-113, and through
-// 8 * F.interpolate in upflow8): every output gradient is scattered to its four source pixels with the forward
-// weights times the magnitude factor.  One thread per output pixel, red.global.add.f32 into d_in (small).
+// 8 * F.interpolate in upflow8), as a gather: one thread per source pixel sums, in ascending output order (row, then
+// column, then the taps 00, 01, 10, 11), the forward weight times the magnitude-scaled gradient of every output tap
+// that lands on it -- the terms ATen's backward scatters, zero-weight taps included.  The taps are recomputed with the
+// forward's own src_index, so no inverted float formula decides which outputs count.  Deterministic: the same bits
+// on every run; d_in is accumulated into with one add per element.
 __global__ void __launch_bounds__(256) resize_bwd_kernel(const float* __restrict__ d_out, float* __restrict__ d_in,
                                                          int NC, int H, int W, int Ho, int Wo, int ac, float rh, float rw,
                                                          float mul_x, float mul_y) {
-    const size_t total = (size_t)NC * Ho * Wo;
+    const size_t total = (size_t)NC * H * W;
     for (size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x; t < total; t += (size_t)gridDim.x * blockDim.x) {
-        const int ox = (int)(t % Wo);
-        const int oy = (int)((t / Wo) % Ho);
-        const int nc = (int)(t / ((size_t)Wo * Ho));
-        const float g = __fmul_rn(__ldg(d_out + t), (nc & 1) ? mul_y : mul_x);
-        int y0, y1, x0, x1; float ly0, ly1, lx0, lx1;
-        src_index(rh, oy, H, Ho, ac != 0, y0, y1, ly0, ly1);
-        src_index(rw, ox, W, Wo, ac != 0, x0, x1, lx0, lx1);
-        float* dst = d_in + (size_t)nc * H * W;
-        atomicAdd(dst + (size_t)y0 * W + x0, ly0 * lx0 * g);
-        atomicAdd(dst + (size_t)y0 * W + x1, ly0 * lx1 * g);
-        atomicAdd(dst + (size_t)y1 * W + x0, ly1 * lx0 * g);
-        atomicAdd(dst + (size_t)y1 * W + x1, ly1 * lx1 * g);
+        const int ix = (int)(t % W);
+        const int iy = (int)((t / W) % H);
+        const int nc = (int)(t / ((size_t)W * H));
+        const float mul = (nc & 1) ? mul_y : mul_x;
+        const float* src = d_out + (size_t)nc * Ho * Wo;
+        int oy0, oy1, ox0, ox1;
+        dst_range(rh, iy, H, Ho, ac != 0, oy0, oy1);
+        dst_range(rw, ix, W, Wo, ac != 0, ox0, ox1);
+        float acc = 0.0f;
+        for (int oy = oy0; oy <= oy1; ++oy) {
+            int y0, y1; float ly0, ly1;
+            src_index(rh, oy, H, Ho, ac != 0, y0, y1, ly0, ly1);
+            const bool hy0 = y0 == iy, hy1 = y1 == iy;
+            if (!hy0 && !hy1) continue;
+            for (int ox = ox0; ox <= ox1; ++ox) {
+                int x0, x1; float lx0, lx1;
+                src_index(rw, ox, W, Wo, ac != 0, x0, x1, lx0, lx1);
+                const bool hx0 = x0 == ix, hx1 = x1 == ix;
+                if (!hx0 && !hx1) continue;
+                const float g = __fmul_rn(__ldg(src + (size_t)oy * Wo + ox), mul);
+                if (hy0 && hx0) acc += ly0 * lx0 * g;
+                if (hy0 && hx1) acc += ly0 * lx1 * g;
+                if (hy1 && hx0) acc += ly1 * lx0 * g;
+                if (hy1 && hx1) acc += ly1 * lx1 * g;
+            }
+        }
+        d_in[t] += acc;
     }
 }
 
@@ -168,8 +206,8 @@ OFB_API int ofb_resize_bilinear_backward_f32(const float* d_out, float* d_in, in
     if (N == 0 || C == 0 || Ho == 0 || Wo == 0) return OFB_OK;   // nothing to do: empty tensors have no storage, their pointers may be null
     if (!d_out || !d_in || N < 0 || C < 0 || H <= 0 || W <= 0 || Ho < 0 || Wo < 0) return OFB_EINVAL;
     if ((C & 1) && (mul_x != mul_y)) return OFB_EINVAL;
-    const size_t total = (size_t)N * C * Ho * Wo;
-    if (total == 0) return OFB_OK;
+    if ((size_t)N * C * Ho * Wo == 0) return OFB_OK;
+    const size_t total = (size_t)N * C * H * W;   // one thread per source pixel
     float rh, rw;
     if (align_corners) {
         rh = Ho > 1 ? (float)(H - 1) / (float)(Ho - 1) : 0.0f;

@@ -5,6 +5,7 @@ Tensors may live on the host or on the GPU: host tensors are staged through the 
 result is returned on the host (the reference's tests/operator build CPU tensors).  fp32 only, except `scale` /
 `normalize` / `denormalize` (dtype-preserving) and `warp` (fp32, fp16 or bf16 frames and flows).
 """
+import warnings
 from typing import Optional, Tuple, Union
 
 import torch
@@ -27,6 +28,21 @@ def _check_f32(*tensors: Tensor) -> None:
 
 
 _WARP_DTYPES = {torch.float32: ofb200.DTYPE_F32, torch.float16: ofb200.DTYPE_F16, torch.bfloat16: ofb200.DTYPE_BF16}
+
+
+def alert_not_deterministic(caller: str) -> None:
+    """What ATen's `alertNotDeterministic` does for its own order-dependent kernels: under
+    `torch.use_deterministic_algorithms(True)` raise RuntimeError, with `warn_only=True` warn instead."""
+    if not torch.are_deterministic_algorithms_enabled():
+        return
+    if torch.is_deterministic_algorithms_warn_only_enabled():
+        warnings.warn(f"{caller} does not have a deterministic implementation, but you set "
+                      "'torch.use_deterministic_algorithms(True, warn_only=True)'.", stacklevel=3)
+        return
+    raise RuntimeError(f"{caller} does not have a deterministic implementation, but you set "
+                       "'torch.use_deterministic_algorithms(True)'. You can turn off determinism just for this "
+                       "operation, or you can use the 'warn_only=True' option, if that's acceptable for your "
+                       "application.")
 
 
 def _run(fn, name: str, *tensors: Tensor, bwd=None) -> Tensor:
@@ -115,9 +131,13 @@ def warp(
     def backward(saved, grad_out: Tensor, needs):
         """d warp / d frame (scatter-add of the bilinear weights) and d warp / d flow, as F.grid_sample's backward
         through warp_grid (reference operator.py:28-33,56).  d_frame is accumulated in fp32 and rounded once to the
-        frame's dtype; d_flow is written in the flow's dtype."""
+        frame's dtype; d_flow is written in the flow's dtype.  d_frame's atomic adds run in no fixed order, so its
+        bits may differ between runs: under `torch.use_deterministic_algorithms(True)` a frame gradient raises, as
+        F.grid_sample's backward does.  d_flow is one store per element and always reproducible."""
         if mode != "bilinear":
             raise NotImplementedError("warp: backward exists for mode='bilinear' only")
+        if needs[0]:
+            alert_not_deterministic("ofb200 warp backward with respect to the frame (ofb_warp_backward d_frame)")
         frame_d, flow_d = saved
         with torch.cuda.device(frame_d.device):
             frame_c, flow_c = frame_d.contiguous(), flow_d.contiguous()
